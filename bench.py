@@ -51,7 +51,26 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-budget-s", type=float, default=12.0)
     ap.add_argument("--skip", default="", help="comma list of optional sections to skip: c1,c5,refgpu,fp32,selfcheck,eval")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the training step of the timed loop behind `value` as it computes from the seeded initial weights, on "
+                         "the batch and dropout stream of that loop's last step (loss, gradient norm, clipped gradients), as "
+                         "DIR/<name>.npy, to compare two builds output for output")
     return ap.parse_args()
+
+
+def dump_outputs(path, arrays, limit=64 << 20, min_rows=4096):
+    """{name: array} -> path/<name>.npy, float64 arrays as float64 and everything else as float32.  When the arrays come to more
+    than `limit` bytes, every array of more than `min_rows` rows keeps a fixed, seeded sample of its rows, in row order, sized so
+    that the sampled arrays take at most half the limit; path/<name>.rows.npy lists the rows kept."""
+    arrays = {k: np.asarray(v, dtype=np.float64 if np.asarray(v).dtype == np.float64 else np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        if total > limit and a.ndim and len(a) > min_rows:
+            rows = np.sort(np.random.default_rng(0).choice(len(a), int(len(a) * (limit // 2) / total), replace=False))
+            np.save(os.path.join(path, f"{k}.rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(path, f"{k}.npy"), a)
 
 
 def peaks():
@@ -356,6 +375,27 @@ def train_section(cx, args, cfg, name, precision, K, W, with_e2e=True, with_kern
                                              "the reference feeds this step from 4 CPU DataLoader workers"}
     out["_tr"], out["_model"] = tr, model
     return out
+
+
+def dump_step(cx, cfg, precision, K, W, pool=8):
+    """--dump-outputs: the step of train_section's device-resident timed loop (the K steps behind `value`; same trainer settings,
+    CUDA graph and precision) taken once more by a fresh trainer, from the seeded initial weights, on the batch and with the dropout
+    stream of that loop's last step.  The trainer sums weight gradients with fp32 atomics, so weights trained for many steps differ
+    from run to run by more than rounding: Adam scales each element's update by that element's own gradient, and an element whose
+    exact gradient is zero (the key bias under softmax) moves by about lr in a direction set by rounding.  One step from fixed
+    weights depends on the arguments only, up to rounding.
+    -> {name: array}: loss, gradient norm, and every parameter's gradient after clipping, as Adam applied it."""
+    from adt_b200.trainer import FusedTrainer
+    model = make_model(cfg, cx.dev)
+    l1, l2 = get_lambdas(cfg["dataset"])
+    tr = FusedTrainer(model, l1, l2, weight_decay=cfg["wd"], lr=1e-3, betas=(0.9, 0.98), clip=5.0, seed=23, use_graph=True, precision=precision)
+    rng = np.random.default_rng(23 + cx.rank)
+    batches = [synth.make_batch(rng, cfg) for _ in range(pool)]     # the batches train_section draws
+    tr.t = W + K - 1                                  # dropout stream of the last device-resident timed step
+    tr.step(*[torch.from_numpy(a).to(cx.dev) for a in batches[(K - 1) % pool]])
+    outs = {"train_loss": np.float64(tr.loss()), "train_grad_norm": np.float64(tr.grad_norm())}
+    outs.update({f"grad.{n}": tr.eng.grad_view(n).cpu().numpy() for n, _ in tr.eng.order})
+    return outs
 
 
 def dominant_roofline(cfg, kern, config_name):
@@ -783,6 +823,12 @@ def main():
                                       "sample": f"{e_n} batches of 512 users: predict(full=True) + mask + argpartition(40) + argsort (median, 1 warm-up)"}
         except Exception as e:   # noqa: BLE001
             cpu = {"unavailable": str(e)[:200]}
+
+    if args.dump_outputs:
+        trace("dump outputs")
+        outs = dump_step(cx, cfg, args.precision, K, W)       # every rank: the step all-reduces when N > 1
+        if rank == 0:
+            dump_outputs(args.dump_outputs, outs)
 
     if rank == 0:
         lps = main_tr.get("gpu_launches_per_step")

@@ -24,16 +24,16 @@ import torch.nn.functional as F
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 STAGED = os.path.join(HERE, "_ref", "sasrec")
-LIVE = "/root/reference/sasrec"
 
 
 def ref_dir():
-    """staged copy (travels to the GPU box) or, in the build container, the read-only reference itself."""
-    if os.path.exists(os.path.join(STAGED, "model.py")):
-        return STAGED
-    if os.path.exists(os.path.join(LIVE, "model.py")):
-        return LIVE
-    raise RuntimeError("reference sources not staged: run `python -m oracle.build_ref` where /root/reference exists")
+    """sasrec/ of the reference checkout (oracle/build_ref.REF: $ADT_REFERENCE_DIR, by default /root/reference), else the copy
+    oracle/build_ref.py staged.  The reference's sources are not part of this repository."""
+    from oracle.build_ref import REF
+    for d in (os.path.join(REF, "sasrec"), STAGED):
+        if os.path.exists(os.path.join(d, "model.py")):
+            return d
+    raise RuntimeError(f"reference sources not found: no checkout at {REF} (set ADT_REFERENCE_DIR) and nothing staged in oracle/_ref")
 
 
 def ref_modules():

@@ -1,71 +1,60 @@
-"""SURVEY 8f-1: device-side batch assembly / negative sampling.  CPU: the oracle restatement against the UNMODIFIED reference
-datasets (when /root/reference is present) for everything that is not random, and the validity of what is.  GPU: the kernels against
-the oracle, bit for bit."""
+"""SURVEY 8f-1: device-side batch assembly / negative sampling.  CPU: the oracle restatement against what the UNMODIFIED reference
+datasets produce (stored in tests/golden, and live where the reference checkout exists) for everything that is not random, and the
+validity of what is.  GPU: the kernels against the oracle, bit for bit."""
 import os
-import sys
-import types
 
 import numpy as np
 import pytest
 import torch
 
-
-def _toy(rng, usernum=40, itemnum=60, maxhist=30):
-    train, valid, test = {}, {}, {}
-    for u in range(1, usernum + 1):
-        n = int(rng.integers(0, maxhist))
-        h = [int(x) for x in rng.integers(1, itemnum + 1, size=n)]
-        if len(h) >= 3:
-            train[u], valid[u], test[u] = h[:-2], [h[-2]], [h[-1]]
-        else:
-            train[u], valid[u], test[u] = h, [], []
-    return train, valid, test, usernum, itemnum
+from oracle import make_golden_sampler as G
+from oracle.make_golden_sampler import toy_histories as _toy
 
 
-def _ref_utils():
-    if not os.path.isdir("/root/reference/sasrec"):
-        pytest.skip("/root/reference not present on this box")
-    for name in ("matplotlib", "matplotlib.pyplot"):
-        sys.modules.setdefault(name, types.ModuleType(name))
-    sys.path.insert(0, "/root/reference/sasrec")
-    import importlib
-    return importlib.import_module("utils")
+def _reference_layouts(part):
+    """what the reference's dataset classes produce on the toy histories: the copy stored in tests/golden/sampler_ref.npz
+    (oracle/make_golden_sampler.py) and, where the reference checkout exists, the live result as well."""
+    got = []
+    if os.path.exists(G.OUT):
+        z = np.load(G.OUT)
+        got.append({k.split("/", 1)[1]: z[k] for k in z.files if k.startswith(part + "/")})
+    if os.path.isdir(os.path.join(G.REF, part)):
+        got.append(getattr(G, part + "_layout")())
+    if not got:
+        pytest.skip(f"neither {G.OUT} nor a reference checkout at {G.REF}: run `python -m oracle.make_golden_sampler` where it exists")
+    return got
 
 
 def test_oracle_batch_layout_matches_reference_datasets():
     """seq / dec / pos of WarpDataset.sample_data and seq / answer of EvalDataset.sample_data are deterministic: the oracle must equal
     the unmodified reference exactly; the random parts must satisfy the reference's constraints."""
     from oracle import sampler_oracle as S
-    R = _ref_utils()
-    rng = np.random.default_rng(0)
-    train, valid, test, usernum, itemnum = _toy(rng)
-    L = 12
-    wd = R.WarpDataset(train, usernum, itemnum, L)
-    for u in range(1, usernum + 1):
-        if len(train[u]) < 1:
-            continue
-        _, seq, dec, pos, neg = wd.sample_data(u)
-        o_seq, o_dec, o_pos, o_neg = S.train_sample(train[u], u, L, itemnum, seed=5, epoch=1)
-        assert np.array_equal(seq, o_seq) and np.array_equal(dec, o_dec) and np.array_equal(pos, o_pos), u
-        assert np.array_equal(neg != 0, o_neg != 0)
-        assert not set(o_neg[o_neg != 0].tolist()) & set(train[u])
-        assert o_neg.max(initial=0) <= itemnum
-    sampler = R.PopularSampler(train, valid, test, usernum, itemnum, 10)
     from adt_b200.sampler import alias_table
-    ap, ai = alias_table(np.asarray(sampler.popular_p, dtype=np.float64))
-    for mode in ("val", "test"):
-        ds = R.EvalDataset(train, valid, test, usernum, itemnum, L, sampler, mode=mode, eval_set=-1)
-        for u in ds.users:
-            _, seq, item_idx, _ = ds.sample_data(u)
-            seen = set(train[u]) | set(valid[u]) | (set(test[u]) if mode == "test" else set())
-            ans = valid[u][0] if mode == "val" else test[u][0]
-            o_seq, o_idx = S.eval_sample(train[u], seen, ans, valid[u][0] if mode == "test" else 0, u, L, itemnum, 10, ap, ai, seed=5, epoch=0)
-            assert np.array_equal(seq, o_seq), (mode, u)
-            assert item_idx[0] == o_idx[0] == ans
-            neg = o_idx[1:]
-            assert len(neg) == 10 and len(set(neg.tolist())) == 10
-            assert not set(neg.tolist()) & seen and neg.max() < itemnum and neg.min() >= 0
-            assert all(sampler.popular_p[i] > 0 for i in neg)        # only items that can be drawn by popularity (quirk B8: never id 0)
+    train, valid, test, usernum, itemnum = _toy(np.random.default_rng(0))
+    L = G.SASREC_L
+    for ref in _reference_layouts("sasrec"):
+        assert list(ref["train_users"]) == [u for u in range(1, usernum + 1) if len(train[u]) >= 1]
+        for b, u in enumerate(int(x) for x in ref["train_users"]):
+            o_seq, o_dec, o_pos, o_neg = S.train_sample(train[u], u, L, itemnum, seed=5, epoch=1)
+            assert np.array_equal(ref["train_seq"][b], o_seq) and np.array_equal(ref["train_dec"][b], o_dec), u
+            assert np.array_equal(ref["train_pos"][b], o_pos), u
+            assert np.array_equal(ref["train_neg_mask"][b], o_neg != 0)
+            assert not set(o_neg[o_neg != 0].tolist()) & set(train[u])
+            assert o_neg.max(initial=0) <= itemnum
+        popular_p = ref["popular_p"]
+        ap, ai = alias_table(np.asarray(popular_p, dtype=np.float64))
+        for mode in ("val", "test"):
+            for b, u in enumerate(int(x) for x in ref[f"{mode}_users"]):
+                seen = set(train[u]) | set(valid[u]) | (set(test[u]) if mode == "test" else set())
+                ans = valid[u][0] if mode == "val" else test[u][0]
+                o_seq, o_idx = S.eval_sample(train[u], seen, ans, valid[u][0] if mode == "test" else 0, u, L, itemnum, 10, ap, ai, seed=5,
+                                             epoch=0)
+                assert np.array_equal(ref[f"{mode}_seq"][b], o_seq), (mode, u)
+                assert ref[f"{mode}_answer"][b] == o_idx[0] == ans
+                neg = o_idx[1:]
+                assert len(neg) == 10 and len(set(neg.tolist())) == 10
+                assert not set(neg.tolist()) & seen and neg.max() < itemnum and neg.min() >= 0
+                assert all(popular_p[i] > 0 for i in neg)        # only items that can be drawn by popularity (quirk B8: never id 0)
 
 
 def test_alias_table_reproduces_the_distribution():
@@ -144,29 +133,17 @@ def test_device_candidates_follow_popularity():
 def test_cloze_instance_table_and_layout_match_reference_dataset():
     """SURVEY 8f-3: the window enumeration of BertTrainDataset._generate_data and the deterministic layout of sample_data / _mask_last
     (right alignment, decoder copy ending in the mask token, labels) against the UNMODIFIED reference dataset class."""
-    if not os.path.isdir("/root/reference/bert4rec"):
-        pytest.skip("/root/reference not present on this box")
-    import importlib
-    pkg = types.ModuleType("refbert_datasets")          # the reference's `datasets/` has no __init__.py: mount it as a package
-    pkg.__path__ = ["/root/reference/bert4rec/datasets"]
-    sys.modules["refbert_datasets"] = pkg
-    try:
-        mod = importlib.import_module("refbert_datasets.dataset")
-    except Exception as e:   # noqa: BLE001
-        pytest.skip(f"reference dataset module not importable here: {e}")
     from adt_b200.sampler import ClozeSampler
     from oracle import sampler_oracle as S
-    rng = np.random.default_rng(2)
-    usernum, itemnum, L = 25, 80, 10
-    train = {u: [int(x) for x in rng.integers(1, itemnum + 1, size=int(rng.integers(0, 35)))] for u in range(1, usernum + 1)}
-    d = mod.BertTrainDataset(train, {}, {}, usernum, itemnum, L, None, 0.0, 1, generate=True, dupe_factor=2, prop_sliding_window=0.5)
-    tab = ClozeSampler.instance_table(train, usernum, L, 2, 0.5)
-    assert len(tab) == len(d.datas)
-    # with mask_prob = 0 nothing is masked: tokens = window, decoder copy = window with the last position masked, labels = 0
-    for row, (data, label) in zip(tab, zip(d.datas, d.labels)):
-        u, st, ln, dup = [int(x) for x in row]
-        tok, dec, lab = S.cloze_sample(train[u], u, st, ln, dup, L, itemnum, 0.0, seed=1, epoch=0)
-        assert np.array_equal(tok, data[0].numpy()) and np.array_equal(dec, data[1].numpy()) and np.array_equal(lab, label.numpy()), row
+    train, L, itemnum = G.bert_histories(), G.BERT_L, G.BERT_ITEMS
+    tab = ClozeSampler.instance_table(train, G.BERT_USERS, L, 2, 0.5)
+    for ref in _reference_layouts("bert4rec"):
+        assert len(tab) == len(ref["tok"])
+        # with mask_prob = 0 nothing is masked: tokens = window, decoder copy = window with the last position masked, labels = 0
+        for b, row in enumerate(tab):
+            u, st, ln, dup = [int(x) for x in row]
+            tok, dec, lab = S.cloze_sample(train[u], u, st, ln, dup, L, itemnum, 0.0, seed=1, epoch=0)
+            assert np.array_equal(tok, ref["tok"][b]) and np.array_equal(dec, ref["dec"][b]) and np.array_equal(lab, ref["labels"][b]), row
 
 
 @pytest.mark.gpu
