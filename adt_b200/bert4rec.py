@@ -106,6 +106,7 @@ class BertModel(nn.Module):
         self.mask_layer_norm = nn.LayerNorm(H, eps=1e-5)
         self.drop_seed, self.drop_step, self.precision = 0, 0, 0
         self.step_dev = None      # optional device-side dropout step counter (adt_b200.dp.GraphedStep)
+        self._scorers = {}        # (K, device) -> CatalogScorer of full_sort_topk (keeps its bf16 table and scratch between calls)
         L.lib()
 
     # ------------------------------------------------------------------------------------------
@@ -226,6 +227,40 @@ class BertModel(nn.Module):
                 if lambda2[l] != 0:
                     total = total + lambda2[l] * F.nll_loss(inds[l].reshape(B * Lq, nh, nh), label)
         return total
+
+    # ---- full-catalog evaluation -------------------------------------------------------------
+    def scoring_catalog(self):
+        """what full-catalog ranking scores (adt_b200.evaluate.catalog_of): score[u, i] = <final_feats[u], E_word[i]> + mask_bias[i]
+        over the real items i = 1..itemnum only -- the padding row 0 and the extra vocabulary rows (mask token itemnum+1 ...) of the
+        tied table are never ranked."""
+        from .evaluate import Catalog
+        I = self.itemnum
+        return Catalog(self.item_emb.word_emb.weight.detach()[1:I + 1], self.mask_bias.detach()[1:I + 1], 1, self.hidden_units)
+
+    @torch.no_grad()
+    def final_feats(self, seqs, seq_pos_ids=None, seq_sent_ids=None):
+        """[U, H] rows the catalog is scored against: encoder in evaluation mode (no dropout, the ops of `predict`), last position,
+        then the head's Linear -> GELU -> LayerNorm (bert.py:81-86).  Position / sentence ids default to 0..L-1 and 0 as in training.
+        No host synchronisation, so a CUDA graph can capture it (GraphedScorer)."""
+        self._check()
+        dev = self.mask_bias.device
+        src = _ids(seqs, dev)
+        B, Lq = src.shape
+        sp = _ids(seq_pos_ids, dev) if seq_pos_ids is not None else torch.arange(Lq, dtype=torch.int32, device=dev).repeat(B, 1)
+        ss = _ids(seq_sent_ids, dev) if seq_sent_ids is not None else torch.zeros(B, Lq, dtype=torch.int32, device=dev)
+        feats, _, _ = self._encode(src, sp, ss, DropCfg(0.0, 0, 0, False))
+        return self._head_hidden(feats.view(B, Lq, -1)[:, -1, :].contiguous())
+
+    @torch.no_grad()
+    def full_sort_topk(self, seqs, seen_indptr=None, seen_idx=None, K=40, answers=None, metric_acc=None):
+        """full-catalog top-K (the bert.py:80-90 score of every item 1..itemnum) -> (scores [U,K] fp32, ids [U,K] int32), best first,
+        ties by ascending id, seen ids (CSR, ascending per user) excluded.  `seqs` is what `predict` takes (history with the mask token
+        last).  Same contract as CatalogScorer.topk, including the fused HIT/NDCG/MRR sums into metric_acc."""
+        from .evaluate import CatalogScorer
+        key = (int(K), self.mask_bias.device)
+        if key not in self._scorers:
+            self._scorers[key] = CatalogScorer(self, K=K)
+        return self._scorers[key].topk(seqs, seen_indptr, seen_idx, answers, metric_acc)
 
     @torch.no_grad()
     def predict(self, user_ids, seqs, seq_pos_ids, seq_sent_ids, candidates):

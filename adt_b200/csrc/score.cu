@@ -27,6 +27,7 @@ struct TopkArgs {
   long long part_stride;                       // elements between two splits' lists in part_scores / part_ids (merge kernel)
   float* dense_out; long long dense_ld;        // WRITE_ALL mode: the whole score row [U][dense_ld] (predict(full=True))
   int U, H, n_items, item_offset, K, n_splits;
+  const float* bias;                           // BIAS kernels: [n_items] added to every score (local index, like E)
 };
 
 // get_full_sort_score (sasrec/utils.py:686-708) for ONE held-out answer per user, accumulated over users:
@@ -60,7 +61,9 @@ __device__ __forceinline__ bool is_seen(const TopkArgs& a, int sb, int se, int i
 // better(a,b): a ranks strictly before b  (score desc, then id asc -- deterministic under exact ties)
 __device__ __forceinline__ bool better(float sa, int ia, float sb, int ib) { return sa > sb || (sa == sb && ia < ib); }
 
-template <bool WRITE_ALL>
+// BIAS: scores are <f, e> + bias[i], the bias added once after the full dot product of the tile, before anything compares them;
+// the re-score kernel of the tensor-core path adds it after the same sequential fmaf chain, so the two stay bit-identical
+template <bool WRITE_ALL, bool BIAS>
 __global__ void __launch_bounds__(NT) score_topk_kernel(TopkArgs a) {
   extern __shared__ __align__(16) float smem[];
   const int H = a.H, K = a.K;
@@ -117,6 +120,15 @@ __global__ void __launch_bounds__(NT) score_topk_kernel(TopkArgs a) {
       __syncthreads();
       mma_nt<4>(acc, Fs, ld, rc * CH, Ws + (rc & 1) * WS_SLOT, min(CH, H - rc * CH));
       __syncthreads();
+    }
+    if constexpr (BIAS) {
+      float b[4];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) b[j] = c0 + 4 * tx + j < it1 ? __ldg(a.bias + c0 + 4 * tx + j) : 0.f;
+#pragma unroll
+      for (int i = 0; i < 4; ++i)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) acc[i][j] += b[j];
     }
 #pragma unroll
     for (int i = 0; i < 4; ++i)
@@ -308,10 +320,16 @@ extern "C" int adt_score_topk(const adt_score_topk_args* a, adt_stream_t s_) {
   k.U = a->U; k.H = a->H; k.n_items = a->n_items; k.item_offset = a->item_offset; k.K = a->K; k.n_splits = a->n_splits;
   k.answers = a->answers; k.metric_acc = a->metric_acc; k.dense_out = nullptr; k.dense_ld = 0; k.user_mask = a->user_mask;
   k.part_stride = (long long)a->U * a->K;
+  k.bias = a->item_bias;
   const size_t smem = ((size_t)UT * (a->H + 4) + (size_t)UT * CHP + WS_FLOATS + (size_t)UT * a->K * 2 + 3 * UT) * sizeof(float);
-  cudaFuncSetAttribute(score_topk_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   dim3 grid(a->n_splits, (a->U + UT - 1) / UT);
-  score_topk_kernel<false><<<grid, NT, smem, s>>>(k);
+  if (a->item_bias) {
+    cudaFuncSetAttribute(score_topk_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    score_topk_kernel<false, true><<<grid, NT, smem, s>>>(k);
+  } else {
+    cudaFuncSetAttribute(score_topk_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    score_topk_kernel<false, false><<<grid, NT, smem, s>>>(k);
+  }
   if (a->out_ids) topk_merge_kernel<<<(a->U + 7) / 8, 256, 0, s>>>(k);
   const cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? ADT_OK : ADT_E_CUDA;
@@ -336,8 +354,8 @@ extern "C" int adt_score_full(const float* feats, int32_t U, int32_t H, const fl
   splits = (n_items + per - 1) / per;
   k.n_splits = splits; k.dense_out = out; k.dense_ld = ld;
   const size_t smem = ((size_t)UT * (H + 4) + (size_t)UT * CHP + WS_FLOATS + (size_t)UT * 2 + 3 * UT) * sizeof(float);
-  cudaFuncSetAttribute(score_topk_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  score_topk_kernel<true><<<dim3(splits, tiles), NT, smem, s>>>(k);
+  cudaFuncSetAttribute(score_topk_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  score_topk_kernel<true, false><<<dim3(splits, tiles), NT, smem, s>>>(k);
   return cudaGetLastError() == cudaSuccess ? ADT_OK : ADT_E_CUDA;
 }
 

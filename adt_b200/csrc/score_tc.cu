@@ -37,6 +37,7 @@ struct TcArgs {
   const float* tau;     // MODE 1: [U] per-user score threshold (from the sample pass): everything above it is a candidate
   int U, n_items, item_offset, KC, n_splits, debug;
   int sstride;          // MODE 2: every sstride-th catalog tile belongs to the sample
+  const float* bias;    // BIAS kernels: [n_items] per-item fp32 bias, local index like the catalog rows
 };
 
 // Which catalog tiles (BN items each) a CTA walks:
@@ -82,7 +83,11 @@ __device__ __forceinline__ bool tc_is_seen(const TcArgs& a, int sb, int se, int 
 // ATM: the user tile (A operand, reused by every MMA of the kernel) lives in TENSOR MEMORY instead of shared memory: the epilogue
 // threads store their own feature row with tcgen05.st once, the MMAs read it from TMEM (tcgen05.mma, A from TMEM).  Frees
 // KB*16 KB of shared memory for a deeper TMA ring and takes the A fragment reads off the shared-memory port.
-template <int KB, int BN, int NS, int MODE, bool MC, bool ATM>
+// BIAS: score = accumulator + bias[item] in fp32, added to every value as it leaves tcgen05.ld and before any comparison, in all three
+// modes (so the streaming lists, the published gthr keys, tau and the appended candidates are all in biased scores).  Every epilogue
+// warp stages the bias of its columns once per tile in its own smem row (loaded from global one tile ahead); each 32-column chunk
+// then reads it back with 8 broadcast LDS.128.  BIAS = false leaves the kernel exactly as without the feature.
+template <int KB, int BN, int NS, int MODE, bool MC, bool ATM, bool BIAS>
 __global__ void __launch_bounds__(TC_THREADS2, 1) score_tc_kernel(const __grid_constant__ CUtensorMap tmA,
                                                                   const __grid_constant__ CUtensorMap tmB, TcArgs a) {
   extern __shared__ uint8_t smem_raw[];
@@ -102,7 +107,8 @@ __global__ void __launch_bounds__(TC_THREADS2, 1) score_tc_kernel(const __grid_c
   int* li = reinterpret_cast<int*>(lk + BM * KCP);                // [KCP][128] item ids      thread that owns a row scans it conflict-free
   float* thr_s = reinterpret_cast<float*>(li + BM * KCP);         // [128] (unused scratch)
   float* vsm = thr_s + BM;                                        // [4][32][32] chunk parking area of the epilogue warps
-  uint64_t* bars = reinterpret_cast<uint64_t*>(vsm + 4 * 1024);
+  float* bsm = vsm + 4 * 1024;                                    // BIAS: [8][64] or [4][128] per-warp bias of the current tile
+  uint64_t* bars = reinterpret_cast<uint64_t*>(bsm + (BIAS ? 512 : 0));
   uint64_t* full = bars;               // [NS] B stage filled (TMA tx)
   uint64_t* empty = bars + NS;         // [NS] B stage consumed (tcgen05.commit)
   uint64_t* tfull = bars + 2 * NS;     // [NACC] accumulator ready (tcgen05.commit)
@@ -224,6 +230,37 @@ __global__ void __launch_bounds__(TC_THREADS2, 1) score_tc_kernel(const __grid_c
       sb = tc_seen_lower_bound(a.seen_idx, a.seen_indptr[u], hi, a.item_offset + it0);
       se = tc_seen_lower_bound(a.seen_idx, sb, hi, a.item_offset + it1);
     }
+    // per-tile bias staging (BIAS only): this warp's BW columns of tile t sit in bs[]; the next tile's are already in registers
+    constexpr int BW = MODE == 0 ? BN : BN / 2;
+    float bnext[BIAS ? BW / 32 : 1];
+    auto bias_fetch = [&](int t) {           // global -> registers, one tile ahead of its use (hides the load latency)
+      if constexpr (BIAS) {
+        const int ib = (tfirst + t * tstep) * BN + CB + lane;
+#pragma unroll
+        for (int j = 0; j < BW / 32; ++j) bnext[j] = (t < ntiles && ib + 32 * j < a.n_items) ? __ldg(a.bias + ib + 32 * j) : 0.f;
+      }
+    };
+    auto bias_stage = [&](int t) {           // registers -> this warp's smem row, then fetch the next tile's
+      if constexpr (BIAS) {
+        float* bs = bsm + (warp - 2) * BW;
+        __syncwarp();
+#pragma unroll
+        for (int j = 0; j < BW / 32; ++j) bs[lane + 32 * j] = bnext[j];
+        __syncwarp();
+        bias_fetch(t + 1);
+      }
+    };
+    auto bias_add = [&](float (&v)[32], int c0) {   // v[c] += bias of column c0 + c (same value in every lane: broadcast loads)
+      if constexpr (BIAS) {
+        const float4* b4 = reinterpret_cast<const float4*>(bsm + (warp - 2) * BW + (c0 - CB));
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          const float4 b = b4[j];
+          v[4 * j] += b.x; v[4 * j + 1] += b.y; v[4 * j + 2] += b.z; v[4 * j + 3] += b.w;
+        }
+      }
+    };
+    bias_fetch(0);
     auto unkey = [](uint32_t k) -> float { return k == 0u ? -INFINITY : __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k); };
     auto fkey = [](float f) -> uint32_t {
       const uint32_t b = __float_as_uint(f);
@@ -239,6 +276,7 @@ __global__ void __launch_bounds__(TC_THREADS2, 1) score_tc_kernel(const __grid_c
       const long long obase = (vsplit * a.U + (u < a.U ? u : 0)) * KC;
       for (int t = 0; t < ntiles; ++t) {
         const int st = t % NACC;
+        bias_stage(t);
         tc::mbar_wait(tfull + st, (t / NACC) & 1);
         tc::tc_fence_after();
         const int tb = (tfirst + t * tstep) * BN;
@@ -251,6 +289,7 @@ __global__ void __launch_bounds__(TC_THREADS2, 1) score_tc_kernel(const __grid_c
             __syncwarp();
             if (lane == 0) tc::mbar_arrive(tempty + st);
           }
+          bias_add(v, c0);
           const int ib = tb + c0;
           const int nvalid = a.n_items - ib;
           if (nvalid < CW) {
@@ -288,6 +327,7 @@ __global__ void __launch_bounds__(TC_THREADS2, 1) score_tc_kernel(const __grid_c
       thr = 0.f;
       for (int t = 0; t < ntiles; ++t) {
         const int st = t % NACC;
+        bias_stage(t);
         tc::mbar_wait(tfull + st, (t / NACC) & 1);
         tc::tc_fence_after();
         const int tb = (tfirst + t * tstep) * BN;
@@ -301,6 +341,7 @@ __global__ void __launch_bounds__(TC_THREADS2, 1) score_tc_kernel(const __grid_c
             __syncwarp();
             if (lane == 0) tc::mbar_arrive(tempty + st);
           }
+          bias_add(v, c0);
           const int nvalid = a.n_items - (tb + c0);
 #pragma unroll
           for (int c = 0; c < CW; ++c) mx = fmaxf(mx, c < nvalid ? v[c] : -INFINITY);
@@ -334,6 +375,7 @@ __global__ void __launch_bounds__(TC_THREADS2, 1) score_tc_kernel(const __grid_c
       const int st = t % NACC;
       // thresholds of the other splits: issue the (L2) load now, consume it after this tile
       const uint32_t gnext = (MODE == 0 && a.gthr && u < a.U) ? __ldcg(a.gthr + u) : 0u;
+      bias_stage(t);
       tc::mbar_wait(tfull + st, (t / NACC) & 1);
       tc::tc_fence_after();
       const int tb = (tfirst + t * tstep) * BN;
@@ -346,6 +388,7 @@ __global__ void __launch_bounds__(TC_THREADS2, 1) score_tc_kernel(const __grid_c
           __syncwarp();
           if (lane == 0) tc::mbar_arrive(tempty + st);
         }
+        bias_add(v, c0);
         const int ib = tb + c0;
         const int nvalid = a.n_items - ib;
         if (nvalid < 32) {
@@ -419,6 +462,7 @@ struct RescoreArgs {
   float* out_scores; int* out_ids; int* flags;
   const int* answers; double* metric_acc;
   int U, H, item_offset, K, KC, n_splits;
+  const float* bias; const float* max_abs_bias;   // BIAS: [n_items] per-item bias (local index) and max |bias|
 };
 
 constexpr int RS_MAXC = 2048;   // candidate slots per user (n_splits * KC)
@@ -437,6 +481,7 @@ __device__ __forceinline__ unsigned long long rs_key(float s, int id) {
   return ((unsigned long long)o << 32) | (unsigned long long)(0xFFFFFFFFu - (unsigned)id);
 }
 
+template <bool BIAS>
 __global__ void __launch_bounds__(RS_NT, 2) rescore_select_kernel(RescoreArgs a) {
   __shared__ int cid[RS_MAXC];
   __shared__ float csc[RS_MAXC];
@@ -512,7 +557,10 @@ __global__ void __launch_bounds__(RS_NT, 2) rescore_select_kernel(RescoreArgs a)
         }
         __syncwarp();
       }
-      if (wbase + l < m) { csc[wbase + l] = acc; ckey[wbase + l] = rs_key(acc, cid[wbase + l]); }
+      if (wbase + l < m) {
+        if constexpr (BIAS) acc += a.bias[cid[wbase + l] - a.item_offset];   // after the whole chain, as in the exact kernel: bit-identical
+        csc[wbase + l] = acc; ckey[wbase + l] = rs_key(acc, cid[wbase + l]);
+      }
     }
   }
   __syncthreads();
@@ -542,7 +590,12 @@ __global__ void __launch_bounds__(RS_NT, 2) rescore_select_kernel(RescoreArgs a)
   __syncthreads();
   if (tid == 0) {
     const float kth = m >= a.K ? kth_s : -INFINITY;
-    const float eps = 0.0078125f * sqrtf(fn) * sqrtf(*a.max_normsq);   // 2^-7 |f| max|e|
+    // a non-candidate's exact score exceeds tau by at most eps: the bf16 operand rounding 2^-7 |f| max|e|, plus with a bias the
+    // rounding of the two fp32 bias additions (epilogue and re-score), each <= 2^-24 |<f,e> + b| <= 2^-24 (|f| max|e| + max|b|);
+    // 2^-22 leaves a factor 2 of margin.  A bias that dwarfs the dot products therefore widens eps until the user is flagged and
+    // re-run exactly, rather than returning a list the bound cannot prove.
+    float eps = 0.0078125f * sqrtf(fn) * sqrtf(*a.max_normsq);        // 2^-7 |f| max|e|
+    if constexpr (BIAS) eps += 2.384185791015625e-07f * (sqrtf(fn) * sqrtf(*a.max_normsq) + *a.max_abs_bias);
     const int flag = (thr_max > -INFINITY && !(kth > thr_max + eps)) ? 1 : 0;
     a.flags[u] = flag;
     // fused get_full_sort_score epilogue (sasrec/utils.py:686-708) for the users whose list is proven exact
@@ -592,11 +645,11 @@ static bool tc_atmem() {
   if (v < 0) { const char* e = getenv("ADT_TC_ATMEM"); v = e ? atoi(e) : 1; }
   return v != 0;
 }
-template <int KB, int BN, int NS, int MODE, bool ATM>
+template <int KB, int BN, int NS, int MODE, bool ATM, bool BIAS>
 int launch_tc_ns(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap* tmBh, const TcArgs& k, dim3 grid, cudaStream_t s, size_t smem) {
   if (tmBh) {      // 2-CTA clusters over pairs of user tiles, grid = (user tiles, splits)
     if (MODE == 0) return ADT_E_SHAPE;
-    cudaFuncSetAttribute(score_tc_kernel<KB, BN, NS, MODE, true, ATM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaFuncSetAttribute(score_tc_kernel<KB, BN, NS, MODE, true, ATM, BIAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));
     cfg.gridDim = dim3(grid.y, grid.x); cfg.blockDim = dim3(MODE == 0 ? TC_THREADS : TC_THREADS2); cfg.dynamicSmemBytes = smem; cfg.stream = s;
@@ -604,29 +657,36 @@ int launch_tc_ns(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorM
     at[0].id = cudaLaunchAttributeClusterDimension;
     at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
     cfg.attrs = at; cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, score_tc_kernel<KB, BN, NS, MODE, true, ATM>, tmA, *tmBh, k) == cudaSuccess ? ADT_OK : ADT_E_CUDA;
+    return cudaLaunchKernelEx(&cfg, score_tc_kernel<KB, BN, NS, MODE, true, ATM, BIAS>, tmA, *tmBh, k) == cudaSuccess ? ADT_OK : ADT_E_CUDA;
   }
-  cudaFuncSetAttribute(score_tc_kernel<KB, BN, NS, MODE, false, ATM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  score_tc_kernel<KB, BN, NS, MODE, false, ATM><<<grid, MODE == 0 ? TC_THREADS : TC_THREADS2, smem, s>>>(tmA, tmB, k);
+  cudaFuncSetAttribute(score_tc_kernel<KB, BN, NS, MODE, false, ATM, BIAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  score_tc_kernel<KB, BN, NS, MODE, false, ATM, BIAS><<<grid, MODE == 0 ? TC_THREADS : TC_THREADS2, smem, s>>>(tmA, tmB, k);
   return cudaGetLastError() == cudaSuccess ? ADT_OK : ADT_E_CUDA;
 }
 // deepest catalog-tile ring (2..4 stages) that fits the 227 KB of shared memory next to the user tile and the top-K lists
-template <int KB, int BN, int MODE, bool ATM>
+template <int KB, int BN, int MODE, bool ATM, bool BIAS>
 int launch_tc_a(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap* tmBh, const TcArgs& k, dim3 grid, cudaStream_t s) {
-  const size_t fixed = 1024 + (ATM ? 0 : (size_t)KB * BM * 128) + (MODE == 0 ? (size_t)(k.KC <= 32 ? 32 : 64) * BM * 8 : 0) + BM * 4 + 4 * 1024 * 4 + 256;
+  const size_t fixed = 1024 + (ATM ? 0 : (size_t)KB * BM * 128) + (MODE == 0 ? (size_t)(k.KC <= 32 ? 32 : 64) * BM * 8 : 0) + BM * 4 + 4 * 1024 * 4 + 256 +
+                       (BIAS ? 512 * 4 : 0);
   const size_t stage = (size_t)KB * BN * 128, cap = 227 * 1024;
   // the ring must hold more than one DRAM round trip (~1 us) of tensor work: a [128 x 128 x 64] tile is only 256 cycles
-  if (fixed + 8 * stage <= cap) return launch_tc_ns<KB, BN, 8, MODE, ATM>(tmA, tmB, tmBh, k, grid, s, fixed + 8 * stage);
-  if (fixed + 6 * stage <= cap) return launch_tc_ns<KB, BN, 6, MODE, ATM>(tmA, tmB, tmBh, k, grid, s, fixed + 6 * stage);
-  if (fixed + 4 * stage <= cap) return launch_tc_ns<KB, BN, 4, MODE, ATM>(tmA, tmB, tmBh, k, grid, s, fixed + 4 * stage);
-  if (fixed + 3 * stage <= cap) return launch_tc_ns<KB, BN, 3, MODE, ATM>(tmA, tmB, tmBh, k, grid, s, fixed + 3 * stage);
-  if (fixed + 2 * stage <= cap) return launch_tc_ns<KB, BN, 2, MODE, ATM>(tmA, tmB, tmBh, k, grid, s, fixed + 2 * stage);
+  if (fixed + 8 * stage <= cap) return launch_tc_ns<KB, BN, 8, MODE, ATM, BIAS>(tmA, tmB, tmBh, k, grid, s, fixed + 8 * stage);
+  if (fixed + 6 * stage <= cap) return launch_tc_ns<KB, BN, 6, MODE, ATM, BIAS>(tmA, tmB, tmBh, k, grid, s, fixed + 6 * stage);
+  if (fixed + 4 * stage <= cap) return launch_tc_ns<KB, BN, 4, MODE, ATM, BIAS>(tmA, tmB, tmBh, k, grid, s, fixed + 4 * stage);
+  if (fixed + 3 * stage <= cap) return launch_tc_ns<KB, BN, 3, MODE, ATM, BIAS>(tmA, tmB, tmBh, k, grid, s, fixed + 3 * stage);
+  if (fixed + 2 * stage <= cap) return launch_tc_ns<KB, BN, 2, MODE, ATM, BIAS>(tmA, tmB, tmBh, k, grid, s, fixed + 2 * stage);
   return ADT_E_SHAPE;
 }
+// with a bias the two-pass kernels always take the user tile in tensor memory (the default; ADT_TC_ATMEM=0 is a measurement switch
+// for the unbiased kernels only), which keeps the number of instantiations down
 template <int KB, int BN, int MODE>
 int launch_tc(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap* tmBh, const TcArgs& k, dim3 grid, cudaStream_t s) {
-  if (MODE != 0 && tc_atmem()) return launch_tc_a<KB, BN, MODE, true>(tmA, tmB, tmBh, k, grid, s);
-  return launch_tc_a<KB, BN, MODE, false>(tmA, tmB, tmBh, k, grid, s);
+  if (k.bias) {
+    if constexpr (MODE != 0) return launch_tc_a<KB, BN, MODE, true, true>(tmA, tmB, tmBh, k, grid, s);
+    else return launch_tc_a<KB, BN, MODE, false, true>(tmA, tmB, tmBh, k, grid, s);
+  }
+  if (MODE != 0 && tc_atmem()) return launch_tc_a<KB, BN, MODE, true, false>(tmA, tmB, tmBh, k, grid, s);
+  return launch_tc_a<KB, BN, MODE, false, false>(tmA, tmB, tmBh, k, grid, s);
 }
 // catalog tile width: 128 items, except that the single-pass H = 256 kernel (user tile 64 KB + lists 32-64 KB on chip) only has room
 // for 64-item tiles.  Wider is better there: a [128 x 64 x 16] MMA re-reads its 4 KB A fragment for 2 KB of B, 192 B/clk of a
@@ -740,6 +800,7 @@ extern "C" int adt_score_topk_tc(const adt_score_topk_tc_args* a, adt_stream_t s
   cudaStream_t s = (cudaStream_t)s_;
   if (a->H % 64 || a->H > 256 || a->K <= 0 || a->K > a->KC || a->KC > 64 || a->n_splits <= 0 || a->n_splits * a->KC > RS_MAXC || a->U <= 0)
     return ADT_E_SHAPE;
+  if (a->item_bias && !a->max_abs_bias) return ADT_E_SHAPE;
   CUtensorMap tmA, tmB;
   const int KB = a->H / 64;
   if (int e = make_map(&tmA, a->feats_bf16, a->U, a->H, BM)) return e;
@@ -747,6 +808,7 @@ extern "C" int adt_score_topk_tc(const adt_score_topk_tc_args* a, adt_stream_t s
   k.seen_indptr = a->seen_indptr; k.seen_idx = a->seen_idx; k.part_scores = a->part_scores; k.part_ids = a->part_ids; k.part_thr = a->part_thr;
   k.U = a->U; k.n_items = a->n_items; k.item_offset = a->item_offset; k.KC = a->KC; k.n_splits = a->n_splits;
   k.feats_bf16 = reinterpret_cast<const __nv_bfloat16*>(a->feats_bf16);
+  k.bias = a->item_bias;
   k.gthr = nullptr;
   if (a->n_splits > 1 && a->flags) {     // `flags` doubles as the threshold exchange buffer until the re-score kernel overwrites it
     k.gthr = reinterpret_cast<unsigned int*>(a->flags);
@@ -809,7 +871,13 @@ extern "C" int adt_score_topk_tc(const adt_score_topk_tc_args* a, adt_stream_t s
   r.U = a->U; r.H = a->H; r.item_offset = a->item_offset; r.K = a->K; r.KC = a->KC; r.n_splits = a->n_splits;
   if (two) { r.KC = a->KC / 2; r.n_splits = 2 * a->n_splits; }     // every (split, column half) wrote its own list and threshold
   r.answers = a->answers; r.metric_acc = a->metric_acc;
-  cudaFuncSetAttribute(rescore_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RS_SMEM);
-  rescore_select_kernel<<<a->U, RS_NT, RS_SMEM, s>>>(r);
+  r.bias = a->item_bias; r.max_abs_bias = a->max_abs_bias;
+  if (a->item_bias) {
+    cudaFuncSetAttribute(rescore_select_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RS_SMEM);
+    rescore_select_kernel<true><<<a->U, RS_NT, RS_SMEM, s>>>(r);
+  } else {
+    cudaFuncSetAttribute(rescore_select_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RS_SMEM);
+    rescore_select_kernel<false><<<a->U, RS_NT, RS_SMEM, s>>>(r);
+  }
   return cudaGetLastError() == cudaSuccess ? ADT_OK : ADT_E_CUDA;
 }

@@ -9,6 +9,8 @@ Item-sharded mode (one 8xB200 box): every rank holds the whole (small) model, sc
 """
 import ctypes
 import math
+from typing import NamedTuple, Optional
+
 import numpy as np
 import torch
 
@@ -16,8 +18,27 @@ from . import _lib as L
 from .model import _as_ids
 
 
+class Catalog(NamedTuple):
+    """What full-catalog evaluation ranks: score(u, row r) = <feats[u], table[r]> (+ bias[r]), reported as global item id first_id + r."""
+    table: torch.Tensor                 # [n_rows, hidden] fp32 rows (a view of the model's item table)
+    bias: Optional[torch.Tensor]        # [n_rows] fp32 per-item term added to every score, or None
+    first_id: int                       # global item id of table row 0
+    hidden: int                         # feature width the encoder produces
+
+
+def catalog_of(model):
+    """The one place that decides which rows of a model are ranked.  Models whose score is not a plain dot product with the whole
+    item table (Bert4Rec: tied head rows 1..itemnum + mask_bias) define `scoring_catalog()`; every other model ranks all rows of
+    `item_emb.weight` from id 0, without a bias."""
+    f = getattr(model, "scoring_catalog", None)
+    if f is not None:
+        return f()
+    E = model.item_emb.weight
+    return Catalog(E, None, 0, E.shape[1])
+
+
 def shard_bounds(n_rows, world, rank):
-    """contiguous, 4-row aligned catalog slice of `rank` (rows 0..n_rows-1 of item_emb, row 0 = padding item)."""
+    """contiguous, 4-row aligned slice of `rank` of the catalog rows 0..n_rows-1 (catalog_of(model).table)."""
     per = (n_rows + world - 1) // world
     per = (per + 3) // 4 * 4
     lo = min(n_rows, rank * per)
@@ -51,23 +72,27 @@ class CatalogScorer:
         self.model, self.K = model, int(K)
         self.use_tc = use_tensor_cores
         self.tc_min_items = tc_min_items   # below this catalog size the exact fp32 kernel is already latency bound and cheaper
-        self._tab = None           # (bf16 copy of this rank's catalog shard, max |e|^2 scalar)
-        self._tab_key = None       # identity/version of the fp32 table the bf16 copy was made from
+        self._tab = None           # (bf16 copy of this rank's catalog shard, max |e|^2 scalar, max |bias| scalar)
+        self._tab_key = None       # identity/version of the fp32 table (and bias) the bf16 copy was made from
         self.lib = L.lib()
         self.pg = process_group
         self.world, self.rank = 1, 0
         if process_group is not None or (torch.distributed.is_available() and torch.distributed.is_initialized()):
             self.world = torch.distributed.get_world_size(process_group)
             self.rank = torch.distributed.get_rank(process_group)
-        n_rows = model.item_emb.weight.shape[0]
+        n_rows = self.catalog().table.shape[0]
         self.sharded = self.world > 1 and (bool(shard) if shard is not None else n_rows >= shard_min_items)
         self.n_splits = n_splits
         self._buf = {}
         self._fallback = None      # device counter: users re-run on the exact fp32 kernel because the bf16 bound was inconclusive
 
     # ------------------------------------------------------------------ helpers
+    def catalog(self):
+        return catalog_of(self.model)
+
     def bounds(self):
-        n_rows = self.model.item_emb.weight.shape[0]
+        """this rank's row range of the catalog (rows, not item ids: id = catalog().first_id + row)"""
+        n_rows = self.catalog().table.shape[0]
         return shard_bounds(n_rows, self.world, self.rank) if self.sharded else (0, n_rows)
 
     @property
@@ -78,24 +103,30 @@ class CatalogScorer:
         return ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
 
     def _table_key(self):
-        E = self.model.item_emb.weight
-        return (E.data_ptr(), E._version, tuple(E.shape), getattr(self.model, "_adt_param_version", 0))
+        c = self.catalog()
+        E, b = c.table, c.bias
+        return (E.data_ptr(), E._version, tuple(E.shape), getattr(self.model, "_adt_param_version", 0),
+                None if b is None else (b.data_ptr(), b._version))
 
     def refresh_table(self):
-        """(re)build the bf16 copy of the catalog shard from the CURRENT item table (in place when the shape is unchanged, so a
-        captured graph keeps reading the same buffer)."""
-        E = self.model.item_emb.weight
+        """(re)build the bf16 copy of the catalog shard and the bound scalars (max |e|^2, max |bias|) from the CURRENT table and bias
+        (in place when the shape is unchanged, so a captured graph keeps reading the same buffers)."""
+        c = self.catalog()
+        E = c.table
         lo, hi = self.bounds()
         shard = E[lo:hi]
         if self._tab is not None and self._tab[0].shape == shard.shape and self._tab[0].device == E.device:
-            tab, mx = self._tab
+            tab, mx, mxb = self._tab
             mx.zero_()
         else:
             tab = torch.empty(shard.shape, dtype=torch.bfloat16, device=E.device)
             mx = torch.zeros(1, dtype=torch.float32, device=E.device)
+            mxb = torch.zeros(1, dtype=torch.float32, device=E.device)
         L.check(self.lib.adt_to_bf16(L.ptr(shard), L.ptr(tab), ctypes.c_int64(shard.shape[0]), ctypes.c_int32(shard.shape[1]), L.ptr(mx),
                                      self._stream(E.device)), "adt_to_bf16")
-        self._tab, self._tab_key = (tab, mx), self._table_key()
+        if c.bias is not None and hi > lo:
+            torch.amax(c.bias[lo:hi].detach().abs(), dim=0, keepdim=True, out=mxb)
+        self._tab, self._tab_key = (tab, mx, mxb), self._table_key()
 
     def ensure_table(self):
         """the bf16 candidates' error bound only holds for the table they were generated from: refresh whenever the fp32 table was
@@ -113,7 +144,7 @@ class CatalogScorer:
         """-> (scores [U,K] fp32, ids [U,K] int32), best first, seen items excluded (utils.py:725).
         answers [U] + metric_acc (float64 device tensor [6]): fused HIT/NDCG@5,10 + MRR sums (get_full_sort_score)."""
         m = self.model
-        dev = m.item_emb.weight.device
+        dev = self.catalog().table.device
         seq = _as_ids(log_seqs, dev)
         feats = m.final_feats(seq)
         return self.topk_from_feats(feats, seen_indptr, seen_idx, answers, metric_acc)
@@ -148,10 +179,10 @@ class CatalogScorer:
         flagged on the device and re-run by the exact kernel in the same stream (masked launch: unflagged tiles exit at once)."""
         dev = feats.device
         U, H = feats.shape
-        E = self.model.item_emb.weight
+        c = self.catalog()
         if self._tab is None:
             self.refresh_table()
-        tab, mx = self._tab
+        tab, mx, mxb = self._tab
         n_items = hi - lo
         K = self.K
         kc, ns = ctypes.c_int32(0), ctypes.c_int32(0)
@@ -170,9 +201,11 @@ class CatalogScorer:
             self._fallback = torch.zeros(1, dtype=torch.int64, device=dev)
         st = self._stream(dev)
         L.check(self.lib.adt_to_bf16(L.ptr(feats), L.ptr(fb), ctypes.c_int64(U), ctypes.c_int32(H), None, st), "adt_to_bf16")
-        a = L.fill(L.adt_score_topk_tc_args(), feats=feats, feats_bf16=fb, U=U, H=H, item_emb=E[lo:hi], item_emb_bf16=tab, n_items=n_items,
-                   item_offset=lo, max_normsq=mx, seen_indptr=ip, seen_idx=ix, K=K, KC=KC, n_splits=S, part_scores=ps, part_ids=pi,
-                   part_thr=pt, out_scores=os_, out_ids=oi, flags=flags, answers=ans, metric_acc=metric_acc)
+        bias = c.bias[lo:hi] if c.bias is not None else None
+        a = L.fill(L.adt_score_topk_tc_args(), feats=feats, feats_bf16=fb, U=U, H=H, item_emb=c.table[lo:hi], item_emb_bf16=tab, n_items=n_items,
+                   item_offset=c.first_id + lo, max_normsq=mx, seen_indptr=ip, seen_idx=ix, K=K, KC=KC, n_splits=S, part_scores=ps, part_ids=pi,
+                   part_thr=pt, out_scores=os_, out_ids=oi, flags=flags, answers=ans, metric_acc=metric_acc,
+                   item_bias=bias, max_abs_bias=mxb if bias is not None else None)
         L.check(self.lib.adt_score_topk_tc(ctypes.byref(a), st), "adt_score_topk_tc")
         self._fallback += flags.sum()
         self._topk_exact(feats, ip, ix, lo, hi, ans, metric_acc, out=(os_, oi), user_mask=flags)
@@ -180,10 +213,9 @@ class CatalogScorer:
 
     @torch.no_grad()
     def _topk_exact(self, feats, ip, ix, lo, hi, ans=None, metric_acc=None, out=None, user_mask=None):
-        m = self.model
+        c = self.catalog()
         dev = feats.device
         U, H = feats.shape
-        E = m.item_emb.weight
         n_items = hi - lo
         tiles = (U + 63) // 64
         S = self.n_splits or max(1, min(256, (2 * 148 + tiles - 1) // tiles, (n_items + 255) // 256))
@@ -195,9 +227,10 @@ class CatalogScorer:
         os_, oi = out if out is not None else (pk[0].view(torch.float32), pk[1])
         if out is None:
             self._last_pk = pk
-        a = L.fill(L.adt_score_topk_args(), feats=feats, U=U, H=H, item_emb=E[lo:hi], n_items=n_items, item_offset=lo,
+        a = L.fill(L.adt_score_topk_args(), feats=feats, U=U, H=H, item_emb=c.table[lo:hi], n_items=n_items, item_offset=c.first_id + lo,
                    seen_indptr=ip, seen_idx=ix, K=self.K, n_splits=S, part_scores=ps, part_ids=pi, out_scores=os_, out_ids=oi,
-                   answers=ans, metric_acc=metric_acc, user_mask=user_mask)
+                   answers=ans, metric_acc=metric_acc, user_mask=user_mask,
+                   item_bias=c.bias[lo:hi] if c.bias is not None else None)
         L.check(self.lib.adt_score_topk(ctypes.byref(a), self._stream(dev)), "adt_score_topk")
         return os_, oi
 
@@ -232,15 +265,15 @@ class GraphedScorer:
 
     def __init__(self, scorer, U, L_, max_seen, capture_collective=True):
         self.sc = scorer
-        m = scorer.model
-        dev = m.item_emb.weight.device
+        cat = scorer.catalog()
+        dev = cat.table.device
         self.U, self.L = int(U), int(L_)
         self.seq = torch.zeros(U, L_, dtype=torch.int32, device=dev)
         self.ip = torch.zeros(U + 1, dtype=torch.int32, device=dev)
         self.ix = torch.zeros(max(1, int(max_seen)), dtype=torch.int32, device=dev)
         self.ans = torch.zeros(U, dtype=torch.int32, device=dev)
         self.metric_acc = torch.zeros(6, dtype=torch.float64, device=dev)
-        self.tc = scorer._uses_tc(m.hidden, *scorer.bounds())
+        self.tc = scorer._uses_tc(cat.hidden, *scorer.bounds())
         if self.tc:
             scorer.refresh_table()
         # the collective of the item-sharded path is captured with the rest when NCCL allows it, else issued between two graphs

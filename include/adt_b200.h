@@ -244,6 +244,9 @@ typedef struct {
   const int32_t* answers; double* metric_acc;
   const int32_t* user_mask;   /* optional [U]: only users with a non-zero entry are scored and written (the exact re-run of the users
                                  adt_score_topk_tc flagged, issued unconditionally so that the whole evaluation stays capturable) */
+  const float* item_bias;     /* optional [n_items], indexed like item_emb (local to the shard): scores[u][i] = <feats[u], item_emb[i]>
+                                 + item_bias[i], the bias added in fp32 once after the full dot product (Bert4Rec's tied head +
+                                 mask_bias).  NULL = no bias */
 } adt_score_topk_args;
 int adt_score_topk(const adt_score_topk_args* a, adt_stream_t stream);
 
@@ -285,6 +288,11 @@ typedef struct {
   float* out_scores; int32_t* out_ids; int32_t* flags;               /* [U][K], [U][K], [U] */
   const int32_t* answers; double* metric_acc;   /* fused metric epilogue as in adt_score_topk, for the users whose result is proven
                                                    exact (flags[u] == 0); flagged users are accumulated by the exact re-run */
+  const float* item_bias;     /* optional [n_items] per-item fp32 bias, as in adt_score_topk (NULL = none).  It is added to every
+                                 accumulator as it leaves tensor memory, so tau, the candidate lists and the exactness test all see
+                                 biased scores; the re-score adds it after the fp32 dot product, bit-identical to adt_score_topk */
+  const float* max_abs_bias;  /* device scalar: max_i |item_bias[i]| (required with item_bias; maintained by the caller like
+                                 max_normsq).  It widens the exactness bound by the rounding of the two fp32 bias additions */
 } adt_score_topk_tc_args;
 int adt_score_topk_tc(const adt_score_topk_tc_args* a, adt_stream_t stream);
 /* Launch plan for adt_score_topk_tc: fills the list capacity KC and the number of catalog splits to pass for (U, n_items, K).
