@@ -7,7 +7,8 @@ attention with the key-padding mask runs in the same attention kernel as SASRec 
 
 `fused_loss` is the B200 training entry: the vocabulary head and the cross entropy are evaluated ONLY on the positions
 that carry a label (~mask_prob of them) instead of the reference's [B*L, V] logits tensor (bert.py:80-90 +
-trainer.py:112-115), in column blocks of the tied item table.
+trainer.py:112-115), in column blocks of the tied item table.  From FUSED_HEAD_MIN_VOCAB items on (bf16 mode, sm_100) the head and the
+cross entropy run fused (ops.linear_cross_entropy): the scores stay on chip, only a per-row log-sum-exp is kept for the backward.
 """
 import ctypes
 import math
@@ -17,7 +18,11 @@ import torch.nn as nn
 
 from . import _lib as L
 from .blocks import DropCfg
-from .ops import AttnFn, DrlFn, Gather3Fn, linear, no_drop
+from .ops import AttnFn, DrlFn, Gather3Fn, linear, linear_cross_entropy, no_drop
+
+# vocabulary size (itemnum + 100) from which fused_loss runs the fused tcgen05 head + cross entropy (adt_linear_ce_*) instead of the
+# [R, V] logits + MaskedCE: at C3 (V 26,844) the materialising path is what runs; at 1M items its [R, V] fp32 tensors no longer fit
+FUSED_HEAD_MIN_VOCAB = 65536
 
 
 def _ids(a, dev):
@@ -215,8 +220,12 @@ class BertModel(nn.Module):
         feats, enc_inputs, dec_outs, inds = self._body(src_ids, dec_ids, pos_ids, sent, pos_ids, sent)
         lab = (labels.to(dev) if isinstance(labels, torch.Tensor) else torch.as_tensor(np.asarray(labels)).to(dev)).view(-1).long()
         rows = torch.nonzero(lab != 0, as_tuple=False).flatten()
-        logits = self.downstream(feats.index_select(0, rows))
-        total = MaskedCE.apply(logits, lab[rows].int())
+        if self._fused_head(rows.numel()):
+            h = self._head_hidden(feats.index_select(0, rows))
+            total = linear_cross_entropy(h, self.item_emb.word_emb.weight, self.mask_bias, lab[rows].int())
+        else:
+            logits = self.downstream(feats.index_select(0, rows))
+            total = MaskedCE.apply(logits, lab[rows].int())
         nh = self.num_heads
         for i in range(self.num_layers):
             if lambda1[i] != 0:
@@ -227,6 +236,13 @@ class BertModel(nn.Module):
                 if lambda2[l] != 0:
                     total = total + lambda2[l] * F.nll_loss(inds[l].reshape(B * Lq, nh, nh), label)
         return total
+
+    def _fused_head(self, R):
+        """fused_loss's choice of vocabulary head: the fused tcgen05 head + cross entropy in the bf16 mode on sm_100 from
+        FUSED_HEAD_MIN_VOCAB on; the [R, V] logits + MaskedCE otherwise (precision 0 is the parity mode and stays there)."""
+        dev = self.mask_bias.device
+        return (self.precision == 1 and R > 0 and self.mask_bias.shape[0] >= FUSED_HEAD_MIN_VOCAB
+                and torch.cuda.get_device_capability(dev) == (10, 0))
 
     # ---- full-catalog evaluation -------------------------------------------------------------
     def scoring_catalog(self):

@@ -24,6 +24,10 @@ static int fail(int code, const char* fmt, const char* what) {
   snprintf(g_err, sizeof(g_err), fmt, what);
   return code;
 }
+// the same message slot for the entry points of the other translation units
+namespace adt {
+int set_error(int code, const char* msg) { return fail(code, "%s", msg); }
+}
 static int check_launch(const char* what) {
   const cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) {

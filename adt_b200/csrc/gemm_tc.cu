@@ -36,6 +36,15 @@ struct GemmTcArgs {
   int stage;                                 // the launch reserved the chunk staging area of the coalesced epilogue
   int batch_inner, nbatch;    // strided batch: blockIdx.z = zo * batch_inner + zi selects the matrices (nbatch <= 1: blockIdx.z = K split)
   long long c_so, c_si;       // element offsets of C per outer / inner batch index
+  // linear + cross-entropy epilogues (MODE 1 / 2 of gemm_tc_kernel; C, pre, act, split K and batching unused there).  Columns are
+  // local to one vocabulary chunk: the B map, bias and g_bias start at its first row, labels are shifted by label_off.
+  const int* labels; int label_off;
+  float2* part;               // MODE 1: per-tile (max, sum exp) of every row, [tiles_n][M]
+  float* zlab;                // MODE 1: z[r, label[r]] when the label falls in this chunk
+  const float* lse;           // MODE 2: per-row log-sum-exp of the forward
+  float coef; const float* coef_dev;     // MODE 2: dS = coef * (*coef_dev) * (softmax - onehot)
+  __nv_bfloat16* ds; long long ld_ds;    // MODE 2: bf16 dS [M][ld_ds]
+  float* g_bias;              // MODE 2: += fp32 column sums of dS (NULL: no bias)
 };
 
 __device__ __forceinline__ float g_gelu(float x) { return 0.5f * x * (1.f + erff(x * 0.70710678118654752f)); }
@@ -124,7 +133,101 @@ __device__ __forceinline__ WorkItem g_item(const GemmTcArgs& a, int w, int BN) {
   return it;
 }
 
-template <int BN, int NS>
+// Epilogue of the fused vocabulary head (adt_linear_ce_fwd / _bwd): z = acc + bias[v] leaves TMEM and is consumed on chip.
+//   MODE 1: the thread owning row r keeps a running (max, sum exp) over the tile's columns and writes it to part[tile_n][r]; it also
+//           takes z[r, label[r]] from the same accumulator when the label falls in the tile.  The scores never reach HBM.
+//   MODE 2: dS = c (exp(z - lse[r]) - [v == label[r]]) in fp32; its column sums go to g_bias (atomics, one per column per warp and
+//           tile), then it is rounded to bf16 and stored as [M][ld_ds] rows, 64 contiguous bytes per half-warp, via the staging chunk.
+template <int BN, int MODE>
+__device__ __forceinline__ void ce_epilogue(const GemmTcArgs& a, uint32_t tmem_base, uint64_t* tfull, uint64_t* tempty, float* __restrict__ stage,
+                                            int q, int lane) {
+  const float c = MODE == 2 ? a.coef * (a.coef_dev ? *a.coef_dev : 1.f) : 0.f;
+  int n = 0;
+  for (int w = blockIdx.x; w < a.n_work; w += gridDim.x) {
+    const WorkItem it = g_item(a, w, BN);
+    const int acc = n & 1;
+    tc::mbar_wait(tfull + acc, (n >> 1) & 1);
+    tc::tc_fence_after();
+    const int row = it.m0 + 32 * q + lane;
+    const bool live = row < a.M;
+    const int lab = live ? __ldg(a.labels + row) - a.label_off : -1;
+    const float ls = MODE == 2 && live ? __ldg(a.lse + row) : 0.f;
+    float m = -INFINITY, s = 0.f, zl = 0.f;
+    bool has = false;
+#pragma unroll 1
+    for (int c0 = 0; c0 < BN; c0 += 32) {
+      float v[32];
+      tc::tmem_ld32(tmem_base + ((uint32_t)(32 * q) << 16) + acc * BN + c0, v);
+      if (c0 + 32 == BN) {
+        tc::tc_fence_before();
+        __syncwarp();
+        if (lane == 0) tc::mbar_arrive(tempty + acc);
+      }
+      const int nb = it.n0 + c0;
+      if (nb >= a.N) continue;             // warp-uniform
+      if (a.bias) {
+#pragma unroll
+        for (int j = 0; j < 32; ++j)
+          if (nb + j < a.N) v[j] += __ldg(a.bias + nb + j);
+      }
+      if constexpr (MODE == 1) {
+        float cm = -INFINITY;
+#pragma unroll
+        for (int j = 0; j < 32; ++j)
+          if (nb + j < a.N) cm = fmaxf(cm, v[j]);
+        if (lab >= nb && lab < nb + 32) {
+          has = true;
+#pragma unroll
+          for (int j = 0; j < 32; ++j)
+            if (nb + j == lab) zl = v[j];
+        }
+        const float mn = fmaxf(m, cm);
+        float t = 0.f;
+#pragma unroll
+        for (int j = 0; j < 32; ++j) t += nb + j < a.N ? __expf(v[j] - mn) : 0.f;
+        s = s * __expf(m - mn) + t;
+        m = mn;
+      } else {
+#pragma unroll
+        for (int j = 0; j < 32; j += 4) {
+          float4 o;
+          o.x = live && nb + j < a.N ? c * (__expf(v[j] - ls) - (nb + j == lab ? 1.f : 0.f)) : 0.f;
+          o.y = live && nb + j + 1 < a.N ? c * (__expf(v[j + 1] - ls) - (nb + j + 1 == lab ? 1.f : 0.f)) : 0.f;
+          o.z = live && nb + j + 2 < a.N ? c * (__expf(v[j + 2] - ls) - (nb + j + 2 == lab ? 1.f : 0.f)) : 0.f;
+          o.w = live && nb + j + 3 < a.N ? c * (__expf(v[j + 3] - ls) - (nb + j + 3 == lab ? 1.f : 0.f)) : 0.f;
+          *reinterpret_cast<float4*>(stage + lane * 36 + j) = o;
+        }
+        __syncwarp();
+        if (a.g_bias) {                    // lane == column: fp32 sum over the warp's 32 rows (dead rows hold 0)
+          float cs = 0.f;
+#pragma unroll 8
+          for (int r = 0; r < 32; ++r) cs += stage[r * 36 + lane];
+          if (nb + lane < a.N) atomicAdd(a.g_bias + nb + lane, cs);
+        }
+        const int hr = lane >> 4, cc = (lane & 15) * 2, row0 = it.m0 + 32 * q;
+#pragma unroll 4
+        for (int r = 0; r < 32; r += 2) {
+          const int rr = r + hr;
+          if (row0 + rr >= a.M || nb + cc >= a.N) continue;
+          const float2 p = *reinterpret_cast<const float2*>(stage + rr * 36 + cc);
+          __nv_bfloat16* dst = a.ds + (long long)(row0 + rr) * a.ld_ds + nb + cc;
+          if (nb + cc + 1 < a.N) *reinterpret_cast<__nv_bfloat162*>(dst) = __floats2bfloat162_rn(p.x, p.y);
+          else *dst = __float2bfloat16_rn(p.x);
+        }
+        __syncwarp();
+      }
+    }
+    if constexpr (MODE == 1) {
+      if (live) {
+        a.part[(long long)(it.n0 / BN) * a.M + row] = make_float2(m, s);
+        if (has) a.zlab[row] = zl;
+      }
+    }
+    ++n;
+  }
+}
+
+template <int BN, int NS, int MODE = 0>
 __global__ void __launch_bounds__(G_THREADS, 1) gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                                                                GemmTcArgs a) {
   extern __shared__ uint8_t smem_raw[];
@@ -209,6 +312,8 @@ __global__ void __launch_bounds__(G_THREADS, 1) gemm_tc_kernel(const __grid_cons
         ++n;
       }
     }
+  } else if constexpr (MODE != 0) {
+    ce_epilogue<BN, MODE>(a, tmem_base, tfull, tempty, stage_all + (warp & 3) * (32 * 36), warp & 3, lane);
   } else {
     const int q = warp & 3;
     const bool vec = ((a.ldc & 3) == 0) && ((reinterpret_cast<uintptr_t>(a.C) & 15) == 0) && (!a.pre || (reinterpret_cast<uintptr_t>(a.pre) & 15) == 0);
@@ -339,11 +444,11 @@ int g_make_map(CUtensorMap* m, const void* base, long long rows, long long cols,
   return r == CUDA_SUCCESS ? ADT_OK : ADT_E_CUDA;
 }
 
-template <int BN, int NS>
+template <int BN, int NS, int MODE = 0>
 int g_launch(const CUtensorMap& tmA, const CUtensorMap& tmB, GemmTcArgs k, int splits, cudaStream_t s, bool stage = false) {
   k.stage = stage ? 1 : 0;
   const size_t smem = 1024 + (size_t)NS * (GM * 128 + BN * 128) + 256 + (stage ? 4 * 32 * 36 * 4 : 0);
-  cudaFuncSetAttribute(gemm_tc_kernel<BN, NS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaFuncSetAttribute(gemm_tc_kernel<BN, NS, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   k.tiles_n = (k.N + BN - 1) / BN; k.tiles_m = (k.M + GM - 1) / GM;
   k.n_split_k = k.nbatch > 1 ? 1 : splits;
   const long long work = (long long)k.tiles_n * k.tiles_m * splits;
@@ -354,11 +459,155 @@ int g_launch(const CUtensorMap& tmA, const CUtensorMap& tmB, GemmTcArgs k, int s
   if (per_sm > 512 / (2 * BN)) per_sm = 512 / (2 * BN);
   if (per_sm < 1) per_sm = 1;
   const int grid = (int)(work < 148ll * per_sm ? work : 148ll * per_sm);
-  gemm_tc_kernel<BN, NS><<<grid, G_THREADS, smem, s>>>(tmA, tmB, k);
+  gemm_tc_kernel<BN, NS, MODE><<<grid, G_THREADS, smem, s>>>(tmA, tmB, k);
   return cudaGetLastError() == cudaSuccess ? ADT_OK : ADT_E_CUDA;
 }
 
+// Folds one vocabulary chunk's per-tile (max, sum exp) into the running per-row state; after the last chunk it writes lse[r] and adds
+// sum_r (lse[r] - z[r, label[r]]) into the fp64 accumulator (as adt_softmax_ce_fwd does).
+__global__ void __launch_bounds__(256) ce_merge_kernel(const float2* __restrict__ part, int ntiles, float2* __restrict__ state,
+                                                       const float* __restrict__ zlab, float* __restrict__ lse, double* __restrict__ acc, int R,
+                                                       int first, int last) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  double loss = 0.0;
+  if (r < R) {
+    float m = -INFINITY, s = 0.f;
+    if (!first) { const float2 st = state[r]; m = st.x; s = st.y; }
+    for (int t = 0; t < ntiles; ++t) {
+      const float2 p = part[(long long)t * R + r];
+      const float mn = fmaxf(m, p.x);
+      s = s * __expf(m - mn) + p.y * __expf(p.x - mn);
+      m = mn;
+    }
+    if (last) {
+      const float l = m + logf(s);
+      lse[r] = l;
+      loss = (double)(l - zlab[r]);
+    } else {
+      state[r] = make_float2(m, s);
+    }
+  }
+  if (last) {
+    for (int o = 16; o; o >>= 1) loss += __shfl_xor_sync(0xffffffffu, loss, o);
+    if ((threadIdx.x & 31) == 0) atomicAdd(acc, loss);
+  }
+}
+
+// Scratch of the fused head for a vocabulary chunk of vc columns (a multiple of 128): bf16 dS [R][vc] (backward), then the forward's
+// per-tile partials [vc / 128][R] float2, the running per-row (max, sum exp) and z[r, label[r]].  Each area is 256-byte aligned.
+struct CeLayout { long long part, state, zlab, total; };
+long long ce_a256(long long b) { return (b + 255) & ~255ll; }
+CeLayout ce_layout(long long R, long long vc) {
+  CeLayout l;
+  l.part = ce_a256(2 * R * vc);
+  l.state = l.part + ce_a256(8 * R * (vc / 128));
+  l.zlab = l.state + ce_a256(8 * R);
+  l.total = l.zlab + ce_a256(4 * R);
+  return l;
+}
+// widest chunk (a multiple of 128, at most V rounded up) whose layout fits in `bytes`; 0 if not even 128 columns fit
+long long ce_chunk128(long long R, long long V, long long bytes) {
+  const long long vmax = (V + 127) / 128 * 128;
+  long long vc = bytes > 12 * R ? (bytes - 12 * R) / (264 * R) * 128 : 0;     // 2 R + 8 R / 128 bytes per column, then the alignment
+  if (vc > vmax) vc = vmax;
+  while (vc >= 128 && ce_layout(R, vc).total > bytes) vc -= 128;
+  return vc >= 128 ? vc : 0;
+}
+
 }  // namespace
+
+namespace adt {
+int set_error(int code, const char* msg);
+}
+
+extern "C" int adt_linear_ce_plan(int32_t R, int32_t V, int32_t H, int64_t scratch_bytes, int32_t* vocab_chunk, int64_t* min_scratch_bytes) {
+  if (R <= 0 || V <= 0 || H <= 0) return set_error(ADT_E_SHAPE, "linear_ce_plan: R, V and H must be positive");
+  if (min_scratch_bytes) *min_scratch_bytes = ce_layout(R, 128).total;
+  const long long vc = ce_chunk128(R, V, scratch_bytes);
+  if (vocab_chunk) *vocab_chunk = (int32_t)(vc < V ? vc : V);
+  if (!vc) return set_error(ADT_E_SHAPE, "linear_ce_plan: scratch_bytes is below the minimum for one 128-column vocabulary chunk");
+  return ADT_OK;
+}
+
+namespace {
+// shared validation of adt_linear_ce_fwd / _bwd: returns the vocabulary chunk (multiple of 128) or an ADT_E_* code (< 0)
+long long ce_check(const adt_linear_ce_args* a, bool bwd) {
+  if (a->R <= 0 || a->V <= 0 || a->H <= 0 || a->ldx < a->H || a->ldw < a->H || (a->ldx & 7) || (a->ldw & 7))
+    return set_error(ADT_E_SHAPE, "linear_ce: R, V, H must be positive, ldx and ldw multiples of 8 and >= H");
+  if (!a->x_bf16 || !a->w_bf16 || !a->labels || !a->lse || !a->scratch || (bwd ? !a->dx || !a->g_w : !a->loss_acc))
+    return set_error(ADT_E_SHAPE, "linear_ce: x_bf16, w_bf16, labels, lse, scratch and loss_acc (forward) or dx, g_w (backward) are required");
+  if ((reinterpret_cast<uintptr_t>(a->x_bf16) | reinterpret_cast<uintptr_t>(a->w_bf16) | reinterpret_cast<uintptr_t>(a->scratch)) & 15)
+    return set_error(ADT_E_ALIGN, "linear_ce: x_bf16, w_bf16 and scratch must be 16-byte aligned");
+  const long long vc = ce_chunk128(a->R, a->V, a->scratch_bytes);
+  if (!vc) return set_error(ADT_E_SHAPE, "linear_ce: scratch_bytes is below adt_linear_ce_plan's min_scratch_bytes");
+  return vc;
+}
+
+template <int MODE>
+int ce_launch(const adt_linear_ce_args* a, GemmTcArgs k, long long v0, int nc, cudaStream_t s) {
+  CUtensorMap tmA, tmB;
+  const __nv_bfloat16* w = reinterpret_cast<const __nv_bfloat16*>(a->w_bf16) + v0 * a->ldw;
+  if (int e = g_make_map(&tmA, a->x_bf16, a->R, a->H, a->ldx, GM)) return e;
+  if (int e = g_make_map(&tmB, w, nc, a->H, a->ldw, 128)) return e;
+  k.M = a->R; k.N = nc; k.K = a->H; k.scale = 1.f; k.nbatch = 1; k.batch_inner = 1;
+  k.bias = a->bias ? a->bias + v0 : nullptr;
+  k.labels = a->labels; k.label_off = (int)v0;
+  const int nkb = (a->H + 63) / 64;
+  k.kb_per_split = nkb;
+  return nkb <= 4 ? g_launch<128, 2, MODE>(tmA, tmB, k, 1, s, MODE == 2)
+       : nkb <= 16 ? g_launch<128, 3, MODE>(tmA, tmB, k, 1, s, MODE == 2) : g_launch<128, 6, MODE>(tmA, tmB, k, 1, s, MODE == 2);
+}
+}  // namespace
+
+extern "C" int adt_linear_ce_fwd(const adt_linear_ce_args* a, adt_stream_t s_) {
+  cudaStream_t s = (cudaStream_t)s_;
+  const long long vc = ce_check(a, false);
+  if (vc < 0) return (int)vc;
+  const CeLayout lay = ce_layout(a->R, vc);
+  uint8_t* base = reinterpret_cast<uint8_t*>(a->scratch);
+  GemmTcArgs k;
+  memset(&k, 0, sizeof(k));
+  k.part = reinterpret_cast<float2*>(base + lay.part);
+  k.zlab = reinterpret_cast<float*>(base + lay.zlab);
+  for (long long v0 = 0; v0 < a->V; v0 += vc) {
+    const int nc = (int)(a->V - v0 < vc ? a->V - v0 : vc);
+    if (ce_launch<1>(a, k, v0, nc, s)) return set_error(ADT_E_CUDA, "linear_ce_fwd: tcgen05 launch failed");
+    ce_merge_kernel<<<(a->R + 255) / 256, 256, 0, s>>>(k.part, (nc + 127) / 128, reinterpret_cast<float2*>(base + lay.state), k.zlab, a->lse, a->loss_acc,
+                                                       a->R, v0 == 0, v0 + nc >= a->V);
+    if (cudaGetLastError() != cudaSuccess) return set_error(ADT_E_CUDA, "linear_ce_fwd: merge launch failed");
+  }
+  return ADT_OK;
+}
+
+extern "C" int adt_linear_ce_bwd(const adt_linear_ce_args* a, adt_stream_t s_) {
+  cudaStream_t s = (cudaStream_t)s_;
+  const long long vc = ce_check(a, true);
+  if (vc < 0) return (int)vc;
+  __nv_bfloat16* ds = reinterpret_cast<__nv_bfloat16*>(a->scratch);
+  GemmTcArgs k;
+  memset(&k, 0, sizeof(k));
+  k.lse = a->lse; k.coef = a->coef; k.coef_dev = a->coef_dev; k.ds = ds; k.ld_ds = vc;
+  const int H = a->H;
+  for (long long v0 = 0; v0 < a->V; v0 += vc) {
+    const int nc = (int)(a->V - v0 < vc ? a->V - v0 : vc);
+    k.g_bias = a->g_bias ? a->g_bias + v0 : nullptr;
+    if (ce_launch<2>(a, k, v0, nc, s)) return set_error(ADT_E_CUDA, "linear_ce_bwd: tcgen05 launch failed");
+    // dx (+)= dS W[v0 : v0 + nc]   (W read MN-major: no transposed copy)
+    adt_gemm_tc_args g;
+    memset(&g, 0, sizeof(g));
+    g.a_bf16 = ds; g.lda = vc; g.b_bf16 = reinterpret_cast<const __nv_bfloat16*>(a->w_bf16) + v0 * a->ldw; g.ldb = a->ldw; g.b_mn = 1;
+    g.c = a->dx; g.ldc = H; g.M = a->R; g.N = H; g.K = nc; g.accumulate = v0 > 0; g.scale = 1.f;
+    if (adt_gemm_tc(&g, s_)) return set_error(ADT_E_CUDA, "linear_ce_bwd: dgrad GEMM failed");
+    // g_W[v0 : v0 + nc] += dS^T x   (dS and x read MN-major, K = R split across CTAs as LinearFn's wgrad does)
+    memset(&g, 0, sizeof(g));
+    g.a_bf16 = ds; g.lda = vc; g.a_mn = 1; g.b_bf16 = a->x_bf16; g.ldb = a->ldx; g.b_mn = 1;
+    g.c = a->g_w + v0 * H; g.ldc = H; g.M = nc; g.N = H; g.K = a->R; g.accumulate = 1; g.scale = 1.f;
+    const int tiles = ((nc + 127) / 128) * ((H + 127) / 128), kspl = 148 / tiles, kmax = (a->R + 63) / 64;
+    g.split_k = kspl < 1 ? 1 : kspl < kmax ? kspl : kmax;
+    if (adt_gemm_tc(&g, s_)) return set_error(ADT_E_CUDA, "linear_ce_bwd: wgrad GEMM failed");
+  }
+  return ADT_OK;
+}
 
 extern "C" int adt_gemm_tc(const adt_gemm_tc_args* a, adt_stream_t s_) {
   cudaStream_t s = (cudaStream_t)s_;

@@ -139,6 +139,79 @@ def linear(x, W, b=None, act=0, scale=1.0, precision=0):
     return LinearFn.apply(x, W, b, act, scale, precision)
 
 
+LINEAR_CE_SCRATCH = 256 << 20   # bytes of the fused head's vocabulary-chunk scratch (bf16 dS [R, Vc] + the forward's per-tile partials)
+
+
+def linear_ce_plan(R, V, H, scratch_bytes):
+    """(vocab_chunk, min_scratch_bytes) of adt_linear_ce_plan; raises when scratch_bytes is below the minimum."""
+    vc, mn = ctypes.c_int32(0), ctypes.c_int64(0)
+    L.check(L.lib().adt_linear_ce_plan(ctypes.c_int32(R), ctypes.c_int32(V), ctypes.c_int32(H), ctypes.c_int64(scratch_bytes), ctypes.byref(vc),
+                                       ctypes.byref(mn)), "adt_linear_ce_plan")
+    return vc.value, mn.value
+
+
+def linear_ce_scratch_bytes(R, V, H, budget=None):
+    """scratch the fused head is given: `budget` (default LINEAR_CE_SCRATCH), at least the planner's minimum, at most what one chunk
+    covering all of V needs."""
+    budget = LINEAR_CE_SCRATCH if budget is None else budget
+    _, mn = linear_ce_plan(R, V, H, 1 << 62)
+    # one chunk covering V: 2 R bytes of dS and 8 R / 128 of partials per column, 12 R of row state, 256-byte alignment of four areas
+    full = 264 * R * ((V + 127) // 128) + 12 * R + 1024
+    return max(mn, min(budget, full))
+
+
+class LinearCE(torch.autograd.Function):
+    """mean over rows of cross_entropy(h W^T + b, labels) on the tcgen05 fused head (adt_linear_ce_fwd / _bwd): the [R, V] logits are
+    never materialised.  Saves the bf16 copies of h and W and the per-row log-sum-exp; the backward recomputes the scores chunk by chunk."""
+
+    @staticmethod
+    def forward(ctx, h, W, b, labels, scratch_bytes):
+        h = h.contiguous()
+        R, H = h.shape
+        V = W.shape[0]
+        dev = h.device
+        x16, ldx = _bf16(h)
+        w16, ldw = _bf16(W.contiguous())
+        b = b.contiguous() if b is not None else None
+        labels = labels.to(device=dev, dtype=torch.int32).contiguous()
+        nbytes = linear_ce_scratch_bytes(R, V, H, scratch_bytes)
+        scratch = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        lse = torch.empty(R, dtype=torch.float32, device=dev)
+        acc = torch.zeros(1, dtype=torch.float64, device=dev)
+        a = L.fill(L.adt_linear_ce_args(), x_bf16=x16, w_bf16=w16, ldx=ldx, ldw=ldw, bias=b, labels=labels, R=R, V=V, H=H, lse=lse,
+                   loss_acc=acc, scratch=scratch, scratch_bytes=nbytes)
+        L.check(L.lib().adt_linear_ce_fwd(ctypes.byref(a), _st(dev)), "adt_linear_ce_fwd")
+        ctx.save_for_backward(x16, w16, b, labels, lse)
+        ctx.cfg = (ldx, ldw, W.shape, nbytes)
+        return (acc / R).float().squeeze(0)
+
+    @staticmethod
+    def backward(ctx, g):
+        x16, w16, b, labels, lse = ctx.saved_tensors
+        ldx, ldw, wshape, nbytes = ctx.cfg
+        R, V, H = lse.shape[0], wshape[0], wshape[1]
+        dev = lse.device
+        g = g.detach().float().reshape(1).contiguous()     # the upstream gradient stays on the device: no host sync
+        dx = torch.empty(R, H, dtype=torch.float32, device=dev)
+        gW = torch.zeros(wshape, dtype=torch.float32, device=dev)
+        gb = torch.zeros(V, dtype=torch.float32, device=dev) if b is not None else None
+        scratch = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        a = L.fill(L.adt_linear_ce_args(), x_bf16=x16, w_bf16=w16, ldx=ldx, ldw=ldw, bias=b, labels=labels, R=R, V=V, H=H,
+                   lse=lse, coef=1.0 / R, coef_dev=g, dx=dx, g_w=gW, g_bias=gb, scratch=scratch, scratch_bytes=nbytes)
+        L.check(L.lib().adt_linear_ce_bwd(ctypes.byref(a), _st(dev)), "adt_linear_ce_bwd")
+        return dx, gW, gb, None, None
+
+
+def linear_cross_entropy(h, W, b, labels, scratch_bytes=None):
+    """mean_r [logsumexp_v(h_r . W_v + b_v) - (h_r . W_{labels[r]} + b_{labels[r]})] with bf16 products and fp32 accumulation, without the
+    [R, V] logits: h [R, H] fp32, W [V, H] fp32, b [V] fp32 or None, labels [R] in [0, V).  Differentiable in h, W and b.  Needs sm_100."""
+    if h.shape[0] < 1:
+        raise L.AdtError("linear_cross_entropy: no rows")
+    if torch.cuda.get_device_capability(h.device) != (10, 0):
+        raise L.AdtError("linear_cross_entropy runs on the sm_100 tensor cores only")
+    return LinearCE.apply(h, W, b, labels, scratch_bytes)
+
+
 class DrlFn(torch.autograd.Function):
     """mode 0: LN(dropout(a) + r) ; mode 1: dropout(LN(a + r)).  r may be None."""
 

@@ -378,6 +378,27 @@ int adt_attention_bwd(const adt_attention_args* a, adt_stream_t stream);
  * fwd: lse[r], *loss_acc += sum_r (lse[r] - logits[r][labels[r]]).  bwd: logits <- (softmax - onehot) * coef, in place. */
 int adt_softmax_ce_fwd(const float* logits, const int32_t* labels, float* lse, double* loss_acc, int32_t R, int32_t V, adt_stream_t stream);
 int adt_softmax_ce_bwd(float* logits, const int32_t* labels, const float* lse, float coef, int32_t R, int32_t V, adt_stream_t stream);
+/* vocabulary head + softmax cross-entropy without the [R,V] logits (bert.py:80-90 + trainer.py:113-115 on the labelled rows):
+ *   z[r][v] = <x[r], W[v]> + bias[v]   (bf16 operands, fp32 accumulation in TMEM, bias added in fp32 as the accumulator leaves it).
+ * fwd: lse[r] = log sum_v exp z[r][v];  *loss_acc += sum_r (lse[r] - z[r][labels[r]]).  The scores stay on chip: the tcgen05 epilogue keeps
+ *      a running (max, sum exp) per row and tile, a merge kernel folds the tiles.
+ * bwd: per vocabulary chunk [v0, v0 + Vc): recompute z, dS = c (exp(z - lse) - onehot) with c = coef * (*coef_dev if non-NULL) rounded to
+ *      bf16 in scratch; g_bias[v] += fp32 column sums of dS; dx (+)= dS W[v0:v0+Vc] and g_w[v0:v0+Vc] += dS^T x on adt_gemm_tc.
+ *      dx [R][H] fp32 is overwritten, g_w [V][H] fp32 and g_bias [V] are accumulated.
+ * x_bf16 [R][ldx], w_bf16 [V][ldw] (ldx, ldw >= H, multiples of 8), labels in [0, V), bias / g_bias / coef_dev may be NULL.
+ * Vc is the widest multiple of 128 whose scratch fits scratch_bytes (adt_linear_ce_plan): memory O(R Vc), not O(R V). */
+typedef struct {
+  const void* x_bf16; const void* w_bf16; int64_t ldx, ldw;
+  const float* bias; const int32_t* labels; int32_t R, V, H;
+  float* lse; double* loss_acc; float coef; const float* coef_dev;
+  float* dx; float* g_w; float* g_bias;
+  void* scratch; int64_t scratch_bytes;
+} adt_linear_ce_args;
+int adt_linear_ce_fwd(const adt_linear_ce_args* a, adt_stream_t stream);
+int adt_linear_ce_bwd(const adt_linear_ce_args* a, adt_stream_t stream);
+/* host only: the vocabulary chunk (*vocab_chunk, = V when one chunk covers it) for scratch_bytes, and the least scratch that works (one
+ * 128-column chunk).  ADT_E_SHAPE when scratch_bytes is below that. */
+int adt_linear_ce_plan(int32_t R, int32_t V, int32_t H, int64_t scratch_bytes, int32_t* vocab_chunk, int64_t* min_scratch_bytes);
 
 /* ---- STOSA-ADT (SURVEY 8a row a20) -------------------------------------------------------------------------------
  * elementwise activation y = act(x) (act codes of adt_linear_fwd); n % 4 == 0. */
