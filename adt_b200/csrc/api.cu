@@ -1415,6 +1415,27 @@ extern "C" int adt_wcatalog_rows(const float* mean, const float* cov, float* out
   wcatalog_kernel<<<min((n + 7) / 8, 148 * 8), NT, 0, (cudaStream_t)s_>>>(mean, cov, out, n, H, is_user);
   return check_launch("wcatalog_rows");
 }
+extern "C" int adt_wcatalog_work_bytes(int32_t H, int64_t* bytes) {
+  if (H <= 0 || 2 * H > NT) return fail(ADT_E_SHAPE, "%s", "wcatalog_work_bytes: H must be 1..128");
+  *bytes = (int64_t)WCAT_PARTS * 2 * H * (int64_t)sizeof(double) + 16;
+  return ADT_OK;
+}
+extern "C" int adt_wcatalog_build(const float* mean, const float* cov, int32_t n, int32_t H, float* mu, float* rows, float* bias, void* work,
+                                  adt_stream_t s_) {
+  if (n <= 0 || H <= 0 || 2 * H > NT) return fail(ADT_E_SHAPE, "%s", "wcatalog_build: dims (n >= 1, H must be 1..128)");
+  const cudaStream_t s = (cudaStream_t)s_;
+  double* part = (double*)work;
+  unsigned int* counter = (unsigned int*)(part + (int64_t)WCAT_PARTS * 2 * H);
+  wcat_mean_kernel<<<WCAT_PARTS, NT, 0, s>>>(mean, cov, n, H, part, counter, mu);
+  wcat_rows_kernel<<<min((n + 7) / 8, 148 * 8), NT, 0, s>>>(mean, cov, mu, n, H, rows, bias);
+  return check_launch("wcatalog_build");
+}
+extern "C" int adt_wcatalog_user(const float* mean, const float* cov, const float* mu, float* out, int32_t U, int32_t H, adt_stream_t s_) {
+  if (U <= 0 || H <= 0) return fail(ADT_E_SHAPE, "%s", "wcatalog_user: dims");
+  const long long blocks = ((long long)U * 2 * H + NT - 1) / NT;
+  wcat_user_kernel<<<(int)min(blocks, 148LL * 8), NT, 0, (cudaStream_t)s_>>>(mean, cov, mu, U, H, out);
+  return check_launch("wcatalog_user");
+}
 
 extern "C" int adt_debug_read(long long* out, int n) {
   cudaDeviceSynchronize();

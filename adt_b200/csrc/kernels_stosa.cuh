@@ -464,4 +464,78 @@ __global__ void __launch_bounds__(NT) wcatalog_kernel(const float* __restrict__ 
   }
 }
 
+// centred catalog for K7 (adt_wcatalog_build / adt_wcatalog_user): item row y_i = [ mean_i | sqrt(elu(cov_i)+1) ], user row
+// x_u = [ mean_u | sqrt(cov_u) ], mu = column mean of the y_i;  rows e_i = y_i - mu, bias b_i = -|e_i|^2, user features f_u = 2 (x_u - mu).
+constexpr int WCAT_PARTS = 296;     // column-sum blocks (2 per SM); fixed, so the summation order depends on n and H only
+
+__device__ __forceinline__ float wcat_col(const float* __restrict__ Em, const float* __restrict__ Ec, long long r, int c, int H) {
+  return c < H ? Em[r * H + c] : wsqrt(elu1(Ec[r * H + c - H]));
+}
+
+// Deterministic column mean of the 2H-wide item rows in one launch of WCAT_PARTS blocks.  Block b sums the fixed row range
+// [b*chunk, (b+1)*chunk): thread t owns column t % 2H of sub-row t / 2H, fp64 accumulation in row order, sub-rows folded in order.
+// The last block to arrive (counter in `work`) folds the WCAT_PARTS partials in block order and resets the counter to 0.
+__global__ void __launch_bounds__(NT) wcat_mean_kernel(const float* __restrict__ Em, const float* __restrict__ Ec, int n, int H,
+                                                       double* __restrict__ part, unsigned int* counter, float* __restrict__ mu) {
+  __shared__ double red[NT];
+  __shared__ bool last;
+  const int W = 2 * H, S = NT / W, c = threadIdx.x % W, s = threadIdx.x / W;
+  const long long chunk = ((long long)n + WCAT_PARTS - 1) / WCAT_PARTS;
+  const long long lo = blockIdx.x * chunk, hi = min((long long)n, lo + chunk);
+  double acc = 0.0;
+  if (s < S) {
+#pragma unroll 4
+    for (long long r = lo + s; r < hi; r += S) acc += (double)wcat_col(Em, Ec, r, c, H);
+  }
+  red[threadIdx.x] = acc;
+  __syncthreads();
+  if (threadIdx.x < W) {
+    double t = red[threadIdx.x];
+    for (int j = 1; j < S; ++j) t += red[j * W + threadIdx.x];
+    part[(long long)blockIdx.x * W + threadIdx.x] = t;
+  }
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) last = atomicAdd(counter, 1u) == WCAT_PARTS - 1;
+  __syncthreads();
+  if (!last) return;
+  __threadfence();
+  if (threadIdx.x < W) {
+    double t = 0.0;
+#pragma unroll 8
+    for (int b = 0; b < WCAT_PARTS; ++b) t += __ldcg(part + (long long)b * W + threadIdx.x);
+    mu[threadIdx.x] = (float)(t / (double)n);
+  }
+  if (threadIdx.x == 0) *counter = 0u;
+}
+
+// warp per item row: rows[i] = y_i - mu, bias[i] = -|rows[i]|^2 (fp32, from the stored values)
+__global__ void __launch_bounds__(NT) wcat_rows_kernel(const float* __restrict__ Em, const float* __restrict__ Ec, const float* __restrict__ mu,
+                                                       int n, int H, float* __restrict__ rows, float* __restrict__ bias) {
+  const int lane = threadIdx.x & 31, wpb = NT / 32, W = 2 * H;
+  for (long long r = blockIdx.x * wpb + (threadIdx.x >> 5); r < n; r += (long long)gridDim.x * wpb) {
+    float nrm = 0.f;
+    for (int c = lane; c < W; c += 32) {
+      const float e = wcat_col(Em, Ec, r, c, H) - mu[c];
+      rows[r * W + c] = e;
+      nrm = fmaf(e, e, nrm);
+    }
+    nrm = warp_sum(nrm);
+    if (lane == 0) bias[r] = -nrm;
+  }
+}
+
+// f[u] = 2 (x_u - mu), [U][2H]; cov already ELU+1 (the encoder's output)
+__global__ void __launch_bounds__(NT) wcat_user_kernel(const float* __restrict__ m, const float* __restrict__ cv, const float* __restrict__ mu,
+                                                       int U, int H, float* __restrict__ f) {
+  const int W = 2 * H;
+  const long long total = (long long)U * W;
+  for (long long i = (long long)blockIdx.x * NT + threadIdx.x; i < total; i += (long long)gridDim.x * NT) {
+    const long long u = i / W;
+    const int c = (int)(i - u * W);
+    const float x = c < H ? m[u * H + c] : wsqrt(cv[u * H + c - H]);
+    f[i] = 2.f * (x - mu[c]);
+  }
+}
+
 }  // namespace adt

@@ -195,6 +195,9 @@ class GraphedStep:
             d.copy_(_to_i32(a, dev), non_blocking=True)
         self.graph.replay()
         self.steps += 1
+        # the replayed Adam kernel wrote the parameters through raw pointers, which moves no tensor version: announce it like
+        # FlatOptimizer.step does, so derived data (scorer bf16 copies, STOSA's ranked catalog) is rebuilt before its next use
+        self.model._adt_param_version = getattr(self.model, "_adt_param_version", 0) + 1
         return self.loss
 
 

@@ -24,12 +24,15 @@ class Catalog(NamedTuple):
     bias: Optional[torch.Tensor]        # [n_rows] fp32 per-item term added to every score, or None
     first_id: int                       # global item id of table row 0
     hidden: int                         # feature width the encoder produces
+    version: object = None              # identity of what a derived table was built from (STOSA rebuilds its rows in place, so the
+                                        # table's own `_version` does not move); None for a view of a parameter
 
 
 def catalog_of(model):
     """The one place that decides which rows of a model are ranked.  Models whose score is not a plain dot product with the whole
-    item table (Bert4Rec: tied head rows 1..itemnum + mask_bias) define `scoring_catalog()`; every other model ranks all rows of
-    `item_emb.weight` from id 0, without a bias."""
+    item table (Bert4Rec: tied head rows 1..itemnum + mask_bias; STOSA: centred rows derived from both item tables + a bias, rebuilt
+    by this call when stale) define `scoring_catalog()`; every other model ranks all rows of `item_emb.weight` from id 0, without a
+    bias."""
     f = getattr(model, "scoring_catalog", None)
     if f is not None:
         return f()
@@ -106,7 +109,7 @@ class CatalogScorer:
         c = self.catalog()
         E, b = c.table, c.bias
         return (E.data_ptr(), E._version, tuple(E.shape), getattr(self.model, "_adt_param_version", 0),
-                None if b is None else (b.data_ptr(), b._version))
+                None if b is None else (b.data_ptr(), b._version), c.version)
 
     def refresh_table(self):
         """(re)build the bf16 copy of the catalog shard and the bound scalars (max |e|^2, max |bias|) from the CURRENT table and bias
@@ -134,6 +137,14 @@ class CatalogScorer:
         Not callable during graph capture -- GraphedScorer calls it before every replay."""
         if self._tab is None or self._tab_key != self._table_key():
             self.refresh_table()
+
+    def ensure_current(self):
+        """bring everything the kernels read up to date with the model: the catalog itself where the model derives it (catalog_of
+        rebuilds STOSA's rows) and, on the tensor-core path, its bf16 copy.  Not callable during graph capture -- GraphedScorer calls
+        it before every replay."""
+        c = self.catalog()
+        if self._uses_tc(c.hidden, *self.bounds()):
+            self.ensure_table()
 
     def _uses_tc(self, H, lo, hi):
         return self.use_tc and H % 64 == 0 and H <= 256 and (hi - lo) >= self.tc_min_items
@@ -320,8 +331,7 @@ class GraphedScorer:
         seq, ip, ix = src(log_seqs), src(seen_indptr), src(seen_idx)
         if tuple(seq.shape) != (self.U, self.L) or ip.numel() != self.U + 1 or ix.numel() > self.ix.numel():
             raise ValueError(f"GraphedScorer was built for [{self.U},{self.L}] batches with at most {self.ix.numel()} seen ids")
-        if self.tc:
-            self.sc.ensure_table()
+        self.sc.ensure_current()
         self.seq.copy_(seq, non_blocking=True)
         self.ip.copy_(ip, non_blocking=True)
         self.ix[:ix.numel()].copy_(ix, non_blocking=True)

@@ -11,7 +11,8 @@ padding*causal mask, softmax, dropout, P.v_mean and P^2.v_cov) is one kernel per
 Wasserstein distances in one kernel with the four table-row gradients scatter-added through the sorted segmented
 scatter, reconstruction and independence terms through the squared-difference / softmax-CE kernels.
 `full_sort_topk` replaces `dist_predict_full` + the host-side argpartition over the whole [U, I] matrix
-(trainer.py:464-479, :604-614) by the fused scoring + top-K kernel on augmented rows.
+(trainer.py:464-479, :604-614) by the shared full-catalog path (adt_b200.evaluate.CatalogScorer): the Wasserstein distance is
+ranked as a centred dot product plus a per-item bias (`scoring_catalog`, `final_feats`).
 """
 import ctypes
 import math
@@ -25,6 +26,7 @@ from .ops import DrlFn, linear, no_drop, _st
 from .bert4rec import MaskedCE, _ids
 
 ELU, ELU1 = 3, 4   # activation codes of adt_linear_fwd / adt_act_fwd
+MAX_CATALOG_HIDDEN = 128   # full-catalog ranking: rows [mean | sqrt cov] of 2H floats, at most 256 for the K7 kernels
 
 
 class _LN(nn.Module):
@@ -95,24 +97,25 @@ class ActFn(torch.autograd.Function):
         return dx, None
 
 
+def _embed_rows(ids, pos_ids, E, P):
+    """E[ids] + P[pos_ids] -> [B*L, H]"""
+    B, Lq = ids.shape
+    H = E.shape[1]
+    s = torch.empty(B * Lq, H, dtype=torch.float32, device=E.device)
+    L.check(L.lib().adt_gather3(L.ptr(ids), L.ptr(E), L.ptr(pos_ids), L.ptr(P), None, None, L.ptr(s), ctypes.c_int32(B * Lq),
+                                ctypes.c_int32(H), _st(E.device)), "adt_gather3")
+    return s
+
+
 class EmbedPairFn(torch.autograd.Function):
     """(E[ids] + P[0..L-1], E[dec_ids] + P[0..L-1]) for one (item, position) table pair; item table has padding_idx=0
     (models.py:169-172), the position table does not."""
 
     @staticmethod
     def forward(ctx, ids, dec_ids, pos_ids, E, P):
-        B, Lq = ids.shape
-        H = E.shape[1]
-        lib = L.lib()
-        outs = []
-        for i in (ids, dec_ids):
-            s = torch.empty(B * Lq, H, dtype=torch.float32, device=E.device)
-            L.check(lib.adt_gather3(L.ptr(i), L.ptr(E), L.ptr(pos_ids), L.ptr(P), None, None, L.ptr(s), ctypes.c_int32(B * Lq),
-                                    ctypes.c_int32(H), _st(E.device)), "adt_gather3")
-            outs.append(s)
         ctx.ids = (ids, dec_ids, pos_ids)
         ctx.shapes = (E.shape, P.shape)
-        return outs[0], outs[1]
+        return _embed_rows(ids, pos_ids, E, P), _embed_rows(dec_ids, pos_ids, E, P)
 
     @staticmethod
     def backward(ctx, d_enc, d_dec):
@@ -239,6 +242,8 @@ class DisenDistSAModel(nn.Module):
         self.pvn_weight = float(getattr(args, "pvn_weight", 0.005))
         self.drop_seed, self.drop_step, self.precision = 0, 0, 0
         self.step_dev = None      # optional device-side dropout step counter (adt_b200.dp.GraphedStep)
+        self._wcat, self._wcat_key = None, None   # ranked catalog (mu, rows, bias, scratch) and the _catalog_key it was built from
+        self._scorers = {}        # (K, device) -> CatalogScorer of full_sort_topk (keeps its bf16 table and scratch between calls)
         self.apply(self.init_weights)
         L.lib()
 
@@ -295,15 +300,10 @@ class DisenDistSAModel(nn.Module):
         h = linear(h, m.dense_2.weight, m.dense_2.bias, 0, 1.0, self.precision)
         return DrlFn.apply(h, x, m.LayerNorm.weight, m.LayerNorm.bias, 0, 1e-12, self._drop(dc, "row", self.dropout_p, Lq))
 
-    def _body(self, input_ids, dec_ids):
-        self._check()
-        dev = self.LayerNorm.weight.device
-        ids, dec = _ids(input_ids, dev), _ids(dec_ids, dev)
+    def _encode(self, ids, m, c, dc):
+        """the encoder stack (models.py:236-241) on the embedded (mean, cov) streams -> (mean, cov, encoder inputs, independence logits)."""
         B, Lq = ids.shape
         nh, H = self.num_heads, self.hidden_units
-        pos_ids = torch.arange(Lq, dtype=torch.int32, device=dev).repeat(B, 1)
-        dc = DropCfg(self.dropout_p, self.drop_seed, self.drop_step, self.training, step_dev=self.step_dev)
-        (m, c), (dm, dcv) = self._embed(ids, dec, pos_ids, dc, Lq)
         enc_inputs, rec_logits = [], []
         for layer in self.item_encoder.layer:
             enc_inputs.append((m, c))
@@ -313,6 +313,17 @@ class DisenDistSAModel(nn.Module):
             mi, ci = layer.mean_independence_layer, layer.cov_independence_layer
             rec_logits.append((linear(rm.view(B * Lq * nh, H // nh), mi.weight, mi.bias, 0, 1.0, 0),
                                linear(rc.view(B * Lq * nh, H // nh), ci.weight, ci.bias, 0, 1.0, 0)))
+        return m, c, enc_inputs, rec_logits
+
+    def _body(self, input_ids, dec_ids):
+        self._check()
+        dev = self.LayerNorm.weight.device
+        ids, dec = _ids(input_ids, dev), _ids(dec_ids, dev)
+        B, Lq = ids.shape
+        pos_ids = torch.arange(Lq, dtype=torch.int32, device=dev).repeat(B, 1)
+        dc = DropCfg(self.dropout_p, self.drop_seed, self.drop_step, self.training, step_dev=self.step_dev)
+        (m, c), (dm, dcv) = self._embed(ids, dec, pos_ids, dc, Lq)
+        m, c, enc_inputs, rec_logits = self._encode(ids, m, c, dc)
         dec_outs = []
         for layer in self.item_decoder.layer:
             # the reference evaluates dec_attention and discards it (modules.py:537-538): only its three dropout sites are consumed
@@ -360,13 +371,20 @@ class DisenDistSAModel(nn.Module):
     # ---- evaluation ---------------------------------------------------------------------------
     @torch.no_grad()
     def _last_states(self, input_ids):
-        was = self.training
-        self.eval()
-        try:
-            m, c, _, _, _, (B, Lq) = self._body(input_ids, input_ids)
-        finally:
-            self.train(was)
-        H = self.hidden_units
+        """(mean, cov) [U, H] of the last position in evaluation mode: embedding + encoder only (the decoder does not feed the
+        ranking)."""
+        self._check()
+        dev = self.LayerNorm.weight.device
+        ids = _ids(input_ids, dev)
+        B, Lq = ids.shape
+        H, ln = self.hidden_units, self.LayerNorm
+        pos_ids = torch.arange(Lq, dtype=torch.int32, device=dev).repeat(B, 1)
+        mc = []
+        for E, P, act in ((self.item_mean_embeddings, self.position_mean_embeddings, ELU),
+                          (self.item_cov_embeddings, self.position_cov_embeddings, ELU1)):
+            s = _embed_rows(ids, pos_ids, E.weight, P.weight)
+            mc.append(ActFn.apply(DrlFn.apply(s, None, ln.weight, ln.bias, 1, 1e-12, no_drop()), act))
+        m, c, _, _ = self._encode(ids, mc[0], mc[1], DropCfg(0.0, 0, 0, False))
         return m.view(B, Lq, H)[:, -1, :].contiguous(), c.view(B, Lq, H)[:, -1, :].contiguous()
 
     def _rows(self, mean, cov, is_user):
@@ -385,18 +403,71 @@ class DisenDistSAModel(nn.Module):
         const = (seq_mean_out ** 2).sum(-1, keepdim=True) + seq_cov_out.sum(-1, keepdim=True)
         return const - neg
 
+    def _catalog_key(self):
+        """what the ranked catalog is derived from, read on the host (launches nothing): storage and in-place version of both item
+        tables, and this package's optimisers' raw-pointer writes (_adt_param_version)."""
+        Em, Ec = self.item_mean_embeddings.weight, self.item_cov_embeddings.weight
+        return (Em.data_ptr(), Em._version, Ec.data_ptr(), Ec._version, getattr(self, "_adt_param_version", 0))
+
+    def _build_catalog(self):
+        """(re)build mu, the centred rows and their bias from the current item tables, in place when the shapes are unchanged so that a
+        captured evaluation graph keeps reading the same buffers."""
+        key = self._catalog_key()
+        Em, Ec = self.item_mean_embeddings.weight.detach(), self.item_cov_embeddings.weight.detach()
+        n, H = Em.shape
+        if H > MAX_CATALOG_HIDDEN or H % 2:
+            raise L.AdtError(f"STOSA full-catalog ranking needs an even hidden size <= {MAX_CATALOG_HIDDEN} (rows of 2H <= 256 floats); "
+                             f"got hidden_units = {H}")
+        self._check()
+        dev = Em.device
+        if self._wcat is None or self._wcat[1].shape != (n, 2 * H) or self._wcat[1].device != dev:
+            nb = ctypes.c_int64(0)
+            L.check(L.lib().adt_wcatalog_work_bytes(ctypes.c_int32(H), ctypes.byref(nb)), "adt_wcatalog_work_bytes")
+            self._wcat = (torch.empty(2 * H, device=dev), torch.empty(n, 2 * H, device=dev), torch.empty(n, device=dev),
+                          torch.zeros(nb.value, dtype=torch.uint8, device=dev))
+        mu, e, b, work = self._wcat
+        L.check(L.lib().adt_wcatalog_build(L.ptr(Em), L.ptr(Ec), ctypes.c_int32(n), ctypes.c_int32(H), L.ptr(mu), L.ptr(e), L.ptr(b),
+                                           L.ptr(work), _st(dev)), "adt_wcatalog_build")
+        self._wcat_key = key
+
+    def scoring_catalog(self):
+        """what full-catalog ranking scores (adt_b200.evaluate.catalog_of): -distance(u, i) + const(u) = <final_feats[u], e_i> + b_i with
+        e_i = y_i - mu, b_i = -|e_i|^2 over all item_size rows from id 0 (y_i = [mean_i | sqrt(elu(cov_i)+1)], mu their column mean).
+        The model-owned rows are rebuilt here, in place, whenever an item table changed since the last build (never during stream
+        capture: a captured graph reads the buffers as they stand).  `version` tells CatalogScorer when its bf16 copy is stale."""
+        from .evaluate import Catalog
+        if self._wcat_key != self._catalog_key():
+            if not (self.item_mean_embeddings.weight.is_cuda and torch.cuda.is_current_stream_capturing()):
+                self._build_catalog()
+            elif self._wcat is None:
+                raise L.AdtError("the STOSA catalog is built outside stream capture: rank once (or call scoring_catalog()) before capturing")
+        _, e, b, _ = self._wcat
+        return Catalog(e, b, 0, e.shape[1], self._wcat_key)
+
     @torch.no_grad()
-    def full_sort_topk(self, input_ids, seen_indptr=None, seen_idx=None, K=40):
-        """trainer.py:596-614 -> ids [U, K] of the K nearest unseen items, nearest first (ties by ascending id)."""
+    def final_feats(self, seqs):
+        """[U, 2H] rows the catalog is scored against: 2 ([mean_u | sqrt(cov_u)] - mu) of the last position, encoder in evaluation
+        mode.  No host synchronisation, so a CUDA graph can capture it (GraphedScorer)."""
+        return self.user_feats(*self._last_states(seqs))
+
+    @torch.no_grad()
+    def user_feats(self, mean, cov):
+        """last-position (mean, cov) [U, H] (cov already ELU+1) -> the [U, 2H] rows 2 ([mean | sqrt(cov)] - mu)."""
+        self.scoring_catalog()
+        mu = self._wcat[0]
+        mean, cov = mean.contiguous(), cov.contiguous()
+        U, H = mean.shape
+        f = torch.empty(U, 2 * H, dtype=torch.float32, device=mean.device)
+        L.check(L.lib().adt_wcatalog_user(L.ptr(mean), L.ptr(cov), L.ptr(mu), L.ptr(f), ctypes.c_int32(U), ctypes.c_int32(H),
+                                          _st(mean.device)), "adt_wcatalog_user")
+        return f
+
+    @torch.no_grad()
+    def full_sort_topk(self, input_ids, seen_indptr=None, seen_idx=None, K=40, answers=None, metric_acc=None):
+        """trainer.py:596-614 -> ids [U, K] of the K nearest unseen items, nearest first (ties by ascending id).  Seen ids: CSR, ascending
+        per user.  answers [U] + metric_acc (float64 device tensor [6]): fused HIT/NDCG@5,10 + MRR sums, as in CatalogScorer.topk."""
         from .evaluate import CatalogScorer
-        um, uc = self._last_states(input_ids)
-        u = self._rows(um, uc, 1)
-        cat = self._rows(self.item_mean_embeddings.weight, self.item_cov_embeddings.weight, 0)
-        holder = type("_Catalog", (), {})()
-        holder.item_emb = type("_W", (), {"weight": cat})()
-        scorer = CatalogScorer(holder, K=K, use_tensor_cores=False)
-        dev = u.device
-        ip = _ids(seen_indptr, dev) if seen_indptr is not None else None
-        ix = _ids(seen_idx, dev) if seen_idx is not None else None
-        _, ids = scorer.topk_from_feats(u, ip, ix)
-        return ids
+        key = (int(K), self.item_mean_embeddings.weight.device)
+        if key not in self._scorers:
+            self._scorers[key] = CatalogScorer(self, K=K)
+        return self._scorers[key].topk(input_ids, seen_indptr, seen_idx, answers, metric_acc)[1]

@@ -444,6 +444,18 @@ int adt_sqdiff_bwd(const float* a, const float* b, const float* g, float scale, 
  *   is_user = 1: [ 2 mean_u | 2 sqrt(cov_u) | 1 | 0 0 0 ]                                        (user rows, cov already ELU+1)
  * so that <user row, catalog row> = -distance(u, i) + const(u): the largest dot product is the smallest distance. */
 int adt_wcatalog_rows(const float* mean, const float* cov, float* out, int32_t n, int32_t H, int32_t is_user, adt_stream_t stream);
+/* the same ranking as a centred, biased dot product for adt_score_topk / adt_score_topk_tc with item_bias.  With item rows
+ * y_i = [ mean_i | sqrt(elu(cov_i)+1) ], user rows x_u = [ mean_u | sqrt(cov_u) ] and any mu,
+ *   -distance(u, i) = -|x_u - y_i|^2 = <2 (x_u - mu), y_i - mu> - |y_i - mu|^2 - |x_u - mu|^2,   the last term constant per user.
+ * mu = the column mean of the y_i removes the component all items share, which keeps the bf16 bound of adt_score_topk_tc tight.
+ * adt_wcatalog_build: mu [2H] (fixed-order fp64 column sums: an unchanged table gives bit-identical output), rows [n][2H] = y_i - mu,
+ *   bias [n] = -|rows[i]|^2, all fp32, H <= 128.  Two launches.  work: adt_wcatalog_work_bytes(H) bytes of scratch (column partials and
+ *   an arrival counter), zero-filled before its first use; every call leaves it zero-filled where the counter is.
+ * adt_wcatalog_user: out [U][2H] = 2 (x_u - mu) from the encoder's (mean, cov) [U][H] (cov already ELU+1); no host synchronisation. */
+int adt_wcatalog_work_bytes(int32_t H, int64_t* bytes);
+int adt_wcatalog_build(const float* mean, const float* cov, int32_t n, int32_t H, float* mu, float* rows, float* bias, void* work,
+                       adt_stream_t stream);
+int adt_wcatalog_user(const float* mean, const float* cov, const float* mu, float* out, int32_t U, int32_t H, adt_stream_t stream);
 
 /* ---- device-side batch assembly and sampling (SURVEY 8f-1) ---------------------------------------------------------------------
  * User histories live in HBM as CSR (hist_indptr [n_users+2] indexed by user id, hist_items in interaction order, hist_sorted the same
