@@ -220,7 +220,7 @@ __global__ void __launch_bounds__(NT) wattn_bwd_kernel(WAttnArgs p) {
   float* sq = mq + WQT * ldk;
   float* nq = sq + WQT * ldk;
   float* P = nq + WQT;
-  float* amk = P + WQT * lp;       // accumulators: sum_i G_ij mq_i, sum_i G_ij sq_i, sum_i P~ dmctx, sum_i P~^2 dcctx
+  float* amk = P + WQT * lp;       // accumulators: sum_i G_ij (mq_i - mk_j), sum_i G_ij (sq_i - sk_j), sum_i P~ dmctx, sum_i P~^2 dcctx
   float* ask = amk + p.L * ldk;
   float* amv = ask + p.L * ldk;
   float* acv = amv + p.L * ldk;
@@ -271,34 +271,39 @@ __global__ void __launch_bounds__(NT) wattn_bwd_kernel(WAttnArgs p) {
         }
       }
       __syncthreads();
-      // query-side gradients (score = (2 mq.mk + 2 sq.sk - nq - nk)/sqrt(hd); the -nq term cancels along the softmax axis)
+      // query-side gradients: d score_ij / d mq_i = 2 (mk_j - mq_i) / sqrt(hd), d score_ij / d cq_i = (sk_j - sq_i) / (sq_i sqrt(hd)).
+      // The differences are formed before the sum over j: every stream shares an offset (~1 for sqrt-cov at initialisation) that the
+      // expanded form sum_j G_ij k_j - (sum_j G_ij) q_i would cancel only after fp32 rounding, at ~100x the gradient's own size.
       for (int t = threadIdx.x; t < rows * hd4; t += NT) {
         const int i = t / hd4, c = (t - i * hd4) * 4;
+        const float4 q = ld4(mq + i * ldk + c), s = ld4(sq + i * ldk + c);
         float4 am = make_float4(0.f, 0.f, 0.f, 0.f), as = am;
         float rs = 0.f;
         for (int j = 0; j < p.L; ++j) {
           const float g = G[i * lp + j];
-          const float4 k = ld4(mk + j * ldk + c), s = ld4(sk + j * ldk + c);
-          am.x += g * k.x; am.y += g * k.y; am.z += g * k.z; am.w += g * k.w;
-          as.x += g * s.x; as.y += g * s.y; as.z += g * s.z; as.w += g * s.w;
+          const float4 k = ld4(mk + j * ldk + c), sj = ld4(sk + j * ldk + c);
+          am.x += g * (k.x - q.x); am.y += g * (k.y - q.y); am.z += g * (k.z - q.z); am.w += g * (k.w - q.w);
+          as.x += g * (sj.x - s.x); as.y += g * (sj.y - s.y); as.z += g * (sj.z - s.z); as.w += g * (sj.w - s.w);
           rs += g;
         }
         const long long go = ((long long)b * p.L + q0 + i) * p.H + h * hd + c;
-        const float4 q = ld4(mq + i * ldk + c), s = ld4(sq + i * ldk + c), cq = ld4(p.cq + go);
-        st4(p.dmq + go, make_float4(2.f * (am.x - rs * q.x), 2.f * (am.y - rs * q.y), 2.f * (am.z - rs * q.z), 2.f * (am.w - rs * q.w)));
-        st4(p.dcq + go, make_float4((cq.x > W_CLAMP ? as.x / s.x : 0.f) - rs, (cq.y > W_CLAMP ? as.y / s.y : 0.f) - rs,
-                                    (cq.z > W_CLAMP ? as.z / s.z : 0.f) - rs, (cq.w > W_CLAMP ? as.w / s.w : 0.f) - rs));
+        const float4 cq = ld4(p.cq + go);
+        st4(p.dmq + go, make_float4(2.f * am.x, 2.f * am.y, 2.f * am.z, 2.f * am.w));
+        st4(p.dcq + go, make_float4(cq.x > W_CLAMP ? as.x / s.x : -rs, cq.y > W_CLAMP ? as.y / s.y : -rs, cq.z > W_CLAMP ? as.z / s.z : -rs,
+                                    cq.w > W_CLAMP ? as.w / s.w : -rs));
       }
       // key-side accumulators (each (j, c) owned by one thread across tiles)
       for (int t = threadIdx.x; t < p.L * hd4; t += NT) {
         const int j = t / hd4, c = (t - j * hd4) * 4;
+        // a1 = sum_i G_ij (mq_i - mk_j), a2 = sum_i G_ij (sq_i - sk_j): differences before the sum, as on the query side
+        const float4 k = ld4(mk + j * ldk + c), sk4 = ld4(sk + j * ldk + c);
         float4 a1 = ld4(amk + j * ldk + c), a2 = ld4(ask + j * ldk + c), a3 = ld4(amv + j * ldk + c), a4 = ld4(acv + j * ldk + c);
         float s = 0.f;
         for (int i = 0; i < rows; ++i) {
           const float g = G[i * lp + j], pt = P[i * lp + j] * Mk[i * lp + j], pt2 = pt * pt;
           const float4 q = ld4(mq + i * ldk + c), sq4 = ld4(sq + i * ldk + c), x = ld4(dm + i * ldk + c), y = ld4(dc + i * ldk + c);
-          a1.x += g * q.x; a1.y += g * q.y; a1.z += g * q.z; a1.w += g * q.w;
-          a2.x += g * sq4.x; a2.y += g * sq4.y; a2.z += g * sq4.z; a2.w += g * sq4.w;
+          a1.x += g * (q.x - k.x); a1.y += g * (q.y - k.y); a1.z += g * (q.z - k.z); a1.w += g * (q.w - k.w);
+          a2.x += g * (sq4.x - sk4.x); a2.y += g * (sq4.y - sk4.y); a2.z += g * (sq4.z - sk4.z); a2.w += g * (sq4.w - sk4.w);
           a3.x += pt * x.x; a3.y += pt * x.y; a3.z += pt * x.z; a3.w += pt * x.w;
           a4.x += pt2 * y.x; a4.y += pt2 * y.y; a4.z += pt2 * y.z; a4.w += pt2 * y.w;
           s += g;
@@ -312,11 +317,10 @@ __global__ void __launch_bounds__(NT) wattn_bwd_kernel(WAttnArgs p) {
       const int j = t / hd4, c = (t - j * hd4) * 4;
       const long long go = ((long long)b * p.L + j) * p.H + h * hd + c;
       const float s = cs[j];
-      const float4 a1 = ld4(amk + j * ldk + c), a2 = ld4(ask + j * ldk + c), k = ld4(mk + j * ldk + c), sk4 = ld4(sk + j * ldk + c),
-                   ck = ld4(p.ck + go);
-      st4(p.dmk + go, make_float4(2.f * (a1.x - s * k.x), 2.f * (a1.y - s * k.y), 2.f * (a1.z - s * k.z), 2.f * (a1.w - s * k.w)));
-      st4(p.dck + go, make_float4((ck.x > W_CLAMP ? a2.x / sk4.x : 0.f) - s, (ck.y > W_CLAMP ? a2.y / sk4.y : 0.f) - s,
-                                  (ck.z > W_CLAMP ? a2.z / sk4.z : 0.f) - s, (ck.w > W_CLAMP ? a2.w / sk4.w : 0.f) - s));
+      const float4 a1 = ld4(amk + j * ldk + c), a2 = ld4(ask + j * ldk + c), sk4 = ld4(sk + j * ldk + c), ck = ld4(p.ck + go);
+      st4(p.dmk + go, make_float4(2.f * a1.x, 2.f * a1.y, 2.f * a1.z, 2.f * a1.w));
+      st4(p.dck + go, make_float4(ck.x > W_CLAMP ? a2.x / sk4.x : -s, ck.y > W_CLAMP ? a2.y / sk4.y : -s, ck.z > W_CLAMP ? a2.z / sk4.z : -s,
+                                  ck.w > W_CLAMP ? a2.w / sk4.w : -s));
       st4(p.dmv + go, ld4(amv + j * ldk + c));
       st4(p.dcv + go, ld4(acv + j * ldk + c));
     }
@@ -366,10 +370,10 @@ __global__ void __launch_bounds__(NT) wbpr_fwd_kernel(WBprArgs p) {
     if (ip <= 0) continue;
     float dp, dn, dpn;
     wbpr_dists(p, r, lane, ip, in, dp, dn, dpn);
-    const float x = dn - dp + 1e-24f;
+    const float d = dn - dp, x = d + 1e-24f;
     s0 += (double)(x > 0.f ? log1pf(expf(-x)) : -x + log1pf(expf(x)));
     s1 += (double)fmaxf(dp - dpn, 0.f);
-    s2 += (double)(((x > 0.f) - (x < 0.f) + 1) * 0.5f);
+    s2 += (double)(((d > 0.f) - (d < 0.f) + 1) * 0.5f);   // the AUC term takes sign(dn - dp) without the 1e-24: a tie counts 1/2
     s3 += 1.0;
   }
   if (lane == 0 && s3 > 0) {

@@ -7,7 +7,8 @@ oracle/make_golden_stosa.py) through tests/golden/stosa_*.npz.
 Reference map (file:line under /root/reference/stosa):
   wdist() / wdist_matmul()  modules.py:22-28 / 30-43
   embed_mean()/embed_cov()  models.py:183-210      (LN(eps=1e-12) -> dropout -> ELU ; cov: ELU(dropout(LN)) + 1)
-  attention()               modules.py:222-275 (self) and :312-361 (encoder-decoder)
+  attention()               modules.py:222-275 (self) and :312-361 (encoder-decoder); its core (scores .. P^2 cv) is attention_core()
+  init_state()              models.py:262-270 (a fresh state dict at any shape)
   intermediate()            modules.py:474-494     (dense 4H, ELU, dense, dropout, LN(+input))
   enc_layer()/dec_layer()   modules.py:509-525 / 527-541 (the decoder's self attention output is DISCARDED, :537-538)
   finetune()                models.py:212-260
@@ -34,6 +35,56 @@ class SCfg:
         self.dropout, self.attention_dropout, self.pvn_weight = dropout, attention_dropout, pvn_weight
 
 
+def init_state(cfg, seed, std=0.02, dtype=torch.float32):
+    """a freshly initialised DisenDistSAModel state dict (names, order and shapes of the reference's state_dict; models.py:262-270:
+    Linear and Embedding weights ~ N(0.01, std) including the padding row, Linear biases 0, LayerNorm 1 / 0), drawn from `seed`."""
+    H, nh = cfg.hidden, cfg.heads
+    g = torch.Generator().manual_seed(int(seed))
+    sd = {}
+
+    def normal(name, *shape):
+        sd[name] = torch.empty(*shape, dtype=torch.float32).normal_(mean=0.01, std=std, generator=g).to(dtype)
+
+    def linear(pre, n_out, n_in):
+        normal(pre + ".weight", n_out, n_in)
+        sd[pre + ".bias"] = torch.zeros(n_out, dtype=dtype)
+
+    def layer_norm(pre):
+        sd[pre + ".weight"], sd[pre + ".bias"] = torch.ones(H, dtype=dtype), torch.zeros(H, dtype=dtype)
+
+    def dist_attention(pre):
+        for n in ("mean_query", "cov_query", "mean_key", "cov_key", "mean_value", "cov_value", "mean_dense", "cov_dense"):
+            linear(f"{pre}.{n}", H, H)
+        layer_norm(pre + ".LayerNorm")
+
+    def intermediate(pre):
+        linear(pre + ".dense_1", 4 * H, H)
+        linear(pre + ".dense_2", H, 4 * H)
+        layer_norm(pre + ".LayerNorm")
+
+    for which in ("mean", "cov"):
+        normal(f"item_{which}_embeddings.weight", cfg.item_size, H)
+    for which in ("mean", "cov"):
+        normal(f"position_{which}_embeddings.weight", cfg.maxlen, H)
+    normal("user_margins.weight", cfg.num_users, 1)
+    for l in range(cfg.layers):
+        pre = f"item_encoder.layer.{l}"
+        dist_attention(pre + ".attention")
+        intermediate(pre + ".mean_intermediate")
+        intermediate(pre + ".cov_intermediate")
+        linear(pre + ".mean_independence_layer", nh, H // nh)
+        linear(pre + ".cov_independence_layer", nh, H // nh)
+    for l in range(cfg.layers):
+        pre = f"item_decoder.layer.{l}"
+        dist_attention(pre + ".dec_attention")
+        dist_attention(pre + ".enc_attention")
+        intermediate(pre + ".mean_intermediate")
+        intermediate(pre + ".cov_intermediate")
+    layer_norm("LayerNorm")
+    layer_norm("decLayerNorm")
+    return sd
+
+
 def wdist(m1, c1, m2, c2):
     s1, s2 = torch.sqrt(torch.clamp(c1, min=1e-24)), torch.sqrt(torch.clamp(c2, min=1e-24))
     return ((m1 - m2) ** 2).sum(-1) + ((s1 - s2) ** 2).sum(-1)
@@ -56,6 +107,26 @@ def embed(sd, which, ids, cfg, drop, sites):
     return F.elu(e) if which == "mean" else F.elu(e) + 1
 
 
+def attention_scores(mq, cq, mk, ck, mask):
+    """modules.py:240-249: masked, scaled scores [B,nh,L,L] of the head-split streams [B,nh,L,hd].
+
+    The additive mask is applied with the reference's fp32 semantics in any working dtype: a masked entry becomes
+    float32(score) + float32(MASK).  In fp32 every |score| < 256 is absorbed into MASK (ulp 512), so a query row whose keys are all
+    masked (left padding) is uniform over its L keys; in plain fp64 the scores would survive and that row would not be uniform.
+    For fp32 inputs this is bit-identical to `score + mask`."""
+    s = -wdist_matmul(mq, cq, mk, ck) / math.sqrt(mq.shape[-1])
+    return torch.where(mask != 0, (s.float() + mask.float()).to(s.dtype), s)
+
+
+def attention_core(mq, cq, mk, ck, mv, cv, mask, drop_p, drop, sites):
+    """modules.py:240-254 on the projected head-split streams [B,nh,L,hd] (cov streams already ELU+1) -> (mean context, cov context),
+    each [B,L,nh,hd]: scores, mask, softmax, dropout, P mv, P^2 cv."""
+    p = _drop(torch.softmax(attention_scores(mq, cq, mk, ck, mask), dim=-1), drop, drop_p, sites)
+    mctx = (p @ mv).permute(0, 2, 1, 3).contiguous()
+    cctx = ((p ** 2) @ cv).permute(0, 2, 1, 3).contiguous()
+    return mctx, cctx
+
+
 def attention(sd, pre, qm, qc, km, kc, mask, cfg, drop, sites):
     """-> (mean', cov', mean context [B,L,nh,hd], cov context)."""
     B, L, H = qm.shape
@@ -64,10 +135,7 @@ def attention(sd, pre, qm, qc, km, kc, mask, cfg, drop, sites):
     sp = lambda x: x.view(B, L, nh, hd).permute(0, 2, 1, 3)
     mq, mk, mv = sp(lin("mean_query", qm)), sp(lin("mean_key", km)), sp(lin("mean_value", km))
     cq, ck, cv = sp(F.elu(lin("cov_query", qc)) + 1), sp(F.elu(lin("cov_key", kc)) + 1), sp(F.elu(lin("cov_value", kc)) + 1)
-    s = -wdist_matmul(mq, cq, mk, ck) / math.sqrt(hd) + mask
-    p = _drop(torch.softmax(s, dim=-1), drop, cfg.attention_dropout, sites)
-    mctx = (p @ mv).permute(0, 2, 1, 3).contiguous()
-    cctx = ((p ** 2) @ cv).permute(0, 2, 1, 3).contiguous()
+    mctx, cctx = attention_core(mq, cq, mk, ck, mv, cv, mask, cfg.attention_dropout, drop, sites)
     mh = ln(sd, pre + "LayerNorm.", _drop(lin("mean_dense", mctx.view(B, L, H)), drop, cfg.dropout, sites) + qm)
     ch = ln(sd, pre + "LayerNorm.", _drop(lin("cov_dense", cctx.view(B, L, H)), drop, cfg.dropout, sites) + qc)
     return mh, ch, mctx, cctx
