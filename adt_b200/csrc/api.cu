@@ -314,13 +314,13 @@ static int launch_attn_bwd(const float* q, const float* k, const float* v, const
   return check_launch("attn_bwd");
 }
 
-// pre_bwd: narrow models (H == 64) in the bf16 mode take the weights-resident 128-thread kernel (ADT_ROW_SMALL=0 disables)
+// pre_bwd: narrow models (H == 64) in the bf16 mode take the weights-resident 256-thread kernel (ADT_ROW_SMALL=0 disables)
 static int launch_pre_bwd(const PreBwdArgs& r, int mma, cudaStream_t s) {
   TIMED("pre_bwd", s);
   if (use_row_small(r.H, mma)) {
     const size_t sm = PreBwdSmall2Smem::TOTAL_BYTES;
     cudaFuncSetAttribute(pre_bwd_small2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-    pre_bwd_small2_kernel<<<(r.M + 63) / 64, AS_NT, sm, s>>>(r);
+    pre_bwd_small2_kernel<<<(r.M + 63) / 64, RS_BWD_NT, sm, s>>>(r);
     return check_launch("pre_bwd_small");
   }
   const int pad = mma ? 8 : 4;
@@ -928,7 +928,7 @@ extern "C" int adt_enc_block_bwd(const adt_enc_block_bwd_args* a, adt_stream_t s
     const size_t sm = PostBwdSmallSmem::TOTAL_BYTES;
     cudaFuncSetAttribute(post_bwd_small_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
     TIMED("enc_post_bwd", s);
-    post_bwd_small_kernel<false><<<(M + 63) / 64, AS_NT, sm, s>>>(p);
+    post_bwd_small_kernel<false><<<(M + 63) / 64, RS_BWD_NT, sm, s>>>(p);
   } else {
     TIMED("enc_post_bwd", s); LAUNCH_TM2(tm, mma, post_bwd_kernel, false, (M + tm - 1) / tm, smem, s, p);
   }
@@ -1034,7 +1034,7 @@ extern "C" int adt_dec_block_bwd(const adt_dec_block_bwd_args* a, adt_stream_t s
     const size_t sm = PostBwdSmallSmem::TOTAL_BYTES;
     cudaFuncSetAttribute(post_bwd_small_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
     TIMED("dec_post_bwd", s);
-    post_bwd_small_kernel<true><<<(M + 63) / 64, AS_NT, sm, s>>>(p);
+    post_bwd_small_kernel<true><<<(M + 63) / 64, RS_BWD_NT, sm, s>>>(p);
   } else {
     TIMED("dec_post_bwd", s); LAUNCH_TM2(tm, mma, post_bwd_kernel, true, (M + tm - 1) / tm, smem, s, p);
   }
@@ -1059,7 +1059,7 @@ extern "C" int adt_dec_block_bwd(const adt_dec_block_bwd_args* a, adt_stream_t s
     const size_t sm = MidBwdSmallSmem::TOTAL_BYTES;
     cudaFuncSetAttribute(mid_bwd_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
     TIMED("mid_bwd", s);
-    mid_bwd_small_kernel<<<(M + 63) / 64, AS_NT, sm, s>>>(m);
+    mid_bwd_small_kernel<<<(M + 63) / 64, RS_BWD_NT, sm, s>>>(m);
   } else {
   tm = pick_tm(3 * (size_t)(H + pad) + (size_t)(2 * H + pad), &smem, 128, M >= 148 * 64 ? 128 : 64);
   if (!tm) return fail(ADT_E_SHAPE, "%s", "mid_bwd: tile does not fit shared memory");

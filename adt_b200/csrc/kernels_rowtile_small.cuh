@@ -15,18 +15,28 @@ constexpr int RS_LD = RS_H + 8;          // halfword stride of every bf16 tile (
 constexpr int RS_TILE = 64 * RS_LD;      // halfwords per [64][72] tile
 constexpr int RS_LF = RS_H + 4;          // float stride of the fp32 input tile (consecutive rows land on different banks)
 
+// The backward kernels (pre_bwd, mid_bwd, post_bwd) run 256-thread CTAs in two roles.  Warps 0-3 (chain warps) run the dgrad chain
+// on their 16-row strips.  Warps 4-7 (wgrad warps) compute every weight gradient; warp 4+w takes the output rows chain warp w took in
+// the 128-thread version.  Nothing downstream reads a weight gradient, so the chain warps hand each operand tile over through a named
+// barrier (bar.arrive) and never wait for the MMAs and atomics of the weight gradients.  Two CTAs stay resident per SM.
+constexpr int RS_BWD_NT = 256;
+constexpr int RS_CHAIN_NT = 128;         // threads of the chain role
+__device__ __forceinline__ void rs_bar_arrive(int id) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "n"(RS_BWD_NT) : "memory"); }
+__device__ __forceinline__ void rs_bar_sync(int id, int n) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n) : "memory"); }
+
 // 64 rows x 64 columns of a row-major fp32 matrix (row stride ld; rows >= nrows read as zero), scaled, into any of: a row-major
 // bf16 tile, a transposed bf16 tile, an fp32 tile [64][64].  N tensors at once: every global load is issued before the first store.
-template <int N>
+// Threads T0 .. T0 + NT - 1 of the CTA take part.
+template <int N, int NT = AS_NT, int T0 = 0>
 __device__ __forceinline__ void rs_load(const float* const (&src)[N], const long long (&ld)[N], const int (&nrows)[N], const float (&scale)[N],
                                         __nv_bfloat16* const (&dst)[N], __nv_bfloat16* const (&dstT)[N], float* const (&dstF)[N]) {
-  constexpr int NIT = 64 * 16 / AS_NT;   // 8 float4 per thread per tensor
+  constexpr int NIT = 64 * 16 / NT;      // float4 per thread per tensor
   float4 v[N][NIT];
 #pragma unroll
   for (int n = 0; n < N; ++n) {
 #pragma unroll
     for (int it = 0; it < NIT; ++it) {
-      const int idx = threadIdx.x + it * AS_NT;
+      const int idx = threadIdx.x - T0 + it * NT;
       const int r = idx >> 4, c = (idx & 15) * 4;
       v[n][it] = r < nrows[n] ? __ldg(reinterpret_cast<const float4*>(src[n] + (long long)r * ld[n] + c)) : make_float4(0.f, 0.f, 0.f, 0.f);
     }
@@ -35,7 +45,7 @@ __device__ __forceinline__ void rs_load(const float* const (&src)[N], const long
   for (int n = 0; n < N; ++n) {
 #pragma unroll
     for (int it = 0; it < NIT; ++it) {
-      const int idx = threadIdx.x + it * AS_NT;
+      const int idx = threadIdx.x - T0 + it * NT;
       const int r = idx >> 4, c = (idx & 15) * 4;
       const float4 x = make_float4(v[n][it].x * scale[n], v[n][it].y * scale[n], v[n][it].z * scale[n], v[n][it].w * scale[n]);
       if (dstF[n]) *reinterpret_cast<float4*>(dstF[n] + r * RS_LF + c) = x;
@@ -119,10 +129,11 @@ __device__ __forceinline__ void rs_dgrad(float (&acc)[8][4], const __nv_bfloat16
   }
 }
 
-// weight gradient of one projection from ROW-MAJOR tiles: gW[j][c] += sum_r T[r][j] X[r][c], gb[j] += sum_r T[r][j]
+// weight gradient of one projection from ROW-MAJOR tiles: gW[j][c] += sum_r T[r][j] X[r][c], gb[j] += sum_r T[r][j]; warp w (0..3)
+// takes the output rows j = 16w..16w+15
 __device__ __forceinline__ void rs_wgrad_rm(const __nv_bfloat16* __restrict__ T, const __nv_bfloat16* __restrict__ X, float* __restrict__ gW,
-                                            float* __restrict__ gb) {
-  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
+                                            float* __restrict__ gb, int w) {
+  const int lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
   float acc[8][4], ones[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
   for (int nb = 0; nb < 8; ++nb) acc[nb][0] = acc[nb][1] = acc[nb][2] = acc[nb][3] = 0.f;
@@ -153,7 +164,12 @@ __device__ __forceinline__ void rs_wgrad_rm(const __nv_bfloat16* __restrict__ T,
     atomicAdd(gb + j1, ones[2]);
   }
 }
+__device__ __forceinline__ void rs_wgrad_rm(const __nv_bfloat16* __restrict__ T, const __nv_bfloat16* __restrict__ X, float* __restrict__ gW,
+                                            float* __restrict__ gb) {
+  rs_wgrad_rm(T, X, gW, gb, threadIdx.x >> 5);
+}
 
+template <int NT = AS_NT, int T0 = 0>
 __device__ __forceinline__ void rs_load1(const float* src, int rows, float scale, __nv_bfloat16* dst) {
   const float* const s[1] = {src};
   const long long ld[1] = {RS_H};
@@ -162,7 +178,7 @@ __device__ __forceinline__ void rs_load1(const float* src, int rows, float scale
   __nv_bfloat16* const d[1] = {dst};
   __nv_bfloat16* const dT[1] = {nullptr};
   float* const dF[1] = {nullptr};
-  rs_load<1>(s, ld, nr, sc, d, dT, dF);
+  rs_load<1, NT, T0>(s, ld, nr, sc, d, dT, dF);
 }
 
 // -------------------------------------------------------------------------------------------------
@@ -485,14 +501,18 @@ __global__ void __launch_bounds__(AS_NT) post_fwd_small_kernel(PostFwdArgs p) {
 
 // -------------------------------------------------------------------------------------------------
 // post_bwd_small_kernel == post_bwd_kernel (kernels_bwd.cuh), H == 64, bf16 mode.  Weights C2, C1, Wo and the attention context
-// stay in shared memory; the gradient stream dO -> dh2 -> da -> dh1 -> dz -> dy -> dctx lives in fragments and is only parked in a
-// bf16 tile where a weight-gradient product needs all rows of the CTA.
+// stay in shared memory; the gradient stream dO -> dh2 -> da -> dh1 -> dz -> dy -> dctx lives in fragments of the chain warps and is
+// only parked in a bf16 tile where a weight-gradient product needs all rows of the CTA.  Each of the three weight gradients has its
+// own operand tiles, so the chain warps never wait for the wgrad warps.
 // -------------------------------------------------------------------------------------------------
 struct PostBwdSmallSmem {
-  static constexpr int W = 0, C = 3 * RS_TILE, T = C + RS_TILE, X = T + RS_TILE;     // C2, C1, Wo | ctx | T | X
-  static constexpr size_t LG_BYTES = (size_t)(X + RS_TILE) * 2;                       // logits / dlogits [64][nh*nh] fp32 (+ nh)
+  // C2, C1, Wo | ctx | dh2, a (dC2) | dh1, z (dC1) | dy (dWo, with ctx)
+  static constexpr int W = 0, C = 3 * RS_TILE, T3 = C + RS_TILE, X3 = T3 + RS_TILE, T5 = X3 + RS_TILE, X5 = T5 + RS_TILE, T8 = X5 + RS_TILE;
+  static constexpr size_t LG_BYTES = (size_t)(T8 + RS_TILE) * 2;                      // logits / dlogits [64][nh*nh] fp32 (+ nh)
   static constexpr size_t TOTAL_BYTES = LG_BYTES + (size_t)(64 * 64 + 8) * 4;
 };
+// named barriers of post_bwd_small_kernel: operand tiles of dC1 / dWo complete, head logits complete, chain warps only
+constexpr int RS_BAR_S5 = 1, RS_BAR_S8 = 2, RS_BAR_HEAD = 3, RS_BAR_CHAIN = 4;
 
 // D[nb] += A * W with A given as fragments (rows of this warp, k = j = 0..63) and W[j][c] a row-major weight tile
 __device__ __forceinline__ void rs_dgrad_frag(float (&out)[8][4], const float (&a_in)[8][4], const __nv_bfloat16* __restrict__ W) {
@@ -597,14 +617,17 @@ __device__ __forceinline__ void frag_ln_bwd(float (&D)[8][4], const float (&Y)[8
 }
 
 template <bool IS_DEC>
-__global__ void __launch_bounds__(AS_NT) post_bwd_small_kernel(PostBwdArgs p) {
+__global__ void __launch_bounds__(RS_BWD_NT, 2) post_bwd_small_kernel(PostBwdArgs p) {
   using SM = PostBwdSmallSmem;
   extern __shared__ __align__(16) uint8_t rs_raw[];
   __nv_bfloat16* hb = reinterpret_cast<__nv_bfloat16*>(rs_raw);
   __nv_bfloat16* Wt = hb + SM::W;            // [0] C2, [1] C1, [2] Wo
   __nv_bfloat16* Cs = hb + SM::C;
-  __nv_bfloat16* T = hb + SM::T;
-  __nv_bfloat16* X = hb + SM::X;
+  __nv_bfloat16* T3 = hb + SM::T3;
+  __nv_bfloat16* X3 = hb + SM::X3;
+  __nv_bfloat16* T5 = hb + SM::T5;
+  __nv_bfloat16* X5 = hb + SM::X5;
+  __nv_bfloat16* T8 = hb + SM::T8;
   float* lgs = reinterpret_cast<float*>(rs_raw + SM::LG_BYTES);
   const int M = p.M;
   const int row0 = blockIdx.x * 64;
@@ -613,8 +636,9 @@ __global__ void __launch_bounds__(AS_NT) post_bwd_small_kernel(PostBwdArgs p) {
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
   const int i0 = 16 * w + g, i1 = i0 + 8;
   const bool v0 = i0 < rows, v1 = i1 < rows;
-  rs_load1(p.ctx + g0, rows, 1.f, Cs);
-  {
+  const bool head = !IS_DEC && (p.nll_coef != 0.f || p.drec);
+  if (w >= 4) {                              // the wgrad warps stage ctx and the weights while the chain warps start
+    rs_load1<RS_BWD_NT - RS_CHAIN_NT, RS_CHAIN_NT>(p.ctx + g0, rows, 1.f, Cs);
     const float* const src[3] = {p.C2, p.C1, p.Wo};
     const long long ld[3] = {RS_H, RS_H, RS_H};
     const int nr[3] = {64, 64, 64};
@@ -622,34 +646,34 @@ __global__ void __launch_bounds__(AS_NT) post_bwd_small_kernel(PostBwdArgs p) {
     __nv_bfloat16* const d[3] = {Wt, Wt + RS_TILE, Wt + 2 * RS_TILE};
     __nv_bfloat16* const dT[3] = {nullptr, nullptr, nullptr};
     float* const dF[3] = {nullptr, nullptr, nullptr};
-    rs_load<3>(src, ld, nr, sc, d, dT, dF);
+    rs_load<3, RS_BWD_NT - RS_CHAIN_NT, RS_CHAIN_NT>(src, ld, nr, sc, d, dT, dF);
   }
   // ---- 1./2. dO, a = relu(h1 m1), dh2 = dO m2 on fragments
-  float G[8][4], A[8][4];
-  frag_load(G, p.dout ? p.dout + g0 : nullptr, i0, i1, v0, v1, t);
-  if (IS_DEC && p.enc_in) {
-    float O[8][4], E[8][4];
-    frag_load(O, p.out + g0, i0, i1, v0, v1, t);
-    frag_load(E, p.enc_in + g0, i0, i1, v0, v1, t);
-#pragma unroll
-    for (int nb = 0; nb < 8; ++nb) {
-#pragma unroll
-      for (int e = 0; e < 4; ++e) { O[nb][e] = p.mse_coef * (O[nb][e] - E[nb][e]); G[nb][e] += O[nb][e]; O[nb][e] = -O[nb][e]; }
-    }
-    if (p.denc) frag_store(p.denc + g0, O, i0, i1, v0, v1, t);
-  }
-  {
-    const int k0 = v0 ? p.ids[row0 + i0] : 0, k1 = v1 ? p.ids[row0 + i1] : 0;
-#pragma unroll
-    for (int nb = 0; nb < 8; ++nb) {
-      if (k0 == 0) { G[nb][0] = 0.f; G[nb][1] = 0.f; }
-      if (k1 == 0) { G[nb][2] = 0.f; G[nb][3] = 0.f; }
-    }
-  }
-  frag_load(A, p.h1 + g0, i0, i1, v0, v1, t);
-  float mk[8][4];
+  float G[8][4], D2[8][4];
   uint32_t m1bits = 0u;                      // bit (4 nb + e): element kept by dropout 1 AND a > 0
-  {
+  if (w < 4) {
+    frag_load(G, p.dout ? p.dout + g0 : nullptr, i0, i1, v0, v1, t);
+    if (IS_DEC && p.enc_in) {
+      float O[8][4], E[8][4];
+      frag_load(O, p.out + g0, i0, i1, v0, v1, t);
+      frag_load(E, p.enc_in + g0, i0, i1, v0, v1, t);
+#pragma unroll
+      for (int nb = 0; nb < 8; ++nb) {
+#pragma unroll
+        for (int e = 0; e < 4; ++e) { O[nb][e] = p.mse_coef * (O[nb][e] - E[nb][e]); G[nb][e] += O[nb][e]; O[nb][e] = -O[nb][e]; }
+      }
+      if (p.denc) frag_store(p.denc + g0, O, i0, i1, v0, v1, t);
+    }
+    {
+      const int k0 = v0 ? p.ids[row0 + i0] : 0, k1 = v1 ? p.ids[row0 + i1] : 0;
+#pragma unroll
+      for (int nb = 0; nb < 8; ++nb) {
+        if (k0 == 0) { G[nb][0] = 0.f; G[nb][1] = 0.f; }
+        if (k1 == 0) { G[nb][2] = 0.f; G[nb][3] = 0.f; }
+      }
+    }
+    float A[8][4], mk[8][4];
+    frag_load(A, p.h1 + g0, i0, i1, v0, v1, t);
     if (p.drop1.enabled) frag_drop(mk, p.drop1, row0 + i0, row0 + i1, t);
 #pragma unroll
     for (int nb = 0; nb < 8; ++nb) {
@@ -661,19 +685,39 @@ __global__ void __launch_bounds__(AS_NT) post_bwd_small_kernel(PostBwdArgs p) {
         if (A[nb][e] > 0.f) m1bits |= 1u << (4 * nb + e);
       }
     }
-  }
-  float D2[8][4];
-  if (p.drop2.enabled) frag_drop(mk, p.drop2, row0 + i0, row0 + i1, t);
+    frag_store_tile(X3, A, i0, i1, t);
+    if (p.drop2.enabled) frag_drop(mk, p.drop2, row0 + i0, row0 + i1, t);
 #pragma unroll
-  for (int nb = 0; nb < 8; ++nb) {
+    for (int nb = 0; nb < 8; ++nb) {
 #pragma unroll
-    for (int e = 0; e < 4; ++e) D2[nb][e] = p.drop2.enabled ? G[nb][e] * mk[nb][e] : G[nb][e];
+      for (int e = 0; e < 4; ++e) D2[nb][e] = p.drop2.enabled ? G[nb][e] * mk[nb][e] : G[nb][e];
+    }
+    frag_store_tile(T3, D2, i0, i1, t);
   }
-  // ---- 3. dC2 += dh2^T a ; dc2 += colsum(dh2)
-  frag_store_tile(T, D2, i0, i1, t);
-  frag_store_tile(X, A, i0, i1, t);
-  __syncthreads();
-  rs_wgrad_rm(T, X, p.gC2, p.gc2);
+  __syncthreads();                           // weights, ctx and the operands of step 3 are in shared memory
+  if (w >= 4) {
+    // ---- wgrad warps: 3. dC2 += dh2^T a ; 5. dC1 += dh1^T z ; 8. dWo += dy^T ctx (and the bias column sums)
+    rs_wgrad_rm(T3, X3, p.gC2, p.gc2, w - 4);
+    rs_bar_sync(RS_BAR_S5, RS_BWD_NT);
+    rs_wgrad_rm(T5, X5, p.gC1, p.gc1, w - 4);
+    rs_bar_sync(RS_BAR_S8, RS_BWD_NT);
+    rs_wgrad_rm(T8, Cs, p.gWo, p.gbo, w - 4);
+    if (head) {
+      // ---- 9. independence-head weight gradient: dWsp[j][d] += sum_{r,c} dl[r][c][j] ctx[r][c*hd+d], dbsp from the CTA's sums
+      const int nh = p.nh, hd = RS_H / nh, n2 = nh * nh;
+      const float* dbs = lgs + 64 * n2;
+      rs_bar_sync(RS_BAR_HEAD, RS_BWD_NT);
+      for (int i = threadIdx.x - RS_CHAIN_NT; i < nh * hd; i += RS_BWD_NT - RS_CHAIN_NT) {
+        const int j = i / hd, dd = i - j * hd;
+        float accw = 0.f;
+        for (int r = 0; r < rows; ++r)
+          for (int c = 0; c < nh; ++c) accw = fmaf(lgs[r * n2 + c * nh + j], __bfloat162float(Cs[r * RS_LD + c * hd + dd]), accw);
+        atomicAdd(p.gWsp + i, accw);
+      }
+      for (int i = threadIdx.x - RS_CHAIN_NT; i < nh; i += RS_BWD_NT - RS_CHAIN_NT) atomicAdd(p.gbsp + i, dbs[i]);
+    }
+    return;
+  }
   // ---- 4. da = dh2 C2 ; dh1 = da [a>0] m1
   float H1[8][4];
 #pragma unroll
@@ -687,10 +731,11 @@ __global__ void __launch_bounds__(AS_NT) post_bwd_small_kernel(PostBwdArgs p) {
       for (int e = 0; e < 4; ++e) H1[nb][e] = (m1bits >> (4 * nb + e)) & 1u ? H1[nb][e] * sc1 : 0.f;
     }
   }
-  // ---- 5. z = LN2(y) (enc) / c (dec) ; dC1 += dh1^T z ; dc1 += colsum(dh1)
+  // ---- 5. z = LN2(y) (enc) / c (dec): operands of dC1 += dh1^T z ; dc1 += colsum(dh1).  Step 6 takes dh1 back from its tile
+  // (the same bf16 values its fragments would pack to), so dh1 is not held in registers next to y and z.
+  frag_store_tile(T5, H1, i0, i1, t);
   float Y[8][4];
   frag_load(Y, p.u + g0, i0, i1, v0, v1, t);
-  __syncthreads();                           // everybody is done with T / X of step 3
   {
     float Z[8][4];
 #pragma unroll
@@ -700,39 +745,36 @@ __global__ void __launch_bounds__(AS_NT) post_bwd_small_kernel(PostBwdArgs p) {
       if (!v0) { for (int nb = 0; nb < 8; ++nb) { Z[nb][0] = 0.f; Z[nb][1] = 0.f; } }
       if (!v1) { for (int nb = 0; nb < 8; ++nb) { Z[nb][2] = 0.f; Z[nb][3] = 0.f; } }
     }
-    frag_store_tile(X, Z, i0, i1, t);
+    frag_store_tile(X5, Z, i0, i1, t);
   }
-  frag_store_tile(T, H1, i0, i1, t);
-  __syncthreads();
-  rs_wgrad_rm(T, X, p.gC1, p.gc1);
+  __syncwarp();                              // step 6 reads this warp's rows of dh1 through ldmatrix
+  rs_bar_arrive(RS_BAR_S5);
   // ---- 6. dz (enc) / dc (dec) = dO + dh1 C1
   float DZ[8][4];
 #pragma unroll
   for (int nb = 0; nb < 8; ++nb) { DZ[nb][0] = G[nb][0]; DZ[nb][1] = G[nb][1]; DZ[nb][2] = G[nb][2]; DZ[nb][3] = G[nb][3]; }
-  rs_dgrad_frag(DZ, H1, Wt + RS_TILE);
+  rs_dgrad(DZ, T5, Wt + RS_TILE, 16 * w);
   if (!IS_DEC) {
     // ---- 7. dy = LN2^T(dz) ; dres = dy
-    frag_ln_bwd(DZ, Y, p.ln2_g, p.gln2_g, p.gln2_b, v0, v1, g, t);
+    frag_ln_bwd(DZ, Y, p.ln2_g, p.gln2_g, p.gln2_b, v0, v1, (threadIdx.x >> 2) & 7, t);   // g recomputed: held live it spills at 128 registers
     frag_store(p.dres + g0, DZ, i0, i1, v0, v1, t);
   } else {
     frag_store(p.dres + g0, G, i0, i1, v0, v1, t);     // dd = dO
   }
-  // ---- 8. dWo += dy^T ctx ; dbo += colsum(dy) ; dctx = dy Wo
-  __syncthreads();                           // everybody is done with T / X of step 5
-  frag_store_tile(T, DZ, i0, i1, t);
-  __syncthreads();
-  rs_wgrad_rm(T, Cs, p.gWo, p.gbo);
+  // ---- 8. operand of dWo += dy^T ctx ; dbo += colsum(dy) ; dctx = dy Wo
+  frag_store_tile(T8, DZ, i0, i1, t);
+  rs_bar_arrive(RS_BAR_S8);
   float DC[8][4];
 #pragma unroll
   for (int nb = 0; nb < 8; ++nb) DC[nb][0] = DC[nb][1] = DC[nb][2] = DC[nb][3] = 0.f;
   rs_dgrad_frag(DC, DZ, Wt + 2 * RS_TILE);
-  if (!IS_DEC && (p.nll_coef != 0.f || p.drec)) {
+  if (head) {
     // ---- 9. independence-head adjoint (per-head logits from the bf16 context tile)
     const int nh = p.nh, hd = RS_H / nh, n2 = nh * nh;
     float* dbs = lgs + 64 * n2;
-    for (int i = threadIdx.x; i < nh; i += AS_NT) dbs[i] = 0.f;
-    __syncthreads();
-    for (int i = threadIdx.x; i < 64 * nh; i += AS_NT) {
+    for (int i = threadIdx.x; i < nh; i += RS_CHAIN_NT) dbs[i] = 0.f;
+    rs_bar_sync(RS_BAR_CHAIN, RS_CHAIN_NT);
+    for (int i = threadIdx.x; i < 64 * nh; i += RS_CHAIN_NT) {
       const int r = i / nh, c = i - r * nh;
       float* lg = lgs + r * n2 + c * nh;
       if (r >= rows) {
@@ -759,7 +801,8 @@ __global__ void __launch_bounds__(AS_NT) post_bwd_small_kernel(PostBwdArgs p) {
         atomicAdd(dbs + j, dl);
       }
     }
-    __syncthreads();
+    rs_bar_arrive(RS_BAR_HEAD);
+    rs_bar_sync(RS_BAR_CHAIN, RS_CHAIN_NT);
     // dctx[r][c*hd+d] += sum_j dl[r][c][j] Wsp[j][d]   (on the fragments)
 #pragma unroll
     for (int nb = 0; nb < 8; ++nb) {
@@ -772,15 +815,6 @@ __global__ void __launch_bounds__(AS_NT) post_bwd_small_kernel(PostBwdArgs p) {
         DC[nb][e] += add;
       }
     }
-    // dWsp[j][d] += sum_{r,c} dl[r][c][j] ctx[r][c*hd+d]
-    for (int i = threadIdx.x; i < nh * hd; i += AS_NT) {
-      const int j = i / hd, dd = i - j * hd;
-      float accw = 0.f;
-      for (int r = 0; r < rows; ++r)
-        for (int c = 0; c < nh; ++c) accw = fmaf(lgs[r * n2 + c * nh + j], __bfloat162float(Cs[r * RS_LD + c * hd + dd]), accw);
-      atomicAdd(p.gWsp + i, accw);
-    }
-    for (int i = threadIdx.x; i < nh; i += AS_NT) atomicAdd(p.gbsp + i, dbs[i]);
   }
   frag_store(p.dctx + g0, DC, i0, i1, v0, v1, t);
 }
@@ -788,14 +822,15 @@ __global__ void __launch_bounds__(AS_NT) post_bwd_small_kernel(PostBwdArgs p) {
 // -------------------------------------------------------------------------------------------------
 // pre_bwd_small2_kernel == pre_bwd_kernel (kernels_bwd.cuh): adjoint of LayerNorm + packed QKV in-projection.  The block input lives in fragments (LayerNorm forward and
 // adjoint without shared memory), all three upstream gradients (dq, dk, dv) are staged as bf16 tiles in the prologue, so the
-// kernel has ONE barrier and no global load on its critical path after the prologue.
+// kernel has ONE barrier and no global load on its critical path after the prologue.  Every weight-gradient operand (Tq, Tk, Tv,
+// Nb, Xb) is complete at that barrier: the wgrad warps need no further handoff.
 // -------------------------------------------------------------------------------------------------
 struct PreBwdSmall2Smem {
   static constexpr int W = 0, TQ = 3 * RS_TILE, TK = TQ + RS_TILE, TV = TK + RS_TILE, X = TV + RS_TILE, N = X + RS_TILE;
   static constexpr size_t TOTAL_BYTES = (size_t)(N + RS_TILE) * 2;
 };
 
-__global__ void __launch_bounds__(AS_NT) pre_bwd_small2_kernel(PreBwdArgs p) {
+__global__ void __launch_bounds__(RS_BWD_NT, 2) pre_bwd_small2_kernel(PreBwdArgs p) {
   using SM = PreBwdSmall2Smem;
   extern __shared__ __align__(16) uint8_t rs_raw[];
   __nv_bfloat16* hb = reinterpret_cast<__nv_bfloat16*>(rs_raw);
@@ -819,7 +854,7 @@ __global__ void __launch_bounds__(AS_NT) pre_bwd_small2_kernel(PreBwdArgs p) {
     __nv_bfloat16* const d[3] = {Tq, Tk, Tv};
     __nv_bfloat16* const dT[3] = {nullptr, nullptr, nullptr};
     float* const dF[3] = {nullptr, nullptr, nullptr};
-    rs_load<3>(src, ld, nr, sc, d, dT, dF);
+    rs_load<3, RS_BWD_NT>(src, ld, nr, sc, d, dT, dF);
   }
   {
     const float* const src[3] = {p.Win, p.Win + RS_H * RS_H, p.Win + 2 * RS_H * RS_H};
@@ -829,11 +864,11 @@ __global__ void __launch_bounds__(AS_NT) pre_bwd_small2_kernel(PreBwdArgs p) {
     __nv_bfloat16* const d[3] = {Wt, Wt + RS_TILE, Wt + 2 * RS_TILE};
     __nv_bfloat16* const dT[3] = {nullptr, nullptr, nullptr};
     float* const dF[3] = {nullptr, nullptr, nullptr};
-    rs_load<3>(src, ld, nr, sc, d, dT, dF);
+    rs_load<3, RS_BWD_NT>(src, ld, nr, sc, d, dT, dF);
   }
   float Xf[8][4];
-  frag_load(Xf, p.x + g0, i0, i1, v0, v1, t);
-  {
+  if (w < 4) {
+    frag_load(Xf, p.x + g0, i0, i1, v0, v1, t);
     float Nf[8][4];
 #pragma unroll
     for (int nb = 0; nb < 8; ++nb) { Nf[nb][0] = Xf[nb][0]; Nf[nb][1] = Xf[nb][1]; Nf[nb][2] = Xf[nb][2]; Nf[nb][3] = Xf[nb][3]; }
@@ -847,11 +882,17 @@ __global__ void __launch_bounds__(AS_NT) pre_bwd_small2_kernel(PreBwdArgs p) {
     if (!p.kv_from_norm) frag_store_tile(Xb, Xf, i0, i1, t);
   }
   __syncthreads();
+  if (w >= 4) {   // ---- wgrad warps: dWq += dq^T LN(x) ; dWk += dk^T xkv ; dWv += dv^T xkv (and the bias column sums)
+    const __nv_bfloat16* Xkv = p.kv_from_norm ? Nb : Xb;
+    rs_wgrad_rm(Tq, Nb, p.gWin, p.gbin, w - 4);
+    rs_wgrad_rm(Tk, Xkv, p.gWin + (long long)RS_H * RS_H, p.gbin + RS_H, w - 4);
+    rs_wgrad_rm(Tv, Xkv, p.gWin + 2ll * RS_H * RS_H, p.gbin + 2 * RS_H, w - 4);
+    return;
+  }
   // ---- q projection
   float D[8][4];
 #pragma unroll
   for (int nb = 0; nb < 8; ++nb) D[nb][0] = D[nb][1] = D[nb][2] = D[nb][3] = 0.f;
-  rs_wgrad_rm(Tq, Nb, p.gWin, p.gbin);
   rs_dgrad(D, Tq, Wt, 16 * w);
   if (p.dnorm_extra) {
     float E[8][4];
@@ -861,10 +902,7 @@ __global__ void __launch_bounds__(AS_NT) pre_bwd_small2_kernel(PreBwdArgs p) {
   }
   if (!p.kv_from_norm) frag_ln_bwd(D, Xf, p.ln_g, p.gln_g, p.gln_b, v0, v1, g, t);     // encoder: k, v come from x itself
   // ---- k and v projections
-  const __nv_bfloat16* Xkv = p.kv_from_norm ? Nb : Xb;
-  rs_wgrad_rm(Tk, Xkv, p.gWin + (long long)RS_H * RS_H, p.gbin + RS_H);
   rs_dgrad(D, Tk, Wt + RS_TILE, 16 * w);
-  rs_wgrad_rm(Tv, Xkv, p.gWin + 2ll * RS_H * RS_H, p.gbin + 2 * RS_H);
   rs_dgrad(D, Tv, Wt + 2 * RS_TILE, 16 * w);
   if (p.kv_from_norm) frag_ln_bwd(D, Xf, p.ln_g, p.gln_g, p.gln_b, v0, v1, g, t);      // decoder: q, k, v all come from LN(x)
   if (p.dx_extra) {
@@ -981,27 +1019,33 @@ __global__ void __launch_bounds__(AS_NT) mid_fwd_small_kernel(const float* __res
 
 // -------------------------------------------------------------------------------------------------
 // mid_bwd_small_kernel == mid_bwd_kernel (kernels_bwd.cuh): adjoint of the decoder's self-attention out-projection and of the
-// cross-attention in-projection (q from the self-attention output a, k/v from the encoder features), H == 64, bf16 mode.
+// cross-attention in-projection (q from the self-attention output a, k/v from the encoder features), H == 64, bf16 mode.  Every
+// operand except da is staged in the prologue; da is the one tile the wgrad warps wait for.
 // -------------------------------------------------------------------------------------------------
 struct MidBwdSmallSmem {
   static constexpr int W = 0;                        // Wq2, Wk2, Wv2, Wo1 row-major
   static constexpr int T = 4 * RS_TILE;              // dq2 * s
-  static constexpr int X = T + RS_TILE;              // a -> feats -> ctx1
-  static constexpr int K = X + RS_TILE;              // dk2
+  static constexpr int A = T + RS_TILE;              // a
+  static constexpr int K = A + RS_TILE;              // dk2
   static constexpr int V = K + RS_TILE;              // dv2
-  static constexpr int DA = V + RS_TILE;             // grad wrt a
+  static constexpr int F = V + RS_TILE;              // feats
+  static constexpr int C = F + RS_TILE;              // ctx1
+  static constexpr int DA = C + RS_TILE;             // grad wrt a
   static constexpr size_t TOTAL_BYTES = (size_t)(DA + RS_TILE) * 2;
 };
+constexpr int RS_BAR_DA = 1;                         // mid_bwd_small_kernel: da tile complete
 
-__global__ void __launch_bounds__(AS_NT) mid_bwd_small_kernel(MidBwdArgs p) {
+__global__ void __launch_bounds__(RS_BWD_NT, 2) mid_bwd_small_kernel(MidBwdArgs p) {
   using SM = MidBwdSmallSmem;
   extern __shared__ __align__(16) uint8_t rs_raw[];
   __nv_bfloat16* hb = reinterpret_cast<__nv_bfloat16*>(rs_raw);
   __nv_bfloat16* Wt = hb + SM::W;
   __nv_bfloat16* T = hb + SM::T;
-  __nv_bfloat16* X = hb + SM::X;
+  __nv_bfloat16* As = hb + SM::A;
   __nv_bfloat16* Kt = hb + SM::K;
   __nv_bfloat16* Vt = hb + SM::V;
+  __nv_bfloat16* Fs = hb + SM::F;
+  __nv_bfloat16* Cs = hb + SM::C;
   __nv_bfloat16* DAs = hb + SM::DA;
   const int row0 = blockIdx.x * 64;
   const int rows = min(64, p.M - row0);
@@ -1009,14 +1053,14 @@ __global__ void __launch_bounds__(AS_NT) mid_bwd_small_kernel(MidBwdArgs p) {
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
   const int i0 = 16 * w + g, i1 = i0 + 8;
   {
-    const float* const src[4] = {p.dq2 + g0, p.a + g0, p.dk2 + g0, p.dv2 + g0};
-    const long long ld[4] = {RS_H, RS_H, RS_H, RS_H};
-    const int nr[4] = {rows, rows, rows, rows};
-    const float sc[4] = {p.qscale, 1.f, 1.f, 1.f};
-    __nv_bfloat16* const d[4] = {T, X, Kt, Vt};
-    __nv_bfloat16* const dT[4] = {nullptr, nullptr, nullptr, nullptr};
-    float* const dF[4] = {nullptr, nullptr, nullptr, nullptr};
-    rs_load<4>(src, ld, nr, sc, d, dT, dF);
+    const float* const src[3] = {p.dq2 + g0, p.dk2 + g0, p.dv2 + g0};
+    const long long ld[3] = {RS_H, RS_H, RS_H};
+    const int nr[3] = {rows, rows, rows};
+    const float sc[3] = {p.qscale, 1.f, 1.f};
+    __nv_bfloat16* const d[3] = {T, Kt, Vt};
+    __nv_bfloat16* const dT[3] = {nullptr, nullptr, nullptr};
+    float* const dF[3] = {nullptr, nullptr, nullptr};
+    rs_load<3, RS_BWD_NT>(src, ld, nr, sc, d, dT, dF);
   }
   {
     const float* const src[4] = {p.Win2, p.Win2 + RS_H * RS_H, p.Win2 + 2 * RS_H * RS_H, p.Wo1};
@@ -1026,26 +1070,41 @@ __global__ void __launch_bounds__(AS_NT) mid_bwd_small_kernel(MidBwdArgs p) {
     __nv_bfloat16* const d[4] = {Wt, Wt + RS_TILE, Wt + 2 * RS_TILE, Wt + 3 * RS_TILE};
     __nv_bfloat16* const dT[4] = {nullptr, nullptr, nullptr, nullptr};
     float* const dF[4] = {nullptr, nullptr, nullptr, nullptr};
-    rs_load<4>(src, ld, nr, sc, d, dT, dF);
+    rs_load<4, RS_BWD_NT>(src, ld, nr, sc, d, dT, dF);
+  }
+  {
+    const float* const src[3] = {p.a + g0, p.feats + g0, p.ctx1 + g0};
+    const long long ld[3] = {RS_H, RS_H, RS_H};
+    const int nr[3] = {rows, rows, rows};
+    const float sc[3] = {1.f, 1.f, 1.f};
+    __nv_bfloat16* const d[3] = {As, Fs, Cs};
+    __nv_bfloat16* const dT[3] = {nullptr, nullptr, nullptr};
+    float* const dF[3] = {nullptr, nullptr, nullptr};
+    rs_load<3, RS_BWD_NT>(src, ld, nr, sc, d, dT, dF);
   }
   __syncthreads();
-  // 1. q projection of the cross attention: dWq2 += (dq2 s)^T a ; da = (dq2 s) Wq2
+  if (w >= 4) {
+    // ---- wgrad warps: dWq2 += (dq2 s)^T a ; dWk2 += dk2^T feats ; dWv2 += dv2^T feats ; dWo1 += da^T ctx1 (and the bias sums)
+    rs_wgrad_rm(T, As, p.gWin2, p.gbin2, w - 4);
+    rs_wgrad_rm(Kt, Fs, p.gWin2 + (long long)RS_H * RS_H, p.gbin2 + RS_H, w - 4);
+    rs_wgrad_rm(Vt, Fs, p.gWin2 + 2ll * RS_H * RS_H, p.gbin2 + 2 * RS_H, w - 4);
+    rs_bar_sync(RS_BAR_DA, RS_BWD_NT);
+    rs_wgrad_rm(DAs, Cs, p.gWo1, p.gbo1, w - 4);
+    return;
+  }
+  // 1. q projection of the cross attention: da = (dq2 s) Wq2
   float D[8][4];
 #pragma unroll
   for (int nb = 0; nb < 8; ++nb) D[nb][0] = D[nb][1] = D[nb][2] = D[nb][3] = 0.f;
-  rs_wgrad_rm(T, X, p.gWin2, p.gbin2);
   rs_dgrad(D, T, Wt, 16 * w);
 #pragma unroll
-  for (int nb = 0; nb < 8; ++nb) {          // da as a bf16 tile (operand of step 3), own rows only
+  for (int nb = 0; nb < 8; ++nb) {          // da as a bf16 tile (operand of step 3 and of dWo1), own rows only
     *reinterpret_cast<uint32_t*>(DAs + i0 * RS_LD + 8 * nb + 2 * t) = pack_bf16(D[nb][0], D[nb][1]);
     *reinterpret_cast<uint32_t*>(DAs + i1 * RS_LD + 8 * nb + 2 * t) = pack_bf16(D[nb][2], D[nb][3]);
   }
-  __syncthreads();                          // everybody is done with X == a
-  rs_load1(p.feats + g0, rows, 1.f, X);
-  __syncthreads();
-  // 2. k/v projections of the encoder features: dWk2 += dk2^T feats, dWv2 += dv2^T feats ; dfeats += dk2 Wk2 + dv2 Wv2
-  rs_wgrad_rm(Kt, X, p.gWin2 + (long long)RS_H * RS_H, p.gbin2 + RS_H);
-  rs_wgrad_rm(Vt, X, p.gWin2 + 2ll * RS_H * RS_H, p.gbin2 + 2 * RS_H);
+  __syncwarp();                             // step 3 reads this warp's rows of da through ldmatrix
+  rs_bar_arrive(RS_BAR_DA);
+  // 2. k/v projections of the encoder features: dfeats += dk2 Wk2 + dv2 Wv2
 #pragma unroll
   for (int nb = 0; nb < 8; ++nb) D[nb][0] = D[nb][1] = D[nb][2] = D[nb][3] = 0.f;
   rs_dgrad(D, Kt, Wt + RS_TILE, 16 * w);
@@ -1056,11 +1115,7 @@ __global__ void __launch_bounds__(AS_NT) mid_bwd_small_kernel(MidBwdArgs p) {
     if (i0 < rows) { float2* d = reinterpret_cast<float2*>(p.dfeats + g0 + (long long)i0 * RS_H + c); const float2 o = *d; *d = make_float2(o.x + D[nb][0], o.y + D[nb][1]); }
     if (i1 < rows) { float2* d = reinterpret_cast<float2*>(p.dfeats + g0 + (long long)i1 * RS_H + c); const float2 o = *d; *d = make_float2(o.x + D[nb][2], o.y + D[nb][3]); }
   }
-  __syncthreads();                          // everybody is done with X == feats
-  rs_load1(p.ctx1 + g0, rows, 1.f, X);
-  __syncthreads();
-  // 3. self-attention out-projection: dWo1 += da^T ctx1 ; dctx1 = da Wo1
-  rs_wgrad_rm(DAs, X, p.gWo1, p.gbo1);
+  // 3. self-attention out-projection: dctx1 = da Wo1
 #pragma unroll
   for (int nb = 0; nb < 8; ++nb) D[nb][0] = D[nb][1] = D[nb][2] = D[nb][3] = 0.f;
   rs_dgrad(D, DAs, Wt + 3 * RS_TILE, 16 * w);
