@@ -128,10 +128,40 @@ static cudaError_t set_smem(K kern, size_t bytes) {
   return cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
 }
 
+// Sequences longer than ATTN_TILE_L positions are served by the fused flash attention (flash_tc.cu) alone, up to FLASH_MAX_L
+static const int ATTN_TILE_L = 256, FLASH_MAX_L = 2048;
 static int check_dims(int B, int L, int H, int nh) {
-  if (B <= 0 || L <= 0 || L > 256 || H <= 0 || H > 256 || (H & 3) || nh <= 0 || nh > 8 || H % nh || ((H / nh) & 3))
-    return fail(ADT_E_SHAPE, "%s", "unsupported shape: need 0<L<=256, H%4==0, H<=256, nh<=8, (H/nh)%4==0");
+  if (L > FLASH_MAX_L) return fail(ADT_E_SHAPE, "%s", "unsupported shape: L > 2048 (the longest sequence the fused flash attention serves)");
+  if (B <= 0 || L <= 0 || H <= 0 || H > 256 || (H & 3) || nh <= 0 || nh > 8 || H % nh || ((H / nh) & 3))
+    return fail(ADT_E_SHAPE, "%s", "unsupported shape: need 0<L<=2048, H%4==0, H<=256, nh<=8, (H/nh)%4==0");
   return ADT_OK;
+}
+// shapes of an attention core or a block: beyond 256 positions only the flash kernels serve (bf16, head size 16, 32, ..., 128)
+static int check_attn_dims(int B, int L, int H, int nh, int precision) {
+  if (int e = check_dims(B, L, H, nh)) return e;
+  if (L <= ATTN_TILE_L) return ADT_OK;
+  if (!precision)
+    return fail(ADT_E_SHAPE, "%s", "unsupported shape: L > 256 needs precision 1 (the fp32 attention cores keep whole score rows in shared "
+                                  "memory and stop at 256 positions)");
+  if ((H / nh) % 16 || H / nh > 128)
+    return fail(ADT_E_SHAPE, "%s", "unsupported shape: L > 256 needs a head size H/nh that is a multiple of 16 and at most 128 (fused flash "
+                                  "attention)");
+  return ADT_OK;
+}
+
+// ---- fused flash attention (flash_tc.cu) --------------------------------------------------------------
+namespace adt {
+int flash_attn_fwd(const __nv_bfloat16* qkv, float* ctx, float* lse, const int* key_ids, int B, int L, int H, int nh, int mask_mode,
+                   const DropDesc& d, cudaStream_t s);
+int flash_attn_bwd(const __nv_bfloat16* qkv, const __nv_bfloat16* dcb, const float* ctx, const float* dctx, float* delta, const float* lse,
+                   const int* key_ids, float* dq, float* dk, float* dv, int B, int L, int H, int nh, int mask_mode, const DropDesc& d,
+                   cudaStream_t s);
+}
+// its area: bf16 [q | k | v] [M][3H] ; backward: + bf16 dctx [M][H] + delta [B][nh][L] fp32.  0 where the flash kernels do not serve
+static long long flash_scratch_bytes(int B, int L, int H, int nh, bool bwd) {
+  if (L <= ATTN_TILE_L) return 0;
+  const long long M = (long long)B * L;
+  return 256 + M * 3 * H * 2 + (bwd ? M * H * 2 + M * nh * 4 : 0);
 }
 
 // Row-tile kernels are launched with programmatic stream serialization (opt-in with ADT_PDL=1: measured neutral at the C2 shape): each of them calls
@@ -181,7 +211,7 @@ extern "C" int adt_version(void) { return 200; }
 // sizes of every buffer the caller allocates for one training step (the library allocates nothing); see include/adt_b200.h
 extern "C" int adt_workspace_bytes(const adt_workspace_query* q, adt_workspace_sizes* out) {
   if (!q || !out) return fail(ADT_E_SHAPE, "%s", "workspace_bytes: null argument");
-  if (int e = check_dims(q->B, q->L, q->H, q->nh > 0 ? q->nh : 1)) return e;
+  if (int e = check_attn_dims(q->B, q->L, q->H, q->nh > 0 ? q->nh : 1, 1)) return e;
   const long long M = (long long)q->B * q->L, H = q->H, nh = q->nh > 0 ? q->nh : 1, nl = q->nl > 0 ? q->nl : 1, f = sizeof(float);
   const long long MH = M * H * f, lse = (long long)q->B * nh * q->L * f;
   // encoder block: q,k,v,ctx,y,h1 + lse + rec ; decoder block: d,q1,k1,v1,ctx1,a,q2,k2,v2,ctx2,c,h1 + 2 lse ; streams x[nl+1], xd[nl+1]
@@ -196,7 +226,9 @@ extern "C" int adt_workspace_bytes(const adt_workspace_query* q, adt_workspace_s
   out->scatter_flags = nb * (long long)sizeof(int);
   out->score_part = (long long)(q->n_splits > 0 ? q->n_splits : 1) * q->B * (q->K > 0 ? q->K : 1) * 8;
   // + the attention area of long sequences: packed bf16 [q|k|v] (+ dctx), scores (+ dP) in fp32 and P (+ dS) in bf16, [B*nh][L][Lp]
-  const long long Lp = (q->L + 7) / 8 * 8, zll = M * nh * Lp;
+  // (sequences beyond 256 positions use the flash kernels and their own O(M H) area instead: no L^2 term)
+  const long long Lp = (q->L + 7) / 8 * 8, zll = q->L > ATTN_TILE_L ? 0 : M * nh * Lp;
+  out->attn_scratch = flash_scratch_bytes(q->B, q->L, q->H, nh, true);
   out->wgrad_scratch = H >= 128 ? 12 * M * H * 2 + 10 * H * H * 2 + 1024 + 4 * M * H * 2 + zll * 12 : 0;   // tcgen05 backward: <= 10 operand slots + weights
   out->fwd_scratch = H >= 128 ? 9 * M * H * 2 + 10 * H * H * 2 + 1024 + 3 * M * H * 2 + zll * 6 : 0;       // decoder block: 7 operands + fp32 h2 + weights
   return ADT_OK;
@@ -485,9 +517,10 @@ static int seq_dec_bwd(const adt_dec_block_bwd_args* a, cudaStream_t s) {
 
 
 static int blk_attn_fwd(const float* q, const float* k, const float* v, float* ctx, float* lse, const int* ids, int B, int L, int H, int nh,
-                        int mask_mode, const adt_dropout& d, int training, int precision, void* area, cudaStream_t s);
-static int blk_attn_bwd(const float* q, const float* k, const float* v, const float* dctx, const float* lse, const int* ids, float* dq, float* dk,
-                        float* dv, int B, int L, int H, int nh, int mask_mode, const adt_dropout& d, int precision, void* area, cudaStream_t s);
+                        int mask_mode, const adt_dropout& d, int training, int precision, void* area, void* flash, cudaStream_t s);
+static int blk_attn_bwd(const float* q, const float* k, const float* v, const float* ctx, const float* dctx, const float* lse, const int* ids,
+                        float* dq, float* dk, float* dv, int B, int L, int H, int nh, int mask_mode, const adt_dropout& d, int precision, void* area,
+                        void* flash, cudaStream_t s);
 // ---- tcgen05 forward path for wide models (block_tc.cuh); ADT_FWD_TC=0 keeps the row-tile kernels ---------------------------------
 static bool use_fwd_tc(const void* scratch, int M, int H, int nh, int mma) {
   static int v = -1;
@@ -551,7 +584,7 @@ static int tc_enc_fwd(const adt_enc_block_fwd_args* a, cudaStream_t s) {
     if (int e = tc_linear(t.op(0), Winb, a->attn.in_b, a->q, nullptr, 0, M, H, H, qscale, 0, s)) return e;
     if (int e = tc_linear(t.op(1), Winb + hh, a->attn.in_b + H, a->k, a->v, H, M, 2 * H, H, 1.f, 0, s)) return e;
     if (int e = blk_attn_fwd(a->q, a->k, a->v, a->ctx, a->lse, a->ids, a->B, a->L, H, a->nh, a->mask_mode, a->drop_attn, a->training, a->precision,
-                             t.wb + 10 * hh, s))
+                             t.wb + 10 * hh, a->attn_scratch, s))
       return e;
     if (a->phase == 1) return ADT_OK;
   }
@@ -592,7 +625,7 @@ static int tc_dec_fwd(const adt_dec_block_fwd_args* a, cudaStream_t s) {
     if (int e = tc_linear(t.op(0), W1b, a->slf.in_b, a->q1, nullptr, 0, M, H, H, qscale, 0, s)) return e;
     if (int e = tc_linear(t.op(0), W1b + hh, a->slf.in_b + H, a->k1, a->v1, H, M, 2 * H, H, 1.f, 0, s)) return e;
     if (int e = blk_attn_fwd(a->q1, a->k1, a->v1, a->ctx1, a->lse1, a->ids, a->B, a->L, H, a->nh, a->mask_mode, a->drop_slf, a->training, a->precision,
-                             t.wb + 10 * hh, s))
+                             t.wb + 10 * hh, a->attn_scratch, s))
       return e;
     if (a->phase == 1) return ADT_OK;
   }
@@ -609,7 +642,7 @@ static int tc_dec_fwd(const adt_dec_block_fwd_args* a, cudaStream_t s) {
   if (int e = tc_linear(t.op(2), W2b, a->enc.in_b, a->q2, nullptr, 0, M, H, H, qscale, 0, s)) return e;
   if (int e = tc_linear(t.op(3), W2b + hh, a->enc.in_b + H, a->k2, a->v2, H, M, 2 * H, H, 1.f, 0, s)) return e;
   if (int e = blk_attn_fwd(a->q2, a->k2, a->v2, a->ctx2, a->lse2, a->ids, a->B, a->L, H, a->nh, a->mask_mode, a->drop_enc, a->training, a->precision,
-                           t.wb + 10 * hh, s))
+                           t.wb + 10 * hh, a->attn_scratch, s))
     return e;
   // c = ctx2 Wo2^T + bo2 ; out = (d + FFN(c) + c) * keep
   tc_cast(a->ctx2, t.op(4), (long long)M * H, s);
@@ -727,14 +760,45 @@ static int tc_attn_bwd(const float* q, const float* k, const float* v, const flo
   if (int e = tc_bgemm(w.Pb, Lp, s_so, s_si, 1, w.dcb, H, c_so, hd, 1, dv, H, c_so, hd, L, hd, L, nh, B, s)) return e;                      // dv = (P m)^T dctx
   return check_launch("tcgen05 attention bwd");
 }
-// attention of the tcgen05 block path: long sequences through the batched GEMMs, short ones through the row-tile / small kernels
+// fused flash attention at any L (flash_tc.cu): the only path beyond 256 positions; `area` holds flash_scratch_bytes(B, max(L, 257), ...)
+static int fl_attn_fwd(const float* q, const float* k, const float* v, float* ctx, float* lse, const int* key_ids, int B, int L, int H, int nh,
+                       int mask_mode, const adt_dropout& d, int training, void* area, cudaStream_t s) {
+  if (!area) return fail(ADT_E_SHAPE, "%s", "attention at L > 256: the fused flash kernels need their scratch area (attn_scratch / tc_scratch)");
+  const int M = B * L;
+  __nv_bfloat16* qkv = reinterpret_cast<__nv_bfloat16*>(align256(area));
+  tc_pack(q, 1.f, nullptr, k, nullptr, v, nullptr, qkv, 3 * H, M, H, s);
+  TIMED("attn_flash_fwd", s);
+  if (int e = flash_attn_fwd(qkv, ctx, lse, key_ids, B, L, H, nh, mask_mode, mk_drop(row_drop(d, training)), s))
+    return fail(e, "%s", "fused flash attention fwd (tensor map or launch)");
+  return check_launch("fused flash attention fwd");
+}
+static int fl_attn_bwd(const float* q, const float* k, const float* v, const float* ctx, const float* dctx, const float* lse, const int* key_ids,
+                       float* dq, float* dk, float* dv, int B, int L, int H, int nh, int mask_mode, const adt_dropout& d, void* area, cudaStream_t s) {
+  if (!area) return fail(ADT_E_SHAPE, "%s", "attention at L > 256: the fused flash kernels need their scratch area (attn_scratch / tc_scratch)");
+  if (!ctx) return fail(ADT_E_SHAPE, "%s", "attention backward at L > 256 reads the forward's output: ctx is NULL");
+  const long long M = (long long)B * L;
+  __nv_bfloat16* qkv = reinterpret_cast<__nv_bfloat16*>(align256(area));
+  __nv_bfloat16* dcb = qkv + M * 3 * H;
+  float* delta = reinterpret_cast<float*>(dcb + M * H);
+  tc_pack(q, 1.f, nullptr, k, nullptr, v, nullptr, qkv, 3 * H, (int)M, H, s);
+  tc_cast(dctx, dcb, M * H, s);
+  TIMED("attn_flash_bwd", s);
+  if (int e = flash_attn_bwd(qkv, dcb, ctx, dctx, delta, lse, key_ids, dq, dk, dv, B, L, H, nh, mask_mode, mk_drop(d), s))
+    return fail(e, "%s", "fused flash attention bwd (tensor map or launch)");
+  return check_launch("fused flash attention bwd");
+}
+// attention of every block path: beyond 256 positions the flash kernels (area `flash`); up to 256, long sequences through the batched
+// GEMMs when `area` is given, short ones through the row-tile / small kernels
 static int blk_attn_fwd(const float* q, const float* k, const float* v, float* ctx, float* lse, const int* ids, int B, int L, int H, int nh,
-                        int mask_mode, const adt_dropout& d, int training, int precision, void* area, cudaStream_t s) {
+                        int mask_mode, const adt_dropout& d, int training, int precision, void* area, void* flash, cudaStream_t s) {
+  if (L > ATTN_TILE_L) return fl_attn_fwd(q, k, v, ctx, lse, ids, B, L, H, nh, mask_mode, d, training, flash, s);
   if (area && use_attn_tc(B, L, H, nh)) return tc_attn_fwd(q, k, v, ctx, lse, ids, B, L, H, nh, mask_mode, d, training, area, s);
   return launch_attn_fwd(q, k, v, ctx, lse, ids, B, L, H, nh, mask_mode, d, training, precision, s);
 }
-static int blk_attn_bwd(const float* q, const float* k, const float* v, const float* dctx, const float* lse, const int* ids, float* dq, float* dk,
-                        float* dv, int B, int L, int H, int nh, int mask_mode, const adt_dropout& d, int precision, void* area, cudaStream_t s) {
+static int blk_attn_bwd(const float* q, const float* k, const float* v, const float* ctx, const float* dctx, const float* lse, const int* ids,
+                        float* dq, float* dk, float* dv, int B, int L, int H, int nh, int mask_mode, const adt_dropout& d, int precision, void* area,
+                        void* flash, cudaStream_t s) {
+  if (L > ATTN_TILE_L) return fl_attn_bwd(q, k, v, ctx, dctx, lse, ids, dq, dk, dv, B, L, H, nh, mask_mode, d, flash, s);
   if (area && use_attn_tc(B, L, H, nh)) return tc_attn_bwd(q, k, v, dctx, lse, ids, dq, dk, dv, B, L, H, nh, mask_mode, d, area, s);
   return launch_attn_bwd(q, k, v, dctx, lse, ids, dq, dk, dv, B, L, H, nh, mask_mode, d, precision, s);
 }
@@ -784,8 +848,8 @@ static int tc_enc_bwd(const adt_enc_block_bwd_args* a, cudaStream_t s) {
                                                         a->g_sparse_b, M, H, a->nh);
   }
   if (int e = check_launch("tcgen05 backward path (enc post)")) return e;
-  if (int e = blk_attn_bwd(a->q, a->k, a->v, a->dctx, a->lse, a->ids, a->dq, a->dk, a->dv, a->B, a->L, H, a->nh, a->mask_mode,
-                           a->drop_attn, a->precision, t.wb + 10 * hh, s))
+  if (int e = blk_attn_bwd(a->q, a->k, a->v, a->ctx, a->dctx, a->lse, a->ids, a->dq, a->dk, a->dv, a->B, a->L, H, a->nh, a->mask_mode,
+                           a->drop_attn, a->precision, t.wb + 10 * hh, a->attn_scratch, s))
     return e;
   // in-projection: [dq*s | dk | dv] packed ; q rows read LN1(x), k / v rows read x
   tc_pack(a->dq, qscale, a->g_attn.in_b, a->dk, a->g_attn.in_b + H, a->dv, a->g_attn.in_b + 2 * H, t.op(0), 3 * H, M, H, s);
@@ -827,8 +891,8 @@ static int tc_dec_bwd(const adt_dec_block_bwd_args* a, cudaStream_t s) {
     if (int e = hoisted_wgrad(t.op(4), H, H, t.op(5), H, H, M, a->g_enc.out_w, s)) return e;
     if (int e = tc_dgrad(t.op(4), H, H, Wo2b, H, a->dctx2, 0, M, s)) return e;
     if (int e = check_launch("tcgen05 backward path (dec post)")) return e;
-    if (int e = blk_attn_bwd(a->q2, a->k2, a->v2, a->dctx2, a->lse2, a->ids, a->dq2, a->dk2, a->dv2, a->B, a->L, H, a->nh, a->mask_mode,
-                             a->drop_enc, a->precision, t.wb + 10 * hh, s))
+    if (int e = blk_attn_bwd(a->q2, a->k2, a->v2, a->ctx2, a->dctx2, a->lse2, a->ids, a->dq2, a->dk2, a->dv2, a->B, a->L, H, a->nh, a->mask_mode,
+                             a->drop_enc, a->precision, t.wb + 10 * hh, a->attn_scratch, s))
       return e;
     // cross-attention in-projection (q rows from a, k / v rows from the encoder features), then the self-attention out-projection
     tc_pack(a->dq2, qscale, a->g_enc.in_b, a->dk2, a->g_enc.in_b + H, a->dv2, a->g_enc.in_b + 2 * H, t.op(0), 3 * H, M, H, s);
@@ -846,8 +910,8 @@ static int tc_dec_bwd(const adt_dec_block_bwd_args* a, cudaStream_t s) {
     if (a->phase == 2) return ADT_OK;
   }
   const __nv_bfloat16* W1b = tc_weight(a->slf.in_w, 3 * hh, a->wm, t.wb, s);
-  if (int e = blk_attn_bwd(a->q1, a->k1, a->v1, a->dctx, a->lse1, a->ids, a->dq, a->dk, a->dv, a->B, a->L, H, a->nh, a->mask_mode,
-                           a->drop_slf, a->precision, t.wb + 10 * hh, s))
+  if (int e = blk_attn_bwd(a->q1, a->k1, a->v1, a->ctx1, a->dctx, a->lse1, a->ids, a->dq, a->dk, a->dv, a->B, a->L, H, a->nh, a->mask_mode,
+                           a->drop_slf, a->precision, t.wb + 10 * hh, a->attn_scratch, s))
     return e;
   // q, k and v all read d = LN(x): one [3H x H] weight gradient, one K = 3H dgrad on top of dd
   tc_pack(a->dq, qscale, a->g_slf.in_b, a->dk, a->g_slf.in_b + H, a->dv, a->g_slf.in_b + 2 * H, t.op(0), 3 * H, M, H, s);
@@ -864,7 +928,7 @@ static int tc_dec_bwd(const adt_dec_block_bwd_args* a, cudaStream_t s) {
 // ---------------------------------------------------------------------------------------------------------
 extern "C" int adt_enc_block_fwd(const adt_enc_block_fwd_args* a, adt_stream_t s_) {
   cudaStream_t s = (cudaStream_t)s_;
-  if (int e = check_dims(a->B, a->L, a->H, a->nh)) return e;
+  if (int e = check_attn_dims(a->B, a->L, a->H, a->nh, a->precision)) return e;
   const int M = a->B * a->L, H = a->H;
   const int mma = a->precision ? 1 : 0, pad = mma ? 8 : 4;
   if (a->phase < 0 || a->phase > 2) return fail(ADT_E_SHAPE, "%s", "enc_block_fwd: phase must be 0, 1 or 2");
@@ -872,7 +936,8 @@ extern "C" int adt_enc_block_fwd(const adt_enc_block_fwd_args* a, adt_stream_t s
   if (a->y && a->h1 && a->out && use_fwd_tc(a->tc_scratch, M, H, a->nh, mma)) return tc_enc_fwd(a, s);
   if (a->phase != 2) {
     if (int e = launch_pre_fwd(a->x, a->ln1_w, a->ln1_b, a->attn, a->q, a->k, a->v, nullptr, M, H, a->nh, 0, a->precision, s)) return e;
-    if (int e = launch_attn_fwd(a->q, a->k, a->v, a->ctx, a->lse, a->ids, a->B, a->L, H, a->nh, a->mask_mode, a->drop_attn, a->training, a->precision, s))
+    if (int e = blk_attn_fwd(a->q, a->k, a->v, a->ctx, a->lse, a->ids, a->B, a->L, H, a->nh, a->mask_mode, a->drop_attn, a->training, a->precision,
+                             nullptr, a->attn_scratch, s))
       return e;
     if (a->phase == 1) return ADT_OK;
   }
@@ -902,7 +967,7 @@ extern "C" int adt_enc_block_fwd(const adt_enc_block_fwd_args* a, adt_stream_t s
 
 extern "C" int adt_enc_block_bwd(const adt_enc_block_bwd_args* a, adt_stream_t s_) {
   cudaStream_t s = (cudaStream_t)s_;
-  if (int e = check_dims(a->B, a->L, a->H, a->nh)) return e;
+  if (int e = check_attn_dims(a->B, a->L, a->H, a->nh, a->precision)) return e;
   const int M = a->B * a->L, H = a->H;
   const int mma = a->precision ? 1 : 0, pad = mma ? 8 : 4;
   if (use_seq(a->L, H, a->nh, mma, SEQ_ENC_BWD)) return seq_enc_bwd(a, s);
@@ -938,8 +1003,8 @@ extern "C" int adt_enc_block_bwd(const adt_enc_block_bwd_args* a, adt_stream_t s
     if (int e = hoisted_wgrad(hz + 2 * hu, H, H, hz + 3 * hu, H, H, M, a->g_ffn.w1, s)) return e;
     if (int e = hoisted_wgrad(hz + 4 * hu, H, H, hz + 5 * hu, H, H, M, a->g_attn.out_w, s)) return e;
   }
-  if (int e = launch_attn_bwd(a->q, a->k, a->v, a->dctx, a->lse, a->ids, a->dq, a->dk, a->dv, a->B, a->L, H, a->nh, a->mask_mode,
-                              a->drop_attn, a->precision, s))
+  if (int e = blk_attn_bwd(a->q, a->k, a->v, a->ctx, a->dctx, a->lse, a->ids, a->dq, a->dk, a->dv, a->B, a->L, H, a->nh, a->mask_mode,
+                           a->drop_attn, a->precision, nullptr, a->attn_scratch, s))
     return e;
   PreBwdArgs r;
   memset(&r, 0, sizeof(r));
@@ -959,14 +1024,15 @@ extern "C" int adt_enc_block_bwd(const adt_enc_block_bwd_args* a, adt_stream_t s
 // ---------------------------------------------------------------------------------------------------------
 extern "C" int adt_dec_block_fwd(const adt_dec_block_fwd_args* a, adt_stream_t s_) {
   cudaStream_t s = (cudaStream_t)s_;
-  if (int e = check_dims(a->B, a->L, a->H, a->nh)) return e;
+  if (int e = check_attn_dims(a->B, a->L, a->H, a->nh, a->precision)) return e;
   const int M = a->B * a->L, H = a->H;
   const int mma = a->precision ? 1 : 0, pad = mma ? 8 : 4;
   if (use_seq(a->L, H, a->nh, mma, SEQ_DEC_FWD)) return seq_dec_fwd(a, s);
   if (a->d && a->a && a->c && a->h1 && use_fwd_tc(a->tc_scratch, M, H, a->nh, mma)) return tc_dec_fwd(a, s);
   if (a->phase != 2) {
     if (int e = launch_pre_fwd(a->x, a->ln_w, a->ln_b, a->slf, a->q1, a->k1, a->v1, a->d, M, H, a->nh, 1, a->precision, s)) return e;
-    if (int e = launch_attn_fwd(a->q1, a->k1, a->v1, a->ctx1, a->lse1, a->ids, a->B, a->L, H, a->nh, a->mask_mode, a->drop_slf, a->training, a->precision, s))
+    if (int e = blk_attn_fwd(a->q1, a->k1, a->v1, a->ctx1, a->lse1, a->ids, a->B, a->L, H, a->nh, a->mask_mode, a->drop_slf, a->training, a->precision,
+                             nullptr, a->attn_scratch, s))
       return e;
     if (a->phase == 1) return ADT_OK;
   }
@@ -986,7 +1052,8 @@ extern "C" int adt_dec_block_fwd(const adt_dec_block_fwd_args* a, adt_stream_t s
               a->q2, a->k2, a->v2, M, H, qscale);
   }
   if (int e = check_launch("mid_fwd")) return e;
-  if (int e = launch_attn_fwd(a->q2, a->k2, a->v2, a->ctx2, a->lse2, a->ids, a->B, a->L, H, a->nh, a->mask_mode, a->drop_enc, a->training, a->precision, s))
+  if (int e = blk_attn_fwd(a->q2, a->k2, a->v2, a->ctx2, a->lse2, a->ids, a->B, a->L, H, a->nh, a->mask_mode, a->drop_enc, a->training, a->precision,
+                           nullptr, a->attn_scratch, s))
     return e;
   PostFwdArgs p;
   memset(&p, 0, sizeof(p));
@@ -1009,7 +1076,7 @@ extern "C" int adt_dec_block_fwd(const adt_dec_block_fwd_args* a, adt_stream_t s
 
 extern "C" int adt_dec_block_bwd(const adt_dec_block_bwd_args* a, adt_stream_t s_) {
   cudaStream_t s = (cudaStream_t)s_;
-  if (int e = check_dims(a->B, a->L, a->H, a->nh)) return e;
+  if (int e = check_attn_dims(a->B, a->L, a->H, a->nh, a->precision)) return e;
   const int M = a->B * a->L, H = a->H;
   const int mma = a->precision ? 1 : 0, pad = mma ? 8 : 4;
   const float qscale = 1.0f / sqrtf((float)(H / a->nh));
@@ -1045,8 +1112,8 @@ extern "C" int adt_dec_block_bwd(const adt_dec_block_bwd_args* a, adt_stream_t s
     if (int e = hoisted_wgrad(hz + 4 * hu, H, H, hz + 5 * hu, H, H, M, a->g_enc.out_w, s)) return e;
   }
   // cross attention (keys/values from the encoder features)
-  if (int e = launch_attn_bwd(a->q2, a->k2, a->v2, a->dctx2, a->lse2, a->ids, a->dq2, a->dk2, a->dv2, a->B, a->L, H, a->nh, a->mask_mode,
-                              a->drop_enc, a->precision, s))
+  if (int e = blk_attn_bwd(a->q2, a->k2, a->v2, a->ctx2, a->dctx2, a->lse2, a->ids, a->dq2, a->dk2, a->dv2, a->B, a->L, H, a->nh, a->mask_mode,
+                           a->drop_enc, a->precision, nullptr, a->attn_scratch, s))
     return e;
   MidBwdArgs m;
   memset(&m, 0, sizeof(m));
@@ -1073,8 +1140,8 @@ extern "C" int adt_dec_block_bwd(const adt_dec_block_bwd_args* a, adt_stream_t s
   }
   if (a->phase == 2) return ADT_OK;
   }
-  if (int e = launch_attn_bwd(a->q1, a->k1, a->v1, a->dctx, a->lse1, a->ids, a->dq, a->dk, a->dv, a->B, a->L, H, a->nh, a->mask_mode,
-                              a->drop_slf, a->precision, s))
+  if (int e = blk_attn_bwd(a->q1, a->k1, a->v1, a->ctx1, a->dctx, a->lse1, a->ids, a->dq, a->dk, a->dv, a->B, a->L, H, a->nh, a->mask_mode,
+                           a->drop_slf, a->precision, nullptr, a->attn_scratch, s))
     return e;
   PreBwdArgs r;
   memset(&r, 0, sizeof(r));
@@ -1326,19 +1393,36 @@ extern "C" int adt_small_table_grad(const int32_t* ids, const float* dx, float* 
 }
 
 extern "C" int64_t adt_attention_scratch_bytes(int32_t B, int32_t L, int32_t H, int32_t nh, int32_t backward) {
-  if (B <= 0 || L <= 0 || H <= 0 || nh <= 0 || !use_attn_tc(B, L, H, nh)) return 0;
+  if (B <= 0 || L <= 0 || H <= 0 || nh <= 0) return 0;
+  if (L > ATTN_TILE_L) return flash_scratch_bytes(B, L, H, nh, backward != 0);
+  if (!use_attn_tc(B, L, H, nh)) return 0;
   const long long M = (long long)B * L, Lp = (L + 7) / 8 * 8, zll = M * nh * Lp;
   return 1024 + (backward ? 4 : 3) * M * H * 2 + zll * (backward ? 12 : 6);
 }
 extern "C" int adt_attention_fwd(const adt_attention_args* a, adt_stream_t s_) {
-  if (int e = check_dims(a->B, a->L, a->H, a->nh)) return e;
+  if (int e = check_attn_dims(a->B, a->L, a->H, a->nh, a->precision)) return e;
   return blk_attn_fwd(a->q, a->k, a->v, a->ctx, a->lse, a->key_ids, a->B, a->L, a->H, a->nh, a->mask_mode, a->drop, a->training,
-                      a->precision ? 1 : 0, a->precision ? a->tc_scratch : nullptr, (cudaStream_t)s_);
+                      a->precision ? 1 : 0, a->precision ? a->tc_scratch : nullptr, a->tc_scratch, (cudaStream_t)s_);
 }
 extern "C" int adt_attention_bwd(const adt_attention_args* a, adt_stream_t s_) {
-  if (int e = check_dims(a->B, a->L, a->H, a->nh)) return e;
-  return blk_attn_bwd(a->q, a->k, a->v, a->dctx, a->lse, a->key_ids, a->dq, a->dk, a->dv, a->B, a->L, a->H, a->nh, a->mask_mode, a->drop,
-                      a->precision ? 1 : 0, a->precision ? a->tc_scratch : nullptr, (cudaStream_t)s_);
+  if (int e = check_attn_dims(a->B, a->L, a->H, a->nh, a->precision)) return e;
+  return blk_attn_bwd(a->q, a->k, a->v, a->ctx, a->dctx, a->lse, a->key_ids, a->dq, a->dk, a->dv, a->B, a->L, a->H, a->nh, a->mask_mode, a->drop,
+                      a->precision ? 1 : 0, a->precision ? a->tc_scratch : nullptr, a->tc_scratch, (cudaStream_t)s_);
+}
+// the flash kernels at any L <= 2048 (for L <= 256 a test / comparison entry: the dispatch above never takes them there)
+static int check_flash(const adt_attention_args* a) {
+  if (int e = check_attn_dims(a->B, a->L > ATTN_TILE_L ? a->L : ATTN_TILE_L + 1, a->H, a->nh, a->precision)) return e;
+  return check_dims(a->B, a->L, a->H, a->nh);
+}
+extern "C" int adt_attention_flash_fwd(const adt_attention_args* a, adt_stream_t s_) {
+  if (int e = check_flash(a)) return e;
+  return fl_attn_fwd(a->q, a->k, a->v, a->ctx, a->lse, a->key_ids, a->B, a->L, a->H, a->nh, a->mask_mode, a->drop, a->training, a->tc_scratch,
+                     (cudaStream_t)s_);
+}
+extern "C" int adt_attention_flash_bwd(const adt_attention_args* a, adt_stream_t s_) {
+  if (int e = check_flash(a)) return e;
+  return fl_attn_bwd(a->q, a->k, a->v, a->ctx, a->dctx, a->lse, a->key_ids, a->dq, a->dk, a->dv, a->B, a->L, a->H, a->nh, a->mask_mode, a->drop,
+                     a->tc_scratch, (cudaStream_t)s_);
 }
 
 extern "C" int adt_softmax_ce_fwd(const float* logits, const int32_t* labels, float* lse, double* loss_acc, int32_t R, int32_t V,

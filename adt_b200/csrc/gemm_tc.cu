@@ -411,6 +411,10 @@ __global__ void __launch_bounds__(256) colsum_kernel(const float* __restrict__ x
   }
 }
 
+}  // namespace
+
+// also used by the fused attention kernels of flash_tc.cu
+namespace adt {
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -443,6 +447,9 @@ int g_make_map(CUtensorMap* m, const void* base, long long rows, long long cols,
                          CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   return r == CUDA_SUCCESS ? ADT_OK : ADT_E_CUDA;
 }
+}  // namespace adt
+
+namespace {
 
 template <int BN, int NS, int MODE = 0>
 int g_launch(const CUtensorMap& tmA, const CUtensorMap& tmB, GemmTcArgs k, int splits, cudaStream_t s, bool stage = false) {

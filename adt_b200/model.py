@@ -235,6 +235,10 @@ class Engine:
         nfs = w["sizes"]["fwd_scratch"] if self.precision else 0
         w["fs"] = torch.empty(nfs, dtype=torch.uint8, device=dev) if nfs else None
         w["side"]["fs"] = torch.empty(nfs, dtype=torch.uint8, device=dev) if nfs else None
+        # bf16 operands of the fused flash attention (L > 256; again one more for the side-stream half of decoder block 0)
+        nas = w["sizes"]["attn_scratch"]
+        w["as"] = torch.empty(nas, dtype=torch.uint8, device=dev) if nas else None
+        w["side"]["as"] = torch.empty(nas, dtype=torch.uint8, device=dev) if nas else None
         N = 4 * M
         i32 = lambda n: torch.empty(n, dtype=torch.int32, device=dev)
         w["keys"], w["vals"], w["keys_tmp"], w["vals_tmp"] = i32(N), i32(N), i32(N), i32(N)
@@ -293,7 +297,7 @@ class Engine:
             sa, s1, s2 = sites[("enc", l)]
             last = l == m.num_layers - 1
             a = L.fill(L.adt_enc_block_fwd_args(), x=w["x"][l], ids=seq, phase=(last_phase if l == m.num_layers - 1 else 0),
-                       wm=wm, out_last=(out_last if last else None), tc_scratch=w.get("fs"),
+                       wm=wm, out_last=(out_last if last else None), tc_scratch=w.get("fs"), attn_scratch=w.get("as"),
                        ln1_w=layer.attention_layernorm.weight, ln1_b=layer.attention_layernorm.bias, attn=_mha_w(layer.attention_layer),
                        ln2_w=layer.forward_layernorm.weight, ln2_b=layer.forward_layernorm.bias, ffn=_ffn_w(layer.forward_layer),
                        sparse_w=layer.sparse.weight, sparse_b=layer.sparse.bias,
@@ -359,6 +363,7 @@ class Engine:
             ss, se, s1, s2 = sites[("dec", j)]
             a = L.fill(L.adt_dec_block_fwd_args(), x=w["xd"][j], feats=w["feats"], ids=dec, wm=self.wm(),
                        tc_scratch=(w["side"]["fs"] if phases[0] == 1 else w["fs"]),     # phase 1 runs beside the encoder on the side stream
+                       attn_scratch=(w["side"]["as"] if phases[0] == 1 else w["as"]),
                        ln_w=layer.layer_norm.weight, ln_b=layer.layer_norm.bias, slf=_mha_w(layer.slf_attn), enc=_mha_w(layer.enc_attn),
                        ffn=_ffn_w(layer.pos_ffn), enc_in=w["x"][nl - 1 - j] if fused_mse else None,
                        out=w["xd"][j + 1], mse_acc=(w["acc"][3 + j:] if fused_mse else None),
@@ -440,7 +445,7 @@ class Engine:
                        dout=dout, denc=w["denc"][i_enc] if fused else None,
                        dq=sb["dq"] if split else w["dq"], dk=sb["dk"] if split else z4[0], dv=sb["dv"] if split else z4[1],
                        dctx=sb["dctx"] if split else w["dctx"], dd=sb["dres"] if split else w["dres"],
-                       dq2=w["dq2"], dk2=z4[2], dv2=z4[3], dctx2=w["dctx2"], phase=2 if split else 0, wgrad_scratch=w["wg"],
+                       dq2=w["dq2"], dk2=z4[2], dv2=z4[3], dctx2=w["dctx2"], phase=2 if split else 0, wgrad_scratch=w["wg"], attn_scratch=w["as"],
                        dfeats=w["dfeats"], dx=out_dx, g_ln_w=g[pre + "layer_norm.weight"], g_ln_b=g[pre + "layer_norm.bias"],
                        g_slf=mg(pre + "slf_attn."), g_enc=mg(pre + "enc_attn."), g_ffn=fg(pre + "pos_ffn."),
                        B=B, L=Lq, H=H, nh=nh, mask_mode=0, precision=self.precision,
@@ -454,6 +459,7 @@ class Engine:
                 with torch.cuda.stream(side):
                     a.phase = 1
                     a.wgrad_scratch = sb["wg"].data_ptr() if sb["wg"] is not None else None
+                    a.attn_scratch = sb["as"].data_ptr() if sb["as"] is not None else None
                     L.check(self.lib.adt_dec_block_bwd(L.ctypes.byref(a), self._stream()), "adt_dec_block_bwd")
             dxd = out_dx
         dx_dec_emb = dxd
@@ -484,7 +490,7 @@ class Engine:
                        q=sv["q"], k=sv["k"], v=sv["v"], ctx=sv["ctx"], lse=sv["lse"], y=sv["y"], h1=sv["h1"],
                        dout=dout, dx_extra=dx_extra, drec=dr[l] if dr is not None else None,
                        nll_coef=(float(lambdas2[nl - 1]) / (Mg * nh)) if (fused and nh > 1) else 0.0,
-                       dq=w["dq"], dk=z4[0], dv=z4[1], dctx=w["dctx"], dy=w["dres"], dx=other, wgrad_scratch=w["wg"],
+                       dq=w["dq"], dk=z4[0], dv=z4[1], dctx=w["dctx"], dy=w["dres"], dx=other, wgrad_scratch=w["wg"], attn_scratch=w["as"],
                        g_ln1_w=g[pre + "attention_layernorm.weight"], g_ln1_b=g[pre + "attention_layernorm.bias"],
                        g_attn=mg(pre + "attention_layer."), g_ln2_w=g[pre + "forward_layernorm.weight"],
                        g_ln2_b=g[pre + "forward_layernorm.bias"], g_ffn=fg(pre + "forward_layer."),

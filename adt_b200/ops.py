@@ -59,8 +59,13 @@ def _use_tc(precision, M, N, K):
     return bool(precision) and M >= 128 and M * N * K >= TC_MIN_WORK and torch.cuda.get_device_capability()[0] >= 10
 
 
+FLASH_MIN_L = 257   # sequences at least this long run in the fused flash attention kernels (adt_attention_fwd / _bwd dispatch)
+
+
 def _attn_scratch(ref, B, Lq, H, nh, precision, backward):
-    """scratch of the tcgen05 attention path (bf16 mode, 65..256 positions): packed bf16 operands, scores and probabilities in HBM"""
+    """scratch of the tcgen05 attention paths (bf16 mode): at 65..256 positions the batched path's packed bf16 operands, scores and
+    probabilities in HBM; at 257..2048 positions the fused flash kernels' packed bf16 operands (+ bf16 dctx and the row sums of
+    dctx * ctx in the backward), O(B L H) with no L^2 term"""
     if not precision or torch.cuda.get_device_capability()[0] < 10:
         return None
     f = L.lib().adt_attention_scratch_bytes
@@ -257,13 +262,14 @@ class AttnFn(torch.autograd.Function):
         a = L.fill(L.adt_attention_args(), q=q, k=k, v=v, ctx=out, lse=lse, key_ids=key_ids, dctx=None, dq=None, dk=None, dv=None, B=B,
                    L=Lq, H=H, nh=nh, mask_mode=mask_mode, training=int(training), drop=drop, precision=precision, tc_scratch=ws)
         L.check(L.lib().adt_attention_fwd(ctypes.byref(a), _st(q.device)), "adt_attention_fwd")
-        ctx.save_for_backward(q, k, v, lse)
+        # the flash backward (L > 256) reads the forward's output for its row sums of dctx * ctx
+        ctx.save_for_backward(q, k, v, lse, out if Lq >= FLASH_MIN_L else None)
         ctx.cfg = (key_ids, dims, drop, training, precision)
         return out
 
     @staticmethod
     def backward(ctx, dctx):
-        q, k, v, lse = ctx.saved_tensors
+        q, k, v, lse, out = ctx.saved_tensors
         key_ids, (B, Lq, nh, mask_mode), drop, training, precision = ctx.cfg
         H = q.shape[1]
         dq, dk, dv = torch.empty_like(q), torch.empty_like(q), torch.empty_like(q)
@@ -271,7 +277,7 @@ class AttnFn(torch.autograd.Function):
         if not training:
             d = no_drop()
         ws = _attn_scratch(q, B, Lq, H, nh, precision, 1)
-        a = L.fill(L.adt_attention_args(), q=q, k=k, v=v, ctx=None, lse=lse, key_ids=key_ids, dctx=dctx.contiguous(), dq=dq, dk=dk, dv=dv,
+        a = L.fill(L.adt_attention_args(), q=q, k=k, v=v, ctx=out, lse=lse, key_ids=key_ids, dctx=dctx.contiguous(), dq=dq, dk=dk, dv=dv,
                    B=B, L=Lq, H=H, nh=nh, mask_mode=mask_mode, training=int(training), drop=d, precision=precision, tc_scratch=ws)
         L.check(L.lib().adt_attention_bwd(ctypes.byref(a), _st(q.device)), "adt_attention_bwd")
         return dq, dk, dv, None, None, None, None, None

@@ -46,9 +46,13 @@ const char* adt_last_error(void);
  * nothing itself.  saved = activations kept from forward for backward; scratch = backward temporaries; sort = keys/vals/tmp/hist of
  * adt_embed_sort; scatter = head/tail/has_tail of adt_embed_bwd; score_part = part_scores + part_ids of adt_score_topk for
  * (U = B, K, n_splits); wgrad_scratch = the bf16 operand copies of the hoisted weight gradients, fwd_scratch = the bf16 operands of the
- * tcgen05 forward path (both 0 when H < 128). */
+ * tcgen05 forward path (both 0 when H < 128).  Sequences of 257..2048 positions need precision 1 and a head size H/nh that is a multiple of
+ * 16 up to 128. */
 typedef struct { int32_t B, L, H, nh, nl, K, n_splits; } adt_workspace_query;
-typedef struct { int64_t saved, scratch, sort_keys, sort_hist, scatter_rows, scatter_flags, score_part, wgrad_scratch, fwd_scratch; } adt_workspace_sizes;
+typedef struct {
+  int64_t saved, scratch, sort_keys, sort_hist, scatter_rows, scatter_flags, score_part, wgrad_scratch, fwd_scratch;
+  int64_t attn_scratch;  /* L > 256: bf16 operands of the fused flash attention (O(B*L*H), one per concurrently running block; 0 for L <= 256) */
+} adt_workspace_sizes;
 int adt_workspace_bytes(const adt_workspace_query* q, adt_workspace_sizes* out);
 
 /* K1. x = dropout(E[ids]*sqrt(H) + P[t]) * (ids != 0)            -- sasrec/model.py:34-41 and :53-58 */
@@ -93,6 +97,7 @@ typedef struct {
                       H == 64, L <= 64, nh in {1,2,4}); otherwise ignored, so callers must check adt_seq_kernels_apply() first */
   void* tc_scratch; /* optional, adt_workspace_sizes.fwd_scratch bytes (precision 1, H >= 128, H % 64 == 0, phase 0): every linear layer
                        then runs as one tcgen05 GEMM over all rows (block_tc.cuh) instead of inside the row-tile kernels */
+  void* attn_scratch; /* adt_workspace_sizes.attn_scratch bytes, required when L > 256 (fused flash attention; NULL otherwise) */
 } adt_enc_block_fwd_args;
 int adt_enc_block_fwd(const adt_enc_block_fwd_args* a, adt_stream_t stream);
 
@@ -115,6 +120,7 @@ typedef struct {
   adt_wmirror wm;
   void* wgrad_scratch;        /* optional, adt_workspace_sizes.wgrad_scratch bytes (precision 1, H >= 128): the row-tile kernels then only write
                                  bf16 copies of their dY / X tiles and every weight gradient becomes ONE split-K tcgen05 GEMM over all rows */
+  void* attn_scratch;         /* as in adt_enc_block_fwd_args */
 } adt_enc_block_bwd_args;
 int adt_enc_block_bwd(const adt_enc_block_bwd_args* a, adt_stream_t stream);
 
@@ -134,6 +140,7 @@ typedef struct {
                     * stream); 2: the rest (cross-attention on `feats`, FFN) */
   adt_wmirror wm;
   void* tc_scratch; /* as in adt_enc_block_fwd_args (phases 0, 1 and 2) */
+  void* attn_scratch; /* as in adt_enc_block_fwd_args */
 } adt_dec_block_fwd_args;
 int adt_dec_block_fwd(const adt_dec_block_fwd_args* a, adt_stream_t stream);
 
@@ -156,6 +163,7 @@ typedef struct {
                     * (produce dx; nothing the encoder backward needs -> may run beside it on another stream) */
   adt_wmirror wm;
   void* wgrad_scratch;        /* as in adt_enc_block_bwd_args */
+  void* attn_scratch;         /* as in adt_enc_block_fwd_args */
 } adt_dec_block_bwd_args;
 int adt_dec_block_bwd(const adt_dec_block_bwd_args* a, adt_stream_t stream);
 
@@ -363,17 +371,24 @@ int adt_gather3(const int32_t* ia, const float* A, const int32_t* ib, const floa
                 int32_t M, int32_t H, adt_stream_t stream);
 int adt_small_table_grad(const int32_t* ids, const float* dx, float* g, int32_t M, int32_t H, int32_t padding_idx, adt_stream_t stream);
 /* multi-head attention core on projected q (pre-scaled), k, v [B*L, H]: softmax(q k^T + mask) -> dropout -> . v
- * mask_mode 0 causal, 1 key padding (key_ids[b][j] == 0 -> -1e9, modules.py:88-91).  lse [B,nh,L] saved for backward. */
+ * mask_mode 0 causal, 1 key padding (key_ids[b][j] == 0 -> -1e9, modules.py:88-91).  lse [B,nh,L] saved for backward.
+ * 1 <= L <= 2048; L > 256 needs precision 1, a head size H/nh that is a multiple of 16 up to 128, tc_scratch, and (backward) ctx. */
 typedef struct {
-  const float* q; const float* k; const float* v; float* ctx; float* lse; const int32_t* key_ids;
+  const float* q; const float* k; const float* v; float* ctx; float* lse; const int32_t* key_ids;   /* backward reads ctx when L > 256 */
   const float* dctx; float* dq; float* dk; float* dv;                       /* backward only */
   int32_t B, L, H, nh, mask_mode, training; adt_dropout drop; int32_t precision;
-  void* tc_scratch;   /* optional, adt_attention_scratch_bytes(B, L, H, nh, backward) bytes: sequences of 65..256 positions in the bf16 mode then run as
-                         strided-batch tcgen05 GEMMs (q k^T, P v, and the three backward products) + one softmax / dropout row kernel */
+  void* tc_scratch;   /* adt_attention_scratch_bytes(B, L, H, nh, backward) bytes.  Sequences of 65..256 positions in the bf16 mode then run as
+                         strided-batch tcgen05 GEMMs (q k^T, P v, and the three backward products) + one softmax / dropout row kernel
+                         (optional there); sequences of 257..2048 positions run in the fused flash kernels (required there) */
 } adt_attention_args;
 int64_t adt_attention_scratch_bytes(int32_t B, int32_t L, int32_t H, int32_t nh, int32_t backward);
 int adt_attention_fwd(const adt_attention_args* a, adt_stream_t stream);
 int adt_attention_bwd(const adt_attention_args* a, adt_stream_t stream);
+/* the fused flash attention (flash_tc.cu) at any 1 <= L <= 2048 (bf16, head size a multiple of 16 up to 128): the kernels every call
+ * above dispatches to for L > 256, exported so that shorter sequences can be compared with the batched path on the same inputs.
+ * tc_scratch: adt_attention_scratch_bytes(B, max(L, 257), H, nh, backward) bytes; the backward reads ctx. */
+int adt_attention_flash_fwd(const adt_attention_args* a, adt_stream_t stream);
+int adt_attention_flash_bwd(const adt_attention_args* a, adt_stream_t stream);
 /* softmax cross-entropy over logits rows [R,V] (nn.CrossEntropyLoss on the rows that carry a label, trainer.py:113-115).
  * fwd: lse[r], *loss_acc += sum_r (lse[r] - logits[r][labels[r]]).  bwd: logits <- (softmax - onehot) * coef, in place. */
 int adt_softmax_ce_fwd(const float* logits, const int32_t* labels, float* lse, double* loss_acc, int32_t R, int32_t V, adt_stream_t stream);
