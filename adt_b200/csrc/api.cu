@@ -346,6 +346,80 @@ static int launch_attn_bwd(const float* q, const float* k, const float* v, const
   return check_launch("attn_bwd");
 }
 
+static adt_dropout row_drop(const adt_dropout& d, int training) {
+  adt_dropout r = d;
+  if (!training) r.enabled = 0;
+  return r;
+}
+
+// Sequences of 33 .. 64 positions on the H = 64 bf16 path: one CTA per sequence runs the attention inside the kernel that produces its
+// operands (LN + in-projection; the decoder's out-projection + cross-attention projections) or consumes its adjoints (in-projection
+// adjoint), which removes a launch and the fp32 round trip of q, k, v (dq, dk, dv) per attention.  The backward needs two or four heads.  ADT_ATTN_FUSED=0 keeps the separate launches.
+static bool use_attn_fused(int L, int H, int nh, int mma, bool bwd) {
+  static int v = -1;
+  if (v < 0) { const char* e = getenv("ADT_ATTN_FUSED"); v = e ? (atoi(e) != 0) : 1; }
+  return v && L > 32 && use_row_small(H, mma) && use_attn_small(L, H / nh, mma) && (!bwd || nh == 2 || nh == 4);
+}
+
+static int launch_pre_attn_fwd(const float* x, const float* ln_w, const float* ln_b, const adt_mha_w& w, float* q, float* k, float* v,
+                               float* norm_out, float* ctx, float* lse, const int* ids, int B, int L, int nh, int kv_from_norm, int mask_mode,
+                               const adt_dropout& d, int training, cudaStream_t s) {
+  RsAttnFwdArgs p;
+  memset(&p, 0, sizeof(p));
+  p.x = x; p.ln_g = ln_w; p.ln_b = ln_b; p.Win = w.in_w; p.bin = w.in_b; p.q = q; p.k = k; p.v = v; p.norm_out = norm_out;
+  p.ctx = ctx; p.lse = lse; p.ids = ids; p.L = L; p.mask_mode = mask_mode; p.kv_from_norm = kv_from_norm;
+  p.qscale = 1.0f / sqrtf((float)(RS_H / nh)); p.drop = mk_drop(row_drop(d, training));
+  const size_t sm = PreAttnFwdSmem::TOTAL_BYTES;
+  TIMED("pre_attn_fwd", s);
+#define ADT_PAF(HD)                                                                                           \
+  do {                                                                                                        \
+    cudaFuncSetAttribute(pre_attn_fwd_small_kernel<HD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm); \
+    pre_attn_fwd_small_kernel<HD><<<B, RS_BWD_NT, sm, s>>>(p);                                                \
+  } while (0)
+  if (nh == 1) ADT_PAF(64);
+  else if (nh == 2) ADT_PAF(32);
+  else ADT_PAF(16);
+#undef ADT_PAF
+  return check_launch("pre_attn_fwd_small");
+}
+
+static int launch_mid_attn_fwd(const adt_dec_block_fwd_args* a, float qscale, cudaStream_t s) {
+  RsMidAttnArgs p;
+  memset(&p, 0, sizeof(p));
+  p.ctx1 = a->ctx1; p.feats = a->feats; p.Wo1 = a->slf.out_w; p.bo1 = a->slf.out_b; p.Win2 = a->enc.in_w; p.bin2 = a->enc.in_b;
+  p.a = a->a; p.q2 = a->q2; p.k2 = a->k2; p.v2 = a->v2; p.ctx2 = a->ctx2; p.lse2 = a->lse2; p.ids = a->ids;
+  p.L = a->L; p.mask_mode = a->mask_mode; p.qscale = qscale; p.drop = mk_drop(row_drop(a->drop_enc, a->training));
+  const size_t sm = MidAttnFwdSmem::TOTAL_BYTES;
+  TIMED("mid_attn_fwd", s);
+#define ADT_MAF(HD)                                                                                           \
+  do {                                                                                                        \
+    cudaFuncSetAttribute(mid_attn_fwd_small_kernel<HD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm); \
+    mid_attn_fwd_small_kernel<HD><<<a->B, RS_BWD_NT, sm, s>>>(p);                                             \
+  } while (0)
+  if (a->nh == 1) ADT_MAF(64);
+  else if (a->nh == 2) ADT_MAF(32);
+  else ADT_MAF(16);
+#undef ADT_MAF
+  return check_launch("mid_attn_fwd_small");
+}
+
+static int launch_attn_pre_bwd(const PreBwdArgs& r, const float* q, const float* k, const float* v, const float* dctx, const float* lse,
+                               const int* ids, int B, int L, int nh, int mask_mode, const adt_dropout& d, cudaStream_t s) {
+  RsAttnBwdArgs p;
+  memset(&p, 0, sizeof(p));
+  p.pre = r; p.q = q; p.k = k; p.v = v; p.dctx = dctx; p.lse = lse; p.ids = ids; p.L = L; p.mask_mode = mask_mode; p.drop = mk_drop(d);
+  const size_t sm = AttnPreBwdSmem::TOTAL_BYTES;
+  TIMED("attn_pre_bwd", s);
+  if (nh == 2) {
+    cudaFuncSetAttribute(attn_pre_bwd_small_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+    attn_pre_bwd_small_kernel<32><<<B, RS_BWD_NT, sm, s>>>(p);
+  } else {
+    cudaFuncSetAttribute(attn_pre_bwd_small_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+    attn_pre_bwd_small_kernel<16><<<B, RS_BWD_NT, sm, s>>>(p);
+  }
+  return check_launch("attn_pre_bwd_small");
+}
+
 // pre_bwd: narrow models (H == 64) in the bf16 mode take the weights-resident 256-thread kernel (ADT_ROW_SMALL=0 disables)
 static int launch_pre_bwd(const PreBwdArgs& r, int mma, cudaStream_t s) {
   TIMED("pre_bwd", s);
@@ -381,12 +455,6 @@ static int hoisted_wgrad(const __nv_bfloat16* dy, long long ldy, int n_out, cons
   TIMED("wgrad_tc", s);
   if (int e = adt_gemm_tc(&g, (adt_stream_t)s)) return fail(e, "%s", "hoisted weight gradient (adt_gemm_tc)");
   return ADT_OK;
-}
-
-static adt_dropout row_drop(const adt_dropout& d, int training) {
-  adt_dropout r = d;
-  if (!training) r.enabled = 0;
-  return r;
 }
 
 // ---- sequence-resident block kernels (kernels_seq.cuh): one CTA per sequence, a whole block per launch ------------------------
@@ -935,10 +1003,16 @@ extern "C" int adt_enc_block_fwd(const adt_enc_block_fwd_args* a, adt_stream_t s
   if (a->phase == 0 && use_seq(a->L, H, a->nh, mma, a->training ? SEQ_ENC_FWD_TRAIN : SEQ_ENC_FWD)) return seq_enc_fwd(a, s);
   if (a->y && a->h1 && a->out && use_fwd_tc(a->tc_scratch, M, H, a->nh, mma)) return tc_enc_fwd(a, s);
   if (a->phase != 2) {
-    if (int e = launch_pre_fwd(a->x, a->ln1_w, a->ln1_b, a->attn, a->q, a->k, a->v, nullptr, M, H, a->nh, 0, a->precision, s)) return e;
-    if (int e = blk_attn_fwd(a->q, a->k, a->v, a->ctx, a->lse, a->ids, a->B, a->L, H, a->nh, a->mask_mode, a->drop_attn, a->training, a->precision,
-                             nullptr, a->attn_scratch, s))
-      return e;
+    if (use_attn_fused(a->L, H, a->nh, mma, false)) {
+      if (int e = launch_pre_attn_fwd(a->x, a->ln1_w, a->ln1_b, a->attn, a->q, a->k, a->v, nullptr, a->ctx, a->lse, a->ids, a->B, a->L, a->nh, 0,
+                                      a->mask_mode, a->drop_attn, a->training, s))
+        return e;
+    } else {
+      if (int e = launch_pre_fwd(a->x, a->ln1_w, a->ln1_b, a->attn, a->q, a->k, a->v, nullptr, M, H, a->nh, 0, a->precision, s)) return e;
+      if (int e = blk_attn_fwd(a->q, a->k, a->v, a->ctx, a->lse, a->ids, a->B, a->L, H, a->nh, a->mask_mode, a->drop_attn, a->training,
+                               a->precision, nullptr, a->attn_scratch, s))
+        return e;
+    }
     if (a->phase == 1) return ADT_OK;
   }
   PostFwdArgs p;
@@ -1003,9 +1077,6 @@ extern "C" int adt_enc_block_bwd(const adt_enc_block_bwd_args* a, adt_stream_t s
     if (int e = hoisted_wgrad(hz + 2 * hu, H, H, hz + 3 * hu, H, H, M, a->g_ffn.w1, s)) return e;
     if (int e = hoisted_wgrad(hz + 4 * hu, H, H, hz + 5 * hu, H, H, M, a->g_attn.out_w, s)) return e;
   }
-  if (int e = blk_attn_bwd(a->q, a->k, a->v, a->ctx, a->dctx, a->lse, a->ids, a->dq, a->dk, a->dv, a->B, a->L, H, a->nh, a->mask_mode,
-                           a->drop_attn, a->precision, nullptr, a->attn_scratch, s))
-    return e;
   PreBwdArgs r;
   memset(&r, 0, sizeof(r));
   r.dq = a->dq; r.dk = a->dk; r.dv = a->dv; r.x = a->x; r.dnorm_extra = a->dy; r.dx_extra = a->dx_extra;
@@ -1013,6 +1084,11 @@ extern "C" int adt_enc_block_bwd(const adt_enc_block_bwd_args* a, adt_stream_t s
   r.gWin = a->g_attn.in_w; r.gbin = a->g_attn.in_b; r.gln_g = a->g_ln1_w; r.gln_b = a->g_ln1_b;
   r.M = M; r.H = H; r.qscale = 1.0f / sqrtf((float)(H / a->nh)); r.kv_from_norm = 0;
   r.hoist = hz;
+  if (use_attn_fused(a->L, H, a->nh, mma, true))
+    return launch_attn_pre_bwd(r, a->q, a->k, a->v, a->dctx, a->lse, a->ids, a->B, a->L, a->nh, a->mask_mode, a->drop_attn, s);
+  if (int e = blk_attn_bwd(a->q, a->k, a->v, a->ctx, a->dctx, a->lse, a->ids, a->dq, a->dk, a->dv, a->B, a->L, H, a->nh, a->mask_mode,
+                           a->drop_attn, a->precision, nullptr, a->attn_scratch, s))
+    return e;
   if (int e = launch_pre_bwd(r, mma, s)) return e;
   if (hz) {   // Wq from LN(x), [Wk; Wv] from x
     if (int e = hoisted_wgrad(hz, 3 * H, H, hz + 3 * hu, H, H, M, a->g_attn.in_w, s)) return e;
@@ -1030,31 +1106,41 @@ extern "C" int adt_dec_block_fwd(const adt_dec_block_fwd_args* a, adt_stream_t s
   if (use_seq(a->L, H, a->nh, mma, SEQ_DEC_FWD)) return seq_dec_fwd(a, s);
   if (a->d && a->a && a->c && a->h1 && use_fwd_tc(a->tc_scratch, M, H, a->nh, mma)) return tc_dec_fwd(a, s);
   if (a->phase != 2) {
-    if (int e = launch_pre_fwd(a->x, a->ln_w, a->ln_b, a->slf, a->q1, a->k1, a->v1, a->d, M, H, a->nh, 1, a->precision, s)) return e;
-    if (int e = blk_attn_fwd(a->q1, a->k1, a->v1, a->ctx1, a->lse1, a->ids, a->B, a->L, H, a->nh, a->mask_mode, a->drop_slf, a->training, a->precision,
-                             nullptr, a->attn_scratch, s))
-      return e;
+    if (use_attn_fused(a->L, H, a->nh, mma, false)) {
+      if (int e = launch_pre_attn_fwd(a->x, a->ln_w, a->ln_b, a->slf, a->q1, a->k1, a->v1, a->d, a->ctx1, a->lse1, a->ids, a->B, a->L, a->nh, 1,
+                                      a->mask_mode, a->drop_slf, a->training, s))
+        return e;
+    } else {
+      if (int e = launch_pre_fwd(a->x, a->ln_w, a->ln_b, a->slf, a->q1, a->k1, a->v1, a->d, M, H, a->nh, 1, a->precision, s)) return e;
+      if (int e = blk_attn_fwd(a->q1, a->k1, a->v1, a->ctx1, a->lse1, a->ids, a->B, a->L, H, a->nh, a->mask_mode, a->drop_slf, a->training,
+                               a->precision, nullptr, a->attn_scratch, s))
+        return e;
+    }
     if (a->phase == 1) return ADT_OK;
   }
   size_t smem;
   int tm = pick_tm(3 * (size_t)(H + pad), &smem);
   if (!tm) return fail(ADT_E_SHAPE, "%s", "mid_fwd: tile does not fit shared memory");
   const float qscale = 1.0f / sqrtf((float)(H / a->nh));
-  if (use_row_small(H, mma)) {
-    const size_t sm = MidFwdSmallSmem::TOTAL_BYTES;
-    cudaFuncSetAttribute(mid_fwd_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-    TIMED("mid_fwd", s);
-    mid_fwd_small_kernel<<<(M + 63) / 64, AS_NT, sm, s>>>(a->ctx1, a->feats, a->slf.out_w, a->slf.out_b, a->enc.in_w, a->enc.in_b, a->a,
-                                                        a->q2, a->k2, a->v2, M, qscale);
+  if (use_attn_fused(a->L, H, a->nh, mma, false)) {
+    if (int e = launch_mid_attn_fwd(a, qscale, s)) return e;
   } else {
-    TIMED("mid_fwd", s);
-    LAUNCH_TM(tm, mma, mid_fwd_kernel, (M + tm - 1) / tm, smem, s, a->ctx1, a->feats, a->slf.out_w, a->slf.out_b, a->enc.in_w, a->enc.in_b, a->a,
-              a->q2, a->k2, a->v2, M, H, qscale);
+    if (use_row_small(H, mma)) {
+      const size_t sm = MidFwdSmallSmem::TOTAL_BYTES;
+      cudaFuncSetAttribute(mid_fwd_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+      TIMED("mid_fwd", s);
+      mid_fwd_small_kernel<<<(M + 63) / 64, AS_NT, sm, s>>>(a->ctx1, a->feats, a->slf.out_w, a->slf.out_b, a->enc.in_w, a->enc.in_b, a->a,
+                                                          a->q2, a->k2, a->v2, M, qscale);
+    } else {
+      TIMED("mid_fwd", s);
+      LAUNCH_TM(tm, mma, mid_fwd_kernel, (M + tm - 1) / tm, smem, s, a->ctx1, a->feats, a->slf.out_w, a->slf.out_b, a->enc.in_w, a->enc.in_b, a->a,
+                a->q2, a->k2, a->v2, M, H, qscale);
+    }
+    if (int e = check_launch("mid_fwd")) return e;
+    if (int e = blk_attn_fwd(a->q2, a->k2, a->v2, a->ctx2, a->lse2, a->ids, a->B, a->L, H, a->nh, a->mask_mode, a->drop_enc, a->training, a->precision,
+                             nullptr, a->attn_scratch, s))
+      return e;
   }
-  if (int e = check_launch("mid_fwd")) return e;
-  if (int e = blk_attn_fwd(a->q2, a->k2, a->v2, a->ctx2, a->lse2, a->ids, a->B, a->L, H, a->nh, a->mask_mode, a->drop_enc, a->training, a->precision,
-                           nullptr, a->attn_scratch, s))
-    return e;
   PostFwdArgs p;
   memset(&p, 0, sizeof(p));
   p.ctx = a->ctx2; p.resid = a->d; p.ids = a->ids; p.Wo = a->enc.out_w; p.bo = a->enc.out_b;
@@ -1140,9 +1226,6 @@ extern "C" int adt_dec_block_bwd(const adt_dec_block_bwd_args* a, adt_stream_t s
   }
   if (a->phase == 2) return ADT_OK;
   }
-  if (int e = blk_attn_bwd(a->q1, a->k1, a->v1, a->ctx1, a->dctx, a->lse1, a->ids, a->dq, a->dk, a->dv, a->B, a->L, H, a->nh, a->mask_mode,
-                           a->drop_slf, a->precision, nullptr, a->attn_scratch, s))
-    return e;
   PreBwdArgs r;
   memset(&r, 0, sizeof(r));
   r.dq = a->dq; r.dk = a->dk; r.dv = a->dv; r.x = a->x; r.dnorm_extra = a->dd; r.dx_extra = nullptr;
@@ -1150,6 +1233,11 @@ extern "C" int adt_dec_block_bwd(const adt_dec_block_bwd_args* a, adt_stream_t s
   r.gWin = a->g_slf.in_w; r.gbin = a->g_slf.in_b; r.gln_g = a->g_ln_w; r.gln_b = a->g_ln_b;
   r.M = M; r.H = H; r.qscale = qscale; r.kv_from_norm = 1;
   r.hoist = hz;
+  if (use_attn_fused(a->L, H, a->nh, mma, true))
+    return launch_attn_pre_bwd(r, a->q1, a->k1, a->v1, a->dctx, a->lse1, a->ids, a->B, a->L, a->nh, a->mask_mode, a->drop_slf, s);
+  if (int e = blk_attn_bwd(a->q1, a->k1, a->v1, a->ctx1, a->dctx, a->lse1, a->ids, a->dq, a->dk, a->dv, a->B, a->L, H, a->nh, a->mask_mode,
+                           a->drop_slf, a->precision, nullptr, a->attn_scratch, s))
+    return e;
   if (int e = launch_pre_bwd(r, mma, s)) return e;
   if (hz) {   // q, k and v all read d = LN(x): one [3H x H] product
     if (int e = hoisted_wgrad(hz, 3 * H, 3 * H, hz + 3 * hu, H, H, M, a->g_slf.in_w, s)) return e;

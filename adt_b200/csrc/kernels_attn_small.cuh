@@ -127,10 +127,9 @@ __device__ __forceinline__ void as_mma_frag(float (&out)[HD / 8][4], const float
 }
 
 // acc[nb] += A[16 rows r0..][0..HD) * Bn[8nb..][0..HD)^T with ldmatrix fragments (tiles [64][HD+8])
-template <int HD>
+template <int HD, int LD = HD + 8>
 __device__ __forceinline__ void as_mma_rows_lm(float (&acc)[8][4], const __nv_bfloat16* __restrict__ A, const __nv_bfloat16* __restrict__ Bn,
                                                int r0, int nbr) {
-  constexpr int LD = HD + 8;
 #pragma unroll
   for (int ks = 0; ks < HD / 16; ++ks) {
     uint32_t a[4];
@@ -145,10 +144,9 @@ __device__ __forceinline__ void as_mma_rows_lm(float (&acc)[8][4], const __nv_bf
     }
   }
 }
-// out[db] += P (fragments, k = key index j) * Bk[j][8db..]   with Bk a row-major [64][HD+8] tile (V or K), via transposing loads
-template <int HD>
+// out[db] += P (fragments, k = key index j) * Bk[j][8db..]   with Bk a row-major [64][LD] tile (V or K), via transposing loads
+template <int HD, int LD = HD + 8>
 __device__ __forceinline__ void as_mma_frag_lm(float (&out)[HD / 8][4], const float (&p)[8][4], const __nv_bfloat16* __restrict__ Bk, int nks) {
-  constexpr int LD = HD + 8;
 #pragma unroll
   for (int ks = 0; ks < 4; ++ks) {
     if (ks < nks) {
@@ -209,30 +207,21 @@ __device__ __forceinline__ void as_drop_all(AsDrop& o, const DropDesc& d, unsign
   }
 }
 
-template <int HD>
-__global__ void __launch_bounds__(AS_NT) attn_small_fwd_kernel(const float* __restrict__ q, const float* __restrict__ k,
-                                                               const float* __restrict__ v, float* __restrict__ ctx,
-                                                               float* __restrict__ lse, const int* __restrict__ key_ids, int L, int H,
-                                                               int nh, int mask_mode, DropDesc drop) {
-  constexpr int LD = HD + 8;
-  __shared__ __align__(16) __nv_bfloat16 Qs[64 * LD], Ks[64 * LD], Vs[64 * LD];
-  const int bh = blockIdx.x, b = bh / nh, h = bh - b * nh;
-  const long long seq_off = (long long)b * L * H + (long long)h * HD;
-  {   // rows >= L are written as zeros by the loader (every row of the 64-row tiles is covered)
-    const float* const src[3] = {q + seq_off, k + seq_off, v + seq_off};
-    __nv_bfloat16* const dst[3] = {Qs, Ks, Vs};
-    __nv_bfloat16* const dstT[3] = {nullptr, nullptr, nullptr};
-    as_load<HD, 3>(src, H, L, dst, dstT);
-  }
-  __syncthreads();
-  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
+// Forward of one head for the 16 query rows 16w .. 16w+15 of the sequence (w = 0..3: the warp's index in its group of four).  Qs, Ks,
+// Vs: bf16 tiles of all 64 rows with row stride LD halfwords, offset to the head's first column; rows >= L hold zeros.  ctx points at
+// the head's first column of the sequence's first row (row stride H), lse (nullable) at the (sequence, head) slice of [B][nh][L], and
+// rb = drop.base + (b nh + h) L is the Philox row counter of query row 0.
+template <int HD, int LD>
+__device__ __forceinline__ void as_fwd_head(const __nv_bfloat16* Qs, const __nv_bfloat16* Ks, const __nv_bfloat16* Vs, int w, int L, int H,
+                                            int mask_mode, const int* __restrict__ kid, float* __restrict__ ctx, float* __restrict__ lse,
+                                            const DropDesc& drop, unsigned long long rb) {
+  const int lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
   const int i0 = 16 * w + g, i1 = i0 + 8;
   const int nbr = (L + 7) >> 3, nks = (L + 15) >> 4;
-  const int* kid = key_ids + (long long)b * L;
   float s[8][4];
 #pragma unroll
   for (int nb = 0; nb < 8; ++nb) s[nb][0] = s[nb][1] = s[nb][2] = s[nb][3] = 0.f;
-  as_mma_rows_lm<HD>(s, Qs, Ks, 16 * w, nbr);
+  as_mma_rows_lm<HD, LD>(s, Qs, Ks, 16 * w, nbr);
   float mx0 = -INFINITY, mx1 = -INFINITY;
 #pragma unroll
   for (int nb = 0; nb < 8; ++nb) {
@@ -263,11 +252,10 @@ __global__ void __launch_bounds__(AS_NT) attn_small_fwd_kernel(const float* __re
   const bool v0 = i0 < L, v1 = i1 < L;
   const float inv0 = v0 ? 1.0f / sum0 : 0.f, inv1 = v1 ? 1.0f / sum1 : 0.f;
   if (lse && t == 0) {
-    if (v0) lse[((long long)b * nh + h) * L + i0] = mx0 + logf(sum0);
-    if (v1) lse[((long long)b * nh + h) * L + i1] = mx1 + logf(sum1);
+    if (v0) lse[i0] = mx0 + logf(sum0);
+    if (v1) lse[i1] = mx1 + logf(sum1);
   }
   const int lp8 = ((L + 7) & ~7) >> 3;
-  const unsigned long long rb = drop.base + ((unsigned long long)b * nh + h) * L;
   if (drop.enabled) {
     AsDrop dm;
     as_drop_all(dm, drop, rb + i0, rb + i1, v0, v1, lp8, nbr, t);
@@ -285,12 +273,32 @@ __global__ void __launch_bounds__(AS_NT) attn_small_fwd_kernel(const float* __re
   float o[HD / 8][4];
 #pragma unroll
   for (int db = 0; db < HD / 8; ++db) o[db][0] = o[db][1] = o[db][2] = o[db][3] = 0.f;
-  as_mma_frag_lm<HD>(o, s, Vs, nks);
+  as_mma_frag_lm<HD, LD>(o, s, Vs, nks);
 #pragma unroll
   for (int db = 0; db < HD / 8; ++db) {
-    if (v0) *reinterpret_cast<float2*>(ctx + seq_off + (long long)i0 * H + 8 * db + 2 * t) = make_float2(o[db][0], o[db][1]);
-    if (v1) *reinterpret_cast<float2*>(ctx + seq_off + (long long)i1 * H + 8 * db + 2 * t) = make_float2(o[db][2], o[db][3]);
+    if (v0) *reinterpret_cast<float2*>(ctx + (long long)i0 * H + 8 * db + 2 * t) = make_float2(o[db][0], o[db][1]);
+    if (v1) *reinterpret_cast<float2*>(ctx + (long long)i1 * H + 8 * db + 2 * t) = make_float2(o[db][2], o[db][3]);
   }
+}
+
+template <int HD>
+__global__ void __launch_bounds__(AS_NT) attn_small_fwd_kernel(const float* __restrict__ q, const float* __restrict__ k,
+                                                               const float* __restrict__ v, float* __restrict__ ctx,
+                                                               float* __restrict__ lse, const int* __restrict__ key_ids, int L, int H,
+                                                               int nh, int mask_mode, DropDesc drop) {
+  constexpr int LD = HD + 8;
+  __shared__ __align__(16) __nv_bfloat16 Qs[64 * LD], Ks[64 * LD], Vs[64 * LD];
+  const int bh = blockIdx.x, b = bh / nh, h = bh - b * nh;
+  const long long seq_off = (long long)b * L * H + (long long)h * HD;
+  {   // rows >= L are written as zeros by the loader (every row of the 64-row tiles is covered)
+    const float* const src[3] = {q + seq_off, k + seq_off, v + seq_off};
+    __nv_bfloat16* const dst[3] = {Qs, Ks, Vs};
+    __nv_bfloat16* const dstT[3] = {nullptr, nullptr, nullptr};
+    as_load<HD, 3>(src, H, L, dst, dstT);
+  }
+  __syncthreads();
+  as_fwd_head<HD, LD>(Qs, Ks, Vs, threadIdx.x >> 5, L, H, mask_mode, key_ids + (long long)b * L, ctx + seq_off,
+                      lse ? lse + ((long long)b * nh + h) * L : nullptr, drop, drop.base + ((unsigned long long)b * nh + h) * L);
 }
 
 // shared memory of the backward kernel (halfwords)
@@ -301,47 +309,28 @@ struct AsBwdSmem {
   static constexpr int TOTAL = 4 * ROW + 2 * SQ;              // Q, K, V, dC [64][HD+8] | dS, P~ [64][72]   (all row-major)
 };
 
-template <int HD>
-__global__ void __launch_bounds__(AS_NT) attn_small_bwd_kernel(const float* __restrict__ q, const float* __restrict__ k,
-                                                               const float* __restrict__ v, const float* __restrict__ dctx,
-                                                               const float* __restrict__ lse, const int* __restrict__ key_ids,
-                                                               float* __restrict__ dq, float* __restrict__ dk, float* __restrict__ dv,
-                                                               int L, int H, int nh, int mask_mode, DropDesc drop) {
-  using SM = AsBwdSmem<HD>;
-  constexpr int LD = SM::LD;
-  extern __shared__ __align__(16) uint8_t as_raw[];
-  __nv_bfloat16* Qs = reinterpret_cast<__nv_bfloat16*>(as_raw);
-  __nv_bfloat16* Ks = Qs + SM::ROW;
-  __nv_bfloat16* Vs = Ks + SM::ROW;
-  __nv_bfloat16* dCs = Vs + SM::ROW;
-  __nv_bfloat16* dSt = dCs + SM::ROW;        // dS[i][j], row-major
-  __nv_bfloat16* Pt = dSt + SM::SQ;          // P~[i][j], row-major
-  const int bh = blockIdx.x, b = bh / nh, h = bh - b * nh;
-  const long long seq_off = (long long)b * L * H + (long long)h * HD;
-  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
+// Backward of one head for the warp's 16 rows 16w .. 16w+15 (w = 0..3 within its group of four warps): query rows for dq, key rows
+// for dk and dv.  Qs, Ks, Vs, dCs: bf16 tiles with row stride LD, offset to the head's columns, zero in rows >= L; dSt, Pt: the group's
+// [64][72] scratch tiles.  ls0 / ls1: lse of query rows i0 / i1.  store(which, o) receives dq (0), dk (1), dv (2) of the warp's rows on
+// accumulator fragments; sync() is a barrier over the group's warps, between the query-side and the key-side products (the key-side
+// products read dS and P~ rows of every warp; after it Ks and Vs are no longer read).
+template <int HD, int LD, class Store, class Sync>
+__device__ __forceinline__ void as_bwd_head(const __nv_bfloat16* Qs, const __nv_bfloat16* Ks, const __nv_bfloat16* Vs, const __nv_bfloat16* dCs,
+                                            __nv_bfloat16* dSt, __nv_bfloat16* Pt, int w, int L, int mask_mode, const int* __restrict__ kid,
+                                            float ls0, float ls1, const DropDesc& drop, unsigned long long rb, Store&& store, Sync&& sync) {
+  const int lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
   const int i0 = 16 * w + g, i1 = i0 + 8;
   const bool v0 = i0 < L, v1 = i1 < L;
-  const float ls0 = v0 ? lse[((long long)b * nh + h) * L + i0] : 0.f;     // issued early: consumed after the first product
-  const float ls1 = v1 ? lse[((long long)b * nh + h) * L + i1] : 0.f;
-  {
-    const float* const src[4] = {q + seq_off, k + seq_off, v + seq_off, dctx + seq_off};
-    __nv_bfloat16* const dst[4] = {Qs, Ks, Vs, dCs};
-    __nv_bfloat16* const dstT[4] = {nullptr, nullptr, nullptr, nullptr};
-    as_load<HD, 4>(src, H, L, dst, dstT);
-  }
-  __syncthreads();
   const int nbr = (L + 7) >> 3, nks = (L + 15) >> 4;
-  const int* kid = key_ids + (long long)b * L;
   float p[8][4], dp[8][4];
 #pragma unroll
   for (int nb = 0; nb < 8; ++nb) {
     p[nb][0] = p[nb][1] = p[nb][2] = p[nb][3] = 0.f;
     dp[nb][0] = dp[nb][1] = dp[nb][2] = dp[nb][3] = 0.f;
   }
-  as_mma_rows_lm<HD>(p, Qs, Ks, 16 * w, nbr);       // S = q k^T
-  as_mma_rows_lm<HD>(dp, dCs, Vs, 16 * w, nbr);     // dP~ = dctx v^T
+  as_mma_rows_lm<HD, LD>(p, Qs, Ks, 16 * w, nbr);       // S = q k^T
+  as_mma_rows_lm<HD, LD>(dp, dCs, Vs, 16 * w, nbr);     // dP~ = dctx v^T
   const int lp8 = ((L + 7) & ~7) >> 3;
-  const unsigned long long rb = drop.base + ((unsigned long long)b * nh + h) * L;
   float dl0 = 0.f, dl1 = 0.f;
   float pt[8][4];                                // P~ = dropout(P)
   AsDrop dm;
@@ -390,20 +379,15 @@ __global__ void __launch_bounds__(AS_NT) attn_small_bwd_kernel(const float* __re
     float o[HD / 8][4];
 #pragma unroll
     for (int db = 0; db < HD / 8; ++db) o[db][0] = o[db][1] = o[db][2] = o[db][3] = 0.f;
-    as_mma_frag_lm<HD>(o, dp, Ks, nks);
-#pragma unroll
-    for (int db = 0; db < HD / 8; ++db) {
-      if (v0) *reinterpret_cast<float2*>(dq + seq_off + (long long)i0 * H + 8 * db + 2 * t) = make_float2(o[db][0], o[db][1]);
-      if (v1) *reinterpret_cast<float2*>(dq + seq_off + (long long)i1 * H + 8 * db + 2 * t) = make_float2(o[db][2], o[db][3]);
-    }
+    as_mma_frag_lm<HD, LD>(o, dp, Ks, nks);
+    store(0, o);
   }
-  __syncthreads();
-  // dk = dS^T q ; dv = P~^T dctx   (this warp owns key rows 16w .. 16w+15; plain stores: the CTA owns the whole head)
+  sync();
+  // dk = dS^T q ; dv = P~^T dctx   (this warp owns key rows 16w .. 16w+15)
 #pragma unroll
   for (int which = 0; which < 2; ++which) {
     const __nv_bfloat16* A = which == 0 ? dSt : Pt;       // [i][j]: used transposed, A[m = j][k = i]
     const __nv_bfloat16* Bk = which == 0 ? Qs : dCs;      // [i][d]: B[k = i][n = d]
-    float* out = which == 0 ? dk : dv;
     float o[HD / 8][4];
 #pragma unroll
     for (int db = 0; db < HD / 8; ++db) o[db][0] = o[db][1] = o[db][2] = o[db][3] = 0.f;
@@ -420,12 +404,51 @@ __global__ void __launch_bounds__(AS_NT) attn_small_bwd_kernel(const float* __re
         }
       }
     }
-#pragma unroll
-    for (int db = 0; db < HD / 8; ++db) {
-      if (v0) *reinterpret_cast<float2*>(out + seq_off + (long long)i0 * H + 8 * db + 2 * t) = make_float2(o[db][0], o[db][1]);
-      if (v1) *reinterpret_cast<float2*>(out + seq_off + (long long)i1 * H + 8 * db + 2 * t) = make_float2(o[db][2], o[db][3]);
-    }
+    store(1 + which, o);
   }
+}
+
+template <int HD>
+__global__ void __launch_bounds__(AS_NT) attn_small_bwd_kernel(const float* __restrict__ q, const float* __restrict__ k,
+                                                               const float* __restrict__ v, const float* __restrict__ dctx,
+                                                               const float* __restrict__ lse, const int* __restrict__ key_ids,
+                                                               float* __restrict__ dq, float* __restrict__ dk, float* __restrict__ dv,
+                                                               int L, int H, int nh, int mask_mode, DropDesc drop) {
+  using SM = AsBwdSmem<HD>;
+  constexpr int LD = SM::LD;
+  extern __shared__ __align__(16) uint8_t as_raw[];
+  __nv_bfloat16* Qs = reinterpret_cast<__nv_bfloat16*>(as_raw);
+  __nv_bfloat16* Ks = Qs + SM::ROW;
+  __nv_bfloat16* Vs = Ks + SM::ROW;
+  __nv_bfloat16* dCs = Vs + SM::ROW;
+  __nv_bfloat16* dSt = dCs + SM::ROW;        // dS[i][j], row-major
+  __nv_bfloat16* Pt = dSt + SM::SQ;          // P~[i][j], row-major
+  const int bh = blockIdx.x, b = bh / nh, h = bh - b * nh;
+  const long long seq_off = (long long)b * L * H + (long long)h * HD;
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
+  const int i0 = 16 * w + g, i1 = i0 + 8;
+  const bool v0 = i0 < L, v1 = i1 < L;
+  const float ls0 = v0 ? lse[((long long)b * nh + h) * L + i0] : 0.f;     // issued early: consumed after the first product
+  const float ls1 = v1 ? lse[((long long)b * nh + h) * L + i1] : 0.f;
+  {
+    const float* const src[4] = {q + seq_off, k + seq_off, v + seq_off, dctx + seq_off};
+    __nv_bfloat16* const dst[4] = {Qs, Ks, Vs, dCs};
+    __nv_bfloat16* const dstT[4] = {nullptr, nullptr, nullptr, nullptr};
+    as_load<HD, 4>(src, H, L, dst, dstT);
+  }
+  __syncthreads();
+  // plain stores: the CTA owns the whole head
+  as_bwd_head<HD, LD>(Qs, Ks, Vs, dCs, dSt, Pt, w, L, mask_mode, key_ids + (long long)b * L, ls0, ls1, drop,
+                      drop.base + ((unsigned long long)b * nh + h) * L,
+                      [&](int which, const float (&o)[HD / 8][4]) {
+                        float* out = which == 0 ? dq : which == 1 ? dk : dv;
+#pragma unroll
+                        for (int db = 0; db < HD / 8; ++db) {
+                          if (v0) *reinterpret_cast<float2*>(out + seq_off + (long long)i0 * H + 8 * db + 2 * t) = make_float2(o[db][0], o[db][1]);
+                          if (v1) *reinterpret_cast<float2*>(out + seq_off + (long long)i1 * H + 8 * db + 2 * t) = make_float2(o[db][2], o[db][3]);
+                        }
+                      },
+                      [] { __syncthreads(); });
 }
 
 }  // namespace adt

@@ -190,6 +190,44 @@ struct PreFwdSmallSmem {
   static constexpr size_t TOTAL_BYTES = XF_BYTES + (size_t)64 * RS_LF * 4;
 };
 
+// LayerNorm of the fp32 tile Xf (rows >= rows: zero in Nb) into the bf16 tile Nb and, when norm_out is given, to global rows row0 ..;
+// two threads per row (threads 0 .. 127), two-pass statistics
+__device__ __forceinline__ void rs_ln_tile(const float* __restrict__ Xf, const float* __restrict__ ln_g, const float* __restrict__ ln_b,
+                                           __nv_bfloat16* __restrict__ Nb, float* __restrict__ norm_out, long long row0, int rows) {
+  const int r = threadIdx.x >> 1, half = threadIdx.x & 1;
+  const float* xr = Xf + r * RS_LF + 32 * half;
+  float s = 0.f;
+#pragma unroll
+  for (int c = 0; c < 32; c += 4) {
+    const float4 u = *reinterpret_cast<const float4*>(xr + c);
+    s += (u.x + u.y) + (u.z + u.w);
+  }
+  s += __shfl_xor_sync(0xffffffffu, s, 1);
+  const float mean = s * (1.0f / RS_H);
+  float qq = 0.f;
+#pragma unroll
+  for (int c = 0; c < 32; c += 4) {
+    const float4 u = *reinterpret_cast<const float4*>(xr + c);
+    const float a = u.x - mean, b = u.y - mean, cc = u.z - mean, d = u.w - mean;
+    qq += (a * a + b * b) + (cc * cc + d * d);
+  }
+  qq += __shfl_xor_sync(0xffffffffu, qq, 1);
+  const float rstd = 1.0f / sqrtf(qq * (1.0f / RS_H) + 1e-8f);
+  const bool ok = r < rows;
+#pragma unroll
+  for (int c = 0; c < 32; c += 4) {
+    const int col = 32 * half + c;
+    const float4 u = *reinterpret_cast<const float4*>(xr + c);
+    const float4 ga = __ldg(reinterpret_cast<const float4*>(ln_g + col)), be = __ldg(reinterpret_cast<const float4*>(ln_b + col));
+    const float4 n = make_float4((u.x - mean) * rstd * ga.x + be.x, (u.y - mean) * rstd * ga.y + be.y, (u.z - mean) * rstd * ga.z + be.z,
+                                 (u.w - mean) * rstd * ga.w + be.w);
+    uint32_t* d = reinterpret_cast<uint32_t*>(Nb + r * RS_LD + col);
+    d[0] = ok ? pack_bf16(n.x, n.y) : 0u;
+    d[1] = ok ? pack_bf16(n.z, n.w) : 0u;
+    if (norm_out && ok) *reinterpret_cast<float4*>(norm_out + (long long)(row0 + r) * RS_H + col) = n;
+  }
+}
+
 __global__ void __launch_bounds__(AS_NT) pre_fwd_small_kernel(const float* __restrict__ x, const float* __restrict__ ln_g,
                                                               const float* __restrict__ ln_b, const float* __restrict__ Win,
                                                               const float* __restrict__ bin, float* __restrict__ q, float* __restrict__ k,
@@ -227,40 +265,7 @@ __global__ void __launch_bounds__(AS_NT) pre_fwd_small_kernel(const float* __res
     rs_load<3>(src, ld, nr, sc, d, dT, dF);
   }
   __syncthreads();
-  {   // LayerNorm: two threads per row, two-pass statistics
-    const int r = threadIdx.x >> 1, half = threadIdx.x & 1;
-    const float* xr = Xf + r * RS_LF + 32 * half;
-    float s = 0.f;
-#pragma unroll
-    for (int c = 0; c < 32; c += 4) {
-      const float4 u = *reinterpret_cast<const float4*>(xr + c);
-      s += (u.x + u.y) + (u.z + u.w);
-    }
-    s += __shfl_xor_sync(0xffffffffu, s, 1);
-    const float mean = s * (1.0f / RS_H);
-    float qq = 0.f;
-#pragma unroll
-    for (int c = 0; c < 32; c += 4) {
-      const float4 u = *reinterpret_cast<const float4*>(xr + c);
-      const float a = u.x - mean, b = u.y - mean, cc = u.z - mean, d = u.w - mean;
-      qq += (a * a + b * b) + (cc * cc + d * d);
-    }
-    qq += __shfl_xor_sync(0xffffffffu, qq, 1);
-    const float rstd = 1.0f / sqrtf(qq * (1.0f / RS_H) + 1e-8f);
-    const bool ok = r < rows;
-#pragma unroll
-    for (int c = 0; c < 32; c += 4) {
-      const int col = 32 * half + c;
-      const float4 u = *reinterpret_cast<const float4*>(xr + c);
-      const float4 ga = __ldg(reinterpret_cast<const float4*>(ln_g + col)), be = __ldg(reinterpret_cast<const float4*>(ln_b + col));
-      const float4 n = make_float4((u.x - mean) * rstd * ga.x + be.x, (u.y - mean) * rstd * ga.y + be.y, (u.z - mean) * rstd * ga.z + be.z,
-                                   (u.w - mean) * rstd * ga.w + be.w);
-      uint32_t* d = reinterpret_cast<uint32_t*>(Nb + r * RS_LD + col);
-      d[0] = ok ? pack_bf16(n.x, n.y) : 0u;
-      d[1] = ok ? pack_bf16(n.z, n.w) : 0u;
-      if (norm_out && ok) *reinterpret_cast<float4*>(norm_out + (long long)(row0 + r) * RS_H + col) = n;
-    }
-  }
+  rs_ln_tile(Xf, ln_g, ln_b, Nb, norm_out, row0, rows);
   __syncthreads();
   const __nv_bfloat16* Akv = kv_from_norm ? Nb : Xb;
 #pragma unroll 1
@@ -830,45 +835,17 @@ struct PreBwdSmall2Smem {
   static constexpr size_t TOTAL_BYTES = (size_t)(N + RS_TILE) * 2;
 };
 
-__global__ void __launch_bounds__(RS_BWD_NT, 2) pre_bwd_small2_kernel(PreBwdArgs p) {
-  using SM = PreBwdSmall2Smem;
-  extern __shared__ __align__(16) uint8_t rs_raw[];
-  __nv_bfloat16* hb = reinterpret_cast<__nv_bfloat16*>(rs_raw);
-  __nv_bfloat16* Wt = hb + SM::W;
-  __nv_bfloat16* Tq = hb + SM::TQ;
-  __nv_bfloat16* Tk = hb + SM::TK;
-  __nv_bfloat16* Tv = hb + SM::TV;
-  __nv_bfloat16* Xb = hb + SM::X;
-  __nv_bfloat16* Nb = hb + SM::N;
-  const int row0 = blockIdx.x * 64;
-  const int rows = min(64, p.M - row0);
-  const long long g0 = (long long)row0 * RS_H;
+// Everything of pre_bwd_small2_kernel after its prologue, for all 256 threads: the bf16 tiles Tq (dq scaled by qscale), Tk, Tv (zero in
+// rows >= rows) and the weights Wt are in shared memory; Xb and Nb are free tiles (x and LN(x) are staged there).  Xf: the block input
+// at the fragment positions of chain warps 0-3 (frag_load of p.x), loaded by the caller so that its latency can hide behind a barrier.
+__device__ __forceinline__ void pre_bwd_small_tail(const PreBwdArgs& p, const float (&Xf)[8][4], const __nv_bfloat16* Wt, const __nv_bfloat16* Tq,
+                                                   const __nv_bfloat16* Tk, const __nv_bfloat16* Tv, __nv_bfloat16* Xb, __nv_bfloat16* Nb,
+                                                   long long row0, int rows) {
+  const long long g0 = row0 * RS_H;
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
   const int i0 = 16 * w + g, i1 = i0 + 8;
   const bool v0 = i0 < rows, v1 = i1 < rows;
-  {
-    const float* const src[3] = {p.dq + g0, p.dk + g0, p.dv + g0};
-    const long long ld[3] = {RS_H, RS_H, RS_H};
-    const int nr[3] = {rows, rows, rows};
-    const float sc[3] = {p.qscale, 1.f, 1.f};
-    __nv_bfloat16* const d[3] = {Tq, Tk, Tv};
-    __nv_bfloat16* const dT[3] = {nullptr, nullptr, nullptr};
-    float* const dF[3] = {nullptr, nullptr, nullptr};
-    rs_load<3, RS_BWD_NT>(src, ld, nr, sc, d, dT, dF);
-  }
-  {
-    const float* const src[3] = {p.Win, p.Win + RS_H * RS_H, p.Win + 2 * RS_H * RS_H};
-    const long long ld[3] = {RS_H, RS_H, RS_H};
-    const int nr[3] = {64, 64, 64};
-    const float sc[3] = {1.f, 1.f, 1.f};
-    __nv_bfloat16* const d[3] = {Wt, Wt + RS_TILE, Wt + 2 * RS_TILE};
-    __nv_bfloat16* const dT[3] = {nullptr, nullptr, nullptr};
-    float* const dF[3] = {nullptr, nullptr, nullptr};
-    rs_load<3, RS_BWD_NT>(src, ld, nr, sc, d, dT, dF);
-  }
-  float Xf[8][4];
   if (w < 4) {
-    frag_load(Xf, p.x + g0, i0, i1, v0, v1, t);
     float Nf[8][4];
 #pragma unroll
     for (int nb = 0; nb < 8; ++nb) { Nf[nb][0] = Xf[nb][0]; Nf[nb][1] = Xf[nb][1]; Nf[nb][2] = Xf[nb][2]; Nf[nb][3] = Xf[nb][3]; }
@@ -912,6 +889,47 @@ __global__ void __launch_bounds__(RS_BWD_NT, 2) pre_bwd_small2_kernel(PreBwdArgs
     for (int nb = 0; nb < 8; ++nb) { D[nb][0] += E[nb][0]; D[nb][1] += E[nb][1]; D[nb][2] += E[nb][2]; D[nb][3] += E[nb][3]; }
   }
   frag_store(p.dx + g0, D, i0, i1, v0, v1, t);
+}
+
+__global__ void __launch_bounds__(RS_BWD_NT, 2) pre_bwd_small2_kernel(PreBwdArgs p) {
+  using SM = PreBwdSmall2Smem;
+  extern __shared__ __align__(16) uint8_t rs_raw[];
+  __nv_bfloat16* hb = reinterpret_cast<__nv_bfloat16*>(rs_raw);
+  __nv_bfloat16* Wt = hb + SM::W;
+  __nv_bfloat16* Tq = hb + SM::TQ;
+  __nv_bfloat16* Tk = hb + SM::TK;
+  __nv_bfloat16* Tv = hb + SM::TV;
+  __nv_bfloat16* Xb = hb + SM::X;
+  __nv_bfloat16* Nb = hb + SM::N;
+  const int row0 = blockIdx.x * 64;
+  const int rows = min(64, p.M - row0);
+  const long long g0 = (long long)row0 * RS_H;
+  {
+    const float* const src[3] = {p.dq + g0, p.dk + g0, p.dv + g0};
+    const long long ld[3] = {RS_H, RS_H, RS_H};
+    const int nr[3] = {rows, rows, rows};
+    const float sc[3] = {p.qscale, 1.f, 1.f};
+    __nv_bfloat16* const d[3] = {Tq, Tk, Tv};
+    __nv_bfloat16* const dT[3] = {nullptr, nullptr, nullptr};
+    float* const dF[3] = {nullptr, nullptr, nullptr};
+    rs_load<3, RS_BWD_NT>(src, ld, nr, sc, d, dT, dF);
+  }
+  {
+    const float* const src[3] = {p.Win, p.Win + RS_H * RS_H, p.Win + 2 * RS_H * RS_H};
+    const long long ld[3] = {RS_H, RS_H, RS_H};
+    const int nr[3] = {64, 64, 64};
+    const float sc[3] = {1.f, 1.f, 1.f};
+    __nv_bfloat16* const d[3] = {Wt, Wt + RS_TILE, Wt + 2 * RS_TILE};
+    __nv_bfloat16* const dT[3] = {nullptr, nullptr, nullptr};
+    float* const dF[3] = {nullptr, nullptr, nullptr};
+    rs_load<3, RS_BWD_NT>(src, ld, nr, sc, d, dT, dF);
+  }
+  float Xf[8][4];
+  {
+    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, i0 = 16 * w + (lane >> 2), i1 = i0 + 8;
+    if (w < 4) frag_load(Xf, p.x + g0, i0, i1, i0 < rows, i1 < rows, lane & 3);
+  }
+  pre_bwd_small_tail(p, Xf, Wt, Tq, Tk, Tv, Xb, Nb, row0, rows);
 }
 
 // -------------------------------------------------------------------------------------------------
@@ -1125,6 +1143,319 @@ __global__ void __launch_bounds__(RS_BWD_NT, 2) mid_bwd_small_kernel(MidBwdArgs 
     if (i0 < rows) *reinterpret_cast<float2*>(p.dctx1 + g0 + (long long)i0 * RS_H + c) = make_float2(D[nb][0], D[nb][1]);
     if (i1 < rows) *reinterpret_cast<float2*>(p.dctx1 + g0 + (long long)i1 * RS_H + c) = make_float2(D[nb][2], D[nb][3]);
   }
+}
+
+// -------------------------------------------------------------------------------------------------
+// Attention fused into the projection kernels, for sequences of 33 .. 64 positions: one 256-thread CTA per sequence, so the rows of
+// its tile are all the keys its queries see.  Warp group g (warps 4g .. 4g+3, 16 rows each) runs the attention of the heads in column
+// half g of the model (one head: group 0 alone); the per-head arithmetic is as_fwd_head / as_bwd_head, the body of the separate
+// kernels, so every row's results are those of the two-launch path.
+// -------------------------------------------------------------------------------------------------
+// Columns 32 grp .. 32 grp + 31 of one projection of the fused kernels below: acc (4 column blocks of this warp's rows i0 / i1) plus
+// bias, times sc -> fp32 rows of `out` below L and the bf16 tile T the attention reads (rows >= L: zero, as as_load writes them)
+__device__ __forceinline__ void rs_store_half(float* __restrict__ out, __nv_bfloat16* __restrict__ T, const float (&acc)[4][4],
+                                              const float* __restrict__ bias, float sc, int grp, int i0, int i1, int L, int t) {
+  const bool v0 = i0 < L, v1 = i1 < L;
+#pragma unroll
+  for (int nb = 0; nb < 4; ++nb) {
+    const int c = 32 * grp + 8 * nb + 2 * t;
+    const float2 bb = __ldg(reinterpret_cast<const float2*>(bias + c));
+    const float2 y0 = make_float2((acc[nb][0] + bb.x) * sc, (acc[nb][1] + bb.y) * sc);
+    const float2 y1 = make_float2((acc[nb][2] + bb.x) * sc, (acc[nb][3] + bb.y) * sc);
+    if (v0) *reinterpret_cast<float2*>(out + (long long)i0 * RS_H + c) = y0;
+    if (v1) *reinterpret_cast<float2*>(out + (long long)i1 * RS_H + c) = y1;
+    *reinterpret_cast<uint32_t*>(T + i0 * RS_LD + c) = v0 ? pack_bf16(y0.x, y0.y) : 0u;
+    *reinterpret_cast<uint32_t*>(T + i1 * RS_LD + c) = v1 ? pack_bf16(y1.x, y1.y) : 0u;
+  }
+}
+
+// acc[nb] += A[rows 16 wl ..][k] * W[32 grp + 8 nb ..][k]^T: column half grp of rs_fgemm, every column accumulated in rs_fgemm's order
+__device__ __forceinline__ void rs_fgemm_half(float (&acc)[4][4], const __nv_bfloat16* __restrict__ A, const __nv_bfloat16* __restrict__ W,
+                                              int wl, int grp) {
+#pragma unroll
+  for (int ks = 0; ks < 4; ++ks) {
+    uint32_t a[4];
+    frag_a(a, A, 16 * wl, 16 * ks);
+#pragma unroll
+    for (int nb = 0; nb < 4; ++nb) {
+      uint32_t b0, b1;
+      frag_b(b0, b1, W, 32 * grp + 8 * nb, 16 * ks);
+      mma16816(acc[nb], a, b0, b1);
+    }
+  }
+}
+
+// attention of the heads in column half grp (one head: group 0 alone) from the tiles Qs, Ks, Vs of sequence b (first row row0)
+template <int HD>
+__device__ __forceinline__ void rs_attn_half(const __nv_bfloat16* Qs, const __nv_bfloat16* Ks, const __nv_bfloat16* Vs, int grp, int wl, int b,
+                                             long long row0, int L, int mask_mode, const int* ids, float* ctx, float* lse, const DropDesc& drop) {
+  constexpr int NH = RS_H / HD, HPG = NH > 1 ? NH / 2 : 1;       // heads, heads per warp group
+  if (NH == 1 && grp == 1) return;
+#pragma unroll 1
+  for (int hh = 0; hh < HPG; ++hh) {
+    const int h = grp * HPG + hh, c0 = h * HD;
+    as_fwd_head<HD, RS_LD>(Qs + c0, Ks + c0, Vs + c0, wl, L, RS_H, mask_mode, ids + row0, ctx + row0 * RS_H + c0,
+                           lse ? lse + ((long long)b * NH + h) * L : nullptr, drop, drop.base + ((unsigned long long)b * NH + h) * L);
+  }
+}
+
+struct RsAttnFwdArgs {
+  const float* x; const float* ln_g; const float* ln_b; const float* Win; const float* bin;
+  float* q; float* k; float* v; float* norm_out;          // norm_out (nullable): LN(x), the decoder's residual d
+  float* ctx; float* lse; const int* ids;
+  int L, mask_mode, kv_from_norm; float qscale; DropDesc drop;
+};
+
+// pre_attn_fwd_small_kernel<HD> == pre_fwd_small_kernel + attn_small_fwd_kernel<HD>.  q, k, v are stored in fp32 (the backward reads
+// them) and, rounded once, as the bf16 tiles the attention reads: the values attn_small_fwd_kernel loads.
+struct PreAttnFwdSmem {
+  static constexpr int W = 0, X = 3 * RS_TILE, N = X + RS_TILE, Q = N + RS_TILE, K = Q + RS_TILE, V = K + RS_TILE, HALF_END = V + RS_TILE;
+  static constexpr size_t XF_BYTES = (size_t)HALF_END * 2;
+  static constexpr size_t TOTAL_BYTES = XF_BYTES + (size_t)64 * RS_LF * 4;
+};
+
+template <int HD>
+__global__ void __launch_bounds__(RS_BWD_NT, 2) pre_attn_fwd_small_kernel(RsAttnFwdArgs p) {
+  using SM = PreAttnFwdSmem;
+  extern __shared__ __align__(16) uint8_t rs_raw[];
+  __nv_bfloat16* hb = reinterpret_cast<__nv_bfloat16*>(rs_raw);
+  __nv_bfloat16* Wt = hb + SM::W;
+  __nv_bfloat16* Xb = hb + SM::X;
+  __nv_bfloat16* Nb = hb + SM::N;
+  __nv_bfloat16* Qs = hb + SM::Q;
+  __nv_bfloat16* Ks = hb + SM::K;
+  __nv_bfloat16* Vs = hb + SM::V;
+  float* Xf = reinterpret_cast<float*>(rs_raw + SM::XF_BYTES);
+  const int b = blockIdx.x, L = p.L;
+  const long long row0 = (long long)b * L;
+  const int w = threadIdx.x >> 5, grp = w >> 2, wl = w & 3, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
+  const int i0 = 16 * wl + g, i1 = i0 + 8;
+  {
+    const float* const src[1] = {p.x + row0 * RS_H};
+    const long long ld[1] = {RS_H};
+    const int nr[1] = {L};
+    const float sc[1] = {1.f};
+    __nv_bfloat16* const d[1] = {Xb};
+    __nv_bfloat16* const dT[1] = {nullptr};
+    float* const dF[1] = {Xf};
+    rs_load<1, RS_BWD_NT>(src, ld, nr, sc, d, dT, dF);
+  }
+  {
+    const float* const src[3] = {p.Win, p.Win + RS_H * RS_H, p.Win + 2 * RS_H * RS_H};
+    const long long ld[3] = {RS_H, RS_H, RS_H};
+    const int nr[3] = {64, 64, 64};
+    const float sc[3] = {1.f, 1.f, 1.f};
+    __nv_bfloat16* const d[3] = {Wt, Wt + RS_TILE, Wt + 2 * RS_TILE};
+    __nv_bfloat16* const dT[3] = {nullptr, nullptr, nullptr};
+    float* const dF[3] = {nullptr, nullptr, nullptr};
+    rs_load<3, RS_BWD_NT>(src, ld, nr, sc, d, dT, dF);
+  }
+  __syncthreads();
+  if (threadIdx.x < AS_NT) rs_ln_tile(Xf, p.ln_g, p.ln_b, Nb, p.norm_out, row0, L);
+  __syncthreads();
+  // packed in-projection, columns 32 grp .. 32 grp + 31 of q, k and v
+  const __nv_bfloat16* Akv = p.kv_from_norm ? Nb : Xb;
+#pragma unroll 1
+  for (int m = 0; m < 3; ++m) {
+    float acc[4][4];
+#pragma unroll
+    for (int nb = 0; nb < 4; ++nb) acc[nb][0] = acc[nb][1] = acc[nb][2] = acc[nb][3] = 0.f;
+    rs_fgemm_half(acc, m == 0 ? Nb : Akv, Wt + m * RS_TILE, wl, grp);
+    rs_store_half((m == 0 ? p.q : m == 1 ? p.k : p.v) + row0 * RS_H, m == 0 ? Qs : m == 1 ? Ks : Vs, acc, p.bin + m * RS_H,
+                  m == 0 ? p.qscale : 1.f, grp, i0, i1, L, t);
+  }
+  __syncthreads();
+  rs_attn_half<HD>(Qs, Ks, Vs, grp, wl, b, row0, L, p.mask_mode, p.ids, p.ctx, p.lse, p.drop);
+}
+
+// mid_attn_fwd_small_kernel<HD> == mid_fwd_small_kernel + attn_small_fwd_kernel<HD> (the decoder's cross attention).  Every warp
+// computes the self-attention out-projection a = ctx1 Wo1^T + bo1 of its 16 rows in full (both groups: a is the A operand of the q
+// projection and stays in fragments, as in mid_fwd_small_kernel); group g then computes column half g of q2, k2, v2 and the
+// attention of the heads in that half.
+struct RsMidAttnArgs {
+  const float* ctx1; const float* feats; const float* Wo1; const float* bo1; const float* Win2; const float* bin2;
+  float* a; float* q2; float* k2; float* v2; float* ctx2; float* lse2; const int* ids;
+  int L, mask_mode; float qscale; DropDesc drop;
+};
+struct MidAttnFwdSmem {
+  // Wo1, Wq2, Wk2, Wv2 | ctx1 | feats | q2 | k2 | v2
+  static constexpr int W = 0, C = 4 * RS_TILE, F = C + RS_TILE, Q = F + RS_TILE, K = Q + RS_TILE, V = K + RS_TILE;
+  static constexpr size_t TOTAL_BYTES = (size_t)(V + RS_TILE) * 2;
+};
+
+template <int HD>
+__global__ void __launch_bounds__(RS_BWD_NT, 2) mid_attn_fwd_small_kernel(RsMidAttnArgs p) {
+  using SM = MidAttnFwdSmem;
+  extern __shared__ __align__(16) uint8_t rs_raw[];
+  __nv_bfloat16* hb = reinterpret_cast<__nv_bfloat16*>(rs_raw);
+  __nv_bfloat16* Wt = hb + SM::W;
+  __nv_bfloat16* Cs = hb + SM::C;
+  __nv_bfloat16* Fs = hb + SM::F;
+  __nv_bfloat16* Qs = hb + SM::Q;
+  __nv_bfloat16* Ks = hb + SM::K;
+  __nv_bfloat16* Vs = hb + SM::V;
+  const int b = blockIdx.x, L = p.L;
+  const long long row0 = (long long)b * L, g0 = row0 * RS_H;
+  const int w = threadIdx.x >> 5, grp = w >> 2, wl = w & 3, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
+  const int i0 = 16 * wl + g, i1 = i0 + 8;
+  {
+    const float* const src[2] = {p.ctx1 + g0, p.feats + g0};
+    const long long ld[2] = {RS_H, RS_H};
+    const int nr[2] = {L, L};
+    const float sc[2] = {1.f, 1.f};
+    __nv_bfloat16* const d[2] = {Cs, Fs};
+    __nv_bfloat16* const dT[2] = {nullptr, nullptr};
+    float* const dF[2] = {nullptr, nullptr};
+    rs_load<2, RS_BWD_NT>(src, ld, nr, sc, d, dT, dF);
+  }
+  {
+    const float* const src[4] = {p.Wo1, p.Win2, p.Win2 + RS_H * RS_H, p.Win2 + 2 * RS_H * RS_H};
+    const long long ld[4] = {RS_H, RS_H, RS_H, RS_H};
+    const int nr[4] = {64, 64, 64, 64};
+    const float sc[4] = {1.f, 1.f, 1.f, 1.f};
+    __nv_bfloat16* const d[4] = {Wt, Wt + RS_TILE, Wt + 2 * RS_TILE, Wt + 3 * RS_TILE};
+    __nv_bfloat16* const dT[4] = {nullptr, nullptr, nullptr, nullptr};
+    float* const dF[4] = {nullptr, nullptr, nullptr, nullptr};
+    rs_load<4, RS_BWD_NT>(src, ld, nr, sc, d, dT, dF);
+  }
+  __syncthreads();
+  {
+    float acc[8][4];
+#pragma unroll
+    for (int nb = 0; nb < 8; ++nb) acc[nb][0] = acc[nb][1] = acc[nb][2] = acc[nb][3] = 0.f;
+    rs_fgemm(acc, Cs, Wt, 16 * wl);
+#pragma unroll
+    for (int nb = 0; nb < 8; ++nb) {
+      const int c = 8 * nb + 2 * t;
+      const float2 bb = __ldg(reinterpret_cast<const float2*>(p.bo1 + c));
+      acc[nb][0] += bb.x; acc[nb][1] += bb.y; acc[nb][2] += bb.x; acc[nb][3] += bb.y;
+      if (p.a && grp == 0) {
+        if (i0 < L) *reinterpret_cast<float2*>(p.a + g0 + (long long)i0 * RS_H + c) = make_float2(acc[nb][0], acc[nb][1]);
+        if (i1 < L) *reinterpret_cast<float2*>(p.a + g0 + (long long)i1 * RS_H + c) = make_float2(acc[nb][2], acc[nb][3]);
+      }
+    }
+    float o[4][4];     // q2 = (a Wq2^T + bq2) s, column half grp, with a taken from the fragments
+#pragma unroll
+    for (int nb = 0; nb < 4; ++nb) o[nb][0] = o[nb][1] = o[nb][2] = o[nb][3] = 0.f;
+#pragma unroll
+    for (int ks = 0; ks < 4; ++ks) {
+      uint32_t a[4];
+      a[0] = pack_bf16(acc[2 * ks][0], acc[2 * ks][1]);
+      a[1] = pack_bf16(acc[2 * ks][2], acc[2 * ks][3]);
+      a[2] = pack_bf16(acc[2 * ks + 1][0], acc[2 * ks + 1][1]);
+      a[3] = pack_bf16(acc[2 * ks + 1][2], acc[2 * ks + 1][3]);
+#pragma unroll
+      for (int nb = 0; nb < 4; ++nb) {
+        uint32_t b0, b1;
+        frag_b(b0, b1, Wt + RS_TILE, 32 * grp + 8 * nb, 16 * ks);
+        mma16816(o[nb], a, b0, b1);
+      }
+    }
+    rs_store_half(p.q2 + g0, Qs, o, p.bin2, p.qscale, grp, i0, i1, L, t);
+  }
+#pragma unroll 1
+  for (int m = 0; m < 2; ++m) {    // k2, v2 from the encoder features
+    float acc[4][4];
+#pragma unroll
+    for (int nb = 0; nb < 4; ++nb) acc[nb][0] = acc[nb][1] = acc[nb][2] = acc[nb][3] = 0.f;
+    rs_fgemm_half(acc, Fs, Wt + (2 + m) * RS_TILE, wl, grp);
+    rs_store_half((m == 0 ? p.k2 : p.v2) + g0, m == 0 ? Ks : Vs, acc, p.bin2 + (1 + m) * RS_H, 1.f, grp, i0, i1, L, t);
+  }
+  __syncthreads();
+  rs_attn_half<HD>(Qs, Ks, Vs, grp, wl, b, row0, L, p.mask_mode, p.ids, p.ctx2, p.lse2, p.drop);
+}
+
+// attn_pre_bwd_small_kernel<HD> == attn_small_bwd_kernel<HD> + pre_bwd_small2_kernel, for two or four heads (one head of 64 columns
+// needs 160 registers in the attention adjoint alone: that would cost the second CTA per SM).  dq (scaled by qscale), dk and dv go
+// from the accumulator fragments straight into the bf16 tiles pre_bwd_small2_kernel stages, rounded as it rounds them; the fp32 dq,
+// dk, dv buffers are not written.  The attention operands alias tiles that are dead by the time they are needed: dk and dv overwrite
+// k and v (read only before the group barrier inside as_bwd_head), LN(x) and x overwrite q and dctx after the attention.
+struct RsAttnBwdArgs {
+  PreBwdArgs pre;
+  const float* q; const float* k; const float* v; const float* dctx; const float* lse; const int* ids;
+  int L, mask_mode; DropDesc drop;
+};
+struct AttnPreBwdSmem {
+  // Wq, Wk, Wv | dq s | k -> dk | v -> dv | q -> LN(x) | dctx -> x | dS, P~ of group 0 | dS, P~ of group 1
+  static constexpr int W = 0, TQ = 3 * RS_TILE, TK = TQ + RS_TILE, TV = TK + RS_TILE, N = TV + RS_TILE, X = N + RS_TILE, S = X + RS_TILE;
+  static constexpr size_t TOTAL_BYTES = (size_t)(S + 4 * RS_TILE) * 2;
+};
+
+template <int HD>
+__global__ void __launch_bounds__(RS_BWD_NT, 2) attn_pre_bwd_small_kernel(RsAttnBwdArgs a) {
+  using SM = AttnPreBwdSmem;
+  constexpr int NH = RS_H / HD, HPG = NH / 2;
+  static_assert(NH == 2 || NH == 4, "one head per warp group or two");
+  extern __shared__ __align__(16) uint8_t rs_raw[];
+  __nv_bfloat16* hb = reinterpret_cast<__nv_bfloat16*>(rs_raw);
+  __nv_bfloat16* Wt = hb + SM::W;
+  __nv_bfloat16* Tq = hb + SM::TQ;
+  __nv_bfloat16* Tk = hb + SM::TK;
+  __nv_bfloat16* Tv = hb + SM::TV;
+  __nv_bfloat16* Nb = hb + SM::N;
+  __nv_bfloat16* Xb = hb + SM::X;
+  const int b = blockIdx.x, L = a.L;
+  const long long row0 = (long long)b * L, g0 = row0 * RS_H;
+  const int w = threadIdx.x >> 5, grp = w >> 2, wl = w & 3, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
+  const int i0 = 16 * wl + g, i1 = i0 + 8;
+  const bool v0 = i0 < L, v1 = i1 < L;
+  const float* lse_g = a.lse + ((long long)b * NH + grp * HPG) * L;     // lse of the group's heads, [HPG][L]
+  float ls0 = v0 ? lse_g[i0] : 0.f, ls1 = v1 ? lse_g[i1] : 0.f;          // issued early: consumed after the first product
+  if (threadIdx.x < 2 * L)                    // the block input, read after the attention: toward L2 now
+    asm volatile("prefetch.global.L2 [%0];" ::"l"(a.pre.x + g0 + 32 * threadIdx.x));
+  {   // q, k, v, dctx into the tiles of LN(x), dk, dv, x
+    const float* const src[4] = {a.q + g0, a.k + g0, a.v + g0, a.dctx + g0};
+    const long long ld[4] = {RS_H, RS_H, RS_H, RS_H};
+    const int nr[4] = {L, L, L, L};
+    const float sc[4] = {1.f, 1.f, 1.f, 1.f};
+    __nv_bfloat16* const d[4] = {Nb, Tk, Tv, Xb};
+    __nv_bfloat16* const dT[4] = {nullptr, nullptr, nullptr, nullptr};
+    float* const dF[4] = {nullptr, nullptr, nullptr, nullptr};
+    rs_load<4, RS_BWD_NT>(src, ld, nr, sc, d, dT, dF);
+  }
+  {
+    const float* const src[3] = {a.pre.Win, a.pre.Win + RS_H * RS_H, a.pre.Win + 2 * RS_H * RS_H};
+    const long long ld[3] = {RS_H, RS_H, RS_H};
+    const int nr[3] = {64, 64, 64};
+    const float sc[3] = {1.f, 1.f, 1.f};
+    __nv_bfloat16* const d[3] = {Wt, Wt + RS_TILE, Wt + 2 * RS_TILE};
+    __nv_bfloat16* const dT[3] = {nullptr, nullptr, nullptr};
+    float* const dF[3] = {nullptr, nullptr, nullptr};
+    rs_load<3, RS_BWD_NT>(src, ld, nr, sc, d, dT, dF);
+  }
+  __syncthreads();
+  __nv_bfloat16* dSt = hb + SM::S + 2 * grp * RS_TILE;
+  __nv_bfloat16* Pt = dSt + RS_TILE;
+  const float qscale = a.pre.qscale;
+  const auto group_sync = [grp] {             // the four warps of this group (immediate barrier ids)
+    if (grp) asm volatile("bar.sync 2, 128;" ::: "memory");
+    else asm volatile("bar.sync 1, 128;" ::: "memory");
+  };
+#pragma unroll 1
+  for (int hh = 0; hh < HPG; ++hh) {
+    const int h = grp * HPG + hh, c0 = h * HD;
+    if (hh) {
+      group_sync();                           // the previous head's key-side products have read dS and P~
+      ls0 = v0 ? lse_g[hh * L + i0] : 0.f;
+      ls1 = v1 ? lse_g[hh * L + i1] : 0.f;
+    }
+    as_bwd_head<HD, RS_LD>(Nb + c0, Tk + c0, Tv + c0, Xb + c0, dSt, Pt, wl, L, a.mask_mode, a.ids + row0, ls0, ls1, a.drop,
+                           a.drop.base + ((unsigned long long)b * NH + h) * L,
+                           [&](int which, const float (&o)[HD / 8][4]) {
+                             __nv_bfloat16* T = (which == 0 ? Tq : which == 1 ? Tk : Tv) + c0;
+                             const float sc = which == 0 ? qscale : 1.f;
+#pragma unroll
+                             for (int db = 0; db < HD / 8; ++db) {
+                               *reinterpret_cast<uint32_t*>(T + i0 * RS_LD + 8 * db + 2 * t) = v0 ? pack_bf16(o[db][0] * sc, o[db][1] * sc) : 0u;
+                               *reinterpret_cast<uint32_t*>(T + i1 * RS_LD + 8 * db + 2 * t) = v1 ? pack_bf16(o[db][2] * sc, o[db][3] * sc) : 0u;
+                             }
+                           },
+                           group_sync);
+  }
+  float Xf[8][4];                             // the block input, issued before the barrier that waits for the other group's heads
+  if (w < 4) frag_load(Xf, a.pre.x + g0, i0, i1, v0, v1, t);
+  __syncthreads();                            // dq s, dk, dv complete; the q and dctx tiles are free
+  pre_bwd_small_tail(a.pre, Xf, Wt, Tq, Tk, Tv, Xb, Nb, row0, L);
 }
 
 }  // namespace adt
