@@ -106,13 +106,11 @@ static DropDesc mk_drop(const adt_dropout& d) {
 
 static const size_t SMEM_MAX = 227 * 1024 - 2048;   // leave room for the kernels' small static arrays
 
-// rows-per-CTA choice: the preferred tile height (ADT_TM = 32 / 64 / 128, default 64) when the tile set fits, else the next smaller
-// `tuned`: per-kernel measured preference used when ADT_TM is not set (C2 shape: mid_bwd is 20 % faster with 128-row tiles -- half
-// the weight-gradient atomics -- every other kernel is fastest at 64)
+// rows-per-CTA choice: the preferred tile height (`tuned`, default 64) when the tile set fits, else the next smaller.  `tuned` is a
+// per-kernel measured preference (C2 shape: mid_bwd is 20 % faster with 128-row tiles -- half the weight-gradient atomics -- every
+// other kernel is fastest at 64)
 static int pick_tm(size_t row_floats, size_t* bytes, int max_tm = 128, int tuned = 0) {
-  static int pref = -1;
-  if (pref < 0) { const char* e = getenv("ADT_TM"); pref = e ? atoi(e) : 0; if (pref != 32 && pref != 64 && pref != 128) pref = 0; }
-  const int want = pref ? pref : (tuned ? tuned : 64);
+  const int want = tuned ? tuned : 64;
   for (int tm = want < max_tm ? want : max_tm; tm >= 32; tm >>= 1) {
     const size_t b = ((size_t)tm * row_floats + WS_FLOATS) * sizeof(float);
     if (b <= SMEM_MAX) {
@@ -164,27 +162,8 @@ static long long flash_scratch_bytes(int B, int L, int H, int nh, bool bwd) {
   return 256 + M * 3 * H * 2 + (bwd ? M * H * 2 + M * nh * 4 : 0);
 }
 
-// Row-tile kernels are launched with programmatic stream serialization (opt-in with ADT_PDL=1: measured neutral at the C2 shape): each of them calls
-// griddepcontrol.launch_dependents on entry and griddepcontrol.wait before it touches activations, so the next kernel's
-// prologue (shared-memory carve-up, weight-ring prefetch) overlaps the tail of the current one.
-static bool use_pdl() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("ADT_PDL"); v = e ? (atoi(e) != 0) : 0; }
-  return v != 0;
-}
-template <class... Exp, class... Act>
-static void launch_pdl(void (*kern)(Exp...), dim3 grid, size_t smem, cudaStream_t stream, Act&&... args) {
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = grid; cfg.blockDim = dim3(NT); cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = use_pdl() ? 1 : 0;
-  cudaLaunchKernelEx(&cfg, kern, static_cast<Exp>(args)...);
-}
 #define LAUNCH_ONE(K, grid, smem, stream, ...) \
-  do { set_smem(K, smem); launch_pdl(K, dim3(grid), smem, stream, __VA_ARGS__); } while (0)
+  do { set_smem(K, smem); K<<<(grid), NT, (smem), (stream)>>>(__VA_ARGS__); } while (0)
 
 #define LAUNCH_TM(tm, mma, KERN, grid, smem, stream, ...)                                        \
   do {                                                                                           \
@@ -457,34 +436,17 @@ static int hoisted_wgrad(const __nv_bfloat16* dy, long long ldy, int n_out, cons
   return ADT_OK;
 }
 
-// ---- sequence-resident block kernels (kernels_seq.cuh): one CTA per sequence, a whole block per launch ------------------------
-// ADT_SEQ_FUSED is a bit mask of the launches served by the sequence-resident kernels: 1 encoder fwd in evaluation mode, 2 decoder
-// fwd, 4 encoder bwd, 8 decoder bwd, 16 encoder fwd in training mode too (0 = the row-tile kernels everywhere).  Default = 1: measured
-// on B200 at the C2 shape (profiles/r02_seq_kernel_variants.md) the one-launch-per-block kernels win where a block runs alone
-// (evaluation: +6 % users/s) but lose inside the training step, whose row-tile kernels overlap across the two streams of the step
-// graph while a sequence-resident CTA pins 83-110 KB of shared memory per SM (0.533 ms -> 0.622 ms with all of them on).
-enum { SEQ_ENC_FWD = 1, SEQ_DEC_FWD = 2, SEQ_ENC_BWD = 4, SEQ_DEC_BWD = 8, SEQ_ENC_FWD_TRAIN = 16, SEQ_DEFAULT = 1 };
-static int seq_mask() {
+// ---- sequence-resident encoder block (kernels_seq.cuh): one CTA per sequence, a whole block per launch, evaluation only --------
+// Measured on B200 at the C2 shape (profiles/r02_seq_kernel_variants.md), the one-launch-per-block kernel wins where a block runs alone
+// (evaluation: +6 % users/s) and loses inside the training step, whose row-tile kernels overlap across the two streams of the step graph
+// while a sequence-resident CTA pins 83 KB of shared memory per SM.  ADT_SEQ_FUSED=0 sends the evaluation encoder to the row-tile
+// kernels too (the reference its parity test compares against).
+static bool use_seq(int L, int H, int nh, int mma) {
   static int v = -1;
-  if (v < 0) { const char* e = getenv("ADT_SEQ_FUSED"); v = e ? atoi(e) : SEQ_DEFAULT; }
-  return v;
-}
-static bool use_seq(int L, int H, int nh, int mma, int which = SEQ_ENC_FWD) {
-  return (seq_mask() & which) && mma && H == RS_H && L <= 64 && (nh == 1 || nh == 2 || nh == 4);
+  if (v < 0) { const char* e = getenv("ADT_SEQ_FUSED"); v = e ? (atoi(e) != 0) : 1; }
+  return v && mma && H == RS_H && L <= 64 && (nh == 1 || nh == 2 || nh == 4);
 }
 extern "C" int adt_seq_kernels_apply(int32_t L, int32_t H, int32_t nh, int32_t precision) { return use_seq(L, H, nh, precision ? 1 : 0) ? 1 : 0; }
-
-static SeqW mk_seqw(const adt_wmirror& m) {
-  SeqW w;
-  w.base32 = m.base32; w.base16 = reinterpret_cast<const __nv_bfloat16*>(m.bf16);
-  return w;
-}
-#define SEQ_LAUNCH(KERN, nh, grid, smem, stream, arg)                                                                  \
-  do {                                                                                                                 \
-    if ((nh) == 1) { cudaFuncSetAttribute(KERN<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smem)); KERN<64><<<grid, SQ_NT, smem, stream>>>(arg); } \
-    else if ((nh) == 2) { cudaFuncSetAttribute(KERN<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smem)); KERN<32><<<grid, SQ_NT, smem, stream>>>(arg); } \
-    else { cudaFuncSetAttribute(KERN<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smem)); KERN<16><<<grid, SQ_NT, smem, stream>>>(arg); } \
-  } while (0)
 
 static int seq_enc_fwd(const adt_enc_block_fwd_args* a, cudaStream_t s) {
   EncSeqFwdArgs p;
@@ -492,97 +454,17 @@ static int seq_enc_fwd(const adt_enc_block_fwd_args* a, cudaStream_t s) {
   p.x = a->x; p.ids = a->ids; p.ln1_g = a->ln1_w; p.ln1_b = a->ln1_b; p.Win = a->attn.in_w; p.bin = a->attn.in_b; p.Wo = a->attn.out_w;
   p.bo = a->attn.out_b; p.ln2_g = a->ln2_w; p.ln2_b = a->ln2_b; p.C1 = a->ffn.w1; p.c1 = a->ffn.b1; p.C2 = a->ffn.w2; p.c2 = a->ffn.b2;
   p.Wsp = a->sparse_w; p.bsp = a->sparse_b;
-  const bool save = a->training != 0;
-  p.q = save ? a->q : nullptr; p.k = save ? a->k : nullptr; p.v = save ? a->v : nullptr; p.ctx = save ? a->ctx : nullptr;
-  p.lse = save ? a->lse : nullptr; p.y = save ? a->y : nullptr; p.h1 = save ? a->h1 : nullptr;
   p.out = a->out; p.out_last = a->out_last; p.rec = a->rec; p.nll_acc = a->nll_acc;
   if (a->nh == 1) { p.rec = nullptr; p.nll_acc = nullptr; }   // a single head has no independence term (main.py:160)
   p.B = a->B; p.L = a->L; p.mask_mode = a->mask_mode; p.qscale = 1.0f / sqrtf((float)(a->H / a->nh));
-  adt_dropout da = a->drop_attn;
-  if (!a->training) da.enabled = 0;
-  p.drop_attn = mk_drop(da); p.drop1 = mk_drop(row_drop(a->drop_ffn1, a->training)); p.drop2 = mk_drop(row_drop(a->drop_ffn2, a->training));
-  p.w = mk_seqw(a->wm);
+  p.w.base32 = a->wm.base32; p.w.base16 = reinterpret_cast<const __nv_bfloat16*>(a->wm.bf16);
+  void (*kern)(EncSeqFwdArgs) = a->nh == 1 ? enc_seq_fwd_kernel<64> : a->nh == 2 ? enc_seq_fwd_kernel<32> : enc_seq_fwd_kernel<16>;
+  const size_t smem = EncSeqFwdSmem::TOTAL_BYTES;
   TIMED("enc_block_fwd", s);
-  SEQ_LAUNCH(enc_seq_fwd_kernel, a->nh, a->B, EncSeqFwdSmem::TOTAL_BYTES, s, p);
+  cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  kern<<<a->B, SQ_NT, smem, s>>>(p);
   return check_launch("enc_seq_fwd");
 }
-
-static int seq_enc_bwd(const adt_enc_block_bwd_args* a, cudaStream_t s) {
-  EncSeqBwdArgs p;
-  memset(&p, 0, sizeof(p));
-  p.x = a->x; p.ids = a->ids; p.q = a->q; p.k = a->k; p.v = a->v; p.ctx = a->ctx; p.lse = a->lse; p.y = a->y; p.h1 = a->h1;
-  p.ln1_g = a->ln1_w; p.ln1_b = a->ln1_b; p.Win = a->attn.in_w; p.Wo = a->attn.out_w; p.ln2_g = a->ln2_w; p.ln2_b = a->ln2_b;
-  p.C1 = a->ffn.w1; p.C2 = a->ffn.w2; p.Wsp = a->sparse_w; p.bsp = a->sparse_b;
-  p.dout = a->dout; p.dx_extra = a->dx_extra; p.drec = a->nh > 1 ? a->drec : nullptr; p.nll_coef = a->nh > 1 ? a->nll_coef : 0.f; p.dx = a->dx;
-  p.gln1_g = a->g_ln1_w; p.gln1_b = a->g_ln1_b; p.gWin = a->g_attn.in_w; p.gbin = a->g_attn.in_b; p.gWo = a->g_attn.out_w; p.gbo = a->g_attn.out_b;
-  p.gln2_g = a->g_ln2_w; p.gln2_b = a->g_ln2_b; p.gC1 = a->g_ffn.w1; p.gc1 = a->g_ffn.b1; p.gC2 = a->g_ffn.w2; p.gc2 = a->g_ffn.b2;
-  p.gWsp = a->g_sparse_w; p.gbsp = a->g_sparse_b;
-  p.B = a->B; p.L = a->L; p.mask_mode = a->mask_mode; p.qscale = 1.0f / sqrtf((float)(a->H / a->nh));
-  p.drop_attn = mk_drop(a->drop_attn); p.drop1 = mk_drop(a->drop_ffn1); p.drop2 = mk_drop(a->drop_ffn2);
-  p.w = mk_seqw(a->wm);
-  TIMED("enc_block_bwd", s);
-  SEQ_LAUNCH(enc_seq_bwd_kernel, a->nh, a->B, SeqBwdSmem::TOTAL_BYTES, s, p);
-  return check_launch("enc_seq_bwd");
-}
-
-static int seq_dec_fwd(const adt_dec_block_fwd_args* a, cudaStream_t s) {
-  DecSeqFwdArgs p;
-  memset(&p, 0, sizeof(p));
-  p.x = a->x; p.feats = a->feats; p.ids = a->ids; p.ln_g = a->ln_w; p.ln_b = a->ln_b;
-  p.Win1 = a->slf.in_w; p.bin1 = a->slf.in_b; p.Wo1 = a->slf.out_w; p.bo1 = a->slf.out_b;
-  p.Win2 = a->enc.in_w; p.bin2 = a->enc.in_b; p.Wo2 = a->enc.out_w; p.bo2 = a->enc.out_b;
-  p.C1 = a->ffn.w1; p.c1 = a->ffn.b1; p.C2 = a->ffn.w2; p.c2 = a->ffn.b2; p.enc_in = a->enc_in;
-  p.d = a->d; p.q1 = a->q1; p.k1 = a->k1; p.v1 = a->v1; p.ctx1 = a->ctx1; p.lse1 = a->lse1; p.a = a->a;
-  p.q2 = a->q2; p.k2 = a->k2; p.v2 = a->v2; p.ctx2 = a->ctx2; p.lse2 = a->lse2; p.c = a->c; p.h1 = a->h1;
-  p.out = a->out; p.mse_acc = a->mse_acc;
-  p.B = a->B; p.L = a->L; p.mask_mode = a->mask_mode; p.qscale = 1.0f / sqrtf((float)(a->H / a->nh));
-  adt_dropout ds = a->drop_slf, de = a->drop_enc;
-  if (!a->training) { ds.enabled = 0; de.enabled = 0; }
-  p.drop_slf = mk_drop(ds); p.drop_enc = mk_drop(de);
-  p.drop1 = mk_drop(row_drop(a->drop_ffn1, a->training)); p.drop2 = mk_drop(row_drop(a->drop_ffn2, a->training));
-  p.w = mk_seqw(a->wm);
-  if (a->phase != 2) {
-    TIMED("dec_block_fwd_p1", s);
-    SEQ_LAUNCH(dec_seq_fwd1_kernel, a->nh, a->B, DecSeqFwd1Smem::TOTAL_BYTES, s, p);
-    if (int e = check_launch("dec_seq_fwd1")) return e;
-  }
-  if (a->phase != 1) {
-    TIMED("dec_block_fwd_p2", s);
-    SEQ_LAUNCH(dec_seq_fwd2_kernel, a->nh, a->B, DecSeqFwd2Smem::TOTAL_BYTES, s, p);
-    if (int e = check_launch("dec_seq_fwd2")) return e;
-  }
-  return ADT_OK;
-}
-
-static int seq_dec_bwd(const adt_dec_block_bwd_args* a, cudaStream_t s) {
-  DecSeqBwdArgs p;
-  memset(&p, 0, sizeof(p));
-  p.x = a->x; p.feats = a->feats; p.ids = a->ids;
-  p.d = a->d; p.q1 = a->q1; p.k1 = a->k1; p.v1 = a->v1; p.ctx1 = a->ctx1; p.lse1 = a->lse1; p.a = a->a;
-  p.q2 = a->q2; p.k2 = a->k2; p.v2 = a->v2; p.ctx2 = a->ctx2; p.lse2 = a->lse2; p.c = a->c; p.h1 = a->h1;
-  p.out = a->out; p.enc_in = a->enc_in; p.mse_coef = a->mse_coef;
-  p.ln_g = a->ln_w; p.ln_b = a->ln_b; p.Win1 = a->slf.in_w; p.Wo1 = a->slf.out_w; p.Win2 = a->enc.in_w; p.Wo2 = a->enc.out_w;
-  p.C1 = a->ffn.w1; p.C2 = a->ffn.w2;
-  p.dout = a->dout; p.denc = a->denc; p.dd = a->dd; p.dctx1 = a->dctx; p.dfeats = a->dfeats; p.dx = a->dx;
-  p.gln_g = a->g_ln_w; p.gln_b = a->g_ln_b; p.gWin1 = a->g_slf.in_w; p.gbin1 = a->g_slf.in_b; p.gWo1 = a->g_slf.out_w; p.gbo1 = a->g_slf.out_b;
-  p.gWin2 = a->g_enc.in_w; p.gbin2 = a->g_enc.in_b; p.gWo2 = a->g_enc.out_w; p.gbo2 = a->g_enc.out_b;
-  p.gC1 = a->g_ffn.w1; p.gc1 = a->g_ffn.b1; p.gC2 = a->g_ffn.w2; p.gc2 = a->g_ffn.b2;
-  p.B = a->B; p.L = a->L; p.mask_mode = a->mask_mode; p.qscale = 1.0f / sqrtf((float)(a->H / a->nh));
-  p.drop_slf = mk_drop(a->drop_slf); p.drop_enc = mk_drop(a->drop_enc); p.drop1 = mk_drop(a->drop_ffn1); p.drop2 = mk_drop(a->drop_ffn2);
-  p.w = mk_seqw(a->wm);
-  if (a->phase != 1) {
-    TIMED("dec_block_bwd_p2", s);
-    SEQ_LAUNCH(dec_seq_bwd2_kernel, a->nh, a->B, SeqBwdSmem::TOTAL_BYTES, s, p);
-    if (int e = check_launch("dec_seq_bwd2")) return e;
-  }
-  if (a->phase != 2) {
-    TIMED("dec_block_bwd_p1", s);
-    SEQ_LAUNCH(dec_seq_bwd1_kernel, a->nh, a->B, SeqBwdSmem::TOTAL_BYTES, s, p);
-    if (int e = check_launch("dec_seq_bwd1")) return e;
-  }
-  return ADT_OK;
-}
-
 
 static int blk_attn_fwd(const float* q, const float* k, const float* v, float* ctx, float* lse, const int* ids, int B, int L, int H, int nh,
                         int mask_mode, const adt_dropout& d, int training, int precision, void* area, void* flash, cudaStream_t s);
@@ -1000,7 +882,7 @@ extern "C" int adt_enc_block_fwd(const adt_enc_block_fwd_args* a, adt_stream_t s
   const int M = a->B * a->L, H = a->H;
   const int mma = a->precision ? 1 : 0, pad = mma ? 8 : 4;
   if (a->phase < 0 || a->phase > 2) return fail(ADT_E_SHAPE, "%s", "enc_block_fwd: phase must be 0, 1 or 2");
-  if (a->phase == 0 && use_seq(a->L, H, a->nh, mma, a->training ? SEQ_ENC_FWD_TRAIN : SEQ_ENC_FWD)) return seq_enc_fwd(a, s);
+  if (a->phase == 0 && !a->training && use_seq(a->L, H, a->nh, mma)) return seq_enc_fwd(a, s);
   if (a->y && a->h1 && a->out && use_fwd_tc(a->tc_scratch, M, H, a->nh, mma)) return tc_enc_fwd(a, s);
   if (a->phase != 2) {
     if (use_attn_fused(a->L, H, a->nh, mma, false)) {
@@ -1044,7 +926,6 @@ extern "C" int adt_enc_block_bwd(const adt_enc_block_bwd_args* a, adt_stream_t s
   if (int e = check_attn_dims(a->B, a->L, a->H, a->nh, a->precision)) return e;
   const int M = a->B * a->L, H = a->H;
   const int mma = a->precision ? 1 : 0, pad = mma ? 8 : 4;
-  if (use_seq(a->L, H, a->nh, mma, SEQ_ENC_BWD)) return seq_enc_bwd(a, s);
   if (use_bwd_tc(a->wgrad_scratch, M, H, a->nh, mma)) return tc_enc_bwd(a, s);
   PostBwdArgs p;
   memset(&p, 0, sizeof(p));
@@ -1103,7 +984,6 @@ extern "C" int adt_dec_block_fwd(const adt_dec_block_fwd_args* a, adt_stream_t s
   if (int e = check_attn_dims(a->B, a->L, a->H, a->nh, a->precision)) return e;
   const int M = a->B * a->L, H = a->H;
   const int mma = a->precision ? 1 : 0, pad = mma ? 8 : 4;
-  if (use_seq(a->L, H, a->nh, mma, SEQ_DEC_FWD)) return seq_dec_fwd(a, s);
   if (a->d && a->a && a->c && a->h1 && use_fwd_tc(a->tc_scratch, M, H, a->nh, mma)) return tc_dec_fwd(a, s);
   if (a->phase != 2) {
     if (use_attn_fused(a->L, H, a->nh, mma, false)) {
@@ -1166,7 +1046,6 @@ extern "C" int adt_dec_block_bwd(const adt_dec_block_bwd_args* a, adt_stream_t s
   const int M = a->B * a->L, H = a->H;
   const int mma = a->precision ? 1 : 0, pad = mma ? 8 : 4;
   const float qscale = 1.0f / sqrtf((float)(H / a->nh));
-  if (use_seq(a->L, H, a->nh, mma, SEQ_DEC_BWD)) return seq_dec_bwd(a, s);
   if (use_bwd_tc(a->wgrad_scratch, M, H, a->nh, mma)) return tc_dec_bwd(a, s);
   __nv_bfloat16* hz = hoist_ptr(a->wgrad_scratch, H, mma);
   const long long hu = (long long)M * H;

@@ -17,11 +17,6 @@ namespace adt {
 __device__ long long g_dbg_clock[64];
 #define ADT_STAMP(i) do { if (blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && threadIdx.x == 0) g_dbg_clock[i] = clock64(); } while (0)
 
-// programmatic dependent launch (no-ops when the kernel was launched without the attribute): the next kernel of the stream may be
-// scheduled while this one still runs; it must not touch anything a predecessor produces before pdl_wait().
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-
 constexpr int NT = 256;        // threads per CTA for all row-tile kernels
 constexpr int CH = 64;         // weight chunk edge (rows and cols)
 constexpr int CHP = CH + 4;    // padded chunk row stride in floats (272 B: 16B aligned, LDS.128 conflict free)

@@ -66,7 +66,6 @@ struct PostBwdArgs {
 template <int TM, bool IS_DEC, bool MMA>
 __global__ void __launch_bounds__(NT) post_bwd_kernel(PostBwdArgs p) {
   extern __shared__ __align__(16) float smem[];
-  pdl_trigger();
   const int H = p.H, M = p.M;
   const int ld = H + tile_pad<MMA>();
   float* G = smem;            // dO -> (enc) dy
@@ -88,7 +87,6 @@ __global__ void __launch_bounds__(NT) post_bwd_kernel(PostBwdArgs p) {
   __syncthreads();
   WStream<WS_NST, MMA> ws;
   ws.start(&wst, Ws);
-  pdl_wait();   // weights may be prefetched early; activations only after the predecessors completed
 
   // 1./2. dO = (dout + mse_coef*(out-enc_in)) * keep ; y/c ; a = relu(h1*m1) ; dh2 = dO*m2
   struct PostLd { float4 g, o, e, y, h; int id; };
@@ -252,7 +250,6 @@ __global__ void __launch_bounds__(NT) attn_bwd_kernel(const float* __restrict__ 
                                                       float* __restrict__ dq, float* __restrict__ dk, float* __restrict__ dv, int L,
                                                       int H, int nh, int mask_mode, DropDesc drop) {
   extern __shared__ __align__(16) float smem[];
-  pdl_trigger();
   const int hd = H / nh;
   const int ldq = hd + tile_pad<MMA>();
   const int lds = ((L + 3) & ~3) + tile_pad<MMA>();
@@ -276,7 +273,6 @@ __global__ void __launch_bounds__(NT) attn_bwd_kernel(const float* __restrict__ 
   }
   __syncthreads();
   WStream<WS_NST, MMA> ws;
-  pdl_wait();   // q/k/v come from the preceding kernel
   ADT_STAMP(36);
   ws.start(&wst, Ws);
   load_tile<TM>(Qs, ldq, q + seq_off, H, 0, hd, i0, L);
@@ -370,7 +366,6 @@ struct MidBwdArgs {
 template <int TM, bool MMA>
 __global__ void __launch_bounds__(NT) mid_bwd_kernel(MidBwdArgs p) {
   extern __shared__ __align__(16) float smem[];
-  pdl_trigger();
   const int H = p.H, M = p.M;
   const int ld = H + tile_pad<MMA>(), ld2 = 2 * H + tile_pad<MMA>();
   float* T0 = smem;              // dq2*scale
@@ -390,7 +385,6 @@ __global__ void __launch_bounds__(NT) mid_bwd_kernel(MidBwdArgs p) {
   __syncthreads();
   WStream<WS_NST, MMA> ws;
   ws.start(&wst, Ws);
-  pdl_wait();   // weights may be prefetched early; activations only after the predecessors completed
   struct Ld2 { float4 a, b; };
   tile_foreach4_ld<TM, 4, Ld2>(H, [&](int r, int c, Ld2& v) {
     v.a = v.b = zero4();
@@ -452,7 +446,6 @@ struct PreBwdArgs {
 template <int TM, bool MMA>
 __global__ void __launch_bounds__(NT) pre_bwd_kernel(PreBwdArgs p) {
   extern __shared__ __align__(16) float smem[];
-  pdl_trigger();
   const int H = p.H, M = p.M;
   const int ld = H + tile_pad<MMA>();
   float* X = smem;
@@ -472,7 +465,6 @@ __global__ void __launch_bounds__(NT) pre_bwd_kernel(PreBwdArgs p) {
   __syncthreads();
   WStream<WS_NST, MMA> ws;
   ws.start(&wst, Ws);
-  pdl_wait();   // weights may be prefetched early; activations only after the predecessors completed
   ADT_STAMP(24);
   struct Ld2 { float4 a, b; };
   tile_foreach4_ld<TM, 4, Ld2>(H, [&](int r, int c, Ld2& v) {

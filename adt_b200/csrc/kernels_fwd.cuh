@@ -49,7 +49,6 @@ __global__ void __launch_bounds__(NT) pre_fwd_kernel(const float* __restrict__ x
                                                      float* __restrict__ v, float* __restrict__ norm_out, int M, int H, float qscale,
                                                      int kv_from_norm) {
   extern __shared__ __align__(16) float smem[];
-  pdl_trigger();
   const int ld = H + tile_pad<MMA>();
   float* Xs = smem;
   float* Ns = Xs + TM * ld;
@@ -66,7 +65,6 @@ __global__ void __launch_bounds__(NT) pre_fwd_kernel(const float* __restrict__ x
   __syncthreads();
   WStream<WS_NST, MMA> ws;
   ws.start(&wst, Ws);
-  pdl_wait();   // weights may be prefetched early; activations only after the predecessors completed
   ADT_STAMP(1);
   load_tile<TM>(Xs, ld, x, H, 0, H, row0, M);
   tile_sync();
@@ -117,7 +115,6 @@ __global__ void __launch_bounds__(NT) attn_fwd_kernel(const float* __restrict__ 
                                                       const int* __restrict__ key_ids, int L, int H, int nh, int mask_mode,
                                                       DropDesc drop) {
   extern __shared__ __align__(16) float smem[];
-  pdl_trigger();
   const int hd = H / nh;
   const int ldq = hd + tile_pad<MMA>();
   const int lds = ((L + 3) & ~3) + tile_pad<MMA>();
@@ -136,7 +133,6 @@ __global__ void __launch_bounds__(NT) attn_fwd_kernel(const float* __restrict__ 
   }
   __syncthreads();
   WStream<WS_NST, MMA> ws;
-  pdl_wait();   // q/k/v come from the preceding kernel
   ws.start(&wst, Ws);
   ADT_STAMP(9);
   load_tile<TM>(Qs, ldq, q + seq_off, H, 0, hd, i0, L);
@@ -215,7 +211,6 @@ __global__ void __launch_bounds__(NT) mid_fwd_kernel(const float* __restrict__ c
                                                      float* __restrict__ a_out, float* __restrict__ q2, float* __restrict__ k2,
                                                      float* __restrict__ v2, int M, int H, float qscale) {
   extern __shared__ __align__(16) float smem[];
-  pdl_trigger();
   const int ld = H + tile_pad<MMA>();
   float* T0 = smem;
   float* T1 = T0 + TM * ld;
@@ -233,7 +228,6 @@ __global__ void __launch_bounds__(NT) mid_fwd_kernel(const float* __restrict__ c
   __syncthreads();
   WStream<WS_NST, MMA> ws;
   ws.start(&wst, Ws);
-  pdl_wait();   // weights may be prefetched early; activations only after the predecessors completed
   load_tile<TM>(T0, ld, ctx1, H, 0, H, row0, M);
   load_tile<TM>(T2, ld, feats, H, 0, H, row0, M);
   tile_sync();
@@ -283,7 +277,6 @@ struct PostFwdArgs {
 template <int TM, bool IS_DEC, bool MMA>
 __global__ void __launch_bounds__(NT) post_fwd_kernel(PostFwdArgs p) {
   extern __shared__ __align__(16) float smem[];
-  pdl_trigger();
   __shared__ double red[NT / 32];
   const int H = p.H, M = p.M;
   const int ld = H + tile_pad<MMA>();
@@ -304,7 +297,6 @@ __global__ void __launch_bounds__(NT) post_fwd_kernel(PostFwdArgs p) {
   __syncthreads();
   WStream<WS_NST, MMA> ws;
   ws.start(&wst, Ws);
-  pdl_wait();   // weights may be prefetched early; activations only after the predecessors completed
   load_tile<TM>(T0, ld, p.ctx, H, 0, H, row0, M);
   if (!IS_DEC) {
     load_tile<TM>(T2, ld, p.resid, H, 0, H, row0, M);

@@ -27,7 +27,6 @@ struct LinearFwdArgs {
 template <int TM, bool MMA>
 __global__ void __launch_bounds__(NT) linear_fwd_kernel(LinearFwdArgs p) {
   extern __shared__ __align__(16) float smem[];
-  pdl_trigger();
   const int ld = p.K + tile_pad<MMA>();
   float* Xs = smem;
   float* Ws = Xs + TM * ld;
@@ -40,7 +39,6 @@ __global__ void __launch_bounds__(NT) linear_fwd_kernel(LinearFwdArgs p) {
   __syncthreads();
   WStream<WS_NST, MMA> ws;
   ws.start(&wst, Ws);
-  pdl_wait();   // weights may be prefetched early; activations only after the predecessors completed
   load_tile<TM>(Xs, ld, p.x, p.K, 0, p.K, row0, p.M);
   tile_sync();
   const bool vec = ((p.N | p.ldy) & 3) == 0;     // output width / stride not a multiple of 4 -> scalar epilogue
@@ -73,7 +71,6 @@ struct LinearBwdArgs {
 template <int TM, bool MMA>
 __global__ void __launch_bounds__(NT) linear_bwd_kernel(LinearBwdArgs p) {
   extern __shared__ __align__(16) float smem[];
-  pdl_trigger();
   const int N4 = (p.N + 3) & ~3;
   const int ldx = p.K + tile_pad<MMA>(), ldy = N4 + tile_pad<MMA>();
   float* Xs = smem;
@@ -89,7 +86,6 @@ __global__ void __launch_bounds__(NT) linear_bwd_kernel(LinearBwdArgs p) {
   __syncthreads();
   WStream<WS_NST, MMA> ws;
   ws.start(&wst, Ws);
-  pdl_wait();   // weights may be prefetched early; activations only after the predecessors completed
   if (p.gW) load_tile<TM>(Xs, ldx, p.x, p.K, 0, p.K, row0, p.M);
   if (((p.N | p.lddy) & 3) == 0) {
     tile_foreach4<TM>(p.N, [&](int r, int c) {

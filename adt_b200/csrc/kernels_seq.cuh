@@ -1,15 +1,16 @@
-// Sequence-resident block kernels for short sequences (L <= 64) of narrow models (H == 64) in the bf16 tensor-core mode:
-// ONE 128-thread CTA owns ONE whole sequence and runs a complete transformer block on it -- LayerNorm -> packed QKV projection ->
-// causal softmax attention (all heads) -> out-projection -> LayerNorm -> FFN -> dropout / residual / pad mask -> loss epilogue --
-// with the sequence's q, k, v, probabilities and context living in shared memory / MMA fragments.  Nothing but the block input,
-// the block output and the tensors saved for the backward pass touches HBM, and a block is ONE launch instead of three (encoder) or
-// five (decoder); the backward kernels mirror that (post adjoint -> attention adjoint -> projection / LayerNorm adjoint on chip).
-// Reference semantics: EncoderLayer.forward sasrec/modules.py:644-655, DecoderLayer.forward :666-677, MultiheadAttentionADT
-// :270-527, PointWiseFeedForward :629-633, SparseInputLinear :696-703 (SURVEY.md appendix A).
+// Sequence-resident encoder block for evaluation: short sequences (L <= 64) of narrow models (H == 64) in the bf16 tensor-core mode.
+// ONE 128-thread CTA owns ONE whole sequence and runs a complete encoder block on it -- LayerNorm -> packed QKV projection -> causal
+// softmax attention (all heads) -> out-projection -> LayerNorm -> FFN -> residual / pad mask (+ the independence head's log-probs) --
+// with the sequence's q, k, v, probabilities and context living in shared memory / MMA fragments.  Nothing but the block input and
+// the block output touches HBM, and a block is ONE launch instead of three.  Training runs the row-tile kernels: they overlap
+// across the two streams of the step graph, and a CTA that pins 83 KB of shared memory per SM would not
+// (profiles/r02_seq_kernel_variants.md).
+// Reference semantics: EncoderLayer.forward sasrec/modules.py:644-655, MultiheadAttentionADT :270-527, PointWiseFeedForward
+// :629-633, SparseInputLinear :696-703 (SURVEY.md appendix A).
 //
-// Weights: the kernels take the fp32 parameters (converted on the fly) or, when the caller keeps a bf16 mirror of the flat
-// parameter buffer (written by the Adam kernel), cp.async them straight into the padded shared-memory tiles.
-// Shared-memory budget: <= 113 KB per CTA so that two CTAs (two sequences) are resident per SM: 256 sequences = one wave.
+// Weights: the kernel takes the fp32 parameters (converted on the fly) or, when the caller keeps a bf16 mirror of the flat
+// parameter buffer (written by the Adam kernel), cp.asyncs them straight into the padded shared-memory tiles.
+// Shared-memory budget: 83 KB per CTA so that two CTAs (two sequences) are resident per SM: 256 sequences = one wave.
 #pragma once
 #include "kernels_rowtile_small.cuh"
 
@@ -76,18 +77,17 @@ __device__ __forceinline__ void frag_bias_scale(float (&v)[8][4], const float* _
 
 // ---------------------------------------------------------------------------------------------------------------------------------
 // causal / key-padding softmax attention of ONE sequence, all heads, operands in full-width bf16 tiles [64][72] (heads are column
-// slices).  Returns the context in fragments (rows i0 / i1 of this thread, all 64 columns).  Same arithmetic, masks and Philox
-// stream as attn_small_fwd_kernel.
+// slices).  Returns the context in fragments (rows i0 / i1 of this thread, all 64 columns).  Same arithmetic and masks as
+// attn_small_fwd_kernel without dropout.
 // ---------------------------------------------------------------------------------------------------------------------------------
 template <int HD>
 __device__ __forceinline__ void sq_attn_fwd(float (&ctxf)[8][4], const __nv_bfloat16* __restrict__ Qs, const __nv_bfloat16* __restrict__ Ks,
-                                            const __nv_bfloat16* __restrict__ Vs, int L, int b, int mask_mode, const int* __restrict__ kid,
-                                            const DropDesc& drop, float* __restrict__ lse) {
+                                            const __nv_bfloat16* __restrict__ Vs, int L, int mask_mode, const int* __restrict__ kid) {
   constexpr int NH = RS_H / HD;
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
   const int i0 = 16 * w + g, i1 = i0 + 8;
   const bool v0 = i0 < L, v1 = i1 < L;
-  const int nbr = (L + 7) >> 3, nks = (L + 15) >> 4, lp8 = ((L + 7) & ~7) >> 3;
+  const int nbr = (L + 7) >> 3, nks = (L + 15) >> 4;
 #pragma unroll
   for (int h = 0; h < NH; ++h) {
     float s[8][4];
@@ -133,23 +133,8 @@ __device__ __forceinline__ void sq_attn_fwd(float (&ctxf)[8][4], const __nv_bflo
     sum0 += __shfl_xor_sync(0xffffffffu, sum0, 1); sum0 += __shfl_xor_sync(0xffffffffu, sum0, 2);
     sum1 += __shfl_xor_sync(0xffffffffu, sum1, 1); sum1 += __shfl_xor_sync(0xffffffffu, sum1, 2);
     const float inv0 = v0 ? 1.0f / sum0 : 0.f, inv1 = v1 ? 1.0f / sum1 : 0.f;
-    if (lse && t == 0) {
-      if (v0) lse[((long long)b * NH + h) * L + i0] = mx0 + logf(sum0);
-      if (v1) lse[((long long)b * NH + h) * L + i1] = mx1 + logf(sum1);
-    }
-    if (drop.enabled) {
-      const unsigned long long rb = drop.base + ((unsigned long long)b * NH + h) * L;
-      AsDrop dm;
-      as_drop_all(dm, drop, rb + i0, rb + i1, v0, v1, lp8, nbr, t);
 #pragma unroll
-      for (int nb = 0; nb < 8; ++nb) {
-        s[nb][0] *= dm.m0[nb].x * inv0; s[nb][1] *= dm.m0[nb].y * inv0;
-        s[nb][2] *= dm.m1[nb].x * inv1; s[nb][3] *= dm.m1[nb].y * inv1;
-      }
-    } else {
-#pragma unroll
-      for (int nb = 0; nb < 8; ++nb) { s[nb][0] *= inv0; s[nb][1] *= inv0; s[nb][2] *= inv1; s[nb][3] *= inv1; }
-    }
+    for (int nb = 0; nb < 8; ++nb) { s[nb][0] *= inv0; s[nb][1] *= inv0; s[nb][2] *= inv1; s[nb][3] *= inv1; }
     float o[HD / 8][4];
 #pragma unroll
     for (int db = 0; db < HD / 8; ++db) o[db][0] = o[db][1] = o[db][2] = o[db][3] = 0.f;
@@ -177,202 +162,47 @@ __device__ __forceinline__ void sq_attn_fwd(float (&ctxf)[8][4], const __nv_bflo
   }
 }
 
-// adjoint of sq_attn_fwd: Q, K, V, dC (grad wrt context) in full-width bf16 tiles; dSt / Pt are [64][72] scratch tiles.
-// Returns dq (rows = queries of this thread), dk, dv (rows = keys of this thread) in full-width fragments.  Contains CTA barriers.
-template <int HD>
-__device__ __forceinline__ void sq_attn_bwd(float (&DQ)[8][4], float (&DK)[8][4], float (&DV)[8][4], const __nv_bfloat16* __restrict__ Qs,
-                                            const __nv_bfloat16* __restrict__ Ks, const __nv_bfloat16* __restrict__ Vs,
-                                            const __nv_bfloat16* __restrict__ dCs, __nv_bfloat16* __restrict__ dSt, __nv_bfloat16* __restrict__ Pt,
-                                            int L, int b, int mask_mode, const int* __restrict__ kid, const DropDesc& drop,
-                                            const float* __restrict__ lse) {
-  constexpr int NH = RS_H / HD;
-  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
-  const int i0 = 16 * w + g, i1 = i0 + 8;
-  const bool v0 = i0 < L, v1 = i1 < L;
-  const int nbr = (L + 7) >> 3, nks = (L + 15) >> 4, lp8 = ((L + 7) & ~7) >> 3;
-#pragma unroll
-  for (int h = 0; h < NH; ++h) {
-    const float ls0 = v0 ? lse[((long long)b * NH + h) * L + i0] : 0.f;
-    const float ls1 = v1 ? lse[((long long)b * NH + h) * L + i1] : 0.f;
-    float p[8][4], dp[8][4];
-    frag_zero(p);
-    frag_zero(dp);
-#pragma unroll
-    for (int ks = 0; ks < HD / 16; ++ks) {
-      uint32_t a[4], c[4];
-      lm_a<RS_LD>(a, Qs + h * HD, 16 * w, 16 * ks);
-      lm_a<RS_LD>(c, dCs + h * HD, 16 * w, 16 * ks);
-#pragma unroll
-      for (int nb = 0; nb < 8; ++nb) {
-        if (nb < nbr) {
-          uint32_t b0, b1;
-          lm_b<RS_LD>(b0, b1, Ks + h * HD, 8 * nb, 16 * ks);
-          mma16816(p[nb], a, b0, b1);                    // S = q k^T
-          lm_b<RS_LD>(b0, b1, Vs + h * HD, 8 * nb, 16 * ks);
-          mma16816(dp[nb], c, b0, b1);                   // dP~ = dctx v^T
-        }
-      }
-    }
-    AsDrop dm;
-    if (drop.enabled) {
-      const unsigned long long rb = drop.base + ((unsigned long long)b * NH + h) * L;
-      as_drop_all(dm, drop, rb + i0, rb + i1, v0, v1, lp8, nbr, t);
-    } else {
-#pragma unroll
-      for (int nb = 0; nb < 8; ++nb) dm.m0[nb] = dm.m1[nb] = make_float2(1.f, 1.f);
-    }
-    float dl0 = 0.f, dl1 = 0.f;
-    float pt[8][4];
-#pragma unroll
-    for (int nb = 0; nb < 8; ++nb) {
-      const float2 m0 = dm.m0[nb], m1 = dm.m1[nb];
-#pragma unroll
-      for (int e = 0; e < 2; ++e) {
-        const int j = 8 * nb + 2 * t + e;
-        const float s0 = as_masked(p[nb][e], i0, j, L, mask_mode, kid), s1 = as_masked(p[nb][2 + e], i1, j, L, mask_mode, kid);
-        const float p0 = s0 == -INFINITY ? 0.f : expf(s0 - ls0), p1 = s1 == -INFINITY ? 0.f : expf(s1 - ls1);
-        const float mm0 = e ? m0.y : m0.x, mm1 = e ? m1.y : m1.x;
-        const float d0 = dp[nb][e] * mm0, d1 = dp[nb][2 + e] * mm1;
-        dl0 = fmaf(d0, p0, dl0); dl1 = fmaf(d1, p1, dl1);
-        p[nb][e] = p0; p[nb][2 + e] = p1;
-        dp[nb][e] = d0; dp[nb][2 + e] = d1;
-        pt[nb][e] = p0 * mm0; pt[nb][2 + e] = p1 * mm1;
-      }
-    }
-    dl0 += __shfl_xor_sync(0xffffffffu, dl0, 1); dl0 += __shfl_xor_sync(0xffffffffu, dl0, 2);
-    dl1 += __shfl_xor_sync(0xffffffffu, dl1, 1); dl1 += __shfl_xor_sync(0xffffffffu, dl1, 2);
-    if (h > 0) __syncthreads();                          // the previous head's key-side products are done with dSt / Pt
-#pragma unroll
-    for (int nb = 0; nb < 8; ++nb) {
-#pragma unroll
-      for (int e = 0; e < 2; ++e) {
-        dp[nb][e] = p[nb][e] * (dp[nb][e] - dl0);
-        dp[nb][2 + e] = p[nb][2 + e] * (dp[nb][2 + e] - dl1);
-      }
-      const int j = 8 * nb + 2 * t;                      // columns >= L of valid rows hold exact zeros (masked probabilities)
-      *reinterpret_cast<uint32_t*>(dSt + i0 * AS_LT + j) = v0 ? pack_bf16(dp[nb][0], dp[nb][1]) : 0u;
-      *reinterpret_cast<uint32_t*>(dSt + i1 * AS_LT + j) = v1 ? pack_bf16(dp[nb][2], dp[nb][3]) : 0u;
-      *reinterpret_cast<uint32_t*>(Pt + i0 * AS_LT + j) = v0 ? pack_bf16(pt[nb][0], pt[nb][1]) : 0u;
-      *reinterpret_cast<uint32_t*>(Pt + i1 * AS_LT + j) = v1 ? pack_bf16(pt[nb][2], pt[nb][3]) : 0u;
-    }
-    {   // dq = dS k
-      float o[HD / 8][4];
-#pragma unroll
-      for (int db = 0; db < HD / 8; ++db) o[db][0] = o[db][1] = o[db][2] = o[db][3] = 0.f;
-#pragma unroll
-      for (int ks = 0; ks < 4; ++ks) {
-        if (ks < nks) {
-          uint32_t a[4];
-          a[0] = pack_bf16(dp[2 * ks][0], dp[2 * ks][1]);
-          a[1] = pack_bf16(dp[2 * ks][2], dp[2 * ks][3]);
-          a[2] = pack_bf16(dp[2 * ks + 1][0], dp[2 * ks + 1][1]);
-          a[3] = pack_bf16(dp[2 * ks + 1][2], dp[2 * ks + 1][3]);
-#pragma unroll
-          for (int db = 0; db < HD / 8; ++db) {
-            uint32_t b0, b1;
-            lm_b_t<RS_LD>(b0, b1, Ks + h * HD, 16 * ks, 8 * db);
-            mma16816(o[db], a, b0, b1);
-          }
-        }
-      }
-#pragma unroll
-      for (int db = 0; db < HD / 8; ++db) {
-        DQ[h * (HD / 8) + db][0] = o[db][0]; DQ[h * (HD / 8) + db][1] = o[db][1];
-        DQ[h * (HD / 8) + db][2] = o[db][2]; DQ[h * (HD / 8) + db][3] = o[db][3];
-      }
-    }
-    __syncthreads();
-    // dk = dS^T q ; dv = P~^T dctx   (this warp owns key rows 16w .. 16w+15)
-#pragma unroll
-    for (int which = 0; which < 2; ++which) {
-      const __nv_bfloat16* A = which == 0 ? dSt : Pt;
-      const __nv_bfloat16* Bk = (which == 0 ? Qs : dCs) + h * HD;
-      float o[HD / 8][4];
-#pragma unroll
-      for (int db = 0; db < HD / 8; ++db) o[db][0] = o[db][1] = o[db][2] = o[db][3] = 0.f;
-#pragma unroll
-      for (int ks = 0; ks < 4; ++ks) {
-        if (ks < nks) {
-          uint32_t a[4];
-          lm_a_t<AS_LT>(a, A, 16 * w, 16 * ks);
-#pragma unroll
-          for (int db = 0; db < HD / 8; ++db) {
-            uint32_t b0, b1;
-            lm_b_t<RS_LD>(b0, b1, Bk, 16 * ks, 8 * db);
-            mma16816(o[db], a, b0, b1);
-          }
-        }
-      }
-#pragma unroll
-      for (int db = 0; db < HD / 8; ++db) {
-#pragma unroll
-        for (int e = 0; e < 4; ++e) {
-          if (which == 0) DK[h * (HD / 8) + db][e] = o[db][e]; else DV[h * (HD / 8) + db][e] = o[db][e];
-        }
-      }
-    }
-  }
-}
-
 // ---------------------------------------------------------------------------------------------------------------------------------
-// FFN tail shared by the encoder and decoder forward kernels: u = z (enc) / c (dec) in fragments ->
-// out = (drop2(relu(drop1(u C1^T + c1)) C2^T + c2) + u [+ res]) * keep
+// FFN tail: u = z in fragments -> out = relu(u C1^T + c1) C2^T + c2 + u
 // ---------------------------------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ void sq_ffn_fwd(float (&y)[8][4], const float (&u)[8][4], const __nv_bfloat16* __restrict__ C1t,
                                            const __nv_bfloat16* __restrict__ C2t, const float* __restrict__ c1, const float* __restrict__ c2,
-                                           const DropDesc& drop1, const DropDesc& drop2, float* __restrict__ h1_save, long long grow0,
-                                           int i0, int i1, bool v0, bool v1, int t) {
+                                           int t) {
   float h[8][4];
   frag_zero(h);
   rs_fgemm_frag(h, u, C1t);
-  float mk[8][4];
-  if (drop1.enabled) frag_drop(mk, drop1, grow0 + i0, grow0 + i1, t);
 #pragma unroll
   for (int nb = 0; nb < 8; ++nb) {
     const int c = 8 * nb + 2 * t;
     const float2 b = __ldg(reinterpret_cast<const float2*>(c1 + c));
     h[nb][0] += b.x; h[nb][1] += b.y; h[nb][2] += b.x; h[nb][3] += b.y;
-    if (h1_save) {
-      if (v0) *reinterpret_cast<float2*>(h1_save + (grow0 + i0) * RS_H + c) = make_float2(h[nb][0], h[nb][1]);
-      if (v1) *reinterpret_cast<float2*>(h1_save + (grow0 + i1) * RS_H + c) = make_float2(h[nb][2], h[nb][3]);
-    }
 #pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      float x = h[nb][e];
-      if (drop1.enabled) x *= mk[nb][e];
-      h[nb][e] = fmaxf(x, 0.f);
-    }
+    for (int e = 0; e < 4; ++e) h[nb][e] = fmaxf(h[nb][e], 0.f);
   }
   frag_zero(y);
   rs_fgemm_frag(y, h, C2t);
-  if (drop2.enabled) frag_drop(mk, drop2, grow0 + i0, grow0 + i1, t);
 #pragma unroll
   for (int nb = 0; nb < 8; ++nb) {
     const int c = 8 * nb + 2 * t;
     const float2 b = __ldg(reinterpret_cast<const float2*>(c2 + c));
     y[nb][0] += b.x; y[nb][1] += b.y; y[nb][2] += b.x; y[nb][3] += b.y;
 #pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      if (drop2.enabled) y[nb][e] *= mk[nb][e];
-      y[nb][e] += u[nb][e];
-    }
+    for (int e = 0; e < 4; ++e) y[nb][e] += u[nb][e];
   }
 }
 
 // ---------------------------------------------------------------------------------------------------------------------------------
-// Encoder block forward, one sequence per CTA.
+// Encoder block forward in evaluation mode, one sequence per CTA.
 // ---------------------------------------------------------------------------------------------------------------------------------
 struct EncSeqFwdArgs {
   const float* x; const int* ids;
   const float* ln1_g; const float* ln1_b; const float* Win; const float* bin; const float* Wo; const float* bo;
   const float* ln2_g; const float* ln2_b; const float* C1; const float* c1; const float* C2; const float* c2;
   const float* Wsp; const float* bsp;
-  float* q; float* k; float* v; float* ctx; float* lse; float* y; float* h1;   // saved for backward (each nullable)
   float* out;                                                                  // [M][64] (nullable when out_last is given)
   float* out_last;                                                             // optional [B][64]: the block output of position L-1 only
   float* rec; double* nll_acc;
   int B, L, mask_mode; float qscale;
-  DropDesc drop_attn, drop1, drop2;
   SeqW w;
 };
 
@@ -421,17 +251,14 @@ __global__ void __launch_bounds__(SQ_NT, 2) enc_seq_fwd_kernel(EncSeqFwdArgs p) 
     frag_zero(o);
     rs_fgemm_frag(o, Nf, Wt);
     frag_bias_scale(o, p.bin, p.qscale, t);
-    if (p.q) frag_store(p.q + g0, o, i0, i1, v0, v1, t);
     frag_store_tile(Qs, o, i0, i1, t);
     frag_zero(o);
     rs_fgemm_frag(o, Xf, Wt + RS_TILE);
     frag_bias_scale(o, p.bin + RS_H, 1.f, t);
-    if (p.k) frag_store(p.k + g0, o, i0, i1, v0, v1, t);
     frag_store_tile(Ks, o, i0, i1, t);
     frag_zero(o);
     rs_fgemm_frag(o, Xf, Wt + 2 * RS_TILE);
     frag_bias_scale(o, p.bin + 2 * RS_H, 1.f, t);
-    if (p.v) frag_store(p.v + g0, o, i0, i1, v0, v1, t);
     frag_store_tile(Vs, o, i0, i1, t);
   }
   ADT_STAMP(51);
@@ -439,9 +266,8 @@ __global__ void __launch_bounds__(SQ_NT, 2) enc_seq_fwd_kernel(EncSeqFwdArgs p) 
   ADT_STAMP(52);
   // ---- attention, all heads
   float Cf[8][4];
-  sq_attn_fwd<HD>(Cf, Qs, Ks, Vs, L, b, p.mask_mode, p.ids + grow0, p.drop_attn, p.lse);
+  sq_attn_fwd<HD>(Cf, Qs, Ks, Vs, L, p.mask_mode, p.ids + grow0);
   ADT_STAMP(53);
-  if (p.ctx) frag_store(p.ctx + g0, Cf, i0, i1, v0, v1, t);
   // ---- y = ctx Wo^T + bo + Qn ; independence head on the per-head context slices
   float u[8][4];
   frag_zero(u);
@@ -451,7 +277,6 @@ __global__ void __launch_bounds__(SQ_NT, 2) enc_seq_fwd_kernel(EncSeqFwdArgs p) 
     const float2 bb = __ldg(reinterpret_cast<const float2*>(p.bo + 8 * nb + 2 * t));
     u[nb][0] += bb.x + Nf[nb][0]; u[nb][1] += bb.y + Nf[nb][1]; u[nb][2] += bb.x + Nf[nb][2]; u[nb][3] += bb.y + Nf[nb][3];
   }
-  if (p.y) frag_store(p.y + g0, u, i0, i1, v0, v1, t);
   ADT_STAMP(54);
   if (p.rec || p.nll_acc) {
     __syncthreads();                                  // every warp is done with Q as the attention operand
@@ -486,7 +311,7 @@ __global__ void __launch_bounds__(SQ_NT, 2) enc_seq_fwd_kernel(EncSeqFwdArgs p) 
   ADT_STAMP(55);
   frag_ln(u, p.ln2_g, p.ln2_b, t);                    // z = LN2(y)
   float o[8][4];
-  sq_ffn_fwd(o, u, Wt + 4 * RS_TILE, Wt + 5 * RS_TILE, p.c1, p.c2, p.drop1, p.drop2, p.h1, grow0, i0, i1, v0, v1, t);
+  sq_ffn_fwd(o, u, Wt + 4 * RS_TILE, Wt + 5 * RS_TILE, p.c1, p.c2, t);
   ADT_STAMP(56);
 #pragma unroll
   for (int nb = 0; nb < 8; ++nb) {
@@ -496,648 +321,6 @@ __global__ void __launch_bounds__(SQ_NT, 2) enc_seq_fwd_kernel(EncSeqFwdArgs p) 
   if (p.out) frag_store(p.out + g0, o, i0, i1, v0, v1, t);
   ADT_STAMP(57);
   if (p.out_last) frag_store(p.out_last + (long long)b * RS_H - (long long)(L - 1) * RS_H, o, i0, i1, i0 == L - 1, i1 == L - 1, t);
-}
-
-// ---------------------------------------------------------------------------------------------------------------------------------
-// Decoder block forward.  Phase 1: d = LN(x), packed self-attention projection, self-attention (needs nothing from the encoder).
-// Phase 2: a = ctx1 Wo1^T + bo1 ; cross-attention on the encoder features ; FFN ; residuals ; pad mask ; reconstruction MSE.
-// ---------------------------------------------------------------------------------------------------------------------------------
-struct DecSeqFwdArgs {
-  const float* x; const float* feats; const int* ids;
-  const float* ln_g; const float* ln_b;
-  const float* Win1; const float* bin1; const float* Wo1; const float* bo1;
-  const float* Win2; const float* bin2; const float* Wo2; const float* bo2;
-  const float* C1; const float* c1; const float* C2; const float* c2;
-  const float* enc_in;
-  float* d; float* q1; float* k1; float* v1; float* ctx1; float* lse1; float* a;
-  float* q2; float* k2; float* v2; float* ctx2; float* lse2; float* c; float* h1;
-  float* out; double* mse_acc;
-  int B, L, mask_mode; float qscale;
-  DropDesc drop_slf, drop_enc, drop1, drop2;
-  SeqW w;
-};
-
-struct DecSeqFwd1Smem {
-  static constexpr int W = 0, Q = 3 * RS_TILE, K = Q + RS_TILE, V = K + RS_TILE;
-  static constexpr size_t TOTAL_BYTES = (size_t)(V + RS_TILE) * 2;
-};
-
-template <int HD>
-__global__ void __launch_bounds__(SQ_NT, 2) dec_seq_fwd1_kernel(DecSeqFwdArgs p) {
-  using SM = DecSeqFwd1Smem;
-  extern __shared__ __align__(16) uint8_t rs_raw[];
-  __nv_bfloat16* hb = reinterpret_cast<__nv_bfloat16*>(rs_raw);
-  __nv_bfloat16* Wt = hb + SM::W;
-  __nv_bfloat16* Qs = hb + SM::Q;
-  __nv_bfloat16* Ks = hb + SM::K;
-  __nv_bfloat16* Vs = hb + SM::V;
-  const int b = blockIdx.x, L = p.L;
-  const long long grow0 = (long long)b * L, g0 = grow0 * RS_H;
-  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
-  const int i0 = 16 * w + g, i1 = i0 + 8;
-  const bool v0 = i0 < L, v1 = i1 < L;
-  {
-    const float* const w3[3] = {p.Win1, p.Win1 + RS_H * RS_H, p.Win1 + 2 * RS_H * RS_H};
-    sq_load_weights<3>(w3, p.w, Wt);
-  }
-  float Nf[8][4];
-  frag_load(Nf, p.x + g0, i0, i1, v0, v1, t);
-  frag_ln(Nf, p.ln_g, p.ln_b, t);                     // d = LN(x): query, key and value all come from d (modules.py:668-670)
-  frag_mask_rows(Nf, v0, v1);
-  if (p.d) frag_store(p.d + g0, Nf, i0, i1, v0, v1, t);
-  sq_weights_wait();
-  __syncthreads();
-  {
-    float o[8][4];
-    frag_zero(o);
-    rs_fgemm_frag(o, Nf, Wt);
-    frag_bias_scale(o, p.bin1, p.qscale, t);
-    if (p.q1) frag_store(p.q1 + g0, o, i0, i1, v0, v1, t);
-    frag_store_tile(Qs, o, i0, i1, t);
-    frag_zero(o);
-    rs_fgemm_frag(o, Nf, Wt + RS_TILE);
-    frag_bias_scale(o, p.bin1 + RS_H, 1.f, t);
-    if (p.k1) frag_store(p.k1 + g0, o, i0, i1, v0, v1, t);
-    frag_store_tile(Ks, o, i0, i1, t);
-    frag_zero(o);
-    rs_fgemm_frag(o, Nf, Wt + 2 * RS_TILE);
-    frag_bias_scale(o, p.bin1 + 2 * RS_H, 1.f, t);
-    if (p.v1) frag_store(p.v1 + g0, o, i0, i1, v0, v1, t);
-    frag_store_tile(Vs, o, i0, i1, t);
-  }
-  __syncthreads();
-  float Cf[8][4];
-  sq_attn_fwd<HD>(Cf, Qs, Ks, Vs, L, b, p.mask_mode, p.ids + grow0, p.drop_slf, p.lse1);
-  frag_store(p.ctx1 + g0, Cf, i0, i1, v0, v1, t);
-}
-
-struct DecSeqFwd2Smem {
-  static constexpr int W = 0, Q = 7 * RS_TILE, K = Q + RS_TILE, V = K + RS_TILE;     // Wo1 Wq2 Wk2 Wv2 Wo2 C1 C2 | Q2 | K2 | V2
-  static constexpr size_t TOTAL_BYTES = (size_t)(V + RS_TILE) * 2;
-};
-
-template <int HD>
-__global__ void __launch_bounds__(SQ_NT, 2) dec_seq_fwd2_kernel(DecSeqFwdArgs p) {
-  using SM = DecSeqFwd2Smem;
-  extern __shared__ __align__(16) uint8_t rs_raw[];
-  __nv_bfloat16* hb = reinterpret_cast<__nv_bfloat16*>(rs_raw);
-  __nv_bfloat16* Wt = hb + SM::W;
-  __nv_bfloat16* Qs = hb + SM::Q;
-  __nv_bfloat16* Ks = hb + SM::K;
-  __nv_bfloat16* Vs = hb + SM::V;
-  const int b = blockIdx.x, L = p.L;
-  const long long grow0 = (long long)b * L, g0 = grow0 * RS_H;
-  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
-  const int i0 = 16 * w + g, i1 = i0 + 8;
-  const bool v0 = i0 < L, v1 = i1 < L;
-  {
-    const float* const wa[4] = {p.Wo1, p.Win2, p.Win2 + RS_H * RS_H, p.Win2 + 2 * RS_H * RS_H};
-    const float* const wb[3] = {p.Wo2, p.C1, p.C2};
-    sq_load_weights<4>(wa, p.w, Wt);
-    sq_load_weights<3>(wb, p.w, Wt + 4 * RS_TILE);
-  }
-  float Cf[8][4], Ff[8][4];
-  frag_load(Cf, p.ctx1 + g0, i0, i1, v0, v1, t);
-  frag_load(Ff, p.feats + g0, i0, i1, v0, v1, t);
-  const int keep0 = v0 ? p.ids[grow0 + i0] : 0, keep1 = v1 ? p.ids[grow0 + i1] : 0;
-  sq_weights_wait();
-  __syncthreads();
-  {
-    float a[8][4], o[8][4];
-    frag_zero(a);
-    rs_fgemm_frag(a, Cf, Wt);                         // a = ctx1 Wo1^T + bo1
-    frag_bias_scale(a, p.bo1, 1.f, t);
-    if (p.a) frag_store(p.a + g0, a, i0, i1, v0, v1, t);
-    frag_zero(o);
-    rs_fgemm_frag(o, a, Wt + RS_TILE);                // q2 = (a Wq2^T + bq2) s
-    frag_bias_scale(o, p.bin2, p.qscale, t);
-    if (p.q2) frag_store(p.q2 + g0, o, i0, i1, v0, v1, t);
-    frag_store_tile(Qs, o, i0, i1, t);
-    frag_zero(o);
-    rs_fgemm_frag(o, Ff, Wt + 2 * RS_TILE);           // k2, v2 from the encoder features
-    frag_bias_scale(o, p.bin2 + RS_H, 1.f, t);
-    if (p.k2) frag_store(p.k2 + g0, o, i0, i1, v0, v1, t);
-    frag_store_tile(Ks, o, i0, i1, t);
-    frag_zero(o);
-    rs_fgemm_frag(o, Ff, Wt + 3 * RS_TILE);
-    frag_bias_scale(o, p.bin2 + 2 * RS_H, 1.f, t);
-    if (p.v2) frag_store(p.v2 + g0, o, i0, i1, v0, v1, t);
-    frag_store_tile(Vs, o, i0, i1, t);
-  }
-  __syncthreads();
-  sq_attn_fwd<HD>(Cf, Qs, Ks, Vs, L, b, p.mask_mode, p.ids + grow0, p.drop_enc, p.lse2);
-  if (p.ctx2) frag_store(p.ctx2 + g0, Cf, i0, i1, v0, v1, t);
-  float u[8][4];
-  frag_zero(u);
-  rs_fgemm_frag(u, Cf, Wt + 4 * RS_TILE);             // c = ctx2 Wo2^T + bo2
-  frag_bias_scale(u, p.bo2, 1.f, t);
-  if (p.c) frag_store(p.c + g0, u, i0, i1, v0, v1, t);
-  float o[8][4];
-  sq_ffn_fwd(o, u, Wt + 5 * RS_TILE, Wt + 6 * RS_TILE, p.c1, p.c2, p.drop1, p.drop2, p.h1, grow0, i0, i1, v0, v1, t);
-  float res[8][4];
-  frag_load(res, p.d + g0, i0, i1, v0, v1, t);        // out = (d + FFN(c) + c) * keep  (modules.py:673-676)
-  double sq = 0.0;
-#pragma unroll
-  for (int nb = 0; nb < 8; ++nb) {
-#pragma unroll
-    for (int e = 0; e < 4; ++e) o[nb][e] += res[nb][e];
-    if (keep0 == 0) { o[nb][0] = 0.f; o[nb][1] = 0.f; }
-    if (keep1 == 0) { o[nb][2] = 0.f; o[nb][3] = 0.f; }
-  }
-  frag_store(p.out + g0, o, i0, i1, v0, v1, t);
-  if (p.enc_in && p.mse_acc) {
-    float e_[8][4];
-    frag_load(e_, p.enc_in + g0, i0, i1, v0, v1, t);
-#pragma unroll
-    for (int nb = 0; nb < 8; ++nb) {
-      if (v0) sq += (double)((e_[nb][0] - o[nb][0]) * (e_[nb][0] - o[nb][0]) + (e_[nb][1] - o[nb][1]) * (e_[nb][1] - o[nb][1]));
-      if (v1) sq += (double)((e_[nb][2] - o[nb][2]) * (e_[nb][2] - o[nb][2]) + (e_[nb][3] - o[nb][3]) * (e_[nb][3] - o[nb][3]));
-    }
-    warp_accumulate(sq, p.mse_acc);
-  }
-}
-
-
-// ---------------------------------------------------------------------------------------------------------------------------------
-// FFN adjoint shared by the encoder and decoder backward kernels (steps 1-6 of post_bwd_small_kernel).  In: G = grad wrt the block
-// output (already pad-masked), Y = saved y (enc) / c (dec) in fragments.  Out: H1-adjoint products accumulated into the weight
-// gradients, DZ = grad wrt z (enc) / c (dec).  Wt: [0] C2, [1] C1 tiles; T, X: scratch tiles.  Contains CTA barriers.
-// ---------------------------------------------------------------------------------------------------------------------------------
-template <bool IS_DEC>
-__device__ __forceinline__ void sq_ffn_bwd(float (&DZ)[8][4], const float (&G)[8][4], const float (&Y)[8][4], const float* __restrict__ h1,
-                                           const __nv_bfloat16* __restrict__ Wt, __nv_bfloat16* __restrict__ T, __nv_bfloat16* __restrict__ X,
-                                           const float* __restrict__ ln2_g, const float* __restrict__ ln2_b, float* gC1, float* gc1, float* gC2,
-                                           float* gc2, const DropDesc& drop1, const DropDesc& drop2, long long grow0, int i0, int i1, bool v0,
-                                           bool v1, int t) {
-  float A[8][4], mk[8][4];
-  frag_load(A, h1 + grow0 * RS_H, i0, i1, v0, v1, t);
-  uint32_t m1bits = 0u;
-  if (drop1.enabled) frag_drop(mk, drop1, grow0 + i0, grow0 + i1, t);
-#pragma unroll
-  for (int nb = 0; nb < 8; ++nb) {
-#pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      float x = A[nb][e];
-      if (drop1.enabled) x *= mk[nb][e];
-      A[nb][e] = fmaxf(x, 0.f);
-      if (A[nb][e] > 0.f) m1bits |= 1u << (4 * nb + e);
-    }
-  }
-  float D2[8][4];
-  if (drop2.enabled) frag_drop(mk, drop2, grow0 + i0, grow0 + i1, t);
-#pragma unroll
-  for (int nb = 0; nb < 8; ++nb) {
-#pragma unroll
-    for (int e = 0; e < 4; ++e) D2[nb][e] = drop2.enabled ? G[nb][e] * mk[nb][e] : G[nb][e];
-  }
-  frag_store_tile(T, D2, i0, i1, t);
-  frag_store_tile(X, A, i0, i1, t);
-  __syncthreads();
-  rs_wgrad_rm(T, X, gC2, gc2);                        // dC2 += dh2^T a ; dc2 += colsum(dh2)
-  float H1[8][4];
-  frag_zero(H1);
-  rs_dgrad_frag(H1, D2, Wt);                          // da = dh2 C2 ; dh1 = da [a > 0] m1
-  {
-    const float sc1 = drop1.enabled ? drop1.scale : 1.f;
-#pragma unroll
-    for (int nb = 0; nb < 8; ++nb) {
-#pragma unroll
-      for (int e = 0; e < 4; ++e) H1[nb][e] = (m1bits >> (4 * nb + e)) & 1u ? H1[nb][e] * sc1 : 0.f;
-    }
-  }
-  __syncthreads();                                    // everybody is done with T / X
-  {
-    float Z[8][4];
-#pragma unroll
-    for (int nb = 0; nb < 8; ++nb) { Z[nb][0] = Y[nb][0]; Z[nb][1] = Y[nb][1]; Z[nb][2] = Y[nb][2]; Z[nb][3] = Y[nb][3]; }
-    if (!IS_DEC) {
-      frag_ln(Z, ln2_g, ln2_b, t);
-      frag_mask_rows(Z, v0, v1);
-    }
-    frag_store_tile(X, Z, i0, i1, t);
-  }
-  frag_store_tile(T, H1, i0, i1, t);
-  __syncthreads();
-  rs_wgrad_rm(T, X, gC1, gc1);                        // dC1 += dh1^T z ; dc1 += colsum(dh1)
-#pragma unroll
-  for (int nb = 0; nb < 8; ++nb) { DZ[nb][0] = G[nb][0]; DZ[nb][1] = G[nb][1]; DZ[nb][2] = G[nb][2]; DZ[nb][3] = G[nb][3]; }
-  rs_dgrad_frag(DZ, H1, Wt + RS_TILE);                // dz (enc) / dc (dec) = dO + dh1 C1
-}
-
-// ---------------------------------------------------------------------------------------------------------------------------------
-// Encoder block backward, one sequence per CTA: post adjoint -> attention adjoint -> in-projection / LayerNorm adjoint.
-// ---------------------------------------------------------------------------------------------------------------------------------
-struct EncSeqBwdArgs {
-  const float* x; const int* ids;
-  const float* q; const float* k; const float* v; const float* ctx; const float* lse; const float* y; const float* h1;
-  const float* ln1_g; const float* ln1_b; const float* Win; const float* Wo; const float* ln2_g; const float* ln2_b;
-  const float* C1; const float* C2; const float* Wsp; const float* bsp;
-  const float* dout; const float* dx_extra; const float* drec; float nll_coef;
-  float* dx;
-  float* gln1_g; float* gln1_b; float* gWin; float* gbin; float* gWo; float* gbo; float* gln2_g; float* gln2_b;
-  float* gC1; float* gc1; float* gC2; float* gc2; float* gWsp; float* gbsp;
-  int B, L, mask_mode; float qscale;
-  DropDesc drop_attn, drop1, drop2;
-  SeqW w;
-};
-
-struct SeqBwdSmem {      // halfword offsets: 4 weight slots + 8 work tiles = 110,592 bytes (two CTAs per SM)
-  static constexpr int W = 0, A0 = 4 * RS_TILE;
-  static constexpr size_t TOTAL_BYTES = (size_t)(A0 + 8 * RS_TILE) * 2;
-};
-
-template <int HD>
-__global__ void __launch_bounds__(SQ_NT, 2) enc_seq_bwd_kernel(EncSeqBwdArgs p) {
-  using SM = SeqBwdSmem;
-  constexpr int NH = RS_H / HD;
-  extern __shared__ __align__(16) uint8_t rs_raw[];
-  __nv_bfloat16* hb = reinterpret_cast<__nv_bfloat16*>(rs_raw);
-  __nv_bfloat16* Wt = hb + SM::W;
-  __nv_bfloat16* Cs = hb + SM::A0;                    // ctx            -> Tq
-  __nv_bfloat16* T = Cs + RS_TILE;                    // T   -> dSt     -> Tk
-  __nv_bfloat16* X = T + RS_TILE;                     // X   -> Pt      -> Tv
-  __nv_bfloat16* A3 = X + RS_TILE;                    // head logits    -> Nb
-  __nv_bfloat16* Qs = A3 + RS_TILE;
-  __nv_bfloat16* Ks = Qs + RS_TILE;
-  __nv_bfloat16* Vs = Ks + RS_TILE;
-  __nv_bfloat16* dCs = Vs + RS_TILE;                  // dctx           -> Xb
-  float* lgs = reinterpret_cast<float*>(A3);
-  const int b = blockIdx.x, L = p.L;
-  const long long grow0 = (long long)b * L, g0 = grow0 * RS_H;
-  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
-  const int i0 = 16 * w + g, i1 = i0 + 8;
-  const bool v0 = i0 < L, v1 = i1 < L;
-  {
-    const float* const w3[3] = {p.C2, p.C1, p.Wo};
-    sq_load_weights<3>(w3, p.w, Wt);
-  }
-  {
-    const float* const src[4] = {p.q + g0, p.k + g0, p.v + g0, p.ctx + g0};
-    const long long ld[4] = {RS_H, RS_H, RS_H, RS_H};
-    const int nr[4] = {L, L, L, L};
-    const float sc[4] = {1.f, 1.f, 1.f, 1.f};
-    __nv_bfloat16* const d[4] = {Qs, Ks, Vs, Cs};
-    __nv_bfloat16* const dT[4] = {nullptr, nullptr, nullptr, nullptr};
-    float* const dF[4] = {nullptr, nullptr, nullptr, nullptr};
-    rs_load<4>(src, ld, nr, sc, d, dT, dF);
-  }
-  // ---- post adjoint
-  float G[8][4], Y[8][4];
-  frag_load(G, p.dout ? p.dout + g0 : nullptr, i0, i1, v0, v1, t);
-  {
-    const int k0 = v0 ? p.ids[grow0 + i0] : 0, k1 = v1 ? p.ids[grow0 + i1] : 0;
-#pragma unroll
-    for (int nb = 0; nb < 8; ++nb) {
-      if (k0 == 0) { G[nb][0] = 0.f; G[nb][1] = 0.f; }
-      if (k1 == 0) { G[nb][2] = 0.f; G[nb][3] = 0.f; }
-    }
-  }
-  frag_load(Y, p.y + g0, i0, i1, v0, v1, t);
-  sq_weights_wait();
-  float DZ[8][4];
-  sq_ffn_bwd<false>(DZ, G, Y, p.h1, Wt, T, X, p.ln2_g, p.ln2_b, p.gC1, p.gc1, p.gC2, p.gc2, p.drop1, p.drop2, grow0, i0, i1, v0, v1, t);
-  frag_ln_bwd(DZ, Y, p.ln2_g, p.gln2_g, p.gln2_b, v0, v1, g, t);          // dy = LN2^T(dz): also the residual grad reaching Qn
-  __syncthreads();                                    // everybody is done with T / X of the FFN adjoint
-  frag_store_tile(T, DZ, i0, i1, t);
-  __syncthreads();
-  rs_wgrad_rm(T, Cs, p.gWo, p.gbo);                   // dWo += dy^T ctx ; dbo += colsum(dy)
-  float DC[8][4];
-  frag_zero(DC);
-  rs_dgrad_frag(DC, DZ, Wt + 2 * RS_TILE);            // dctx = dy Wo
-  if (p.nll_coef != 0.f || p.drec) {                  // independence-head adjoint (per-head logits from the bf16 context tile)
-    constexpr int n2 = NH * NH;
-    float* dbs = lgs + 64 * n2;
-    for (int i = threadIdx.x; i < NH; i += SQ_NT) dbs[i] = 0.f;
-    __syncthreads();
-    for (int i = threadIdx.x; i < 64 * NH; i += SQ_NT) {
-      const int r = i / NH, c = i - r * NH;
-      float* lg = lgs + r * n2 + c * NH;
-      if (r >= L) {
-#pragma unroll
-        for (int j = 0; j < NH; ++j) lg[j] = 0.f;
-        continue;
-      }
-      float l_[NH];
-      float mx = -INFINITY;
-#pragma unroll
-      for (int j = 0; j < NH; ++j) {
-        float sacc = 0.f;
-        for (int dd = 0; dd < HD; ++dd) sacc = fmaf(__bfloat162float(Cs[r * RS_LD + c * HD + dd]), __ldg(p.Wsp + j * HD + dd), sacc);
-        l_[j] = sacc + __ldg(p.bsp + j);
-        mx = fmaxf(mx, l_[j]);
-      }
-      float se = 0.f;
-#pragma unroll
-      for (int j = 0; j < NH; ++j) se += expf(l_[j] - mx);
-      const float* dr = p.drec ? p.drec + ((grow0 + r) * NH + c) * NH : nullptr;
-      float gsum = 0.f;
-      if (dr) {
-#pragma unroll
-        for (int j = 0; j < NH; ++j) gsum += dr[j];
-      }
-#pragma unroll
-      for (int j = 0; j < NH; ++j) {
-        const float pj = expf(l_[j] - mx) / se;
-        float dl = p.nll_coef * (pj - (j == c ? 1.f : 0.f));
-        if (dr) dl += dr[j] - pj * gsum;
-        lg[j] = dl;
-        atomicAdd(dbs + j, dl);
-      }
-    }
-    __syncthreads();
-#pragma unroll
-    for (int nb = 0; nb < 8; ++nb) {
-#pragma unroll
-      for (int e = 0; e < 4; ++e) {
-        const int r = e < 2 ? i0 : i1, col = 8 * nb + 2 * t + (e & 1), c = col / HD, dd = col - c * HD;
-        const float* dl = lgs + r * n2 + c * NH;
-        float add = 0.f;
-#pragma unroll
-        for (int j = 0; j < NH; ++j) add = fmaf(dl[j], __ldg(p.Wsp + j * HD + dd), add);
-        DC[nb][e] += add;
-      }
-    }
-    for (int i = threadIdx.x; i < NH * HD; i += SQ_NT) {
-      const int j = i / HD, dd = i - j * HD;
-      float accw = 0.f;
-      for (int r = 0; r < L; ++r)
-#pragma unroll
-        for (int c = 0; c < NH; ++c) accw = fmaf(lgs[r * n2 + c * NH + j], __bfloat162float(Cs[r * RS_LD + c * HD + dd]), accw);
-      atomicAdd(p.gWsp + i, accw);
-    }
-    for (int i = threadIdx.x; i < NH; i += SQ_NT) atomicAdd(p.gbsp + i, dbs[i]);
-  }
-  // ---- attention adjoint (the in-projection weights stream into the weight slots meanwhile)
-  __syncthreads();                                    // everybody is done with the stage-1 weights, T, X, Cs and the head scratch
-  {
-    const float* const w3[3] = {p.Win, p.Win + RS_H * RS_H, p.Win + 2 * RS_H * RS_H};
-    sq_load_weights<3>(w3, p.w, Wt);
-  }
-  frag_store_tile(dCs, DC, i0, i1, t);
-  __syncthreads();
-  float DQ[8][4], DK[8][4], DV[8][4];
-  sq_attn_bwd<HD>(DQ, DK, DV, Qs, Ks, Vs, dCs, T, X, L, b, p.mask_mode, p.ids + grow0, p.drop_attn, p.lse);
-  __syncthreads();                                    // everybody is done with the attention operands and scratch
-  // ---- in-projection + LayerNorm adjoint
-  __nv_bfloat16* Tq = Cs; __nv_bfloat16* Tk = T; __nv_bfloat16* Tv = X; __nv_bfloat16* Nb = A3; __nv_bfloat16* Xb = dCs;
-#pragma unroll
-  for (int nb = 0; nb < 8; ++nb) {
-#pragma unroll
-    for (int e = 0; e < 4; ++e) DQ[nb][e] *= p.qscale;
-  }
-  frag_store_tile(Tq, DQ, i0, i1, t);
-  frag_store_tile(Tk, DK, i0, i1, t);
-  frag_store_tile(Tv, DV, i0, i1, t);
-  float Xf[8][4];
-  frag_load(Xf, p.x + g0, i0, i1, v0, v1, t);
-  {
-    float Nf[8][4];
-#pragma unroll
-    for (int nb = 0; nb < 8; ++nb) { Nf[nb][0] = Xf[nb][0]; Nf[nb][1] = Xf[nb][1]; Nf[nb][2] = Xf[nb][2]; Nf[nb][3] = Xf[nb][3]; }
-    frag_ln(Nf, p.ln1_g, p.ln1_b, t);
-    frag_mask_rows(Nf, v0, v1);
-    frag_store_tile(Nb, Nf, i0, i1, t);
-    frag_store_tile(Xb, Xf, i0, i1, t);
-  }
-  sq_weights_wait();
-  __syncthreads();
-  float D[8][4];
-  frag_zero(D);
-  rs_wgrad_rm(Tq, Nb, p.gWin, p.gbin);
-  rs_dgrad_frag(D, DQ, Wt);
-#pragma unroll
-  for (int nb = 0; nb < 8; ++nb) { D[nb][0] += DZ[nb][0]; D[nb][1] += DZ[nb][1]; D[nb][2] += DZ[nb][2]; D[nb][3] += DZ[nb][3]; }
-  frag_ln_bwd(D, Xf, p.ln1_g, p.gln1_g, p.gln1_b, v0, v1, g, t);          // encoder: k, v come from x itself
-  rs_wgrad_rm(Tk, Xb, p.gWin + (long long)RS_H * RS_H, p.gbin + RS_H);
-  rs_dgrad_frag(D, DK, Wt + RS_TILE);
-  rs_wgrad_rm(Tv, Xb, p.gWin + 2ll * RS_H * RS_H, p.gbin + 2 * RS_H);
-  rs_dgrad_frag(D, DV, Wt + 2 * RS_TILE);
-  if (p.dx_extra) {
-    float E[8][4];
-    frag_load(E, p.dx_extra + g0, i0, i1, v0, v1, t);
-#pragma unroll
-    for (int nb = 0; nb < 8; ++nb) { D[nb][0] += E[nb][0]; D[nb][1] += E[nb][1]; D[nb][2] += E[nb][2]; D[nb][3] += E[nb][3]; }
-  }
-  frag_store(p.dx + g0, D, i0, i1, v0, v1, t);
-}
-
-// ---------------------------------------------------------------------------------------------------------------------------------
-// Decoder block backward.  Phase 2: FFN + cross-attention adjoints + the adjoint of (self-attention out-projection, cross-attention
-// in-projection) -> dfeats (+=), dctx1, dd.  Phase 1: self-attention + LayerNorm adjoints -> dx (needs nothing the encoder backward
-// waits for, so it may run beside it on another stream).
-// ---------------------------------------------------------------------------------------------------------------------------------
-struct DecSeqBwdArgs {
-  const float* x; const float* feats; const int* ids;
-  const float* d; const float* q1; const float* k1; const float* v1; const float* ctx1; const float* lse1; const float* a;
-  const float* q2; const float* k2; const float* v2; const float* ctx2; const float* lse2; const float* c; const float* h1;
-  const float* out; const float* enc_in; float mse_coef;
-  const float* ln_g; const float* ln_b; const float* Win1; const float* Wo1; const float* Win2; const float* Wo2; const float* C1; const float* C2;
-  const float* dout; float* denc;
-  float* dd; float* dctx1; float* dfeats; float* dx;
-  float* gln_g; float* gln_b; float* gWin1; float* gbin1; float* gWo1; float* gbo1; float* gWin2; float* gbin2; float* gWo2; float* gbo2;
-  float* gC1; float* gc1; float* gC2; float* gc2;
-  int B, L, mask_mode; float qscale;
-  DropDesc drop_slf, drop_enc, drop1, drop2;
-  SeqW w;
-};
-
-template <int HD>
-__global__ void __launch_bounds__(SQ_NT, 2) dec_seq_bwd2_kernel(DecSeqBwdArgs p) {
-  using SM = SeqBwdSmem;
-  extern __shared__ __align__(16) uint8_t rs_raw[];
-  __nv_bfloat16* hb = reinterpret_cast<__nv_bfloat16*>(rs_raw);
-  __nv_bfloat16* Wt = hb + SM::W;
-  __nv_bfloat16* Cs = hb + SM::A0;                    // ctx2           -> Tq2 (dq2 s)
-  __nv_bfloat16* T = Cs + RS_TILE;                    // T   -> dSt     -> dk2
-  __nv_bfloat16* X = T + RS_TILE;                     // X   -> Pt      -> dv2
-  __nv_bfloat16* A3 = X + RS_TILE;                    //                   a -> feats -> ctx1
-  __nv_bfloat16* Qs = A3 + RS_TILE;
-  __nv_bfloat16* Ks = Qs + RS_TILE;
-  __nv_bfloat16* Vs = Ks + RS_TILE;
-  __nv_bfloat16* dCs = Vs + RS_TILE;                  // dctx2          -> da
-  const int b = blockIdx.x, L = p.L;
-  const long long grow0 = (long long)b * L, g0 = grow0 * RS_H;
-  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
-  const int i0 = 16 * w + g, i1 = i0 + 8;
-  const bool v0 = i0 < L, v1 = i1 < L;
-  {
-    const float* const w3[3] = {p.C2, p.C1, p.Wo2};
-    sq_load_weights<3>(w3, p.w, Wt);
-  }
-  {
-    const float* const src[4] = {p.q2 + g0, p.k2 + g0, p.v2 + g0, p.ctx2 + g0};
-    const long long ld[4] = {RS_H, RS_H, RS_H, RS_H};
-    const int nr[4] = {L, L, L, L};
-    const float sc[4] = {1.f, 1.f, 1.f, 1.f};
-    __nv_bfloat16* const d[4] = {Qs, Ks, Vs, Cs};
-    __nv_bfloat16* const dT[4] = {nullptr, nullptr, nullptr, nullptr};
-    float* const dF[4] = {nullptr, nullptr, nullptr, nullptr};
-    rs_load<4>(src, ld, nr, sc, d, dT, dF);
-  }
-  float G[8][4], Y[8][4];
-  frag_load(G, p.dout ? p.dout + g0 : nullptr, i0, i1, v0, v1, t);
-  if (p.enc_in) {                                     // reconstruction term: d/d out of lambda1 * mean((enc_in - out)^2)
-    float O[8][4], E[8][4];
-    frag_load(O, p.out + g0, i0, i1, v0, v1, t);
-    frag_load(E, p.enc_in + g0, i0, i1, v0, v1, t);
-#pragma unroll
-    for (int nb = 0; nb < 8; ++nb) {
-#pragma unroll
-      for (int e = 0; e < 4; ++e) { O[nb][e] = p.mse_coef * (O[nb][e] - E[nb][e]); G[nb][e] += O[nb][e]; O[nb][e] = -O[nb][e]; }
-    }
-    if (p.denc) frag_store(p.denc + g0, O, i0, i1, v0, v1, t);
-  }
-  {
-    const int k0 = v0 ? p.ids[grow0 + i0] : 0, k1 = v1 ? p.ids[grow0 + i1] : 0;
-#pragma unroll
-    for (int nb = 0; nb < 8; ++nb) {
-      if (k0 == 0) { G[nb][0] = 0.f; G[nb][1] = 0.f; }
-      if (k1 == 0) { G[nb][2] = 0.f; G[nb][3] = 0.f; }
-    }
-  }
-  frag_store(p.dd + g0, G, i0, i1, v0, v1, t);        // dd = dO (the residual on d)
-  frag_load(Y, p.c + g0, i0, i1, v0, v1, t);
-  sq_weights_wait();
-  float DZ[8][4];
-  sq_ffn_bwd<true>(DZ, G, Y, p.h1, Wt, T, X, nullptr, nullptr, p.gC1, p.gc1, p.gC2, p.gc2, p.drop1, p.drop2, grow0, i0, i1, v0, v1, t);
-  __syncthreads();
-  frag_store_tile(T, DZ, i0, i1, t);
-  __syncthreads();
-  rs_wgrad_rm(T, Cs, p.gWo2, p.gbo2);                 // dWo2 += dc^T ctx2
-  float DC[8][4];
-  frag_zero(DC);
-  rs_dgrad_frag(DC, DZ, Wt + 2 * RS_TILE);            // dctx2 = dc Wo2
-  __syncthreads();
-  {
-    const float* const w4[4] = {p.Win2, p.Win2 + RS_H * RS_H, p.Win2 + 2 * RS_H * RS_H, p.Wo1};
-    sq_load_weights<4>(w4, p.w, Wt);
-  }
-  frag_store_tile(dCs, DC, i0, i1, t);
-  __syncthreads();
-  float DQ[8][4], DK[8][4], DV[8][4];
-  sq_attn_bwd<HD>(DQ, DK, DV, Qs, Ks, Vs, dCs, T, X, L, b, p.mask_mode, p.ids + grow0, p.drop_enc, p.lse2);
-  __syncthreads();
-  // ---- adjoint of: a = ctx1 Wo1^T + bo1 ; q2 = (a Wq2^T + bq2) s ; k2, v2 = feats Wkv2^T + bkv2
-  __nv_bfloat16* Tq = Cs; __nv_bfloat16* Tk = T; __nv_bfloat16* Tv = X; __nv_bfloat16* Xa = A3; __nv_bfloat16* DAs = dCs;
-#pragma unroll
-  for (int nb = 0; nb < 8; ++nb) {
-#pragma unroll
-    for (int e = 0; e < 4; ++e) DQ[nb][e] *= p.qscale;
-  }
-  frag_store_tile(Tq, DQ, i0, i1, t);
-  frag_store_tile(Tk, DK, i0, i1, t);
-  frag_store_tile(Tv, DV, i0, i1, t);
-  rs_load1(p.a + g0, L, 1.f, Xa);
-  sq_weights_wait();
-  __syncthreads();
-  rs_wgrad_rm(Tq, Xa, p.gWin2, p.gbin2);
-  float DA[8][4];
-  frag_zero(DA);
-  rs_dgrad_frag(DA, DQ, Wt);                          // da = (dq2 s) Wq2
-  frag_store_tile(DAs, DA, i0, i1, t);
-  __syncthreads();                                    // everybody is done with Xa == a
-  rs_load1(p.feats + g0, L, 1.f, Xa);
-  __syncthreads();
-  rs_wgrad_rm(Tk, Xa, p.gWin2 + (long long)RS_H * RS_H, p.gbin2 + RS_H);
-  rs_wgrad_rm(Tv, Xa, p.gWin2 + 2ll * RS_H * RS_H, p.gbin2 + 2 * RS_H);
-  {
-    float D[8][4];
-    frag_zero(D);
-    rs_dgrad_frag(D, DK, Wt + RS_TILE);
-    rs_dgrad_frag(D, DV, Wt + 2 * RS_TILE);
-#pragma unroll
-    for (int nb = 0; nb < 8; ++nb) {                  // dfeats += : the sequence's rows belong to this CTA alone
-      const int c = 8 * nb + 2 * t;
-      if (v0) { float2* dp = reinterpret_cast<float2*>(p.dfeats + g0 + (long long)i0 * RS_H + c); const float2 o = *dp; *dp = make_float2(o.x + D[nb][0], o.y + D[nb][1]); }
-      if (v1) { float2* dp = reinterpret_cast<float2*>(p.dfeats + g0 + (long long)i1 * RS_H + c); const float2 o = *dp; *dp = make_float2(o.x + D[nb][2], o.y + D[nb][3]); }
-    }
-  }
-  __syncthreads();                                    // everybody is done with Xa == feats
-  rs_load1(p.ctx1 + g0, L, 1.f, Xa);
-  __syncthreads();
-  rs_wgrad_rm(DAs, Xa, p.gWo1, p.gbo1);
-  {
-    float D[8][4];
-    frag_zero(D);
-    rs_dgrad_frag(D, DA, Wt + 3 * RS_TILE);           // dctx1 = da Wo1
-    frag_store(p.dctx1 + g0, D, i0, i1, v0, v1, t);
-  }
-}
-
-template <int HD>
-__global__ void __launch_bounds__(SQ_NT, 2) dec_seq_bwd1_kernel(DecSeqBwdArgs p) {
-  using SM = SeqBwdSmem;
-  extern __shared__ __align__(16) uint8_t rs_raw[];
-  __nv_bfloat16* hb = reinterpret_cast<__nv_bfloat16*>(rs_raw);
-  __nv_bfloat16* Wt = hb + SM::W;
-  __nv_bfloat16* Tq = hb + SM::A0;
-  __nv_bfloat16* T = Tq + RS_TILE;                    // dSt -> Tk
-  __nv_bfloat16* X = T + RS_TILE;                     // Pt  -> Tv
-  __nv_bfloat16* Nb = X + RS_TILE;
-  __nv_bfloat16* Qs = Nb + RS_TILE;
-  __nv_bfloat16* Ks = Qs + RS_TILE;
-  __nv_bfloat16* Vs = Ks + RS_TILE;
-  __nv_bfloat16* dCs = Vs + RS_TILE;
-  const int b = blockIdx.x, L = p.L;
-  const long long grow0 = (long long)b * L, g0 = grow0 * RS_H;
-  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
-  const int i0 = 16 * w + g, i1 = i0 + 8;
-  const bool v0 = i0 < L, v1 = i1 < L;
-  {
-    const float* const w3[3] = {p.Win1, p.Win1 + RS_H * RS_H, p.Win1 + 2 * RS_H * RS_H};
-    sq_load_weights<3>(w3, p.w, Wt);
-  }
-  {
-    const float* const src[4] = {p.q1 + g0, p.k1 + g0, p.v1 + g0, p.dctx1 + g0};
-    const long long ld[4] = {RS_H, RS_H, RS_H, RS_H};
-    const int nr[4] = {L, L, L, L};
-    const float sc[4] = {1.f, 1.f, 1.f, 1.f};
-    __nv_bfloat16* const d[4] = {Qs, Ks, Vs, dCs};
-    __nv_bfloat16* const dT[4] = {nullptr, nullptr, nullptr, nullptr};
-    float* const dF[4] = {nullptr, nullptr, nullptr, nullptr};
-    rs_load<4>(src, ld, nr, sc, d, dT, dF);
-  }
-  float Xf[8][4];
-  frag_load(Xf, p.x + g0, i0, i1, v0, v1, t);
-  {
-    float Nf[8][4];
-#pragma unroll
-    for (int nb = 0; nb < 8; ++nb) { Nf[nb][0] = Xf[nb][0]; Nf[nb][1] = Xf[nb][1]; Nf[nb][2] = Xf[nb][2]; Nf[nb][3] = Xf[nb][3]; }
-    frag_ln(Nf, p.ln_g, p.ln_b, t);
-    frag_mask_rows(Nf, v0, v1);
-    frag_store_tile(Nb, Nf, i0, i1, t);
-  }
-  __syncthreads();
-  float DQ[8][4], DK[8][4], DV[8][4];
-  sq_attn_bwd<HD>(DQ, DK, DV, Qs, Ks, Vs, dCs, T, X, L, b, p.mask_mode, p.ids + grow0, p.drop_slf, p.lse1);
-  __syncthreads();
-  __nv_bfloat16* Tk = T; __nv_bfloat16* Tv = X;
-#pragma unroll
-  for (int nb = 0; nb < 8; ++nb) {
-#pragma unroll
-    for (int e = 0; e < 4; ++e) DQ[nb][e] *= p.qscale;
-  }
-  frag_store_tile(Tq, DQ, i0, i1, t);
-  frag_store_tile(Tk, DK, i0, i1, t);
-  frag_store_tile(Tv, DV, i0, i1, t);
-  sq_weights_wait();
-  __syncthreads();
-  float D[8][4];
-  frag_zero(D);
-  rs_wgrad_rm(Tq, Nb, p.gWin1, p.gbin1);
-  rs_dgrad_frag(D, DQ, Wt);
-  rs_wgrad_rm(Tk, Nb, p.gWin1 + (long long)RS_H * RS_H, p.gbin1 + RS_H);
-  rs_dgrad_frag(D, DK, Wt + RS_TILE);
-  rs_wgrad_rm(Tv, Nb, p.gWin1 + 2ll * RS_H * RS_H, p.gbin1 + 2 * RS_H);
-  rs_dgrad_frag(D, DV, Wt + 2 * RS_TILE);
-  {
-    float E[8][4];
-    frag_load(E, p.dd + g0, i0, i1, v0, v1, t);       // the residual on d = LN(x) (and the grad reaching d through nothing else)
-#pragma unroll
-    for (int nb = 0; nb < 8; ++nb) { D[nb][0] += E[nb][0]; D[nb][1] += E[nb][1]; D[nb][2] += E[nb][2]; D[nb][3] += E[nb][3]; }
-  }
-  frag_ln_bwd(D, Xf, p.ln_g, p.gln_g, p.gln_b, v0, v1, g, t);             // decoder: q, k, v all come from LN(x)
-  frag_store(p.dx + g0, D, i0, i1, v0, v1, t);
 }
 
 }  // namespace adt

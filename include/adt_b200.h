@@ -71,7 +71,7 @@ typedef struct { float* w1; float* b1; float* w2; float* b2; } adt_ffn_g;
  * adt_adam (mirror / mirror_n) or adt_to_bf16; base32 segments must start on 8-element boundaries.  bf16 == NULL: kernels convert the
  * fp32 weights on the fly. */
 typedef struct { const float* base32; const void* bf16; } adt_wmirror;
-/* 1 when the sequence-resident block kernels (one CTA per sequence, a whole block per launch) serve this shape / precision */
+/* 1 when the sequence-resident encoder forward (evaluation; one CTA per sequence, a whole block per launch) serves this shape / precision */
 int adt_seq_kernels_apply(int32_t L, int32_t H, int32_t nh, int32_t precision);
 
 /* Encoder block -- EncoderLayer.forward, sasrec/modules.py:644-655 (+ MultiheadAttentionADT :270-527,
@@ -93,8 +93,8 @@ typedef struct {
                       the tail of the LAST block on those rows only */
   adt_wmirror wm;  /* optional bf16 mirror of the parameters (see adt_wmirror) */
   float* out_last; /* optional [B][H]: the block output of the LAST position of every sequence (predict reads nothing else,
-                      sasrec/model.py:89); `out` may then be NULL.  Only honoured by the sequence-resident kernels (phase 0, precision 1,
-                      H == 64, L <= 64, nh in {1,2,4}); otherwise ignored, so callers must check adt_seq_kernels_apply() first */
+                      sasrec/model.py:89); `out` may then be NULL.  Only honoured by the sequence-resident kernel (phase 0, training 0,
+                      precision 1, H == 64, L <= 64, nh in {1,2,4}); otherwise ignored, so callers must check adt_seq_kernels_apply() first */
   void* tc_scratch; /* optional, adt_workspace_sizes.fwd_scratch bytes (precision 1, H >= 128, H % 64 == 0, phase 0): every linear layer
                        then runs as one tcgen05 GEMM over all rows (block_tc.cuh) instead of inside the row-tile kernels */
   void* attn_scratch; /* adt_workspace_sizes.attn_scratch bytes, required when L > 256 (fused flash attention; NULL otherwise) */

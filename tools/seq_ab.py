@@ -1,4 +1,4 @@
-"""A/B of the sequence-resident block kernels against the three/five-kernel row-tile path on the C2 shape (run twice, with
+"""A/B of the sequence-resident evaluation encoder against the three-kernel row-tile forward on the C2 shape (run twice, with
 ADT_SEQ_FUSED=0 and =1; tests/test_round2_gpu.py compares the two JSON lines), and -- with a hidden size >= 128 -- of the hoisted tcgen05
 weight gradients against the in-kernel ones (ADT_WGRAD_HOIST=1 / 0).   python tools/seq_ab.py [nh] [L] [hidden]"""
 import json, os, sys, types
