@@ -1409,11 +1409,12 @@ extern "C" int adt_act_fwd(const float* x, float* y, int64_t n, int32_t act, adt
   act_fwd_kernel<<<(int)(blocks < 148 * 16 ? (blocks > 0 ? blocks : 1) : 148 * 16), 256, 0, (cudaStream_t)s_>>>(x, y, n4, act);
   return check_launch("act_fwd");
 }
+static const size_t WATTN_SMEM_MAX = 220 * 1024;   // shared memory of the resident Wasserstein attention kernels
 static int launch_wattn(const adt_wattention_args* a, bool bwd, cudaStream_t s) {
   if (a->B <= 0 || a->L <= 0 || a->nh <= 0 || a->H % a->nh || ((a->H / a->nh) & 3)) return fail(ADT_E_SHAPE, "%s", "wattention: dims");
   const int hd = a->H / a->nh;
   const size_t smem = wattn_smem_floats(a->L, hd, bwd) * sizeof(float);
-  if (smem > 220 * 1024) return fail(ADT_E_SHAPE, "%s", "wattention: (L, H/nh) tile does not fit shared memory");
+  if (smem > WATTN_SMEM_MAX) return fail(ADT_E_SHAPE, "%s", "wattention: (L, H/nh) tile does not fit shared memory");
   WAttnArgs p;
   p.mq = a->mq; p.cq = a->cq; p.mk = a->mk; p.ck = a->ck; p.mv = a->mv; p.cv = a->cv; p.mctx = a->mctx; p.cctx = a->cctx; p.lse = a->lse;
   p.key_ids = a->key_ids; p.dmctx = a->dmctx; p.dcctx = a->dcctx; p.dmq = a->dmq; p.dcq = a->dcq; p.dmk = a->dmk; p.dck = a->dck;
@@ -1431,6 +1432,44 @@ static int launch_wattn(const adt_wattention_args* a, bool bwd, cudaStream_t s) 
 }
 extern "C" int adt_wattention_fwd(const adt_wattention_args* a, adt_stream_t s_) { return launch_wattn(a, false, (cudaStream_t)s_); }
 extern "C" int adt_wattention_bwd(const adt_wattention_args* a, adt_stream_t s_) { return launch_wattn(a, true, (cudaStream_t)s_); }
+extern "C" int adt_wattention_resident_fits(int32_t L, int32_t H, int32_t nh, int32_t backward) {
+  if (L <= 0 || nh <= 0 || H <= 0 || H % nh || ((H / nh) & 3)) return fail(ADT_E_SHAPE, "%s", "wattention_resident_fits: dims");
+  return wattn_smem_floats(L, H / nh, backward != 0) * sizeof(float) <= WATTN_SMEM_MAX ? 1 : 0;
+}
+
+// ---- the same core beyond the resident kernels' shared memory: fused tcgen05 Wasserstein flash attention (wflash_tc.cu) ----------
+namespace adt {
+long long wflash_scratch_bytes(int B, int L, int H, int nh, bool bwd);
+int wattn_flash(const adt_wattention_args* a, const DropDesc& d, bool bwd, cudaStream_t s);
+}
+static int check_wflash_dims(int B, int L, int H, int nh) {
+  if (B <= 0 || L <= 0 || nh <= 0 || H <= 0 || H % nh) return fail(ADT_E_SHAPE, "%s", "wattention flash: dims (B, L, nh > 0, H % nh == 0)");
+  if (L > FLASH_MAX_L) return fail(ADT_E_SHAPE, "%s", "wattention flash: L > 2048 (the longest sequence the Wasserstein flash attention serves)");
+  if ((H / nh) % 16) return fail(ADT_E_SHAPE, "%s", "wattention flash: the head size H/nh must be a multiple of 16");
+  if (H / nh > 64)
+    return fail(ADT_E_SHAPE, "%s", "wattention flash: the head size H/nh must be at most 64 (score operands [mean | sqrt cov] of 2 H/nh <= 128 "
+                                  "columns)");
+  return ADT_OK;
+}
+extern "C" int64_t adt_wattention_scratch_bytes(int32_t B, int32_t L, int32_t H, int32_t nh, int32_t backward) {
+  if (check_wflash_dims(B, L, H, nh)) return -1;
+  return wflash_scratch_bytes(B, L, H, nh, backward != 0);
+}
+static int launch_wflash(const adt_wattention_args* a, bool bwd, cudaStream_t s) {
+  if (int e = check_wflash_dims(a->B, a->L, a->H, a->nh)) return e;
+  if (!a->tc_scratch) return fail(ADT_E_SHAPE, "%s", "wattention flash: tc_scratch is NULL (adt_wattention_scratch_bytes bytes)");
+  if (!a->key_ids || !a->lse) return fail(ADT_E_SHAPE, "%s", "wattention flash: key_ids and lse are required");
+  if (bwd && (!a->mctx_in || !a->cctx_in || !a->dmctx || !a->dcctx))
+    return fail(ADT_E_SHAPE, "%s", "wattention flash backward: mctx_in / cctx_in (the forward's outputs) and dmctx / dcctx are required");
+  const char* what = bwd ? "wattention_flash_bwd" : "wattention_flash_fwd";
+  if (int e = wattn_flash(a, mk_drop(a->drop), bwd, s)) {
+    if (int c = check_launch(what)) return c;
+    return fail(e, "%s", "wattention flash: TMA descriptor encoding failed");
+  }
+  return check_launch(what);
+}
+extern "C" int adt_wattention_flash_fwd(const adt_wattention_args* a, adt_stream_t s_) { return launch_wflash(a, false, (cudaStream_t)s_); }
+extern "C" int adt_wattention_flash_bwd(const adt_wattention_args* a, adt_stream_t s_) { return launch_wflash(a, true, (cudaStream_t)s_); }
 
 static WBprArgs mk_wbpr(const adt_wbpr_args* a) {
   WBprArgs p;

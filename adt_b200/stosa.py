@@ -5,7 +5,9 @@ num_layers, num_heads, dropout, attention_dropout, initializer_range`; `finetune
 7-tuple; parameter names/shapes identical so reference checkpoints load) and stosa/modules.py (DistAttention,
 DistEDAttention, DistIntermediate, DistLayer, DistDecLayer).  Two streams (mean, covariance) run through the generic
 linear / dropout+residual+LayerNorm kernels; the Wasserstein attention core (scores in matmul form, additive
-padding*causal mask, softmax, dropout, P.v_mean and P^2.v_cov) is one kernel per direction (adt_wattention_fwd/bwd).
+padding*causal mask, softmax, dropout, P.v_mean and P^2.v_cov) is one kernel per direction (adt_wattention_fwd/bwd); with
+`precision = 1`, shapes whose attention tile does not fit shared memory (up to L 2048, H/nh a multiple of 16 up to 64) run in the
+fused tcgen05 flash kernels instead (adt_wattention_flash_fwd/bwd).
 
 `fused_loss` is the B200 training entry (stosa/trainer.py:358-378 + :517-533): BPR + pvn terms on elementwise
 Wasserstein distances in one kernel with the four table-row gradients scatter-added through the sorted segmented
@@ -134,35 +136,65 @@ class EmbedPairFn(torch.autograd.Function):
         return None, None, None, dE, dP
 
 
+def _resident_fits(Lq, H, nh, backward):
+    """the resident (fp32, shared-memory) Wasserstein attention kernels serve this shape; False also for dims they refuse outright"""
+    return L.lib().adt_wattention_resident_fits(ctypes.c_int32(Lq), ctypes.c_int32(H), ctypes.c_int32(nh), ctypes.c_int32(int(backward))) == 1
+
+
+def _wflash_scratch(ref, B, Lq, H, nh, backward):
+    f = L.lib().adt_wattention_scratch_bytes
+    f.restype = ctypes.c_int64
+    n = int(f(ctypes.c_int32(B), ctypes.c_int32(Lq), ctypes.c_int32(H), ctypes.c_int32(nh), ctypes.c_int32(int(backward))))
+    return torch.empty(n, dtype=torch.uint8, device=ref.device) if n > 0 else None    # n < 0: refused shape, the launch names why
+
+
 class WAttnFn(torch.autograd.Function):
-    """Wasserstein attention core (modules.py:240-254): six projected streams [B*L,H] -> (mean ctx, cov ctx)."""
+    """Wasserstein attention core (modules.py:240-254): six projected streams [B*L,H] -> (mean ctx, cov ctx).
+
+    precision 0 runs the resident fp32 kernels (adt_wattention_fwd/bwd), which refuse shapes whose tile does not fit shared memory.
+    precision 1 runs the same kernels where they fit and the tcgen05 flash kernels (adt_wattention_flash_fwd/bwd: bf16 operands, L up to
+    2048, H/nh a multiple of 16 up to 64) where they do not: the backward tile decides when a gradient will be needed, else the forward
+    tile, so a forward and its backward always take the same path."""
 
     @staticmethod
-    def forward(ctx, mq, cq, mk, ck, mv, cv, key_ids, dims, drop):
+    def forward(ctx, mq, cq, mk, ck, mv, cv, key_ids, dims, drop, precision=0):
         B, Lq, nh = dims
         t = [x.contiguous() for x in (mq, cq, mk, ck, mv, cv)]
         H = t[0].shape[1]
         mctx, cctx = torch.empty_like(t[0]), torch.empty_like(t[0])
         lse = torch.empty(B, nh, Lq, 2, dtype=torch.float32, device=mctx.device)
+        ctx.flash = precision == 1 and not _resident_fits(Lq, H, nh, any(ctx.needs_input_grad[:6]))
         a = L.fill(L.adt_wattention_args(), mq=t[0], cq=t[1], mk=t[2], ck=t[3], mv=t[4], cv=t[5], mctx=mctx, cctx=cctx, lse=lse,
                    key_ids=key_ids, dmctx=None, dcctx=None, dmq=None, dcq=None, dmk=None, dck=None, dmv=None, dcv=None, B=B, L=Lq, H=H,
                    nh=nh, drop=drop)
-        L.check(L.lib().adt_wattention_fwd(ctypes.byref(a), _st(mctx.device)), "adt_wattention_fwd")
-        ctx.save_for_backward(*t, lse)
+        if ctx.flash:
+            ws = _wflash_scratch(mctx, B, Lq, H, nh, 0)
+            a.tc_scratch = None if ws is None else ws.data_ptr()
+            L.check(L.lib().adt_wattention_flash_fwd(ctypes.byref(a), _st(mctx.device)), "adt_wattention_flash_fwd")
+            ctx.save_for_backward(*t, lse, mctx, cctx)
+        else:
+            L.check(L.lib().adt_wattention_fwd(ctypes.byref(a), _st(mctx.device)), "adt_wattention_fwd")
+            ctx.save_for_backward(*t, lse)
         ctx.cfg = (key_ids, dims, drop)
         return mctx, cctx
 
     @staticmethod
     def backward(ctx, dm, dc):
-        mq, cq, mk, ck, mv, cv, lse = ctx.saved_tensors
+        mq, cq, mk, ck, mv, cv, lse = ctx.saved_tensors[:7]
         key_ids, (B, Lq, nh), drop = ctx.cfg
         H = mq.shape[1]
         g = [torch.empty_like(mq) for _ in range(6)]
         a = L.fill(L.adt_wattention_args(), mq=mq, cq=cq, mk=mk, ck=ck, mv=mv, cv=cv, mctx=None, cctx=None, lse=lse, key_ids=key_ids,
                    dmctx=dm.contiguous(), dcctx=dc.contiguous(), dmq=g[0], dcq=g[1], dmk=g[2], dck=g[3], dmv=g[4], dcv=g[5], B=B, L=Lq,
                    H=H, nh=nh, drop=drop)
-        L.check(L.lib().adt_wattention_bwd(ctypes.byref(a), _st(mq.device)), "adt_wattention_bwd")
-        return (*g, None, None, None)
+        if ctx.flash:
+            ws = _wflash_scratch(mq, B, Lq, H, nh, 1)
+            a.tc_scratch = None if ws is None else ws.data_ptr()
+            a.mctx_in, a.cctx_in = ctx.saved_tensors[7].data_ptr(), ctx.saved_tensors[8].data_ptr()
+            L.check(L.lib().adt_wattention_flash_bwd(ctypes.byref(a), _st(mq.device)), "adt_wattention_flash_bwd")
+        else:
+            L.check(L.lib().adt_wattention_bwd(ctypes.byref(a), _st(mq.device)), "adt_wattention_bwd")
+        return (*g, None, None, None, None)
 
 
 class WBprFn(torch.autograd.Function):
@@ -288,7 +320,7 @@ class DisenDistSAModel(nn.Module):
         mq, mk, mv = lin(m.mean_query, qm), lin(m.mean_key, km), lin(m.mean_value, km)
         cq, ck, cv = lin(m.cov_query, qc, ELU1), lin(m.cov_key, kc, ELU1), lin(m.cov_value, kc, ELU1)
         d = self._drop(dc, "attn", self.attention_dropout_p, Lq)
-        mctx, cctx = WAttnFn.apply(mq, cq, mk, ck, mv, cv, key_ids, (B, Lq, self.num_heads), d)
+        mctx, cctx = WAttnFn.apply(mq, cq, mk, ck, mv, cv, key_ids, (B, Lq, self.num_heads), d, self.precision)
         ln = m.LayerNorm
         mh = DrlFn.apply(lin(m.mean_dense, mctx), qm, ln.weight, ln.bias, 0, 1e-12, self._drop(dc, "row", self.dropout_p, Lq))
         ch = DrlFn.apply(lin(m.cov_dense, cctx), qc, ln.weight, ln.bias, 0, 1e-12, self._drop(dc, "row", self.dropout_p, Lq))

@@ -423,7 +423,11 @@ int adt_act_fwd(const float* x, float* y, int64_t n, int32_t act, adt_stream_t s
  *   S_ij = -( |mq_i - mk_j|^2 in matmul form + sum cq_i + sum ck_j - 2 sqrt(cq_i).sqrt(ck_j) ) / sqrt(hd) + mask_ij,
  *   mask_ij = 0 if key_ids[b][j] > 0 and j <= i else float(-2^32+1) (additive, models.py:229-233), P = dropout(softmax(S)),
  *   mctx = P mv, cctx = P^2 cv.  bwd returns the gradients of all six streams.  Needs (8 L + 64)(hd + 4) + 96 L floats of
- *   shared memory in bwd (L=100, hd=16 -> 108 KB); larger shapes return ADT_E_SHAPE. */
+ *   shared memory in bwd (L=100, hd=16 -> 108 KB); larger shapes return ADT_E_SHAPE (adt_wattention_resident_fits tells which).
+ * adt_wattention_flash_fwd / _bwd: the same core on the tensor cores for any 1 <= L <= 2048 with a head size hd = H/nh that is a
+ *   multiple of 16 up to 64 (bf16 operands centred per (sequence, head), fp32 accumulation; the same mask, dropout stream and row
+ *   statistics).  tc_scratch: adt_wattention_scratch_bytes(B, L, H, nh, backward) bytes; the backward also reads the forward's outputs
+ *   (mctx_in, cctx_in).  Both write every output element once: no zeroed buffers, bitwise reproducible. */
 typedef struct {
   const float* mq; const float* cq; const float* mk; const float* ck; const float* mv; const float* cv;
   float* mctx; float* cctx; float* lse;            /* softmax row statistics (max, 1/sum) [B, nh, L, 2]: written by fwd, read by bwd */
@@ -431,9 +435,17 @@ typedef struct {
   const float* dmctx; const float* dcctx;          /* bwd only */
   float* dmq; float* dcq; float* dmk; float* dck; float* dmv; float* dcv;
   int32_t B, L, H, nh; adt_dropout drop;           /* attention-probability site (base = row offset) */
+  void* tc_scratch;                                /* flash only */
+  const float* mctx_in; const float* cctx_in;      /* flash bwd only: mctx, cctx of the forward */
 } adt_wattention_args;
 int adt_wattention_fwd(const adt_wattention_args* a, adt_stream_t stream);
 int adt_wattention_bwd(const adt_wattention_args* a, adt_stream_t stream);
+int adt_wattention_flash_fwd(const adt_wattention_args* a, adt_stream_t stream);
+int adt_wattention_flash_bwd(const adt_wattention_args* a, adt_stream_t stream);
+/* host only: 1 when the resident kernels serve (L, H/nh) in the forward (backward = 0) or the backward, 0 when not, ADT_E_SHAPE for
+ * invalid dims; the scratch of the flash kernels (O(B L H), -1 for shapes they do not serve) */
+int adt_wattention_resident_fits(int32_t L, int32_t H, int32_t nh, int32_t backward);
+int64_t adt_wattention_scratch_bytes(int32_t B, int32_t L, int32_t H, int32_t nh, int32_t backward);
 /* BPR + positive-vs-negative loss on elementwise Wasserstein distances (stosa/trainer.py:358-391).
  * fwd: acc[0] += sum_t softplus(-(d_neg - d_pos + 1e-24)), acc[1] += sum_t max(d_pos - d_pn, 0), acc[2] += sum_t (sign(d_neg-d_pos)+1)/2,
  *      acc[3] += #targets (pos id > 0).  bwd: gcoef[0] = dLoss/d(acc[0]), gcoef[1] = dLoss/d(acc[1]) (device scalars) ->
