@@ -128,15 +128,33 @@ static cudaError_t set_smem(K kern, size_t bytes) {
 
 // Sequences longer than ATTN_TILE_L positions are served by the fused flash attention (flash_tc.cu) alone, up to FLASH_MAX_L
 static const int ATTN_TILE_L = 256, FLASH_MAX_L = 2048;
+// Hidden sizes beyond ROW_TILE_H (the widest row the row-tile kernels hold) are served by the tcgen05 block path alone (bf16 GEMMs +
+// warp-per-row kernels of four float4 per lane), up to WIDE_MAX_H
+static const int ROW_TILE_H = 256, WIDE_MAX_H = 512;
 static int check_dims(int B, int L, int H, int nh) {
   if (L > FLASH_MAX_L) return fail(ADT_E_SHAPE, "%s", "unsupported shape: L > 2048 (the longest sequence the fused flash attention serves)");
-  if (B <= 0 || L <= 0 || H <= 0 || H > 256 || (H & 3) || nh <= 0 || nh > 8 || H % nh || ((H / nh) & 3))
-    return fail(ADT_E_SHAPE, "%s", "unsupported shape: need 0<L<=2048, H%4==0, H<=256, nh<=8, (H/nh)%4==0");
+  if (H > WIDE_MAX_H)
+    return fail(ADT_E_SHAPE, "%s", "unsupported shape: H > 512 (the widest row the warp-per-row kernels of the tcgen05 block path hold)");
+  if (H > ROW_TILE_H && H % 64)
+    return fail(ADT_E_SHAPE, "%s", "unsupported shape: H > 256 needs H % 64 == 0 (the tcgen05 block path and catalog scorer take 64-column K "
+                                  "blocks)");
+  if (B <= 0 || L <= 0 || H <= 0 || (H & 3) || nh <= 0 || nh > 8 || H % nh || ((H / nh) & 3))
+    return fail(ADT_E_SHAPE, "%s", H > ROW_TILE_H ? "unsupported shape: need 0<L<=2048, H%64==0, H<=512, nh<=8, (H/nh)%4==0"
+                                                   : "unsupported shape: need 0<L<=2048, H%4==0, H<=256, nh<=8, (H/nh)%4==0");
   return ADT_OK;
 }
-// shapes of an attention core or a block: beyond 256 positions only the flash kernels serve (bf16, head size 16, 32, ..., 128)
+// shapes of an attention core or a block: beyond 256 positions only the flash kernels serve (bf16, head size 16, 32, ..., 128); beyond
+// H = 256 only the tcgen05 block path (bf16, head size 32, 64, 96, 128)
 static int check_attn_dims(int B, int L, int H, int nh, int precision) {
   if (int e = check_dims(B, L, H, nh)) return e;
+  if (H > ROW_TILE_H) {
+    if (!precision)
+      return fail(ADT_E_SHAPE, "%s", "unsupported shape: H > 256 needs precision 1 (the fp32 row-tile kernels keep whole rows in shared "
+                                    "memory and stop at H = 256)");
+    if ((H / nh) % 32 || H / nh > 128)
+      return fail(ADT_E_SHAPE, "%s", "unsupported shape: H > 256 needs a head size H/nh that is a multiple of 32 and at most 128 (tcgen05 "
+                                    "block path)");
+  }
   if (L <= ATTN_TILE_L) return ADT_OK;
   if (!precision)
     return fail(ADT_E_SHAPE, "%s", "unsupported shape: L > 256 needs precision 1 (the fp32 attention cores keep whole score rows in shared "
@@ -471,11 +489,12 @@ static int blk_attn_fwd(const float* q, const float* k, const float* v, float* c
 static int blk_attn_bwd(const float* q, const float* k, const float* v, const float* ctx, const float* dctx, const float* lse, const int* ids,
                         float* dq, float* dk, float* dv, int B, int L, int H, int nh, int mask_mode, const adt_dropout& d, int precision, void* area,
                         void* flash, cudaStream_t s);
-// ---- tcgen05 forward path for wide models (block_tc.cuh); ADT_FWD_TC=0 keeps the row-tile kernels ---------------------------------
+// ---- tcgen05 forward path for wide models (block_tc.cuh); ADT_FWD_TC=0 keeps the row-tile kernels up to H = 256, beyond it the
+// tcgen05 path is the only one and serves every row count ---------------------------------
 static bool use_fwd_tc(const void* scratch, int M, int H, int nh, int mma) {
   static int v = -1;
   if (v < 0) { const char* e = getenv("ADT_FWD_TC"); v = e ? (atoi(e) != 0) : 1; }
-  return v && mma && scratch && H >= 128 && H <= 256 && (H & 7) == 0 && M >= 512 && nh <= 8;
+  return (v || H > ROW_TILE_H) && mma && scratch && H >= 128 && (H & 7) == 0 && (M >= 512 || H > ROW_TILE_H) && nh <= 8;
 }
 struct TcScratch {
   __nv_bfloat16* base; long long mh; __nv_bfloat16* wb;     // M*H elements per operand; weights after 9 operands
@@ -515,7 +534,7 @@ static int tc_ffn_out(const TcScratch& t, const __nv_bfloat16* zb, int a_op, int
   float* h2 = reinterpret_cast<float*>(t.op(h2_op));
   if (int e = tc_linear(t.op(a_op), C2b, ffn.b2, h2, nullptr, 0, M, H, H, 1.f, 0, s)) return e;
   o.h2 = h2; o.M = M; o.H = H; o.drop2 = mk_drop(row_drop(d2, training));
-  { TIMED("row_tc", s); row_out_kernel<<<row_grid(M), 256, 0, s>>>(o); }
+  { TIMED("row_tc", s); rv_kernel(row_out_kernel, H)<<<row_grid(M), 256, 0, s>>>(o); }
   return check_launch("tcgen05 forward path");
 }
 
@@ -529,7 +548,7 @@ static int tc_enc_fwd(const adt_enc_block_fwd_args* a, cudaStream_t s) {
     RowLnArgs r;
     memset(&r, 0, sizeof(r));
     r.x = a->x; r.g = a->ln1_w; r.b = a->ln1_b; r.yb = t.op(0); r.xb = t.op(1); r.M = M; r.H = H;
-    { TIMED("row_tc", s); row_ln_cast_kernel<<<row_grid(M), 256, 0, s>>>(r); }
+    { TIMED("row_tc", s); rv_kernel(row_ln_cast_kernel, H)<<<row_grid(M), 256, 0, s>>>(r); }
     // q = (LN1(x) Wq^T + bq) * scale ; [k | v] = x [Wk; Wv]^T + [bk | bv]
     if (int e = tc_linear(t.op(0), Winb, a->attn.in_b, a->q, nullptr, 0, M, H, H, qscale, 0, s)) return e;
     if (int e = tc_linear(t.op(1), Winb + hh, a->attn.in_b + H, a->k, a->v, H, M, 2 * H, H, 1.f, 0, s)) return e;
@@ -545,7 +564,7 @@ static int tc_enc_fwd(const adt_enc_block_fwd_args* a, cudaStream_t s) {
   RowLnArgs r;
   memset(&r, 0, sizeof(r));
   r.x = a->x; r.g = a->ln1_w; r.b = a->ln1_b; r.y = a->y; r.M = M; r.H = H;
-  { TIMED("row_tc", s); row_ln_cast_kernel<<<row_grid(M), 256, 0, s>>>(r); }
+  { TIMED("row_tc", s); rv_kernel(row_ln_cast_kernel, H)<<<row_grid(M), 256, 0, s>>>(r); }
   tc_cast(a->ctx, t.op(2), (long long)M * H, s);
   if (a->rec || a->nll_acc) {
     TIMED("row_tc", s);
@@ -554,7 +573,7 @@ static int tc_enc_fwd(const adt_enc_block_fwd_args* a, cudaStream_t s) {
   if (int e = tc_linear(t.op(2), Wob, a->attn.out_b, a->y, nullptr, 0, M, H, H, 1.f, 1, s)) return e;
   memset(&r, 0, sizeof(r));
   r.x = a->y; r.g = a->ln2_w; r.b = a->ln2_b; r.yb = t.op(3); r.M = M; r.H = H;
-  { TIMED("row_tc", s); row_ln_cast_kernel<<<row_grid(M), 256, 0, s>>>(r); }
+  { TIMED("row_tc", s); rv_kernel(row_ln_cast_kernel, H)<<<row_grid(M), 256, 0, s>>>(r); }
   RowOutArgs o;
   memset(&o, 0, sizeof(o));
   o.u = a->y; o.ln_g = a->ln2_w; o.ln_b = a->ln2_b; o.ids = a->ids; o.out = a->out; o.is_dec = 0;
@@ -571,7 +590,7 @@ static int tc_dec_fwd(const adt_dec_block_fwd_args* a, cudaStream_t s) {
     RowLnArgs r;
     memset(&r, 0, sizeof(r));
     r.x = a->x; r.g = a->ln_w; r.b = a->ln_b; r.y = a->d; r.yb = t.op(0); r.M = M; r.H = H;
-    { TIMED("row_tc", s); row_ln_cast_kernel<<<row_grid(M), 256, 0, s>>>(r); }
+    { TIMED("row_tc", s); rv_kernel(row_ln_cast_kernel, H)<<<row_grid(M), 256, 0, s>>>(r); }
     if (int e = tc_linear(t.op(0), W1b, a->slf.in_b, a->q1, nullptr, 0, M, H, H, qscale, 0, s)) return e;
     if (int e = tc_linear(t.op(0), W1b + hh, a->slf.in_b + H, a->k1, a->v1, H, M, 2 * H, H, 1.f, 0, s)) return e;
     if (int e = blk_attn_fwd(a->q1, a->k1, a->v1, a->ctx1, a->lse1, a->ids, a->B, a->L, H, a->nh, a->mask_mode, a->drop_slf, a->training, a->precision,
@@ -604,11 +623,12 @@ static int tc_dec_fwd(const adt_dec_block_fwd_args* a, cudaStream_t s) {
   return tc_ffn_out(t, t.op(5), 6, 7, a->ffn, C1b, C2b, a->h1, a->drop_ffn1, a->drop_ffn2, a->training, o, M, H, s);
 }
 
-// ---- tcgen05 backward path for wide models (block_tc.cuh); ADT_BWD_TC=0 keeps the row-tile kernels (with hoisted weight gradients) -----
+// ---- tcgen05 backward path for wide models (block_tc.cuh); ADT_BWD_TC=0 keeps the row-tile kernels (with hoisted weight gradients) up to
+// H = 256; beyond it the tcgen05 path is the only one -----
 static bool use_bwd_tc(const void* scratch, int M, int H, int nh, int mma) {
   static int v = -1;
   if (v < 0) { const char* e = getenv("ADT_BWD_TC"); v = e ? (atoi(e) != 0) : 1; }
-  return v && mma && scratch && H >= 128 && H <= 256 && (H & 7) == 0 && M >= 512 && nh <= 8 && ((H / nh) & 31) == 0;
+  return (v || H > ROW_TILE_H) && mma && scratch && H >= 128 && (H & 7) == 0 && (M >= 512 || H > ROW_TILE_H) && nh <= 8 && ((H / nh) & 31) == 0;
 }
 struct TcBwdScratch {
   __nv_bfloat16* base; long long mh; __nv_bfloat16* wb;     // 12 operand slots of M*H bf16, then the bf16 weights
@@ -638,7 +658,7 @@ static void tc_pack(const float* s0, float sc0, float* gb0, const float* s1, flo
   p.src[0] = s0; p.scale[0] = sc0; p.gb[0] = gb0; p.src[1] = s1; p.scale[1] = 1.f; p.gb[1] = gb1; p.src[2] = s2; p.scale[2] = 1.f; p.gb[2] = gb2;
   p.n = s2 ? 3 : (s1 ? 2 : 1); p.dst = dst; p.ld = ld; p.M = M; p.H = H;
   TIMED("row_tc", s);
-  row_pack_kernel<<<rows_grid2(M), 256, 0, s>>>(p);
+  rv_kernel(row_pack_kernel, H)<<<rows_grid2(M), 256, 0, s>>>(p);
 }
 // ---- attention of long sequences as strided-batch tcgen05 GEMMs (block_tc.cuh); ADT_ATTN_TC=0 keeps the generic row-tile attention ------
 static bool use_attn_tc(int B, int L, int H, int nh) {
@@ -756,10 +776,10 @@ static int blk_attn_bwd(const float* q, const float* k, const float* v, const fl
 static int tc_ffn_bwd(const TcBwdScratch& t, RowPostPrepArgs pp, const adt_ffn_w& ffn, const adt_ffn_g& gf, const __nv_bfloat16* C1b,
                       const __nv_bfloat16* C2b, const __nv_bfloat16* zb, int M, int H, cudaStream_t s) {
   pp.g = t.f32(6); pp.dh2b = t.op(0); pp.ab = t.op(1); pp.gc2 = gf.b2; pp.M = M; pp.H = H;
-  { TIMED("row_tc", s); row_post_prep_kernel<<<rows_grid2(M), 256, 0, s>>>(pp); }
+  { TIMED("row_tc", s); rv_kernel(row_post_prep_kernel, H)<<<rows_grid2(M), 256, 0, s>>>(pp); }
   if (int e = hoisted_wgrad(t.op(0), H, H, t.op(1), H, H, M, gf.w2, s)) return e;
   if (int e = tc_dgrad(t.op(0), H, H, C2b, H, t.f32(8), 0, M, s)) return e;                       // da = dh2 C2
-  { TIMED("row_tc", s); row_dh1_kernel<<<rows_grid2(M), 256, 0, s>>>(t.f32(8), pp.h1, t.op(2), gf.b1, M, H, pp.drop1); }
+  { TIMED("row_tc", s); rv_kernel(row_dh1_kernel, H)<<<rows_grid2(M), 256, 0, s>>>(t.f32(8), pp.h1, t.op(2), gf.b1, M, H, pp.drop1); }
   if (int e = hoisted_wgrad(t.op(2), H, H, zb, H, H, M, gf.w1, s)) return e;
   return tc_dgrad(t.op(2), H, H, C1b, H, t.f32(6), 1, M, s);                                      // dz / dc = dO + dh1 C1
 }
@@ -777,7 +797,7 @@ static int tc_enc_bwd(const adt_enc_block_bwd_args* a, cudaStream_t s) {
   RowLnArgs r;
   memset(&r, 0, sizeof(r));
   r.x = a->y; r.g = a->ln2_w; r.b = a->ln2_b; r.yb = t.op(3); r.M = M; r.H = H;
-  { TIMED("row_tc", s); row_ln_cast_kernel<<<row_grid(M), 256, 0, s>>>(r); }
+  { TIMED("row_tc", s); rv_kernel(row_ln_cast_kernel, H)<<<row_grid(M), 256, 0, s>>>(r); }
   RowPostPrepArgs pp;
   memset(&pp, 0, sizeof(pp));
   pp.dout = a->dout; pp.ids = a->ids; pp.h1 = a->h1; pp.is_dec = 0;
@@ -788,13 +808,13 @@ static int tc_enc_bwd(const adt_enc_block_bwd_args* a, cudaStream_t s) {
   memset(&lb, 0, sizeof(lb));
   lb.x = a->y; lb.g = t.f32(6); lb.ln_g = a->ln2_w; lb.dx = a->dy; lb.dxb = t.op(4); lb.gln_g = a->g_ln2_w; lb.gln_b = a->g_ln2_b;
   lb.gb = a->g_attn.out_b; lb.M = M; lb.H = H;
-  { TIMED("row_tc", s); row_ln_bwd_kernel<<<rows_grid2(M), 256, 0, s>>>(lb); }
+  { TIMED("row_tc", s); rv_kernel(row_ln_bwd_kernel, H)<<<rows_grid2(M), 256, 0, s>>>(lb); }
   tc_cast(a->ctx, t.op(5), (long long)M * H, s);
   if (int e = hoisted_wgrad(t.op(4), H, H, t.op(5), H, H, M, a->g_attn.out_w, s)) return e;
   if (int e = tc_dgrad(t.op(4), H, H, Wob, H, a->dctx, 0, M, s)) return e;
   if (a->nll_coef != 0.f || a->drec) {
     TIMED("row_tc", s);
-    sparse_head_bwd_kernel<<<attn_rows_grid(M), 256, 0, s>>>(a->ctx, a->sparse_w, a->sparse_b, a->drec, a->nll_coef, a->dctx, a->g_sparse_w,
+    rv_kernel(sparse_head_bwd_kernel, H)<<<attn_rows_grid(M), 256, 0, s>>>(a->ctx, a->sparse_w, a->sparse_b, a->drec, a->nll_coef, a->dctx, a->g_sparse_w,
                                                         a->g_sparse_b, M, H, a->nh);
   }
   if (int e = check_launch("tcgen05 backward path (enc post)")) return e;
@@ -805,14 +825,14 @@ static int tc_enc_bwd(const adt_enc_block_bwd_args* a, cudaStream_t s) {
   tc_pack(a->dq, qscale, a->g_attn.in_b, a->dk, a->g_attn.in_b + H, a->dv, a->g_attn.in_b + 2 * H, t.op(0), 3 * H, M, H, s);
   memset(&r, 0, sizeof(r));
   r.x = a->x; r.g = a->ln1_w; r.b = a->ln1_b; r.yb = t.op(3); r.xb = t.op(4); r.M = M; r.H = H;
-  { TIMED("row_tc", s); row_ln_cast_kernel<<<row_grid(M), 256, 0, s>>>(r); }
+  { TIMED("row_tc", s); rv_kernel(row_ln_cast_kernel, H)<<<row_grid(M), 256, 0, s>>>(r); }
   if (int e = hoisted_wgrad(t.op(0), 3 * H, H, t.op(3), H, H, M, a->g_attn.in_w, s)) return e;
   if (int e = hoisted_wgrad(t.op(0) + H, 3 * H, 2 * H, t.op(4), H, H, M, a->g_attn.in_w + hh, s)) return e;
   if (int e = tc_dgrad(t.op(0), 3 * H, H, Winb, H, a->dy, 1, M, s)) return e;                    // dN = dy + dq*s Wq
   memset(&lb, 0, sizeof(lb));
   lb.x = a->x; lb.g = a->dy; lb.ln_g = a->ln1_w; lb.extra = a->dx_extra; lb.dx = a->dx; lb.gln_g = a->g_ln1_w; lb.gln_b = a->g_ln1_b;
   lb.M = M; lb.H = H;
-  { TIMED("row_tc", s); row_ln_bwd_kernel<<<rows_grid2(M), 256, 0, s>>>(lb); }
+  { TIMED("row_tc", s); rv_kernel(row_ln_bwd_kernel, H)<<<rows_grid2(M), 256, 0, s>>>(lb); }
   if (int e = tc_dgrad(t.op(0) + H, 3 * H, 2 * H, Winb + hh, H, a->dx, 1, M, s)) return e;       // dx += dk Wk + dv Wv
   return check_launch("tcgen05 backward path (enc pre)");
 }
@@ -871,7 +891,7 @@ static int tc_dec_bwd(const adt_dec_block_bwd_args* a, cudaStream_t s) {
   RowLnBwdArgs lb;
   memset(&lb, 0, sizeof(lb));
   lb.x = a->x; lb.g = a->dd; lb.ln_g = a->ln_w; lb.dx = a->dx; lb.gln_g = a->g_ln_w; lb.gln_b = a->g_ln_b; lb.M = M; lb.H = H;
-  { TIMED("row_tc", s); row_ln_bwd_kernel<<<rows_grid2(M), 256, 0, s>>>(lb); }
+  { TIMED("row_tc", s); rv_kernel(row_ln_bwd_kernel, H)<<<rows_grid2(M), 256, 0, s>>>(lb); }
   return check_launch("tcgen05 backward path (dec pre)");
 }
 
@@ -884,6 +904,9 @@ extern "C" int adt_enc_block_fwd(const adt_enc_block_fwd_args* a, adt_stream_t s
   if (a->phase < 0 || a->phase > 2) return fail(ADT_E_SHAPE, "%s", "enc_block_fwd: phase must be 0, 1 or 2");
   if (a->phase == 0 && !a->training && use_seq(a->L, H, a->nh, mma)) return seq_enc_fwd(a, s);
   if (a->y && a->h1 && a->out && use_fwd_tc(a->tc_scratch, M, H, a->nh, mma)) return tc_enc_fwd(a, s);
+  if (H > ROW_TILE_H)
+    return fail(ADT_E_SHAPE, "%s", "enc_block_fwd at H > 256 runs on the tcgen05 block path only: tc_scratch (adt_workspace_sizes.fwd_scratch), "
+                                  "y, h1 and out are required");
   if (a->phase != 2) {
     if (use_attn_fused(a->L, H, a->nh, mma, false)) {
       if (int e = launch_pre_attn_fwd(a->x, a->ln1_w, a->ln1_b, a->attn, a->q, a->k, a->v, nullptr, a->ctx, a->lse, a->ids, a->B, a->L, a->nh, 0,
@@ -927,6 +950,9 @@ extern "C" int adt_enc_block_bwd(const adt_enc_block_bwd_args* a, adt_stream_t s
   const int M = a->B * a->L, H = a->H;
   const int mma = a->precision ? 1 : 0, pad = mma ? 8 : 4;
   if (use_bwd_tc(a->wgrad_scratch, M, H, a->nh, mma)) return tc_enc_bwd(a, s);
+  if (H > ROW_TILE_H)
+    return fail(ADT_E_SHAPE, "%s", "enc_block_bwd at H > 256 runs on the tcgen05 block path only: wgrad_scratch (adt_workspace_sizes.wgrad_scratch) "
+                                  "is required");
   PostBwdArgs p;
   memset(&p, 0, sizeof(p));
   p.dout = a->dout; p.ids = a->ids; p.ctx = a->ctx; p.u = a->y; p.h1 = a->h1;
@@ -985,6 +1011,9 @@ extern "C" int adt_dec_block_fwd(const adt_dec_block_fwd_args* a, adt_stream_t s
   const int M = a->B * a->L, H = a->H;
   const int mma = a->precision ? 1 : 0, pad = mma ? 8 : 4;
   if (a->d && a->a && a->c && a->h1 && use_fwd_tc(a->tc_scratch, M, H, a->nh, mma)) return tc_dec_fwd(a, s);
+  if (H > ROW_TILE_H)
+    return fail(ADT_E_SHAPE, "%s", "dec_block_fwd at H > 256 runs on the tcgen05 block path only: tc_scratch (adt_workspace_sizes.fwd_scratch), "
+                                  "d, a, c and h1 are required");
   if (a->phase != 2) {
     if (use_attn_fused(a->L, H, a->nh, mma, false)) {
       if (int e = launch_pre_attn_fwd(a->x, a->ln_w, a->ln_b, a->slf, a->q1, a->k1, a->v1, a->d, a->ctx1, a->lse1, a->ids, a->B, a->L, a->nh, 1,
@@ -1047,6 +1076,9 @@ extern "C" int adt_dec_block_bwd(const adt_dec_block_bwd_args* a, adt_stream_t s
   const int mma = a->precision ? 1 : 0, pad = mma ? 8 : 4;
   const float qscale = 1.0f / sqrtf((float)(H / a->nh));
   if (use_bwd_tc(a->wgrad_scratch, M, H, a->nh, mma)) return tc_dec_bwd(a, s);
+  if (H > ROW_TILE_H)
+    return fail(ADT_E_SHAPE, "%s", "dec_block_bwd at H > 256 runs on the tcgen05 block path only: wgrad_scratch (adt_workspace_sizes.wgrad_scratch) "
+                                  "is required");
   __nv_bfloat16* hz = hoist_ptr(a->wgrad_scratch, H, mma);
   const long long hu = (long long)M * H;
   size_t smem;
@@ -1127,17 +1159,17 @@ extern "C" int adt_dec_block_bwd(const adt_dec_block_bwd_args* a, adt_stream_t s
 // ---------------------------------------------------------------------------------------------------------
 extern "C" int adt_final_logits_loss_fwd(const adt_final_fwd_args* a, adt_stream_t s_) {
   cudaStream_t s = (cudaStream_t)s_;
-  if (a->H > 256 || (a->H & 3)) return fail(ADT_E_SHAPE, "%s", "final_fwd: H");
+  if (a->H > WIDE_MAX_H || (a->H & 3)) return fail(ADT_E_SHAPE, "%s", "final_fwd: H");
   const int grid = min((a->M + 7) / 8, 148 * 8);
   TIMED("final_fwd", s);
-  final_fwd_kernel<<<grid, NT, 0, s>>>(a->x, a->ln_w, a->ln_b, a->item_emb, a->pos, a->neg, a->feats, a->pos_logits, a->neg_logits, a->acc,
+  (a->H > 256 ? final_fwd_kernel<16> : final_fwd_kernel<8>)<<<grid, NT, 0, s>>>(a->x, a->ln_w, a->ln_b, a->item_emb, a->pos, a->neg, a->feats, a->pos_logits, a->neg_logits, a->acc,
                                        a->M, a->H);
   return check_launch("final_fwd");
 }
 
 extern "C" int adt_final_logits_loss_bwd(const adt_final_bwd_args* a, adt_stream_t s_) {
   cudaStream_t s = (cudaStream_t)s_;
-  if (a->H > 256 || (a->H & 3)) return fail(ADT_E_SHAPE, "%s", "final_bwd: H");
+  if (a->H > WIDE_MAX_H || (a->H & 3)) return fail(ADT_E_SHAPE, "%s", "final_bwd: H");
   FinalBwdArgs p;
   p.x = a->x; p.ln_g = a->ln_w; p.E = a->item_emb; p.pos = a->pos; p.neg = a->neg;
   p.pos_logits = a->pos_logits; p.neg_logits = a->neg_logits; p.dfeats_in = a->dfeats_in; p.n_valid = a->n_valid;
@@ -1145,7 +1177,7 @@ extern "C" int adt_final_logits_loss_bwd(const adt_final_bwd_args* a, adt_stream
   p.dx = a->dx; p.cpos = a->cpos; p.cneg = a->cneg; p.gln_g = a->g_ln_w; p.gln_b = a->g_ln_b; p.M = a->M; p.H = a->H;
   const int grid = min((a->M + 7) / 8, 148 * 4);
   TIMED("final_bwd", s);
-  final_bwd_kernel<<<grid, NT, 0, s>>>(p);
+  (a->H > 256 ? final_bwd_kernel<16> : final_bwd_kernel<8>)<<<grid, NT, 0, s>>>(p);
   return check_launch("final_bwd");
 }
 
@@ -1213,8 +1245,9 @@ extern "C" int adt_embed_bwd(const adt_embed_bwd_args* a, adt_stream_t s_) {
   sa.dE = a->d_item_emb; sa.head = a->head; sa.tail = a->tail; sa.has_tail = a->has_tail;
   const int nb = (sa.N + 31) / 32;
   if (a->H <= 128) scatter_phase1_kernel<1><<<(nb + 7) / 8, 256, 0, s>>>(sa);
-  else scatter_phase1_kernel<2><<<(nb + 7) / 8, 256, 0, s>>>(sa);
-  scatter_phase2_kernel<<<(nb + 7) / 8, 256, 0, s>>>(sa);
+  else if (a->H <= 256) scatter_phase1_kernel<2><<<(nb + 7) / 8, 256, 0, s>>>(sa);
+  else scatter_phase1_kernel<4><<<(nb + 7) / 8, 256, 0, s>>>(sa);
+  (a->H > 256 ? scatter_phase2_kernel<4> : scatter_phase2_kernel<2>)<<<(nb + 7) / 8, 256, 0, s>>>(sa);
   return check_launch("adt_embed_bwd");
 }
 
@@ -1332,15 +1365,15 @@ static DrlArgs mk_drl(const adt_drl_args* a) {
   return p;
 }
 extern "C" int adt_drop_res_ln_fwd(const adt_drl_args* a, adt_stream_t s_) {
-  if (a->H > 256 || a->H <= 0) return fail(ADT_E_SHAPE, "%s", "drop_res_ln: H <= 256");
+  if (a->H > WIDE_MAX_H || a->H <= 0) return fail(ADT_E_SHAPE, "%s", "drop_res_ln: 0 < H <= 512");
   const int grid = min((a->M + 7) / 8, 148 * 8);
-  drl_fwd_kernel<<<grid, NT, 0, (cudaStream_t)s_>>>(mk_drl(a));
+  (a->H > 256 ? drl_fwd_kernel<16> : drl_fwd_kernel<8>)<<<grid, NT, 0, (cudaStream_t)s_>>>(mk_drl(a));
   return check_launch("drop_res_ln_fwd");
 }
 extern "C" int adt_drop_res_ln_bwd(const adt_drl_args* a, adt_stream_t s_) {
-  if (a->H > 256 || a->H <= 0) return fail(ADT_E_SHAPE, "%s", "drop_res_ln: H <= 256");
+  if (a->H > WIDE_MAX_H || a->H <= 0) return fail(ADT_E_SHAPE, "%s", "drop_res_ln: 0 < H <= 512");
   const int grid = min((a->M + 7) / 8, 148 * 4);
-  drl_bwd_kernel<<<grid, NT, 0, (cudaStream_t)s_>>>(mk_drl(a));
+  (a->H > 256 ? drl_bwd_kernel<16> : drl_bwd_kernel<8>)<<<grid, NT, 0, (cudaStream_t)s_>>>(mk_drl(a));
   return check_launch("drop_res_ln_bwd");
 }
 

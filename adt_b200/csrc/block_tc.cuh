@@ -9,8 +9,9 @@
 
 namespace adt {
 
-// columns of a row owned by a lane: float4 at 4*lane + 128*j, j < RV_MAX (H <= 256)
-constexpr int RV_MAX = 2;
+// columns of a row owned by a lane: float4 at 4*lane + 128*j, j < RV.  Every warp-per-row kernel below is instantiated for RV = 2
+// (H <= 256) and RV = 4 (256 < H <= 512); rv_kernel picks the instantiation from H at launch.
+#define rv_kernel(K, H) ((H) > 256 ? K<4> : K<2>)
 
 struct RowLnArgs {
   const float* x; const float* g; const float* b;
@@ -26,23 +27,24 @@ __device__ __forceinline__ void st_bf16x4(__nv_bfloat16* p, float4 v) {
   *reinterpret_cast<uint2*>(p) = o;
 }
 
-// LayerNorm of a row held as v[RV_MAX] by the warp (eps 1e-8, two-pass statistics like ln_tile)
-__device__ __forceinline__ void warp_ln(float4 (&v)[RV_MAX], int H, int lane, const float* __restrict__ g, const float* __restrict__ b) {
+// LayerNorm of a row held as v[RV] by the warp (eps 1e-8, two-pass statistics like ln_tile)
+template <int RV>
+__device__ __forceinline__ void warp_ln(float4 (&v)[RV], int H, int lane, const float* __restrict__ g, const float* __restrict__ b) {
   float sum = 0.f;
 #pragma unroll
-  for (int j = 0; j < RV_MAX; ++j)
+  for (int j = 0; j < RV; ++j)
     if (4 * lane + 128 * j < H) sum += (v[j].x + v[j].y) + (v[j].z + v[j].w);
   const float mean = warp_sum(sum) / (float)H;
   float var = 0.f;
 #pragma unroll
-  for (int j = 0; j < RV_MAX; ++j)
+  for (int j = 0; j < RV; ++j)
     if (4 * lane + 128 * j < H) {
       const float a0 = v[j].x - mean, a1 = v[j].y - mean, a2 = v[j].z - mean, a3 = v[j].w - mean;
       var += (a0 * a0 + a1 * a1) + (a2 * a2 + a3 * a3);
     }
   const float rstd = 1.0f / sqrtf(warp_sum(var) / (float)H + 1e-8f);
 #pragma unroll
-  for (int j = 0; j < RV_MAX; ++j) {
+  for (int j = 0; j < RV; ++j) {
     const int c = 4 * lane + 128 * j;
     if (c < H) {
       const float4 ga = __ldg(reinterpret_cast<const float4*>(g + c)), be = __ldg(reinterpret_cast<const float4*>(b + c));
@@ -52,20 +54,21 @@ __device__ __forceinline__ void warp_ln(float4 (&v)[RV_MAX], int H, int lane, co
   }
 }
 
+template <int RV>
 __global__ void __launch_bounds__(256) row_ln_cast_kernel(RowLnArgs a) {
   const int lane = threadIdx.x & 31;
   for (int row = blockIdx.x * 8 + (threadIdx.x >> 5); row < a.M; row += gridDim.x * 8) {
     const long long off = (long long)row * a.H;
-    float4 v[RV_MAX];
+    float4 v[RV];
 #pragma unroll
-    for (int j = 0; j < RV_MAX; ++j) {
+    for (int j = 0; j < RV; ++j) {
       const int c = 4 * lane + 128 * j;
       v[j] = c < a.H ? *reinterpret_cast<const float4*>(a.x + off + c) : make_float4(0.f, 0.f, 0.f, 0.f);
       if (a.xb && c < a.H) st_bf16x4(a.xb + off + c, v[j]);
     }
-    warp_ln(v, a.H, lane, a.g, a.b);
+    warp_ln<RV>(v, a.H, lane, a.g, a.b);
 #pragma unroll
-    for (int j = 0; j < RV_MAX; ++j) {
+    for (int j = 0; j < RV; ++j) {
       const int c = 4 * lane + 128 * j;
       if (c < a.H) {
         if (a.y) *reinterpret_cast<float4*>(a.y + off + c) = v[j];
@@ -133,22 +136,23 @@ struct RowOutArgs {
   DropDesc drop2;
 };
 
+template <int RV>
 __global__ void __launch_bounds__(256) row_out_kernel(RowOutArgs a) {
   __shared__ double red[8];
   const int lane = threadIdx.x & 31;
   double sq = 0.0;
   for (int row = blockIdx.x * 8 + (threadIdx.x >> 5); row < a.M; row += gridDim.x * 8) {
     const long long off = (long long)row * a.H;
-    float4 v[RV_MAX];
+    float4 v[RV];
 #pragma unroll
-    for (int j = 0; j < RV_MAX; ++j) {
+    for (int j = 0; j < RV; ++j) {
       const int c = 4 * lane + 128 * j;
       v[j] = c < a.H ? *reinterpret_cast<const float4*>(a.u + off + c) : make_float4(0.f, 0.f, 0.f, 0.f);
     }
-    if (!a.is_dec) warp_ln(v, a.H, lane, a.ln_g, a.ln_b);
+    if (!a.is_dec) warp_ln<RV>(v, a.H, lane, a.ln_g, a.ln_b);
     const bool keep = a.ids[row] != 0;
 #pragma unroll
-    for (int j = 0; j < RV_MAX; ++j) {
+    for (int j = 0; j < RV; ++j) {
       const int c = 4 * lane + 128 * j;
       if (c >= a.H) continue;
       float4 h2 = *reinterpret_cast<const float4*>(a.h2 + off + c);
@@ -177,9 +181,10 @@ __global__ void __launch_bounds__(256) row_out_kernel(RowOutArgs a) {
 // =====================================================================================================================
 namespace adt {
 
-__device__ __forceinline__ void lane_cols_to_smem(float* __restrict__ sm, const float4 (&p)[RV_MAX], int H, int lane) {
+template <int RV>
+__device__ __forceinline__ void lane_cols_to_smem(float* __restrict__ sm, const float4 (&p)[RV], int H, int lane) {
 #pragma unroll
-  for (int j = 0; j < RV_MAX; ++j) {
+  for (int j = 0; j < RV; ++j) {
     const int c = 4 * lane + 128 * j;
     if (c < H) { atomicAdd(sm + c, p[j].x); atomicAdd(sm + c + 1, p[j].y); atomicAdd(sm + c + 2, p[j].z); atomicAdd(sm + c + 3, p[j].w); }
   }
@@ -202,19 +207,20 @@ struct RowPostPrepArgs {
   DropDesc drop1, drop2;
 };
 
+template <int RV>
 __global__ void __launch_bounds__(256) row_post_prep_kernel(RowPostPrepArgs a) {
-  __shared__ float cs[256];
+  __shared__ float cs[128 * RV];
   const int lane = threadIdx.x & 31;
   for (int c = threadIdx.x; c < a.H; c += 256) cs[c] = 0.f;
   __syncthreads();
-  float4 part[RV_MAX];
+  float4 part[RV];
 #pragma unroll
-  for (int j = 0; j < RV_MAX; ++j) part[j] = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int j = 0; j < RV; ++j) part[j] = make_float4(0.f, 0.f, 0.f, 0.f);
   for (int row = blockIdx.x * 8 + (threadIdx.x >> 5); row < a.M; row += gridDim.x * 8) {
     const long long off = (long long)row * a.H;
     const bool keep = a.ids[row] != 0;
 #pragma unroll
-    for (int j = 0; j < RV_MAX; ++j) {
+    for (int j = 0; j < RV; ++j) {
       const int c = 4 * lane + 128 * j;
       if (c >= a.H) continue;
       const long long gi = off + c;
@@ -237,24 +243,25 @@ __global__ void __launch_bounds__(256) row_post_prep_kernel(RowPostPrepArgs a) {
       part[j] = f4_add(part[j], d2);
     }
   }
-  lane_cols_to_smem(cs, part, a.H, lane);
+  lane_cols_to_smem<RV>(cs, part, a.H, lane);
   __syncthreads();
   smem_cols_to_global(cs, a.gc2, a.H);
 }
 
 // dh1 = da * [h1 m1 > 0] * m1 -> bf16 ; gc1 += colsum(dh1)        (post_bwd step 4)
+template <int RV>
 __global__ void __launch_bounds__(256) row_dh1_kernel(const float* __restrict__ da, const float* __restrict__ h1, __nv_bfloat16* __restrict__ dh1b,
                                                       float* __restrict__ gc1, int M, int H, DropDesc drop1) {
-  __shared__ float cs[256];
+  __shared__ float cs[128 * RV];
   const int lane = threadIdx.x & 31;
   for (int c = threadIdx.x; c < H; c += 256) cs[c] = 0.f;
   __syncthreads();
-  float4 part[RV_MAX];
+  float4 part[RV];
 #pragma unroll
-  for (int j = 0; j < RV_MAX; ++j) part[j] = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int j = 0; j < RV; ++j) part[j] = make_float4(0.f, 0.f, 0.f, 0.f);
   for (int row = blockIdx.x * 8 + (threadIdx.x >> 5); row < M; row += gridDim.x * 8) {
 #pragma unroll
-    for (int j = 0; j < RV_MAX; ++j) {
+    for (int j = 0; j < RV; ++j) {
       const int c = 4 * lane + 128 * j;
       if (c >= H) continue;
       const long long gi = (long long)row * H + c;
@@ -267,7 +274,7 @@ __global__ void __launch_bounds__(256) row_dh1_kernel(const float* __restrict__ 
       part[j] = f4_add(part[j], o);
     }
   }
-  lane_cols_to_smem(cs, part, H, lane);
+  lane_cols_to_smem<RV>(cs, part, H, lane);
   __syncthreads();
   smem_cols_to_global(cs, gc1, H);
 }
@@ -279,20 +286,21 @@ struct RowLnBwdArgs {
   int M, H;
 };
 
+template <int RV>
 __global__ void __launch_bounds__(256) row_ln_bwd_kernel(RowLnBwdArgs a) {
-  __shared__ float cs[3 * 256];
+  __shared__ float cs[3 * 128 * RV];
   const int lane = threadIdx.x & 31, H = a.H;
   for (int c = threadIdx.x; c < 3 * H; c += 256) cs[c] = 0.f;
   __syncthreads();
-  float4 pg[RV_MAX], pb[RV_MAX], pc[RV_MAX];
+  float4 pg[RV], pb[RV], pc[RV];
 #pragma unroll
-  for (int j = 0; j < RV_MAX; ++j) pg[j] = pb[j] = pc[j] = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int j = 0; j < RV; ++j) pg[j] = pb[j] = pc[j] = make_float4(0.f, 0.f, 0.f, 0.f);
   for (int row = blockIdx.x * 8 + (threadIdx.x >> 5); row < a.M; row += gridDim.x * 8) {
     const long long off = (long long)row * H;
-    float4 xv[RV_MAX], gv[RV_MAX];
+    float4 xv[RV], gv[RV];
     float sum = 0.f;
 #pragma unroll
-    for (int j = 0; j < RV_MAX; ++j) {
+    for (int j = 0; j < RV; ++j) {
       const int c = 4 * lane + 128 * j;
       xv[j] = gv[j] = make_float4(0.f, 0.f, 0.f, 0.f);
       if (c < H) {
@@ -304,16 +312,16 @@ __global__ void __launch_bounds__(256) row_ln_bwd_kernel(RowLnBwdArgs a) {
     const float mean = warp_sum(sum) / (float)H;
     float var = 0.f;
 #pragma unroll
-    for (int j = 0; j < RV_MAX; ++j)
+    for (int j = 0; j < RV; ++j)
       if (4 * lane + 128 * j < H) {
         const float a0 = xv[j].x - mean, a1 = xv[j].y - mean, a2 = xv[j].z - mean, a3 = xv[j].w - mean;
         var += (a0 * a0 + a1 * a1) + (a2 * a2 + a3 * a3);
       }
     const float rstd = 1.0f / sqrtf(warp_sum(var) / (float)H + 1e-8f);
     float s1 = 0.f, s2 = 0.f;
-    float4 gg[RV_MAX];
+    float4 gg[RV];
 #pragma unroll
-    for (int j = 0; j < RV_MAX; ++j) {
+    for (int j = 0; j < RV; ++j) {
       const int c = 4 * lane + 128 * j;
       gg[j] = make_float4(0.f, 0.f, 0.f, 0.f);
       if (c < H) {
@@ -329,7 +337,7 @@ __global__ void __launch_bounds__(256) row_ln_bwd_kernel(RowLnBwdArgs a) {
     s1 = warp_sum(s1) / (float)H;
     s2 = warp_sum(s2) / (float)H;
 #pragma unroll
-    for (int j = 0; j < RV_MAX; ++j) {
+    for (int j = 0; j < RV; ++j) {
       const int c = 4 * lane + 128 * j;
       if (c >= H) continue;
       float4 d = make_float4(rstd * (gg[j].x - s1 - xv[j].x * s2), rstd * (gg[j].y - s1 - xv[j].y * s2), rstd * (gg[j].z - s1 - xv[j].z * s2),
@@ -340,9 +348,9 @@ __global__ void __launch_bounds__(256) row_ln_bwd_kernel(RowLnBwdArgs a) {
       pc[j] = f4_add(pc[j], d);
     }
   }
-  lane_cols_to_smem(cs, pg, H, lane);
-  lane_cols_to_smem(cs + H, pb, H, lane);
-  if (a.gb) lane_cols_to_smem(cs + 2 * H, pc, H, lane);
+  lane_cols_to_smem<RV>(cs, pg, H, lane);
+  lane_cols_to_smem<RV>(cs + H, pb, H, lane);
+  if (a.gb) lane_cols_to_smem<RV>(cs + 2 * H, pc, H, lane);
   __syncthreads();
   smem_cols_to_global(cs, a.gln_g, H);
   smem_cols_to_global(cs + H, a.gln_b, H);
@@ -355,22 +363,23 @@ struct RowPackArgs {
   __nv_bfloat16* dst; long long ld; int n, M, H;
 };
 
+template <int RV>
 __global__ void __launch_bounds__(256) row_pack_kernel(RowPackArgs a) {
-  __shared__ float cs[3 * 256];
+  __shared__ float cs[3 * 128 * RV];
   const int lane = threadIdx.x & 31, H = a.H;
   for (int c = threadIdx.x; c < 3 * H; c += 256) cs[c] = 0.f;
   __syncthreads();
-  float4 part[3][RV_MAX];
+  float4 part[3][RV];
 #pragma unroll
   for (int i = 0; i < 3; ++i)
 #pragma unroll
-    for (int j = 0; j < RV_MAX; ++j) part[i][j] = make_float4(0.f, 0.f, 0.f, 0.f);
+    for (int j = 0; j < RV; ++j) part[i][j] = make_float4(0.f, 0.f, 0.f, 0.f);
   for (int row = blockIdx.x * 8 + (threadIdx.x >> 5); row < a.M; row += gridDim.x * 8) {
 #pragma unroll
     for (int i = 0; i < 3; ++i) {
       if (i >= a.n) continue;
 #pragma unroll
-      for (int j = 0; j < RV_MAX; ++j) {
+      for (int j = 0; j < RV; ++j) {
         const int c = 4 * lane + 128 * j;
         if (c >= H) continue;
         const float4 v = f4_scale(*reinterpret_cast<const float4*>(a.src[i] + (long long)row * H + c), a.scale[i]);
@@ -381,7 +390,7 @@ __global__ void __launch_bounds__(256) row_pack_kernel(RowPackArgs a) {
   }
 #pragma unroll
   for (int i = 0; i < 3; ++i)
-    if (i < a.n && a.gb[i]) lane_cols_to_smem(cs + i * H, part[i], H, lane);
+    if (i < a.n && a.gb[i]) lane_cols_to_smem<RV>(cs + i * H, part[i], H, lane);
   __syncthreads();
 #pragma unroll
   for (int i = 0; i < 3; ++i)
@@ -389,12 +398,13 @@ __global__ void __launch_bounds__(256) row_pack_kernel(RowPackArgs a) {
 }
 
 // adjoint of the independence head (post_bwd step 9): dl = nll_coef (softmax - onehot) [+ log-softmax adjoint of drec] ;
-//   dctx[r, head c] += dl[c] Ws ; gWs += sum dl[c]^T ctx[r, head c] ; gbs += sum dl[c]          (hd a multiple of 32, nh <= 8)
+//   dctx[r, head c] += dl[c] Ws ; gWs += sum dl[c]^T ctx[r, head c] ; gbs += sum dl[c]          (hd a multiple of 32, nh <= 8, H <= 128 RV)
+template <int RV>
 __global__ void __launch_bounds__(256) sparse_head_bwd_kernel(const float* __restrict__ ctx, const float* __restrict__ Wsp,
                                                               const float* __restrict__ bsp, const float* __restrict__ drec, float nll_coef,
                                                               float* __restrict__ dctx, float* __restrict__ gWsp, float* __restrict__ gbsp, int M,
                                                               int H, int nh) {
-  __shared__ float gw[256];
+  __shared__ float gw[128 * RV];
   __shared__ float gbv[8];
   __shared__ float dls[8][8];          // per warp: dl[j] of the (row, head) being processed
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, hd = H / nh, tpd = hd >> 5, nflat = H >> 5;
@@ -402,9 +412,11 @@ __global__ void __launch_bounds__(256) sparse_head_bwd_kernel(const float* __res
   if (threadIdx.x < 8) gbv[threadIdx.x] = 0.f;
   __syncthreads();
   // this lane's share of gWs: flat slot i <-> (class j = i / tpd, column d = lane + 32 (i % tpd)); slots are compile-time indices
-  float accw[8], accb[8];
+  float accw[4 * RV], accb[8];
 #pragma unroll
-  for (int i = 0; i < 8; ++i) accw[i] = accb[i] = 0.f;
+  for (int i = 0; i < 8; ++i) accb[i] = 0.f;
+#pragma unroll
+  for (int i = 0; i < 4 * RV; ++i) accw[i] = 0.f;
   for (int row = blockIdx.x * 8 + w; row < M; row += gridDim.x * 8) {
     const float* xr = ctx + (long long)row * H;
     float* dr_out = dctx + (long long)row * H;
@@ -445,7 +457,7 @@ __global__ void __launch_bounds__(256) sparse_head_bwd_kernel(const float* __res
         dr_out[c * hd + d] += add;
       }
 #pragma unroll
-      for (int i = 0; i < 8; ++i)
+      for (int i = 0; i < 4 * RV; ++i)
         if (i < nflat) {
           const int j = i / tpd, t = i - j * tpd;
           accw[i] = fmaf(dls[w][j], xr[c * hd + lane + 32 * t], accw[i]);
@@ -453,7 +465,7 @@ __global__ void __launch_bounds__(256) sparse_head_bwd_kernel(const float* __res
     }
   }
 #pragma unroll
-  for (int i = 0; i < 8; ++i)
+  for (int i = 0; i < 4 * RV; ++i)
     if (i < nflat) {
       const int j = i / tpd, t = i - j * tpd;
       atomicAdd(gw + j * hd + lane + 32 * t, accw[i]);

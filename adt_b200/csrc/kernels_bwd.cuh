@@ -542,14 +542,15 @@ struct FinalBwdArgs {
   int M, H;
 };
 
+template <int U>
 __global__ void __launch_bounds__(NT) final_bwd_kernel(FinalBwdArgs p) {
-  __shared__ float red[2 * (NT / 32) * 256];
+  __shared__ float red[2 * (NT / 32) * 32 * U];
   const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
   const int H = p.H;
   constexpr int NW = NT / 32;
-  float dg[8], db[8];
+  float dg[U], db[U];
 #pragma unroll
-  for (int u = 0; u < 8; ++u) dg[u] = db[u] = 0.f;
+  for (int u = 0; u < U; ++u) dg[u] = db[u] = 0.f;
   const float inv_n = p.bce_weight != 0.f ? (float)(1.0 / fmax(*p.n_valid, 1.0)) * p.bce_weight : 0.f;
   for (int row = blockIdx.x * NW + w; row < p.M; row += gridDim.x * NW) {
     const int pi = p.pos[row], ni = p.neg[row];
@@ -563,10 +564,10 @@ __global__ void __launch_bounds__(NT) final_bwd_kernel(FinalBwdArgs p) {
     if (p.dnl_ext) dnl += p.dnl_ext[row];
     if (l == 0) { p.cpos[row] = dpl; p.cneg[row] = dnl; }
     const float* xr = p.x + (long long)row * H;
-    float xv[8], gv[8];
+    float xv[U], gv[U];
     float sum = 0.f;
 #pragma unroll
-    for (int u = 0; u < 8; ++u) {
+    for (int u = 0; u < U; ++u) {
       const int c = l + 32 * u;
       xv[u] = c < H ? xr[c] : 0.f;
       sum += xv[u];
@@ -580,19 +581,19 @@ __global__ void __launch_bounds__(NT) final_bwd_kernel(FinalBwdArgs p) {
     }
     if (!p.ln_g) {
 #pragma unroll
-      for (int u = 0; u < 8; ++u)
+      for (int u = 0; u < U; ++u)
         if (l + 32 * u < H) p.dx[(long long)row * H + l + 32 * u] = gv[u];
       continue;
     }
     const float mean = warp_sum(sum) / (float)H;
     float var = 0.f;
 #pragma unroll
-    for (int u = 0; u < 8; ++u)
+    for (int u = 0; u < U; ++u)
       if (l + 32 * u < H) { const float t = xv[u] - mean; var += t * t; }
     const float rstd = 1.0f / sqrtf(warp_sum(var) / (float)H + 1e-8f);
     float s1 = 0.f, s2 = 0.f;
 #pragma unroll
-    for (int u = 0; u < 8; ++u) {
+    for (int u = 0; u < U; ++u) {
       const int c = l + 32 * u;
       if (c < H) {
         const float xh = (xv[u] - mean) * rstd;
@@ -604,7 +605,7 @@ __global__ void __launch_bounds__(NT) final_bwd_kernel(FinalBwdArgs p) {
     s1 = warp_sum(s1) / (float)H;
     s2 = warp_sum(s2) / (float)H;
 #pragma unroll
-    for (int u = 0; u < 8; ++u) {
+    for (int u = 0; u < U; ++u) {
       const int c = l + 32 * u;
       if (c < H) {
         const float xh = (xv[u] - mean) * rstd;
@@ -614,7 +615,7 @@ __global__ void __launch_bounds__(NT) final_bwd_kernel(FinalBwdArgs p) {
   }
   if (p.ln_g) {
 #pragma unroll
-    for (int u = 0; u < 8; ++u) {
+    for (int u = 0; u < U; ++u) {
       const int c = l + 32 * u;
       if (c < H) { red[w * H + c] = dg[u]; red[(NW + w) * H + c] = db[u]; }
     }

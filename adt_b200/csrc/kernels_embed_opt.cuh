@@ -187,7 +187,7 @@ __device__ __forceinline__ float4 scatter_row4(const ScatterArgs& a, int e, int 
   return f4_scale(ld4(a.feats + gi), cf);
 }
 
-// NS = float4 per lane: 1 for H <= 128, 2 for H <= 256
+// NS = float4 per lane: 1 for H <= 128, 2 for H <= 256, 4 for H <= 512 (phase 2: 2 up to H = 256, else 4)
 template <int NS>
 __global__ void __launch_bounds__(256) scatter_phase1_kernel(ScatterArgs a) {
   const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
@@ -276,6 +276,7 @@ __global__ void __launch_bounds__(256) scatter_phase1_kernel(ScatterArgs a) {
   if (l == 0) a.has_tail[g] = tail_written ? 1 : 0;
 }
 
+template <int NS>
 __global__ void __launch_bounds__(256) scatter_phase2_kernel(ScatterArgs a) {
   const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
   const int g = blockIdx.x * 8 + w;
@@ -283,9 +284,9 @@ __global__ void __launch_bounds__(256) scatter_phase2_kernel(ScatterArgs a) {
   if (g >= nb || !a.has_tail[g]) return;
   const int key = a.keys[g * 32 + 31];
   const int h4 = a.H >> 2;
-  float4 acc[2];
+  float4 acc[NS];
 #pragma unroll
-  for (int s = 0; s < 2; ++s) {
+  for (int s = 0; s < NS; ++s) {
     const int c4 = l + 32 * s;
     acc[s] = c4 < h4 ? ld4(a.tail + (long long)g * a.H + 4 * c4) : zero4();
   }
@@ -299,11 +300,11 @@ __global__ void __launch_bounds__(256) scatter_phase2_kernel(ScatterArgs a) {
     const unsigned ok = __ballot_sync(0xffffffffu, same);
     const int len = ok == 0xffffffffu ? 32 : __ffs(~ok) - 1;     // leading blocks that belong to the run
     for (int b0 = 0; b0 < len; b0 += 8) {
-      float4 hv[8][2];
+      float4 hv[8][NS];
 #pragma unroll
       for (int u = 0; u < 8; ++u) {
 #pragma unroll
-        for (int s = 0; s < 2; ++s) {
+        for (int s = 0; s < NS; ++s) {
           const int c4 = l + 32 * s;
           hv[u][s] = (b0 + u < len && c4 < h4) ? ld4(a.head + (long long)(g2 + b0 + u) * a.H + 4 * c4) : zero4();
         }
@@ -312,7 +313,7 @@ __global__ void __launch_bounds__(256) scatter_phase2_kernel(ScatterArgs a) {
       for (int u = 0; u < 8; ++u) {
         if (b0 + u < len) {
 #pragma unroll
-          for (int s = 0; s < 2; ++s) acc[s] = f4_add(acc[s], hv[u][s]);
+          for (int s = 0; s < NS; ++s) acc[s] = f4_add(acc[s], hv[u][s]);
         }
       }
     }
@@ -320,7 +321,7 @@ __global__ void __launch_bounds__(256) scatter_phase2_kernel(ScatterArgs a) {
     g2 += 32;
   }
 #pragma unroll
-  for (int s = 0; s < 2; ++s) {
+  for (int s = 0; s < NS; ++s) {
     const int c4 = l + 32 * s;
     if (c4 < h4) st4(a.dE + (long long)key * a.H + 4 * c4, acc[s]);
   }

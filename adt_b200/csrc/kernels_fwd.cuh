@@ -381,6 +381,7 @@ __global__ void __launch_bounds__(NT) post_fwd_kernel(PostFwdArgs p) {
 // -------------------------------------------------------------------------------------------------
 __device__ __forceinline__ float softplusf(float z) { return fmaxf(z, 0.f) + log1pf(expf(-fabsf(z))); }
 
+template <int U>
 __global__ void __launch_bounds__(NT) final_fwd_kernel(const float* __restrict__ x, const float* __restrict__ ln_g,
                                                        const float* __restrict__ ln_b, const float* __restrict__ E,
                                                        const int* __restrict__ pos, const int* __restrict__ neg,
@@ -391,10 +392,10 @@ __global__ void __launch_bounds__(NT) final_fwd_kernel(const float* __restrict__
   double a0 = 0.0, a1 = 0.0, a2 = 0.0;
   for (int row = blockIdx.x * (NT / 32) + w; row < M; row += gridDim.x * (NT / 32)) {
     const float* xr = x + (long long)row * H;
-    float xv[8];
+    float xv[U];
     float sum = 0.f;
 #pragma unroll
-    for (int u = 0; u < 8; ++u) {
+    for (int u = 0; u < U; ++u) {
       const int c = l + 32 * u;
       xv[u] = c < H ? xr[c] : 0.f;
       sum += xv[u];
@@ -404,14 +405,14 @@ __global__ void __launch_bounds__(NT) final_fwd_kernel(const float* __restrict__
       mean = warp_sum(sum) / (float)H;
       float var = 0.f;
 #pragma unroll
-      for (int u = 0; u < 8; ++u)
+      for (int u = 0; u < U; ++u)
         if (l + 32 * u < H) { const float t = xv[u] - mean; var += t * t; }
       rstd = 1.0f / sqrtf(warp_sum(var) / (float)H + 1e-8f);
     }
     const int pi = pos ? pos[row] : 0, ni = neg ? neg[row] : 0;
     float dp = 0.f, dn = 0.f;
 #pragma unroll
-    for (int u = 0; u < 8; ++u) {
+    for (int u = 0; u < U; ++u) {
       const int c = l + 32 * u;
       if (c < H) {
         const float f = ln_g ? (xv[u] - mean) * rstd * ln_g[c] + ln_b[c] : xv[u];

@@ -128,20 +128,21 @@ __global__ void __launch_bounds__(256) act_bwd_kernel(const float* __restrict__ 
 
 // mode 0 (DropResidualNormalizeLayer, modules.py:104-117): y = LN(dropout(a) + r)
 // mode 1 (BertEmbedding, modules.py:42-48)               : y = dropout(LN(a + r))
-// Warp per row, H <= 256.
+// Warp per row, U columns per lane (H <= 32 U): U = 8 up to H = 256, 16 up to 512.
 struct DrlArgs {
   const float* a; const float* r; const float* gamma; const float* beta; float* y;
   const float* dy; float* da; float* dr; float* ggamma; float* gbeta;
   int M, H, mode; float eps; DropDesc drop;
 };
+template <int U>
 __global__ void __launch_bounds__(NT) drl_fwd_kernel(DrlArgs p) {
   const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
   const int H = p.H;
   for (int row = blockIdx.x * (NT / 32) + w; row < p.M; row += gridDim.x * (NT / 32)) {
-    float s[8];
+    float s[U];
     float sum = 0.f;
 #pragma unroll
-    for (int u = 0; u < 8; ++u) {
+    for (int u = 0; u < U; ++u) {
       const int c = l + 32 * u;
       float v = 0.f;
       if (c < H) {
@@ -156,11 +157,11 @@ __global__ void __launch_bounds__(NT) drl_fwd_kernel(DrlArgs p) {
     const float mean = warp_sum(sum) / (float)H;
     float var = 0.f;
 #pragma unroll
-    for (int u = 0; u < 8; ++u)
+    for (int u = 0; u < U; ++u)
       if (l + 32 * u < H) { const float t = s[u] - mean; var += t * t; }
     const float rstd = 1.0f / sqrtf(warp_sum(var) / (float)H + p.eps);
 #pragma unroll
-    for (int u = 0; u < 8; ++u) {
+    for (int u = 0; u < U; ++u) {
       const int c = l + 32 * u;
       if (c < H) {
         const long long gi = (long long)row * H + c;
@@ -172,19 +173,20 @@ __global__ void __launch_bounds__(NT) drl_fwd_kernel(DrlArgs p) {
   }
 }
 
+template <int U>
 __global__ void __launch_bounds__(NT) drl_bwd_kernel(DrlArgs p) {
-  __shared__ float red[2 * (NT / 32) * 256];
+  __shared__ float red[2 * (NT / 32) * 32 * U];
   const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
   const int H = p.H;
   constexpr int NW = NT / 32;
-  float dg[8], db[8];
+  float dg[U], db[U];
 #pragma unroll
-  for (int u = 0; u < 8; ++u) dg[u] = db[u] = 0.f;
+  for (int u = 0; u < U; ++u) dg[u] = db[u] = 0.f;
   for (int row = blockIdx.x * NW + w; row < p.M; row += gridDim.x * NW) {
-    float s[8], g[8], m[8];
+    float s[U], g[U], m[U];
     float sum = 0.f;
 #pragma unroll
-    for (int u = 0; u < 8; ++u) {
+    for (int u = 0; u < U; ++u) {
       const int c = l + 32 * u;
       float v = 0.f, gg = 0.f, mm = 1.f;
       if (c < H) {
@@ -202,12 +204,12 @@ __global__ void __launch_bounds__(NT) drl_bwd_kernel(DrlArgs p) {
     const float mean = warp_sum(sum) / (float)H;
     float var = 0.f;
 #pragma unroll
-    for (int u = 0; u < 8; ++u)
+    for (int u = 0; u < U; ++u)
       if (l + 32 * u < H) { const float t = s[u] - mean; var += t * t; }
     const float rstd = 1.0f / sqrtf(warp_sum(var) / (float)H + p.eps);
     float s1 = 0.f, s2 = 0.f;
 #pragma unroll
-    for (int u = 0; u < 8; ++u) {
+    for (int u = 0; u < U; ++u) {
       const int c = l + 32 * u;
       if (c < H) {
         const float xh = (s[u] - mean) * rstd, gg = g[u] * p.gamma[c];
@@ -218,7 +220,7 @@ __global__ void __launch_bounds__(NT) drl_bwd_kernel(DrlArgs p) {
     s1 = warp_sum(s1) / (float)H;
     s2 = warp_sum(s2) / (float)H;
 #pragma unroll
-    for (int u = 0; u < 8; ++u) {
+    for (int u = 0; u < U; ++u) {
       const int c = l + 32 * u;
       if (c < H) {
         const long long gi = (long long)row * H + c;
@@ -230,7 +232,7 @@ __global__ void __launch_bounds__(NT) drl_bwd_kernel(DrlArgs p) {
     }
   }
 #pragma unroll
-  for (int u = 0; u < 8; ++u) {
+  for (int u = 0; u < U; ++u) {
     const int c = l + 32 * u;
     if (c < H) { red[w * H + c] = dg[u]; red[(NW + w) * H + c] = db[u]; }
   }

@@ -4,6 +4,7 @@
 //
 // Exact path (this file, fp32 FFMA tiles): scores never leave the SM; every CTA keeps a sorted top-K list per
 // user in shared memory and only [splits][U][K] (score,id) pairs are written; a second kernel merges the splits.
+// H <= 512: the [64 x H] fp32 user tile, the staging ring and K = 64 lists take 215 KB of shared memory at H = 512.
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdio.h>
@@ -313,7 +314,7 @@ __global__ void __launch_bounds__(256) rank_metrics_kernel(const int* __restrict
 
 extern "C" int adt_score_topk(const adt_score_topk_args* a, adt_stream_t s_) {
   cudaStream_t s = (cudaStream_t)s_;
-  if (a->K <= 0 || a->K > KMAX || a->H > 256 || (a->H & 3) || a->n_splits <= 0 || a->n_splits > 256 || a->U <= 0) return ADT_E_SHAPE;
+  if (a->K <= 0 || a->K > KMAX || a->H > 512 || (a->H & 3) || a->n_splits <= 0 || a->n_splits > 256 || a->U <= 0) return ADT_E_SHAPE;
   TopkArgs k;
   k.feats = a->feats; k.E = a->item_emb; k.seen_indptr = a->seen_indptr; k.seen_idx = a->seen_idx;
   k.part_scores = a->part_scores; k.part_ids = a->part_ids; k.out_scores = a->out_scores; k.out_ids = a->out_ids;
@@ -339,7 +340,7 @@ extern "C" int adt_score_topk(const adt_score_topk_args* a, adt_stream_t s_) {
 extern "C" int adt_score_full(const float* feats, int32_t U, int32_t H, const float* item_emb, int32_t n_items, int32_t item_offset,
                               float* out, int64_t ld, adt_stream_t s_) {
   cudaStream_t s = (cudaStream_t)s_;
-  if (H > 256 || (H & 3) || U <= 0 || n_items <= 0 || ld < (int64_t)item_offset + n_items) return ADT_E_SHAPE;
+  if (H > 512 || (H & 3) || U <= 0 || n_items <= 0 || ld < (int64_t)item_offset + n_items) return ADT_E_SHAPE;
   TopkArgs k;
   memset(&k, 0, sizeof(k));
   k.feats = feats; k.E = item_emb; k.U = U; k.H = H; k.n_items = n_items; k.item_offset = item_offset; k.K = 1;

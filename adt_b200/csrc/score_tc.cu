@@ -83,6 +83,9 @@ __device__ __forceinline__ bool tc_is_seen(const TcArgs& a, int sb, int se, int 
 // ATM: the user tile (A operand, reused by every MMA of the kernel) lives in TENSOR MEMORY instead of shared memory: the epilogue
 // threads store their own feature row with tcgen05.st once, the MMAs read it from TMEM (tcgen05.mma, A from TMEM).  Frees
 // KB*16 KB of shared memory for a deeper TMA ring and takes the A fragment reads off the shared-memory port.
+// KB > 4 (H = 320 .. 512): a full-K catalog tile (KB*BN*128 B, 128 KB at H = 512) no longer fits two ring stages beside the lists, so
+// the ring holds ONE 64-column K block of a catalog tile per stage and the MMA warp consumes KB stages per tile; the user tile always
+// sits in tensor memory there (KB*32 <= 256 columns beside two 128-column accumulators).  KB <= 4 keeps the full-K stages.
 // BIAS: score = accumulator + bias[item] in fp32, added to every value as it leaves tcgen05.ld and before any comparison, in all three
 // modes (so the streaming lists, the published gthr keys, tau and the appended candidates are all in biased scores).  Every epilogue
 // warp stages the bias of its columns once per tile in its own smem row (loaded from global one tile ahead); each 32-column chunk
@@ -92,6 +95,8 @@ __global__ void __launch_bounds__(TC_THREADS2, 1) score_tc_kernel(const __grid_c
                                                                   const __grid_constant__ CUtensorMap tmB, TcArgs a) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
+  constexpr bool KBLK = KB > 4;
+  static_assert(!KBLK || ATM, "the K-blocked ring takes the user tile from tensor memory");
   constexpr int A_BYTES = ATM ? 0 : KB * BM * 128;
   // accumulator ring in tensor memory: MMA(t + NACC - 1) may be issued while tile t is still being read out.  The per-tile chain
   // (commit -> barrier -> tcgen05.ld -> filter -> arrive -> next MMA) costs ~2k cycles against ~130 of MMA at H = 64, so the depth of
@@ -99,7 +104,7 @@ __global__ void __launch_bounds__(TC_THREADS2, 1) score_tc_kernel(const __grid_c
   constexpr int NACC = (3 * BN + (ATM ? KB * 32 : 0) <= 512) ? 3 : 2;
   constexpr int TM_COLS = (ATM || NACC * BN > 256) ? 512 : (NACC * BN > 128 ? 256 : 128);   // accumulators NACC x BN (+ KB*32 columns of A behind them)
   constexpr uint32_t A_COL = NACC * BN;
-  constexpr int B_STAGE = KB * BN * 128;
+  constexpr int B_STAGE = KBLK ? BN * 128 : KB * BN * 128;
   uint8_t* sA = smem;
   uint8_t* sB = sA + A_BYTES;
   const int KCP = MODE == 0 ? (a.KC <= 32 ? 32 : 64) : 0;     // list slots reserved per user row (the two-pass modes keep no lists on chip)
@@ -150,6 +155,19 @@ __global__ void __launch_bounds__(TC_THREADS2, 1) score_tc_kernel(const __grid_c
         tc::mbar_arrive_expect_tx(abar, A_BYTES);
         for (int kb = 0; kb < KB; ++kb) tc::tma_load_2d(sA + kb * BM * 128, &tmA, kb * 64, u0, abar);
       }
+      if constexpr (KBLK) {
+        for (int t = 0; t < ntiles; ++t)
+          for (int kb = 0; kb < KB; ++kb) {
+            const int g = t * KB + kb, st = g % NS;
+            tc::mbar_wait(empty + st, ((g / NS) & 1) ^ 1);
+            tc::mbar_arrive_expect_tx(full + st, B_STAGE);
+            if (MC)
+              tc::tma_load_2d_mc(sB + st * B_STAGE + crank * (BN / 2) * 128, &tmB, kb * 64, (tfirst + t * tstep) * BN + (int)crank * (BN / 2),
+                                 full + st, (uint16_t)3);
+            else
+              tc::tma_load_2d(sB + st * B_STAGE, &tmB, kb * 64, (tfirst + t * tstep) * BN, full + st);
+          }
+      } else
       for (int t = 0; t < ntiles; ++t) {
         const int st = t % NS;
         tc::mbar_wait(empty + st, ((t / NS) & 1) ^ 1);
@@ -170,6 +188,21 @@ __global__ void __launch_bounds__(TC_THREADS2, 1) score_tc_kernel(const __grid_c
       for (int t = 0; t < ntiles; ++t) {
         const int st = t % NS, acc = t % NACC;
         tc::mbar_wait(tempty + acc, ((t / NACC) & 1) ^ 1);
+        if constexpr (KBLK) {
+          const uint32_t d_tmem = tmem_base + acc * BN;
+          for (int kb = 0; kb < KB; ++kb) {
+            const int g = t * KB + kb, gs = g % NS;
+            tc::mbar_wait(full + gs, (g / NS) & 1);
+            tc::tc_fence_after();
+            const uint64_t bd = tc::smem_desc_k_sw128(tc::smem_u32(sB + gs * B_STAGE));
+#pragma unroll
+            for (int k4 = 0; k4 < 4; ++k4)
+              tc::mma_bf16_ts(d_tmem, tmem_base + A_COL + kb * 32 + k4 * 8, bd + (uint64_t)(k4 * 2), idesc, (kb | k4) != 0);
+            if (MC) tc::mma_commit_mc(empty + gs, (uint16_t)3); else tc::mma_commit(empty + gs);
+          }
+          tc::mma_commit(tfull + acc);
+          continue;
+        }
         tc::mbar_wait(full + st, (t / NS) & 1);
         tc::tc_fence_after();
         const uint32_t d_tmem = tmem_base + acc * BN;
@@ -468,7 +501,8 @@ struct RescoreArgs {
 constexpr int RS_MAXC = 2048;   // candidate slots per user (n_splits * KC)
 constexpr int RS_NT = 256;
 constexpr int RS_STAGES = 2, RS_CW = 32, RS_LD = RS_CW + 4;   // re-score ring: stages per warp, columns per stage, floats per staged row (+4: conflict-free float4 reads)
-constexpr size_t RS_SMEM = (256 + (size_t)(RS_NT / 32) * RS_STAGES * 32 * RS_LD) * sizeof(float);
+// dynamic shared memory of the re-score kernel for rows of up to HMAX floats: the user vector, then the per-warp rings
+constexpr size_t rs_smem(int HMAX) { return (HMAX + (size_t)(RS_NT / 32) * RS_STAGES * 32 * RS_LD) * sizeof(float); }
 
 // One CTA per user: (1) compact the valid candidates of all splits, (2) one THREAD per candidate (rows staged through a per-warp cp.async ring) recomputes its score in fp32 with
 // the same sequential fmaf order as the exact kernel (bit-identical scores, so the two paths can be mixed and compared), 16 row
@@ -481,7 +515,7 @@ __device__ __forceinline__ unsigned long long rs_key(float s, int id) {
   return ((unsigned long long)o << 32) | (unsigned long long)(0xFFFFFFFFu - (unsigned)id);
 }
 
-template <bool BIAS>
+template <bool BIAS, int HMAX>
 __global__ void __launch_bounds__(RS_NT, 2) rescore_select_kernel(RescoreArgs a) {
   __shared__ int cid[RS_MAXC];
   __shared__ float csc[RS_MAXC];
@@ -518,7 +552,7 @@ __global__ void __launch_bounds__(RS_NT, 2) rescore_select_kernel(RescoreArgs a)
   {
     extern __shared__ __align__(16) float rs_dyn[];
     float* fs = rs_dyn;                                           // [H] user vector
-    float* ring = rs_dyn + 256 + w * (RS_STAGES * 32 * RS_LD);    // this warp's stages
+    float* ring = rs_dyn + HMAX + w * (RS_STAGES * 32 * RS_LD);   // this warp's stages
     for (int c = tid; c < a.H; c += RS_NT) fs[c] = f[c];
     __syncthreads();
     const int nch = a.H / RS_CW;
@@ -677,16 +711,31 @@ int launch_tc_a(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMa
   if (fixed + 2 * stage <= cap) return launch_tc_ns<KB, BN, 2, MODE, ATM, BIAS>(tmA, tmB, tmBh, k, grid, s, fixed + 2 * stage);
   return ADT_E_SHAPE;
 }
+// the K-blocked ring (KB > 4): 16 KB stages, eight of them (one H = 512 catalog tile, 128 KB in flight), every mode with the user tile in
+// tensor memory.  Shared memory: 86 KB of lists, parking area and barriers beside the ring in mode 0 (214 KB), 22 KB in the two-pass modes.
+template <int KB, int BN, int MODE, bool BIAS>
+int launch_tc_k(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap* tmBh, const TcArgs& k, dim3 grid, cudaStream_t s) {
+  constexpr int NS = 8;
+  const size_t fixed = 1024 + (MODE == 0 ? (size_t)(k.KC <= 32 ? 32 : 64) * BM * 8 : 0) + BM * 4 + 4 * 1024 * 4 + 256 + (BIAS ? 512 * 4 : 0);
+  const size_t smem = fixed + (size_t)NS * BN * 128;
+  if (smem > 227 * 1024) return ADT_E_SHAPE;
+  return launch_tc_ns<KB, BN, NS, MODE, true, BIAS>(tmA, tmB, tmBh, k, grid, s, smem);
+}
 // with a bias the two-pass kernels always take the user tile in tensor memory (the default; ADT_TC_ATMEM=0 is a measurement switch
 // for the unbiased kernels only), which keeps the number of instantiations down
 template <int KB, int BN, int MODE>
 int launch_tc(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap* tmBh, const TcArgs& k, dim3 grid, cudaStream_t s) {
-  if (k.bias) {
-    if constexpr (MODE != 0) return launch_tc_a<KB, BN, MODE, true, true>(tmA, tmB, tmBh, k, grid, s);
-    else return launch_tc_a<KB, BN, MODE, false, true>(tmA, tmB, tmBh, k, grid, s);
+  if constexpr (KB > 4) {
+    if (k.bias) return launch_tc_k<KB, BN, MODE, true>(tmA, tmB, tmBh, k, grid, s);
+    return launch_tc_k<KB, BN, MODE, false>(tmA, tmB, tmBh, k, grid, s);
+  } else {
+    if (k.bias) {
+      if constexpr (MODE != 0) return launch_tc_a<KB, BN, MODE, true, true>(tmA, tmB, tmBh, k, grid, s);
+      else return launch_tc_a<KB, BN, MODE, false, true>(tmA, tmB, tmBh, k, grid, s);
+    }
+    if (MODE != 0 && tc_atmem()) return launch_tc_a<KB, BN, MODE, true, false>(tmA, tmB, tmBh, k, grid, s);
+    return launch_tc_a<KB, BN, MODE, false, false>(tmA, tmB, tmBh, k, grid, s);
   }
-  if (MODE != 0 && tc_atmem()) return launch_tc_a<KB, BN, MODE, true, false>(tmA, tmB, tmBh, k, grid, s);
-  return launch_tc_a<KB, BN, MODE, false, false>(tmA, tmB, tmBh, k, grid, s);
 }
 // catalog tile width: 128 items, except that the single-pass H = 256 kernel (user tile 64 KB + lists 32-64 KB on chip) only has room
 // for 64-item tiles.  Wider is better there: a [128 x 64 x 16] MMA re-reads its 4 KB A fragment for 2 KB of B, 192 B/clk of a
@@ -698,6 +747,10 @@ int launch_tc_h(int KB, int BN, const CUtensorMap& tmA, const CUtensorMap& tmB, 
   if (KB == 2) return launch_tc<2, 128, MODE>(tmA, tmB, tmBh, k, grid, s);
   if (KB == 3) return launch_tc<3, 128, MODE>(tmA, tmB, tmBh, k, grid, s);
   if (KB == 4) return BN == 64 ? launch_tc<4, 64, MODE>(tmA, tmB, tmBh, k, grid, s) : launch_tc<4, 128, MODE>(tmA, tmB, tmBh, k, grid, s);
+  if (KB == 5) return launch_tc<5, 128, MODE>(tmA, tmB, tmBh, k, grid, s);
+  if (KB == 6) return launch_tc<6, 128, MODE>(tmA, tmB, tmBh, k, grid, s);
+  if (KB == 7) return launch_tc<7, 128, MODE>(tmA, tmB, tmBh, k, grid, s);
+  if (KB == 8) return launch_tc<8, 128, MODE>(tmA, tmB, tmBh, k, grid, s);
   return ADT_E_SHAPE;
 }
 
@@ -798,7 +851,7 @@ extern "C" int adt_score_tc_plan(int32_t U, int32_t H, int32_t n_items, int32_t 
 
 extern "C" int adt_score_topk_tc(const adt_score_topk_tc_args* a, adt_stream_t s_) {
   cudaStream_t s = (cudaStream_t)s_;
-  if (a->H % 64 || a->H > 256 || a->K <= 0 || a->K > a->KC || a->KC > 64 || a->n_splits <= 0 || a->n_splits * a->KC > RS_MAXC || a->U <= 0)
+  if (a->H % 64 || a->H > 512 || a->K <= 0 || a->K > a->KC || a->KC > 64 || a->n_splits <= 0 || a->n_splits * a->KC > RS_MAXC || a->U <= 0)
     return ADT_E_SHAPE;
   if (a->item_bias && !a->max_abs_bias) return ADT_E_SHAPE;
   CUtensorMap tmA, tmB;
@@ -872,12 +925,11 @@ extern "C" int adt_score_topk_tc(const adt_score_topk_tc_args* a, adt_stream_t s
   if (two) { r.KC = a->KC / 2; r.n_splits = 2 * a->n_splits; }     // every (split, column half) wrote its own list and threshold
   r.answers = a->answers; r.metric_acc = a->metric_acc;
   r.bias = a->item_bias; r.max_abs_bias = a->max_abs_bias;
-  if (a->item_bias) {
-    cudaFuncSetAttribute(rescore_select_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RS_SMEM);
-    rescore_select_kernel<true><<<a->U, RS_NT, RS_SMEM, s>>>(r);
-  } else {
-    cudaFuncSetAttribute(rescore_select_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RS_SMEM);
-    rescore_select_kernel<false><<<a->U, RS_NT, RS_SMEM, s>>>(r);
-  }
+  const bool wide = a->H > 256;
+  void (*rk)(RescoreArgs) = a->item_bias ? (wide ? rescore_select_kernel<true, 512> : rescore_select_kernel<true, 256>)
+                                         : (wide ? rescore_select_kernel<false, 512> : rescore_select_kernel<false, 256>);
+  const size_t rsm = rs_smem(wide ? 512 : 256);
+  cudaFuncSetAttribute(rk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rsm);
+  rk<<<a->U, RS_NT, rsm, s>>>(r);
   return cudaGetLastError() == cudaSuccess ? ADT_OK : ADT_E_CUDA;
 }

@@ -147,7 +147,7 @@ class CatalogScorer:
             self.ensure_table()
 
     def _uses_tc(self, H, lo, hi):
-        return self.use_tc and H % 64 == 0 and H <= 256 and (hi - lo) >= self.tc_min_items
+        return self.use_tc and H % 64 == 0 and H <= 512 and (hi - lo) >= self.tc_min_items
 
     # ------------------------------------------------------------------ public
     @torch.no_grad()

@@ -328,7 +328,9 @@ class Engine:
         svs["ctx"].copy_(sv["ctx"].view(B, Lq, H)[:, Lq - 1])
         ids_last = seq[:, Lq - 1].contiguous()
         nodrop = self._drop(0, "row", False, B, 1)
-        a = L.fill(L.adt_enc_block_fwd_args(), x=ws["x"][nl - 1], ids=ids_last, phase=2,
+        # beyond H = 256 only the tcgen05 block path serves, at any row count: it runs phase 2 on the B last rows from its own scratch
+        tc = {"wm": self.wm(), "tc_scratch": ws["fs"]} if H > 256 else {}
+        a = L.fill(L.adt_enc_block_fwd_args(), x=ws["x"][nl - 1], ids=ids_last, phase=2, **tc,
                    ln1_w=layer.attention_layernorm.weight, ln1_b=layer.attention_layernorm.bias, attn=_mha_w(layer.attention_layer),
                    ln2_w=layer.forward_layernorm.weight, ln2_b=layer.forward_layernorm.bias, ffn=_ffn_w(layer.forward_layer),
                    sparse_w=layer.sparse.weight, sparse_b=layer.sparse.bias,

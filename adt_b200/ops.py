@@ -13,6 +13,7 @@ def _st(dev):
 
 
 NBLK = 1024   # column block of wide linear layers
+ROWTILE_BWD_COLS = 1512   # (K + 8) + (N + 8) floats per row (N rounded up to 4): the most a 32-row adt_linear_bwd tile holds beside its staging ring
 
 
 def no_drop():
@@ -116,7 +117,9 @@ class LinearFn(torch.autograd.Function):
         dx = torch.empty_like(x)
         gW = torch.zeros_like(W)
         gb = torch.zeros(N, dtype=torch.float32, device=x.device) if has_b else None
-        if _use_tc(precision, M, N, K):
+        # the row-tile backward keeps 32-row tiles of x and of a column block of dy in shared memory; wide models' layers with fewer
+        # than 128 rows (a vocabulary head over a few labelled rows, H > 256) exceed it and run on the tensor cores at any row count
+        if _use_tc(precision, M, N, K) or (precision and K + ((min(N, NBLK) + 3) & ~3) + 16 > ROWTILE_BWD_COLS):
             # dx = scale * dy W ; dW = scale * dy^T x ; db = scale * colsum(dy): three more products on the tensor cores
             # (W, dy and x are read MN-major where the product needs their transpose: no transposed copies)
             dy16, ldd = _bf16(dy)

@@ -7,7 +7,8 @@
  *
  * Conventions
  *   - every pointer is a DEVICE pointer owned by the caller (fp32 activations/weights, int32 ids), 16-byte aligned;
- *   - activations are row-major [M = B*L, H]; H % 4 == 0, H <= 256, (H/nh) % 4 == 0, L <= 256, nh <= 8;
+ *   - activations are row-major [M = B*L, H]; H % 4 == 0, H <= 256, (H/nh) % 4 == 0, L <= 256, nh <= 8; longer sequences (L <= 2048)
+ *     and wider rows (256 < H <= 512: precision 1, H % 64 == 0, H/nh a multiple of 32 up to 128) as stated where they apply;
  *   - all calls are asynchronous on `stream` (a cudaStream_t), never synchronise, allocate nothing;
  *   - return 0 on success, a negative ADT_E_* otherwise; adt_last_error() gives the thread-local message;
  *   - gradient buffers are ACCUMULATED into (+=, atomics) unless stated: zero them once per step.
@@ -47,7 +48,8 @@ const char* adt_last_error(void);
  * adt_embed_sort; scatter = head/tail/has_tail of adt_embed_bwd; score_part = part_scores + part_ids of adt_score_topk for
  * (U = B, K, n_splits); wgrad_scratch = the bf16 operand copies of the hoisted weight gradients, fwd_scratch = the bf16 operands of the
  * tcgen05 forward path (both 0 when H < 128).  Sequences of 257..2048 positions need precision 1 and a head size H/nh that is a multiple of
- * 16 up to 128. */
+ * 16 up to 128.  Hidden sizes of 257..512 need precision 1, H % 64 == 0 and a head size H/nh that is a multiple of 32 up to 128; the
+ * block entry points then run on the tcgen05 path at every row count, so tc_scratch / wgrad_scratch are required there. */
 typedef struct { int32_t B, L, H, nh, nl, K, n_splits; } adt_workspace_query;
 typedef struct {
   int64_t saved, scratch, sort_keys, sort_hist, scatter_rows, scatter_flags, score_part, wgrad_scratch, fwd_scratch;
@@ -96,7 +98,8 @@ typedef struct {
                       sasrec/model.py:89); `out` may then be NULL.  Only honoured by the sequence-resident kernel (phase 0, training 0,
                       precision 1, H == 64, L <= 64, nh in {1,2,4}); otherwise ignored, so callers must check adt_seq_kernels_apply() first */
   void* tc_scratch; /* optional, adt_workspace_sizes.fwd_scratch bytes (precision 1, H >= 128, H % 64 == 0, phase 0): every linear layer
-                       then runs as one tcgen05 GEMM over all rows (block_tc.cuh) instead of inside the row-tile kernels */
+                       then runs as one tcgen05 GEMM over all rows (block_tc.cuh) instead of inside the row-tile kernels (at >= 512 rows
+                       up to H = 256).  Required beyond H = 256, with y, h1 and out, in every phase */
   void* attn_scratch; /* adt_workspace_sizes.attn_scratch bytes, required when L > 256 (fused flash attention; NULL otherwise) */
 } adt_enc_block_fwd_args;
 int adt_enc_block_fwd(const adt_enc_block_fwd_args* a, adt_stream_t stream);
@@ -119,7 +122,8 @@ typedef struct {
   int32_t precision;
   adt_wmirror wm;
   void* wgrad_scratch;        /* optional, adt_workspace_sizes.wgrad_scratch bytes (precision 1, H >= 128): the row-tile kernels then only write
-                                 bf16 copies of their dY / X tiles and every weight gradient becomes ONE split-K tcgen05 GEMM over all rows */
+                                 bf16 copies of their dY / X tiles and every weight gradient becomes ONE split-K tcgen05 GEMM over all rows
+                                 (>= 512 rows: the whole backward on the tcgen05 path).  Required beyond H = 256 */
   void* attn_scratch;         /* as in adt_enc_block_fwd_args */
 } adt_enc_block_bwd_args;
 int adt_enc_block_bwd(const adt_enc_block_bwd_args* a, adt_stream_t stream);
@@ -280,7 +284,8 @@ typedef struct {
 } adt_candidate_scores_args;
 int adt_candidate_scores(const adt_candidate_scores_args* a, adt_stream_t stream);
 
-/* K7 on the tensor cores (H % 64 == 0): bf16 TMA-fed tcgen05.mma GEMM (fp32 accumulators in TMEM) with a fused
+/* K7 on the tensor cores (H % 64 == 0, H <= 512; beyond 256 the catalog ring holds one 64-column K block per stage): bf16
+ * TMA-fed tcgen05.mma GEMM (fp32 accumulators in TMEM) with a fused
  * streaming top-KC epilogue per (catalog split, user), then an exact fp32 re-score of the <= n_splits*KC candidates
  * per user and the final top-K.  flags[u] = 1 when the bf16 rounding bound cannot prove that the fp32 top-K is
  * contained in the candidate set; the caller re-runs those users through adt_score_topk (exact).  n_splits*KC <= 2048. */
