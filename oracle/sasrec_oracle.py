@@ -95,49 +95,66 @@ def embed(sd, ids, drop, site):
     return x * (ids != 0).unsqueeze(-1).to(x.dtype)
 
 
-def mha(q_in, kv_in, w_in, b_in, w_o, b_o, nh, drop, site, causal=True):
+class Products:
+    """The matrix products of a block: every x W^T + b and the attention core.  The default evaluates them as the reference does;
+    a test may pass a subclass that evaluates them differently (for instance on bf16-rounded operands, as the tensor-core kernels
+    do) while LayerNorm, biases, residuals, dropout and the independence head stay the oracle's own."""
+
+    def linear(self, x, w, b):
+        return F.linear(x, w, b)
+
+    def attention(self, q, k, v, drop, site, causal=True):
+        """q (already scaled by 1/sqrt(hd)), k, v: [B, nh, L, hd] -> softmax(q k^T + mask) v, [B, nh, L, hd]"""
+        L = q.shape[2]
+        s = q @ k.transpose(-1, -2)
+        if causal:
+            neg = torch.full((L, L), float("-inf"), dtype=s.dtype).triu(1)
+            s = s + neg
+        p = torch.softmax(s, dim=-1)
+        p = drop.apply(p, site)
+        return p @ v
+
+
+PRODUCTS = Products()
+
+
+def mha(q_in, kv_in, w_in, b_in, w_o, b_o, nh, drop, site, causal=True, prod=PRODUCTS):
     """Batch-first restatement of multi_head_attention_forward (modules.py:270-527).
     q is projected from q_in with rows [0:H) of w_in, k/v from kv_in with rows
     [H:3H).  Returns (out [B,L,H], ctx [B,L,H] head-concatenated)."""
     B, L, H = q_in.shape
     hd = H // nh
-    q = F.linear(q_in, w_in[:H], b_in[:H])
-    k = F.linear(kv_in, w_in[H:2 * H], b_in[H:2 * H])
-    v = F.linear(kv_in, w_in[2 * H:], b_in[2 * H:])
+    q = prod.linear(q_in, w_in[:H], b_in[:H])
+    k = prod.linear(kv_in, w_in[H:2 * H], b_in[H:2 * H])
+    v = prod.linear(kv_in, w_in[2 * H:], b_in[2 * H:])
     q = q.view(B, L, nh, hd).transpose(1, 2) / math.sqrt(hd)  # modules.py:54
     k = k.view(B, L, nh, hd).transpose(1, 2)
     v = v.view(B, L, nh, hd).transpose(1, 2)
-    s = q @ k.transpose(-1, -2)
-    if causal:
-        neg = torch.full((L, L), float("-inf"), dtype=s.dtype).triu(1)
-        s = s + neg
-    p = torch.softmax(s, dim=-1)
-    p = drop.apply(p, site)
-    ctx = (p @ v).transpose(1, 2).reshape(B, L, H)
-    return F.linear(ctx, w_o, b_o), ctx
+    ctx = prod.attention(q, k, v, drop, site, causal).transpose(1, 2).reshape(B, L, H)
+    return prod.linear(ctx, w_o, b_o), ctx
 
 
-def ffn(x, w1, b1, w2, b2, drop, site1, site2):
+def ffn(x, w1, b1, w2, b2, drop, site1, site2, prod=PRODUCTS):
     """dropout2(conv2(relu(dropout1(conv1(x))))) + x  -- modules.py:629-633 (Conv1d k=1 == Linear)"""
-    h = F.linear(x, w1.squeeze(-1), b1)
+    h = prod.linear(x, w1.squeeze(-1), b1)
     h = torch.relu(drop.apply(h, site1))
-    h = F.linear(h, w2.squeeze(-1), b2)
+    h = prod.linear(h, w2.squeeze(-1), b2)
     return drop.apply(h, site2) + x
 
 
-def encoder_layer(sd, pre, x, keep, nh, drop, sites, l):
+def encoder_layer(sd, pre, x, keep, nh, drop, sites, l, prod=PRODUCTS):
     """modules.py:644-655.  Returns (out, rec_true [B,L,nh,nh], ctx)."""
     Qn = layer_norm(x, sd[pre + "attention_layernorm.weight"], sd[pre + "attention_layernorm.bias"])
     mha_out, ctx = mha(Qn, x, sd[pre + "attention_layer.in_proj_weight"], sd[pre + "attention_layer.in_proj_bias"],
                        sd[pre + "attention_layer.out_proj.weight"], sd[pre + "attention_layer.out_proj.bias"],
-                       nh, drop, sites[f"enc{l}_attn"])
+                       nh, drop, sites[f"enc{l}_attn"], prod=prod)
     B, L, H = x.shape
     rec_true = F.log_softmax(F.linear(ctx.view(B, L, nh, H // nh), sd[pre + "sparse.weight"], sd[pre + "sparse.bias"]), dim=3)
     y = Qn + mha_out
     z = layer_norm(y, sd[pre + "forward_layernorm.weight"], sd[pre + "forward_layernorm.bias"])
     out = ffn(z, sd[pre + "forward_layer.conv1.weight"], sd[pre + "forward_layer.conv1.bias"],
               sd[pre + "forward_layer.conv2.weight"], sd[pre + "forward_layer.conv2.bias"],
-              drop, sites[f"enc{l}_ffn1"], sites[f"enc{l}_ffn2"])
+              drop, sites[f"enc{l}_ffn1"], sites[f"enc{l}_ffn2"], prod)
     return out * keep, rec_true, ctx
 
 
@@ -148,15 +165,17 @@ def misview(rec_true):
     return rec_true.transpose(0, 1).contiguous().view(B, L, *rec_true.shape[2:])
 
 
-def decoder_layer(sd, pre, xd, feats, keep_d, nh, drop, sites, l):
+def decoder_layer(sd, pre, xd, feats, keep_d, nh, drop, sites, l, prod=PRODUCTS):
     """modules.py:666-677 (pos_ffn_layernorm is never applied)."""
     d = layer_norm(xd, sd[pre + "layer_norm.weight"], sd[pre + "layer_norm.bias"])
     a, _ = mha(d, d, sd[pre + "slf_attn.in_proj_weight"], sd[pre + "slf_attn.in_proj_bias"],
-               sd[pre + "slf_attn.out_proj.weight"], sd[pre + "slf_attn.out_proj.bias"], nh, drop, sites[f"dec{l}_self"])
+               sd[pre + "slf_attn.out_proj.weight"], sd[pre + "slf_attn.out_proj.bias"], nh, drop, sites[f"dec{l}_self"],
+               prod=prod)
     c, _ = mha(a, feats, sd[pre + "enc_attn.in_proj_weight"], sd[pre + "enc_attn.in_proj_bias"],
-               sd[pre + "enc_attn.out_proj.weight"], sd[pre + "enc_attn.out_proj.bias"], nh, drop, sites[f"dec{l}_cross"])
+               sd[pre + "enc_attn.out_proj.weight"], sd[pre + "enc_attn.out_proj.bias"], nh, drop, sites[f"dec{l}_cross"],
+               prod=prod)
     f = ffn(c, sd[pre + "pos_ffn.conv1.weight"], sd[pre + "pos_ffn.conv1.bias"],
-            sd[pre + "pos_ffn.conv2.weight"], sd[pre + "pos_ffn.conv2.bias"], drop, sites[f"dec{l}_ffn1"], sites[f"dec{l}_ffn2"])
+            sd[pre + "pos_ffn.conv2.weight"], sd[pre + "pos_ffn.conv2.bias"], drop, sites[f"dec{l}_ffn1"], sites[f"dec{l}_ffn2"], prod)
     return (d + f) * keep_d
 
 

@@ -11,6 +11,8 @@ import numpy as np
 import pytest
 import torch
 
+from block_ref import attention_core as _reference
+
 pytestmark = pytest.mark.gpu
 
 
@@ -72,34 +74,6 @@ def _run(fwd, bwd, q, k, v, dctx, ids, B, L, H, nh, mask_mode, drop, precision=1
     L_.check(getattr(lib, bwd)(ctypes.byref(a), _st(dev)), bwd)
     torch.cuda.synchronize()
     return tuple(t.cpu() for t in (ctx, lse, dq, dk, dv))
-
-
-def _reference(q, k, v, dctx, ids, B, L, H, nh, mask_mode, p, seed, step, base):
-    """fp64 attention core on bf16-rounded operands; the backward uses the fp32-rounded lse (see module docstring)"""
-    from oracle.philox import keep_mask_attn
-    hd = H // nh
-    r = lambda t: t.to(torch.bfloat16).double().view(B, L, nh, hd).permute(0, 2, 1, 3)
-    Q, K, V = r(q), r(k), r(v)
-    dO = dctx.double().view(B, L, nh, hd).permute(0, 2, 1, 3)
-    S = Q @ K.transpose(-1, -2)
-    if mask_mode == 0:
-        S = S.masked_fill(torch.ones(L, L, dtype=torch.bool).triu(1), float("-inf"))
-    else:
-        S = torch.where((ids == 0).view(B, 1, 1, L), torch.full_like(S, -1e9), S)
-    lse = torch.logsumexp(S, -1)
-    P = torch.exp(S - lse[..., None])
-    if p > 0:
-        keep = keep_mask_attn(B * nh * L, L, p, seed, step, 5, row_offset=base)
-        m = torch.from_numpy(keep.astype(np.float64)).view(B, nh, L, L) / (1.0 - np.float32(p))
-    else:
-        m = torch.ones_like(P)
-    ctx = (P * m) @ V
-    Pb = torch.exp(S - lse.float().double()[..., None])
-    dPd = dO @ V.transpose(-1, -2)
-    delta = (dO * ctx).sum(-1, keepdim=True)
-    dS = Pb * (dPd * m - delta)
-    back = lambda t: t.permute(0, 2, 1, 3).reshape(B * L, H)
-    return back(ctx), lse, back(dS @ K), back(dS.transpose(-1, -2) @ Q), back((Pb * m).transpose(-1, -2) @ dO)
 
 
 def _err(a, b):
